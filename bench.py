@@ -4,6 +4,7 @@
     python bench.py --gpus 1 --steps 10 --warmup 3            # one JSON line on stdout
     python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...                      # the reference's CPU algorithm (oracle port)
+    python bench.py --steps 10 --warmup 3 --dump-outputs DIR  # also write the timed path's outputs as DIR/<name>.npy
 
 Workload (config.workload): synthetic planted-partition graph of BASELINE.json's shape, README-Cora flag
 profile ("Profile A": --w1=0.01 --w6=10 --w7=10 --w9=10 --w10=1000 --lr=-2 --measure=MSELoss, all three priors,
@@ -39,6 +40,7 @@ PROFILES = {"A": dict(w=PROFILE_A, measure="MSELoss", lr=-2.0,
                       flags="Profile B: README Polblogs HSIC w1=.01 w2=.01 w6=1e4 w7=100 w9=.001 w10=1000 lr=10^-2.5 "
                             "(n x n HSIC stage on library GEMMs, DESIGN.md 1)")}
 SAMPLE_N = int(os.environ.get("MCGRA_BENCH_SAMPLE_N", "3072"))   # CPU baseline sample size (the reference algorithm is O(n^3) per iteration)
+DUMP_SAMPLE = 1 << 22     # --dump-outputs keeps at most this many entries of an array: two 16 MB samples + loss histories
 
 
 class Args:
@@ -416,6 +418,28 @@ def measure_tf32_peak(device):
         torch.backends.cuda.matmul.allow_tf32 = old
 
 
+def sample_flat(t, seed):
+    """Flattened float32 host copy of a device tensor: all of it up to DUMP_SAMPLE entries, else the entries at a fixed
+    seeded set of sorted, distinct flat indices (np.unique of RandomState(seed).randint(0, numel, DUMP_SAMPLE)), so that
+    two runs or two builds at the same size compare entry for entry."""
+    import torch
+    flat = t.reshape(-1)
+    if flat.numel() > DUMP_SAMPLE:
+        idx = np.unique(np.random.RandomState(seed).randint(0, flat.numel(), DUMP_SAMPLE, dtype=np.int64))
+        flat = flat[torch.from_numpy(idx).to(flat.device)]
+    return flat.float().cpu().numpy()
+
+
+def write_outputs(path, arrays, rank):
+    """--dump-outputs: rank 0 writes every array as <path>/<name>.npy, float32 arrays as they are, the rest as float64."""
+    if rank != 0:
+        return
+    os.makedirs(path, exist_ok=True)
+    for name, v in arrays.items():
+        v = np.asarray(v)
+        np.save(os.path.join(path, name + ".npy"), v if v.dtype == np.float32 else v.astype(np.float64))
+
+
 def run_native(a):
     import torch
     import torch.distributed as dist
@@ -496,7 +520,12 @@ def run_native(a):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
         dist.barrier()
-    losses = eng.losses()["loss"]
+    hist = eng.losses()
+    losses = hist["loss"]
+    if a.dump_outputs:      # the K timed iterations' loss terms and the parameter after the last one (collective at N > 1)
+        dump = {("loss" if k == "loss" else "loss_" + k): v[-K:] for k, v in hist.items()}
+        dump["adj_changes"] = sample_flat(eng.packed_parameter(), seed=0)
+        write_outputs(a.dump_outputs, dump, rank)
     del eng, atk
     torch.cuda.empty_cache()
     parity_large = None
@@ -536,6 +565,9 @@ def run_native(a):
             t = torch.tensor([dt], device=device, dtype=torch.float64)
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
             dt = float(t.item())
+        if a.dump_outputs:      # what PGDAttack.attack + AUC hand back (gathering the row bands is collective at N > 1)
+            write_outputs(a.dump_outputs, {"e2e_loss": loss_hist, "e2e_auc_ap": [auc, ap],
+                                           "e2e_modified_adj": sample_flat(atk.gather_modified_adj(), seed=1)}, rank)
         if world == 1:
             fa_bytes = prob["feature_adj"].numel() * 4
         else:       # all ranks' row bands together
@@ -670,9 +702,9 @@ def run_reference(a):
     torch.set_num_threads(threads)
     n = min(SAMPLE_N, wl["n"])
     O, prob, cfg = cpu_problem(n, wl["f"], wl["c"])
-    for _ in range(min(a.warmup, 1)):
+    for _ in range(a.warmup):
         O.attack(prob, cfg, 1, bookkeeping=True)
-    K = max(1, min(a.steps, 3))
+    K = a.steps
     t0 = time.perf_counter()
     O.attack(prob, cfg, K, bookkeeping=True)
     dt = time.perf_counter() - t0
@@ -680,7 +712,7 @@ def run_reference(a):
     sample = (f"oracle port of the reference loop at n={n} (bounded sample; the reference needs >0.9 TB and "
               f"O(n^3) work per iteration at n={wl['n']}), {K} timed iterations")
     out = {"impl": "reference", "metric": "PGD attack iterations/s (fwd+bwd+prior losses+Adam+projection)", "value": v,
-           "unit": "iterations/s", "n_gpus": int(os.environ.get("WORLD_SIZE", 1)), "steps": K, "warmup": min(a.warmup, 1),
+           "unit": "iterations/s", "n_gpus": int(os.environ.get("WORLD_SIZE", 1)), "steps": K, "warmup": a.warmup,
            "ms_per_step": dt / K * 1e3, "higher_is_better": True, "scaling": "strong", "vs_baseline": None,
            "dtype": "f32", "data": "synthetic",
            "config": {"workload": f"bounded sample n={n} of: " + wl["name"], "n": n, "sample_n": n,
@@ -705,7 +737,17 @@ def main():
     ap.add_argument("--no-e2e", dest="no_e2e", action="store_true")
     ap.add_argument("--no-cpu", dest="no_cpu", action="store_true")
     ap.add_argument("--no-parity", dest="no_parity", action="store_true", help="skip the untimed large-size precision check")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR",
+                    help="after the timed steps write what they computed as DIR/<name>.npy: the loss terms of the K timed "
+                         "iterations and the parameter after the last one, and of the e2e run its loss history, AUC / AP "
+                         f"and modified_adj (arrays over {DUMP_SAMPLE} entries as a fixed seeded sample).  The inputs are "
+                         "the same in every run; fp32 atomics make two runs of one build differ in the last bits, so "
+                         "compare with a tolerance")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "native":
+        ap.error("--dump-outputs writes the native path's outputs (--impl native)")
     if a.impl == "reference":
         run_reference(a)
     else:
