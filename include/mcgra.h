@@ -121,6 +121,14 @@ typedef struct {
 int64_t mcgra_propagate_ws_bytes(int64_t n, int K);
 int mcgra_propagate(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw,
                     const float* B, int K, float* Y, const mcgra_elem_args* elem, void* ws, void* stream);
+/* the same with a product selector: with L the stored strict lower triangle (entry (i,j), i > j, at tile (I,J)),
+ * DIRECT adds L*B, MIRRORED adds L^T*B, BOTH (= mcgra_propagate) their sum.  The noisy path (mcgra_noise_stage) keeps
+ * the two orientations of a non-symmetric M in two tile planes and forms M*B / M^T*B from one product of each.
+ * elem must be NULL unless products == MCGRA_PROD_BOTH.                                                          */
+enum { MCGRA_PROD_DIRECT = 1, MCGRA_PROD_MIRRORED = 2, MCGRA_PROD_BOTH = 3 };
+int mcgra_propagate_sel(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw,
+                        const float* B, int K, float* Y, const mcgra_elem_args* elem, void* ws, int products,
+                        void* stream);
 /* the same element-wise terms as a stand-alone streaming pass (x and F tiles read once): lets every propagation
  * use the plain tensor-core kernels; values into elem->acc, row sums into elem->eps_row.                        */
 int mcgra_elem_stats(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw,
@@ -176,6 +184,9 @@ int mcgra_node_head(const mcgra_node_args* a, void* stream);   /* after pass 2: 
 int mcgra_node_bwd2(const mcgra_node_args* a, void* stream);   /* dQ2, B3                              */
 int mcgra_node_bwd1(const mcgra_node_args* a, void* stream);   /* after pass 3: dZ1,dQ1,B4             */
 int mcgra_node_rho(const mcgra_node_args* a, void* stream);    /* after pass 4: rho, fold factors Wt   */
+/* mcgra_node_rho for an estimate with a non-zero diagonal M_ii = mdiag[i] (the noisy path): the diagonal entry of
+ * A_hat is r_i^2 (1 + M_ii) in the element-wise terms and in rho.                                                    */
+int mcgra_node_rho_diag(const mcgra_node_args* a, const float* mdiag, void* stream);
 
 /* ---- pair pass over the decode gram M1 = relu(zhat zhat^T) (dot_product_decode :414-419,
  *      get_modified_adj_after :381-395): c7 entropy (:233-236) and c2 MSE (:221-229) values, their
@@ -423,6 +434,42 @@ int mcgra_nd_measure(const mcgra_nd_args* a, void* stream);
 /* ---- stand-alone helpers of the class surface ----
  * M <- clamp(M + eps * noise, 0, 1) (PGDAttack.adding_noise, topology_attack.py:474-478; noise = the caller's N(0,1) draw) */
 int mcgra_noise_clamp(float* M, const float* noise, float eps, int64_t count, void* stream);
+
+/* ---- attack() with adjacency noise (--eps != 0, topology_attack.py:165, 474-478), single GPU, MSELoss ----
+ * Per iteration M = clamp(p + N*eps, 0, 1) with a fresh dense n x n N (row-major fp32) and p the parameter view of
+ * the tiles (off the diagonal; the diagonal is clamp(N_ii*eps, 0, 1)).  M is not symmetric: its two orientations are
+ * kept as tile planes Lt (M_ij at (i,j), i > j) and Ut (M_ji at (i,j)), read by mcgra_propagate_sel with raw = 2:
+ *     M B = DIRECT(Lt) + MIRRORED(Ut) + diag(mdiag) B,     M^T B = DIRECT(Ut) + MIRRORED(Lt) + diag(mdiag) B.
+ * The clamp masks are not stored: the gradient pass recomputes p + N*eps with the same two roundings.             */
+int mcgra_noise_stage(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* noise,
+                      float eps, float* Lt, float* Ut, float* mdiag, float* d, void* stream);   /* d = 1 + row sums of M */
+/* Y[i, :] += mdiag[i] * B[i, :]  (B, Y row-major [n x K]) */
+int mcgra_diag_axpy(const float* mdiag, const float* B, int K, int64_t n, float* Y, void* stream);
+typedef struct {
+  int64_t n, npad;
+  int tr0, tr1;
+  const float* tiles;      /* parameter tiles and their view (mu, raw) as given to mcgra_noise_stage        */
+  const float* mu;
+  int raw;
+  const float* noise;      /* [n x n] this iteration's draw                                                 */
+  float eps;
+  const float *Lt, *Ut;    /* the two orientations written by mcgra_noise_stage                             */
+  const float *FLt, *FUt;  /* feature_adj: F_ij and F_ji at (i,j) (mcgra_dense_to_tiles of F and F^T), or NULL */
+  const float* zhat;       /* [n x 16] row-normalised embedding (c2: M1 = relu(zhat zhat^T))                */
+  const float* r;          /* [n] D^-1/2                                                                    */
+  const float* rho;        /* [n] degree gradient (mcgra_node_rho_diag)                                     */
+  const float* Wt;         /* [128 x npad] factors U, V (mcgra_node_rho_diag)                               */
+  float k1, k2, k6;        /* as in mcgra_node_args (c1 and c2 under MSELoss, c6)                           */
+  double* acc;             /* slots C1, C2, C6 (+=)                                                         */
+  float* eps_row;          /* [n] += row and column parts of the element-wise degree gradient               */
+  float* dzhat;            /* [n x 16] += gradient of c2 through M1                                         */
+  float* Gt;               /* gradient tiles: dL/dx_ij (consumed by mcgra_fold_adam as Gtiles)              */
+} mcgra_noisy_args;
+/* c1 (MSE), c2 (MSE, both orientations of A_hat against the symmetric M1) and c6 over the off-diagonal entries:
+ * values, eps_row, dzhat */
+int mcgra_noisy_terms(const mcgra_noisy_args* a, void* stream);
+/* dL/dx_ij = mask_ij dL/dM_ij + mask_ji dL/dM_ji with dL/dM_ij = U_i.V_j + r_i r_j e'_ij + rho_i, written to Gt */
+int mcgra_noisy_grad(const mcgra_noisy_args* a, void* stream);
 /* out[0] += sum_rows KL(softmax(X_i) || softmax(Y_i)) (PGDAttack.calc_kl, :483-487; divide by rows for batchmean)      */
 int mcgra_row_kl(const float* X, const float* Y, int64_t rows, int64_t cols, int64_t ldx, int64_t ldy, double* out,
                  void* stream);

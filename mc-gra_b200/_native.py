@@ -53,6 +53,17 @@ class FoldArgs(C.Structure):
                 ("plain_gd", C.c_int), ("Gtiles", c_fp)]
 
 
+class NoisyArgs(C.Structure):
+    """mcgra_noisy_args (include/mcgra.h): the --eps != 0 stages."""
+    _fields_ = [("n", i64), ("npad", i64), ("tr0", C.c_int), ("tr1", C.c_int), ("tiles", c_fp), ("mu", c_fp),
+                ("raw", C.c_int), ("noise", c_fp), ("eps", C.c_float), ("Lt", c_fp), ("Ut", c_fp), ("FLt", c_fp),
+                ("FUt", c_fp), ("zhat", c_fp), ("r", c_fp), ("rho", c_fp), ("Wt", c_fp), ("k1", C.c_float),
+                ("k2", C.c_float), ("k6", C.c_float), ("acc", c_fp), ("eps_row", c_fp), ("dzhat", c_fp), ("Gt", c_fp)]
+
+
+PROD_DIRECT, PROD_MIRRORED, PROD_BOTH = 1, 2, 3
+
+
 class Image(C.Structure):
     """mcgra_image: fp16x2 operand image of an fp32 matrix (include/mcgra.h)."""
     _fields_ = [("hi", c_fp), ("lo", c_fp), ("inv_scale", c_fp), ("rows", i64), ("cols", i64), ("ld", i64)]
@@ -102,6 +113,14 @@ _SIGS = {
     "mcgra_propagate_ws_bytes": (i64, [i64, C.c_int]),
     "mcgra_propagate": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, C.c_int, c_fp,
                                   C.POINTER(ElemArgs), c_fp, c_fp]),
+    "mcgra_propagate_sel": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, C.c_int, c_fp,
+                                      C.POINTER(ElemArgs), c_fp, C.c_int, c_fp]),
+    "mcgra_noise_stage": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, C.c_float, c_fp, c_fp, c_fp, c_fp,
+                                    c_fp]),
+    "mcgra_diag_axpy": (C.c_int, [c_fp, c_fp, C.c_int, i64, c_fp, c_fp]),
+    "mcgra_noisy_terms": (C.c_int, [C.POINTER(NoisyArgs), c_fp]),
+    "mcgra_noisy_grad": (C.c_int, [C.POINTER(NoisyArgs), c_fp]),
+    "mcgra_node_rho_diag": (C.c_int, [C.POINTER(NodeArgs), c_fp, c_fp]),
     "mcgra_elem_stats": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, C.POINTER(ElemArgs), c_fp]),
     "mcgra_row_sumexp": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, c_fp, c_fp]),
     "mcgra_node_pre": (C.c_int, [C.POINTER(NodeArgs), c_fp]),
@@ -221,7 +240,7 @@ LAUNCHES = {"count": 0, "kernels": 0}
 # hand-written kernels launched per C entry with the default engines (everything else launches exactly one):
 # propagate = k_colmax + k_prep_b16 + k_propagate_h; fold_adam = k_prep_w + k_fold_tc; auc_ap = compact + 4 x (hist, scan,
 # scatter) + rank + finish; argsort_desc = make_keys + 4 x 3
-KERNELS_PER_CALL = {"mcgra_propagate": 3, "mcgra_fold_adam": 2, "mcgra_auc_ap": 15, "mcgra_argsort_desc": 13,
+KERNELS_PER_CALL = {"mcgra_propagate": 3, "mcgra_propagate_sel": 3, "mcgra_noise_stage": 2, "mcgra_fold_adam": 2, "mcgra_auc_ap": 15, "mcgra_argsort_desc": 13,
                     "mcgra_version": 0, "mcgra_set_engine": 0, "mcgra_tiles_in_rows": 0, "mcgra_propagate_ws_bytes": 0,
                     "mcgra_fold_ws_bytes": 0, "mcgra_auc_workspace_bytes": 0, "mcgra_sort_workspace_bytes": 0,
                     "mcgra_pairs_ws_bytes": 0, "mcgra_auc_hist_offset": 0, "mcgra_auc_stage": 5, "mcgra_nd_scratch_doubles": 0, "mcgra_nd_scratch_floats": 0, "mcgra_nd_measure": 5,

@@ -118,6 +118,7 @@ k_fold_adam(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restri
   float* mt = mbuf + (int64_t)blockIdx.x * TILE_ELEMS;
   float* vt = vbuf + (int64_t)blockIdx.x * TILE_ELEMS;
   const float* ft = fa.Ftiles ? fa.Ftiles + (int64_t)blockIdx.x * TILE_ELEMS : nullptr;
+  const float* gt_up = fa.Gtiles ? fa.Gtiles + (int64_t)blockIdx.x * TILE_ELEMS : nullptr;
 
   float s_clamp = 0.f, s_sq = 0.f, xmin = INFINITY, xmax = -INFINITY;
   float colp[8];
@@ -171,6 +172,7 @@ k_fold_adam(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restri
           esym += 4.f * fa.k2 * (ah - fmaxf(s, 0.f));
         }
         float g = ri * rj * esym + rhoi + sm.rhoJ[b] + acc[p][cg * 4 + k];
+        if (gt_up != nullptr) g += gt_up[off + k];
         g = pv.mask(xs[k]) * g + fa.norm_coef * p_ * inv_norm;
         const float mn = fa.beta1 * ms[k] + omb1 * g;
         const float vn = fa.beta2 * vs[k] + omb2 * g * g;

@@ -321,7 +321,10 @@ __global__ void k_node_bwd1(mcgra_node_args a) {
   zero16(a.Y4 + i * HID);
 }
 
-__global__ void k_node_rho(mcgra_node_args a) {
+// DIAG: the estimate has a non-zero diagonal M_ii = mdiag[i] (noisy path): A_hat_ii = r^2 (1 + M_ii), and the diagonal
+// entry enters rho's row and column parts with (M + I)_ii = 1 + M_ii
+template <bool DIAG>
+__global__ void k_node_rho(mcgra_node_args a, const float* __restrict__ mdiag) {
   __shared__ double red[32];
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const bool live = i < a.n;
@@ -355,7 +358,8 @@ __global__ void k_node_rho(mcgra_node_args a) {
       t = fmaf(s2[k], p3[k] + r * dz2[k], t);
     }
     // diagonal entry A_hat_ii = r^2 of the element-wise terms
-    const float aii = r * r;
+    const float mi1 = DIAG ? 1.f + mdiag[i] : 1.f;
+    const float aii = DIAG ? (r * mi1) * r : r * r;
     float eii = 0.f;
     if (a.k1 != 0.f && a.measure_nn == MCGRA_M_MSE) {
       const float f = a.Fdiag ? a.Fdiag[i] : 0.f;
@@ -378,7 +382,7 @@ __global__ void k_node_rho(mcgra_node_args a) {
       v2 = (double)a.k2 * (double)(aii * aii);
     }
     if (a.k7 != 0.f) v7 = (double)a.k7 * (double)ent_val(0.f);
-    const float tot = t + a.eps_row[i] + 2.f * eii * r;
+    const float tot = t + a.eps_row[i] + 2.f * eii * (DIAG ? mi1 * r : r);
     a.rho[i] = -0.5f * tot / (d * sqrtf(d));
     // fold factors, transposed: rows 0-63 U = [r dZ1 | r dZ2 | dQ1 | dQ2], rows 64-127 V = [r S1 | r S2 | S1 | T2]
     float* W = a.Wt + i;
@@ -434,7 +438,13 @@ int mcgra_node_bwd1(const mcgra_node_args* a, void* stream) {
   return 0;
 }
 int mcgra_node_rho(const mcgra_node_args* a, void* stream) {
-  k_node_rho<<<nblk(a->n), 128, 0, (cudaStream_t)stream>>>(*a);
+  k_node_rho<false><<<nblk(a->n), 128, 0, (cudaStream_t)stream>>>(*a, nullptr);
+  MCGRA_LAUNCH_CHECK();
+  return 0;
+}
+int mcgra_node_rho_diag(const mcgra_node_args* a, const float* mdiag, void* stream) {
+  if (mdiag == nullptr) return -1;
+  k_node_rho<true><<<nblk(a->n), 128, 0, (cudaStream_t)stream>>>(*a, mdiag);
   MCGRA_LAUNCH_CHECK();
   return 0;
 }

@@ -39,7 +39,7 @@ struct PropSmem {
 template <int KC, bool ELEM>
 __global__ void __launch_bounds__(128, 2)
 k_propagate(const float* __restrict__ tiles, int64_t n, int64_t t0, const float* mu, int raw,
-            const float* __restrict__ B, float* __restrict__ Y, mcgra_elem_args ea) {
+            const float* __restrict__ B, float* __restrict__ Y, mcgra_elem_args ea, int products) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   PropSmem<KC>& sm = *reinterpret_cast<PropSmem<KC>*>(smem_raw);
   int I, J;
@@ -139,6 +139,8 @@ k_propagate(const float* __restrict__ tiles, int64_t n, int64_t t0, const float*
 
   // ---- compute: warps 0-1 direct product (rows of I), warps 2-3 mirrored product (rows of J) -------------
   const int u = tid & 63;
+  // product selector (MCGRA_PROD_*): warps 0-1 carry the direct product, warps 2-3 the mirrored one
+  if (!(products & (warp < 2 ? MCGRA_PROD_DIRECT : MCGRA_PROD_MIRRORED))) return;
   float acc0[KC], acc1[KC];
 #pragma unroll
   for (int c = 0; c < KC; ++c) acc0[c] = acc1[c] = 0.f;
@@ -463,7 +465,8 @@ __device__ __forceinline__ void h_flush2(float* __restrict__ Y, int64_t n, int64
 template <int KC>
 __global__ void __launch_bounds__(H_THREADS, 1)
 k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* mu, int raw,
-              const unsigned char* __restrict__ Bk, const float* __restrict__ scale, float* __restrict__ Y, int dbg) {
+              const unsigned char* __restrict__ Bk, const float* __restrict__ scale, float* __restrict__ Y, int dbg,
+              int products) {
   const int I = tr0 + (int)blockIdx.y;
   const int Jbeg = (int)blockIdx.x * H_RUN;
   if (Jbeg > I) return;
@@ -483,6 +486,7 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
   constexpr uint32_t COL_D1 = 0, COL_D2 = 192;    // D1 of the even / odd tiles at 0 / 96, D2[b] at 192 + 96 b
   const bool tcwarp = warp == 12 || warp == 14;   // two issuing lanes: even / odd tiles of the run
   const bool rows_ok = (i0 + TILE <= n) && (pv.raw == 2);
+  const bool do_dir = (products & MCGRA_PROD_DIRECT) != 0, do_mir = (products & MCGRA_PROD_MIRRORED) != 0;
   const int64_t tix0 = tri((int64_t)I) - tri((int64_t)tr0);
 
   if (warp == 0) tc::tmem_alloc(&sm.tmem_base, 512);
@@ -538,11 +542,15 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
           const uint64_t db = (uint64_t)((uint32_t)ks * ((2u * LBO_B) >> 4));
           const uint32_t acc1 = (k > par || ks > 0) ? 1u : 0u, acc2 = ks > 0 ? 1u : 0u;
           // direct: A K-major (M = row: SBO 128 between 8-row groups; K = column: LBO H_SJ between 8-column groups)
-          mma_f16(d1, tc::make_desc(p0 + (uint32_t)ks * 2u * H_SJ, H_SJ, 128u), bJ0 + db, id_cat, acc1);
-          mma_f16(d1 + 2 * KC, tc::make_desc(p1 + (uint32_t)ks * 2u * H_SJ, H_SJ, 128u), bJ0 + db, id_one, acc1);
+          if (do_dir) {
+            mma_f16(d1, tc::make_desc(p0 + (uint32_t)ks * 2u * H_SJ, H_SJ, 128u), bJ0 + db, id_cat, acc1);
+            mma_f16(d1 + 2 * KC, tc::make_desc(p1 + (uint32_t)ks * 2u * H_SJ, H_SJ, 128u), bJ0 + db, id_one, acc1);
+          }
           // mirrored: the same image as an MN-major A operand (M = column: SBO H_SJ; K = row: LBO 128)
-          mma_f16(d2, tc::make_desc(p0 + (uint32_t)ks * 256u, 128u, H_SJ), bI0 + db, id_cat_t, acc2);
-          mma_f16(d2 + 2 * KC, tc::make_desc(p1 + (uint32_t)ks * 256u, 128u, H_SJ), bI0 + db, id_one_t, acc2);
+          if (do_mir) {
+            mma_f16(d2, tc::make_desc(p0 + (uint32_t)ks * 256u, 128u, H_SJ), bI0 + db, id_cat_t, acc2);
+            mma_f16(d2 + 2 * KC, tc::make_desc(p1 + (uint32_t)ks * 256u, 128u, H_SJ), bI0 + db, id_one_t, acc2);
+          }
         }
         tc::mma_commit(&sm.tile_done[b]);
         tc::mma_commit(&sm.bfree[r]);
@@ -559,7 +567,7 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
       const int b = k & 1;
       tc::mbar_wait(&sm.tile_done[b], (uint32_t)((k >> 1) & 1));
       tc::fence_after();
-      if (on) {
+      if (on && do_mir) {
 #pragma unroll
         for (int cg = 0; cg < KC / 16; ++cg)
           h_flush<KC>(Y, n, (int64_t)tile_of(k) * TILE + ltid, tlane + COL_D2 + (uint32_t)b * 96u, cg * 16, sm.inv_s + cg * 16);
@@ -567,7 +575,7 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
       tc::fence_before();
       mbar_arrive(&sm.flushed[b]);
     }
-    if (on) {                                            // the run's direct result (complete with the last tile_done)
+    if (on && do_dir) {                                  // the run's direct result (complete with the last tile_done)
 #pragma unroll
       for (int cg = 0; cg < KC / 16; ++cg) {
         if (nt >= 2) h_flush2<KC>(Y, n, i0 + ltid, tlane + COL_D1, tlane + COL_D1 + 96u, cg * 16, sm.inv_s + cg * 16);
@@ -638,7 +646,7 @@ inline int64_t prop_ws_bk_bytes(int64_t n, int K) {
 
 template <int KC>
 int launch_prop_h(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* B, float* Y,
-                  void* ws, cudaStream_t st) {
+                  void* ws, cudaStream_t st, int products) {
   const int64_t npad = (n + TILE - 1) / TILE * TILE;
   unsigned char* Bk = reinterpret_cast<unsigned char*>(ws);
   float* scale = reinterpret_cast<float*>(Bk + prop_ws_bk_bytes(n, KC));        // [s_c | 1/s_c | max bits]
@@ -652,7 +660,7 @@ int launch_prop_h(const float* tiles, int64_t n, int tr0, int tr1, const float* 
   if (e != cudaSuccess) return (int)e;
   if (tr1 - tr0 > 65535) return -3;
   dim3 grid((unsigned)((tr1 + H_RUN - 1) / H_RUN), (unsigned)(tr1 - tr0));
-  k_propagate_h<KC><<<grid, H_THREADS, smem, st>>>(tiles, n, tr0, mu, raw, Bk, scale, Y, g_prop_dbg);
+  k_propagate_h<KC><<<grid, H_THREADS, smem, st>>>(tiles, n, tr0, mu, raw, Bk, scale, Y, g_prop_dbg, products);
   MCGRA_LAUNCH_CHECK();
   return 0;
 }
@@ -972,13 +980,13 @@ k_elem_rs(const float* __restrict__ tiles, int64_t n, int tr0, int64_t ntiles, c
 
 template <int KC, bool ELEM>
 int launch_prop(const float* tiles, int64_t n, int64_t t0, int64_t nt, const float* mu, int raw, const float* B,
-                float* Y, const mcgra_elem_args* elem, cudaStream_t st) {
+                float* Y, const mcgra_elem_args* elem, cudaStream_t st, int products) {
   const size_t smem = sizeof(PropSmem<KC>);
   cudaError_t e = cudaFuncSetAttribute(k_propagate<KC, ELEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
   mcgra_elem_args ea = {};
   if (ELEM) ea = *elem;
-  k_propagate<KC, ELEM><<<(unsigned)nt, 128, smem, st>>>(tiles, n, t0, mu, raw, B, Y, ea);
+  k_propagate<KC, ELEM><<<(unsigned)nt, 128, smem, st>>>(tiles, n, t0, mu, raw, B, Y, ea, products);
   MCGRA_LAUNCH_CHECK();
   return 0;
 }
@@ -1062,26 +1070,33 @@ int64_t mcgra_propagate_ws_bytes(int64_t n, int K) {
   return prop_ws_bk_bytes(n, K) + npad * 2 * K * (int64_t)sizeof(float) + 256;
 }
 
-int mcgra_propagate(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* B, int K,
-                    float* Y, const mcgra_elem_args* elem, void* ws, void* stream) {
+int mcgra_propagate_sel(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* B, int K,
+                        float* Y, const mcgra_elem_args* elem, void* ws, int products, void* stream) {
   const int64_t nt = tri(tr1) - tri(tr0);
+  if (products < MCGRA_PROD_DIRECT || products > MCGRA_PROD_BOTH) return -1;
+  if (elem != nullptr && products != MCGRA_PROD_BOTH) return -1;     // the fused terms cover both orientations
   if (nt <= 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t t0 = tri(tr0);
   if (ws != nullptr && g_prop_engine == 5 && elem == nullptr) {
-    if (K == 32) return launch_prop_h<32>(tiles, n, tr0, tr1, mu, raw, B, Y, ws, st);
-    if (K == 16) return launch_prop_h<16>(tiles, n, tr0, tr1, mu, raw, B, Y, ws, st);
+    if (K == 32) return launch_prop_h<32>(tiles, n, tr0, tr1, mu, raw, B, Y, ws, st, products);
+    if (K == 16) return launch_prop_h<16>(tiles, n, tr0, tr1, mu, raw, B, Y, ws, st, products);
     return -1;
   }
   if (K == 32) {
-    return elem ? launch_prop<32, true>(tiles, n, t0, nt, mu, raw, B, Y, elem, st)
-                : launch_prop<32, false>(tiles, n, t0, nt, mu, raw, B, Y, nullptr, st);
+    return elem ? launch_prop<32, true>(tiles, n, t0, nt, mu, raw, B, Y, elem, st, products)
+                : launch_prop<32, false>(tiles, n, t0, nt, mu, raw, B, Y, nullptr, st, products);
   }
   if (K == 16) {
-    return elem ? launch_prop<16, true>(tiles, n, t0, nt, mu, raw, B, Y, elem, st)
-                : launch_prop<16, false>(tiles, n, t0, nt, mu, raw, B, Y, nullptr, st);
+    return elem ? launch_prop<16, true>(tiles, n, t0, nt, mu, raw, B, Y, elem, st, products)
+                : launch_prop<16, false>(tiles, n, t0, nt, mu, raw, B, Y, nullptr, st, products);
   }
   return -1;
+}
+
+int mcgra_propagate(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* B, int K,
+                    float* Y, const mcgra_elem_args* elem, void* ws, void* stream) {
+  return mcgra_propagate_sel(tiles, n, tr0, tr1, mu, raw, B, K, Y, elem, ws, MCGRA_PROD_BOTH, stream);
 }
 
 }  // extern "C"

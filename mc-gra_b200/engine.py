@@ -76,10 +76,24 @@ def output_band(n, rank, world):
     return min(n, rank * rb), min(n, (rank + 1) * rb)
 
 
+def check_noise_supported(measure, world, feature_adj, device):
+    """Scope of attack() with adjacency noise (--eps != 0): MSELoss on one CUDA device.  Raised before any device work."""
+    if measure != "MSELoss":
+        raise NotImplementedError(f"--eps != 0 is implemented for --measure MSELoss only (got {measure!r}): the other "
+                                  "measures' passes and closed forms assume a symmetric A_hat")
+    if world > 1 or isinstance(feature_adj, HostBands):
+        raise NotImplementedError("--eps != 0 runs on one GPU: the sharded (world > 1) / row-band noisy path is not built")
+    if torch.device(device).type != "cuda":
+        raise NotImplementedError(f"--eps != 0 needs a CUDA device (got {device!r}); there is no CPU fallback")
+
+
 class PGDEngine:
     def __init__(self, n, S1, W2, b1, b2, Wl, bl, labels, idx_attack, HA, YA, feature_adj, measure, weights,
                  lr, weight_sup=1.0, num_edges=None, x0=None, device="cuda", rank=0, world=1, group=None,
-                 max_epochs=1024, plain_gd=False):
+                 max_epochs=1024, plain_gd=False, eps=0.0, noise=None):
+        self.eps = float(eps)
+        if self.eps != 0.0:
+            check_noise_supported(measure, world, feature_adj, device)
         if not torch.cuda.is_available():
             raise N.NativeError("mcgra_b200 needs a CUDA device (sm_100a); there is no CPU fallback")
         N.lib()
@@ -178,6 +192,16 @@ class PGDEngine:
                 #  mirrored entries live on other ranks, so the band is taken as is instead of (F_ij + F_ji) / 2)
                 call("mcgra_dense_to_tiles", fa.data_ptr() - fa_row0 * n * 4, n, n, self.tr0, self.tr1,
                      0 if isinstance(feature_adj, HostBands) else 1, ptr(self.Ft), ptr(self.Fdiag), N.stream_ptr())
+                if self.eps != 0.0:
+                    # the noisy A_hat is not symmetric: c1 pairs A_hat_ij with F_ij and A_hat_ji with F_ji, so both
+                    # orientations of feature_adj are tiled as they are (F, then F^T)
+                    fdg = torch.zeros(n, **f32)
+                    self.FLt = torch.zeros(ntl, **f32)
+                    call("mcgra_dense_to_tiles", ptr(fa), n, n, 0, self.T, 0, ptr(self.FLt), ptr(fdg), N.stream_ptr())
+                    faT = fa.t().contiguous()
+                    self.FUt = torch.zeros(ntl, **f32)
+                    call("mcgra_dense_to_tiles", ptr(faT), n, n, 0, self.T, 0, ptr(self.FUt), ptr(fdg), N.stream_ptr())
+                    del faT, fdg
                 if world > 1:     # each rank wrote the diagonal of its own tile rows only
                     self._allreduce(self.Fdiag)
                 self.meas_nn = self.measure
@@ -271,7 +295,7 @@ class PGDEngine:
         # scalar and two consecutive iterations can be replayed as ONE CUDA graph (run()).  Large graphs keep the direct
         # history rows: launch overhead is < 1 % there and per-kernel CUDA-event timing stays possible.
         self.ring_mode = (GRAPH_MAX_N > 0 and n <= GRAPH_MAX_N and world == 1 and self.nn_mode in ("native", "off")
-                          and self.measure == N.M_MSE)
+                          and self.measure == N.M_MSE and self.eps == 0.0)
         self.acc_ring = torch.zeros(2, N.ACC_N, dtype=torch.float64, device=dev)
         self.step_dev = torch.zeros(1, dtype=torch.int32, device=dev)
         self._graph = None
@@ -323,6 +347,18 @@ class PGDEngine:
             self.nd_coef = z(int(N.lib().mcgra_nd_scratch_floats(self.nclass)))
             self.nd_m = float(idx.numel())
         _tick("state + node buffers")
+        if self.eps != 0.0:
+            # noisy path: the two orientations of M, its diagonal, the gradient tiles handed to the fold, and zero
+            # factors / rho for that fold (its own product and degree terms are already inside the gradient tiles)
+            self.Lt, self.Ut, self.Gn = (torch.zeros(nel, **f32) for _ in range(3))
+            self.mdiag = z(n)
+            self.Wt0, self.rho0 = z(128, self.npad), z(n)
+            if not self.c1_active or self.nn_mode != "native":
+                self.FLt = self.FUt = None
+            # (the default draw captures no reference to the engine: a cycle would keep its device memory alive
+            #  after attack() drops the engine)
+            self._noise_fn = noise if noise is not None else (
+                lambda t, n=n, dev=dev: torch.randn((n, n), dtype=torch.float32, device=dev))
         self.split_elem = True     # element-wise c1/c6 terms as a separate streaming pass (faster than fused, see DESIGN)
         self.set_parameter(x0)
         _tick("set_parameter")
@@ -433,6 +469,8 @@ class PGDEngine:
         t = self.step
         if t >= self.max_epochs:
             raise RuntimeError("acc history exhausted; construct the engine with a larger max_epochs")
+        if self.eps != 0.0:
+            return self._iterate_noisy(t)
         st = N.stream_ptr()
         n, tr0, tr1, mu, raw = self.n, self.tr0, self.tr1, ptr(self.mu), self.raw
         a = self.forward_stages(t)
@@ -504,6 +542,78 @@ class PGDEngine:
             call("mcgra_history_push", self._acc_row(t).data_ptr(), ptr(self.acc_hist), self.acc_hist.shape[0],
                  ptr(self.step_dev), st)
         self.step = t + 1
+
+    def _propagate_noisy(self, B, K, Y, transpose):
+        """Y += M B (transpose=False) or M^T B from the two orientation planes and the diagonal (mcgra.h)."""
+        st, n = N.stream_ptr(), self.n
+        first, second = (self.Ut, self.Lt) if transpose else (self.Lt, self.Ut)
+        for plane, sel in ((first, N.PROD_DIRECT), (second, N.PROD_MIRRORED)):
+            call("mcgra_propagate_sel", ptr(plane), n, self.tr0, self.tr1, None, 2, ptr(B), K, ptr(Y), None,
+                 ptr(self.prop_ws), sel, st, tag=f"propagate{K}_sel")
+        call("mcgra_diag_axpy", ptr(self.mdiag), ptr(B), K, n, ptr(Y), st)
+
+    def _iterate_noisy(self, t):
+        """One iteration with adjacency noise (--eps != 0, topology_attack.py:165, 474-478): single GPU, MSELoss.
+        noise stage -> node_pre -> M B1 -> node_mid -> M B2 -> node_head -> pairs (c7) -> noisy terms (c1, c2, c6)
+        -> node_bwd2 -> M^T B3 -> node_bwd1 -> M^T B4 -> node_rho_diag -> noisy gradient -> fold (Adam, clamp, sums)."""
+        st = N.stream_ptr()
+        n, tr0, tr1, mu, raw = self.n, self.tr0, self.tr1, ptr(self.mu), self.raw
+        noise = self._noise_fn(t)
+        if tuple(noise.shape) != (n, n):
+            raise ValueError(f"noise draw of shape {tuple(noise.shape)}, expected ({n}, {n})")
+        noise = noise.to(device=self.dev, dtype=torch.float32).contiguous()
+        call("mcgra_noise_stage", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(noise), self.eps, ptr(self.Lt), ptr(self.Ut),
+             ptr(self.mdiag), ptr(self.d), st)
+        a = self._node_args(t)
+        ap = C.byref(a)
+        call("mcgra_node_pre", ap, st)
+        self._propagate_noisy(self.B1, 32, self.Y1, False)
+        call("mcgra_node_mid", ap, st)
+        self._propagate_noisy(self.B2, 32, self.Y2, False)
+        call("mcgra_node_head", ap, st)
+        if self.k7 != 0.0:        # c7 is a function of the symmetric decode M1 only: the existing pass
+            call("mcgra_pairs", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.zhat), ptr(self.r), self.k7, 0.0, None, None,
+                 ptr(self.dzhat), ptr(self.eps_row), self._acc_row(t).data_ptr(), ptr(self.pairs_ws), st)
+        na = N.NoisyArgs()
+        na.n, na.npad, na.tr0, na.tr1 = n, self.npad, tr0, tr1
+        na.tiles, na.mu, na.raw, na.noise, na.eps = ptr(self.xt), mu, raw, ptr(noise), self.eps
+        na.Lt, na.Ut, na.FLt, na.FUt = ptr(self.Lt), ptr(self.Ut), ptr(self.FLt), ptr(self.FUt)
+        na.zhat, na.r, na.rho, na.Wt = ptr(self.zhat), ptr(self.r), ptr(self.rho), ptr(self.Wt)
+        na.k1 = self.k1 if self.FLt is not None else 0.0
+        na.k2, na.k6 = self.k2, self.k6
+        na.acc, na.eps_row, na.dzhat, na.Gt = self._acc_row(t).data_ptr(), ptr(self.eps_row), ptr(self.dzhat), ptr(self.Gn)
+        nap = C.byref(na)
+        call("mcgra_noisy_terms", nap, st)
+        call("mcgra_node_bwd2", ap, st)
+        self._propagate_noisy(self.B3, 32, self.Y3, True)
+        call("mcgra_node_bwd1", ap, st)
+        self._propagate_noisy(self.B4, 16, self.Y4, True)
+        call("mcgra_node_rho_diag", ap, ptr(self.mdiag), st)
+        call("mcgra_noisy_grad", nap, st)
+
+        f = N.FoldArgs()
+        f.n, f.npad, f.Wt, f.r, f.rho = n, self.npad, ptr(self.Wt0), ptr(self.r), ptr(self.rho0)
+        f.Ftiles, f.lseA, f.lseF, f.zhat = None, None, None, None
+        f.measure = N.M_NONE
+        f.k1, f.k6, f.k2 = 0.0, 0.0, 0.0
+        f.norm_coef = self.weight_sup * 0.001
+        f.lr, f.beta1, f.beta2, f.adam_eps = self.lr, 0.9, 0.999, 1e-8
+        f.step = t + 1
+        f.acc_prev = self._acc_row(t).data_ptr()
+        f.acc_next = self._acc_row(t + 1).data_ptr()
+        f.step_ptr = None
+        f.d_next = ptr(self.d_next)
+        f.store_clamped = 0 if self.proj_possible else 1
+        f.Wk = ptr(self.fold_ws)
+        f.plain_gd = 0
+        f.Gtiles = ptr(self.Gn)
+        call("mcgra_fold_adam", ptr(self.xt), ptr(self.mt), ptr(self.vt), tr0, tr1, mu, raw, C.byref(f),
+             ptr(self.minmax), st)
+        self.raw = 0 if self.proj_possible else 2
+        self.mu.zero_()
+        if self.proj_possible:
+            self._project(t)
+        self.step = t + 1     # (the degree of the next iteration comes from its own noise stage)
 
     def run(self, epochs, on_iter=None, use_graph="auto"):
         """`epochs` iterations.  In ring mode (small graphs) two consecutive iterations are captured once as a CUDA graph

@@ -22,7 +22,7 @@ from torch.nn.parameter import Parameter
 from . import _native as N
 from ._native import call, ptr
 from .base_attack import BaseAttack
-from .engine import HID, HostBands, PGDEngine, output_band
+from .engine import HID, HostBands, PGDEngine, check_noise_supported, output_band
 
 Align_Parameter_Cora = {"c1": 100, "c2": 1000, "c3": 100, "c4": 10, "c5": 10, "c6": 10, "c7": 10, "c8": 0.01,
                         "c9": 1, "c10": 1}
@@ -122,8 +122,11 @@ class PGDAttack(BaseAttack):
         self.args = args
         if self.loss_type != 'CE':
             raise NotImplementedError("native path implements loss_type='CE' (the reference driver's choice)")
-        if float(getattr(args, "eps", 0) or 0) != 0.0:
-            raise NotImplementedError("--eps != 0 (un-symmetrised n x n Gaussian noise, :474-478) is not built yet")
+        eps = float(getattr(args, "eps", 0) or 0)
+        if eps != 0.0:        # scope of the noisy path, checked before any device work
+            world_ = (torch.distributed.get_world_size()
+                      if torch.distributed.is_available() and torch.distributed.is_initialized() else 1)
+            check_noise_supported(args.measure, world_, feature_adj, self.device)
         dev = torch.device(self.device)
         n = self.nnodes
         timing = {} if kwargs.get("_timing") else None      # bench hook: phase wall-clock (adds synchronisations)
@@ -192,7 +195,8 @@ class PGDAttack(BaseAttack):
         self.engine = PGDEngine(n, S1, W2, b1, b2, Wl, bl, labels_t, idx_attack, HA_loop, YA_loop, fa,
                                 args.measure, weights, lr_ori, weight_sup=weight_supervised, num_edges=num_edges,
                                 x0=x0, device=dev, rank=rank, world=world,
-                                max_epochs=max(int(epochs), int(kwargs.get('_engine_epochs', 1)), 1))
+                                max_epochs=max(int(epochs), int(kwargs.get('_engine_epochs', 1)), 1),
+                                eps=eps, noise=kwargs.get("_noise"))
         eng = self.engine
         fa_on_host = not isinstance(feature_adj, HostBands) and not (torch.is_tensor(feature_adj) and feature_adj.is_cuda)
         if eng.nn_mode == "dense" and fa_on_host:
@@ -201,6 +205,7 @@ class PGDAttack(BaseAttack):
         self._trace = []
         self._timing = timing
         # test hook `_trace`: parameter after every iteration's projection; `_graph`: True / False force or forbid CUDA-graph replay (default: auto)
+        # `_noise`: callable(t) -> n x n draw of iteration t for --eps != 0 (default: torch.randn on the attack's device)
         on_iter = (lambda: self._trace.append(eng.packed_parameter())) if kwargs.get("_trace") else None
         eng.run(int(epochs), on_iter=on_iter, use_graph=kwargs.get("_graph", "auto"))
         if kwargs.get("_skip_finalize"):         # bench hook: engine is driven by the caller
