@@ -464,9 +464,12 @@ typedef struct {
   float* eps_row;          /* [n] += row and column parts of the element-wise degree gradient               */
   float* dzhat;            /* [n x 16] += gradient of c2 through M1                                         */
   float* Gt;               /* gradient tiles: dL/dx_ij (consumed by mcgra_fold_adam as Gtiles)              */
+  const float* gslab;      /* [n x nb] dL/dA_hat_ij for j < nb computed upstream (--measure KDE), or NULL;
+                              added to e'_ij (j < nb) and e'_ji (i < nb) of the stored entries                 */
+  int nb;                  /* columns of gslab, 1 <= nb <= MCGRA_TILE when gslab != NULL                     */
 } mcgra_noisy_args;
 /* c1 (MSE), c2 (MSE, both orientations of A_hat against the symmetric M1) and c6 over the off-diagonal entries:
- * values, eps_row, dzhat */
+ * values, eps_row, dzhat; gslab's part of eps_row.  Launches when any of k1, k2, k6 is non-zero or gslab != NULL. */
 int mcgra_noisy_terms(const mcgra_noisy_args* a, void* stream);
 /* dL/dx_ij = mask_ij dL/dM_ij + mask_ji dL/dM_ji with dL/dM_ij = U_i.V_j + r_i r_j e'_ij + rho_i, written to Gt */
 int mcgra_noisy_grad(const mcgra_noisy_args* a, void* stream);
@@ -503,6 +506,19 @@ int mcgra_kde_scalars(const double* mom, int d, double m, double weight, double*
 /* slab [n x NB] += first NB columns of A_hat from this rank's tile rows (caller zero-fills; all-reduce across ranks)     */
 int mcgra_slab_ahat(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* r, int NB,
                     float* slab, void* stream);
+/* the same for the noisy estimate (mcgra_noise_stage): A_hat_ij = r_i Lt_ij r_j below the diagonal, the entry above it
+ * (i < j < NB) from the U orientation of the stored entry (j, i), and A_hat_jj = r_j^2 (1 + mdiag[j])                    */
+int mcgra_slab_ahat_noisy(const float* Lt, const float* Ut, const float* mdiag, int64_t n, int tr0, int tr1,
+                          const float* r, int NB, float* slab, void* stream);
+/* fp64 MI of two value slabs X, Y [m x d] that share the bins j * bin_step (c1 / c2 on the noisy path, where MI is ~1e-6
+ * of the entropies it is the difference of): mcgra_kde_moments64 recomputes the kernel values in fp64 and adds
+ * wt * [sum kvX (d) | sum kvY (d) | sum kvX kvY^T (d*d)] to mom (caller zero-fills; layout of mcgra_kde_scalars, whose
+ * Syy block it leaves untouched); mcgra_kde_chain64 adds the gradient w.r.t. the values, given gmom = d loss / d mom,
+ * to gX and gY (either may be NULL).                                                                                    */
+int mcgra_kde_moments64(const float* X, const float* Y, int d, int64_t m, double bin_step, double wt, double* mom,
+                        void* stream);
+int mcgra_kde_chain64(const float* X, const float* Y, int d, int64_t m, double bin_step, double wt, const double* gmom,
+                      float* gX, float* gY, void* stream);
 int mcgra_slab_m1(const float* zhat, int64_t n, int NB, float* slab, void* stream);
 /* gradient slab G [n x NB] -> tiles (I, 0), I in [tr0, tr1), of G_ij + G_ji; diag[i] = G_ii for the rows of those tiles */
 int mcgra_slab_to_tiles(const float* G, int64_t n, int tr0, int tr1, int NB, float* tiles, float* diag, void* stream);

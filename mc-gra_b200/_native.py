@@ -58,7 +58,8 @@ class NoisyArgs(C.Structure):
     _fields_ = [("n", i64), ("npad", i64), ("tr0", C.c_int), ("tr1", C.c_int), ("tiles", c_fp), ("mu", c_fp),
                 ("raw", C.c_int), ("noise", c_fp), ("eps", C.c_float), ("Lt", c_fp), ("Ut", c_fp), ("FLt", c_fp),
                 ("FUt", c_fp), ("zhat", c_fp), ("r", c_fp), ("rho", c_fp), ("Wt", c_fp), ("k1", C.c_float),
-                ("k2", C.c_float), ("k6", C.c_float), ("acc", c_fp), ("eps_row", c_fp), ("dzhat", c_fp), ("Gt", c_fp)]
+                ("k2", C.c_float), ("k6", C.c_float), ("acc", c_fp), ("eps_row", c_fp), ("dzhat", c_fp), ("Gt", c_fp),
+                ("gslab", c_fp), ("nb", C.c_int)]
 
 
 PROD_DIRECT, PROD_MIRRORED, PROD_BOTH = 1, 2, 3
@@ -174,6 +175,9 @@ _SIGS = {
     "mcgra_kde_chain": (C.c_int, [c_fp, i64, c_fp, c_fp, C.c_int, i64, C.c_float, c_fp, C.c_int, c_fp]),
     "mcgra_kde_scalars": (C.c_int, [c_fp, C.c_int, C.c_double, C.c_double, c_fp, c_fp, c_fp]),
     "mcgra_slab_ahat": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, C.c_int, c_fp, c_fp]),
+    "mcgra_slab_ahat_noisy": (C.c_int, [c_fp, c_fp, c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, c_fp]),
+    "mcgra_kde_moments64": (C.c_int, [c_fp, c_fp, C.c_int, i64, C.c_double, C.c_double, c_fp, c_fp]),
+    "mcgra_kde_chain64": (C.c_int, [c_fp, c_fp, C.c_int, i64, C.c_double, C.c_double, c_fp, c_fp, c_fp, c_fp]),
     "mcgra_slab_m1": (C.c_int, [c_fp, i64, C.c_int, c_fp, c_fp]),
     "mcgra_slab_to_tiles": (C.c_int, [c_fp, i64, C.c_int, C.c_int, C.c_int, c_fp, c_fp, c_fp]),
     "mcgra_softmax_rows": (C.c_int, [c_fp, c_fp, c_fp, i64, C.c_int, c_fp, c_fp]),

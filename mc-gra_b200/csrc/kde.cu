@@ -78,12 +78,17 @@ __global__ void k_kde_scalars(const double* __restrict__ mom, int d, double m, d
   *acc_slot += weight * value;
 }
 
-// first NB columns of A_hat from the tiled triangle (tile column 0): slab[i][j] += r_i M_ij r_j (+ r_i^2 on the diagonal)
-__global__ void k_slab_ahat(const float* __restrict__ tiles, int64_t n, int tr0, int tr1, const float* mu, int raw,
-                            const float* __restrict__ r, int NB, float* __restrict__ slab) {
+// first NB columns of A_hat from the tiled triangle (tile column 0): slab[i][j] += r_i M_ij r_j (+ r_i^2 on the diagonal).
+// NOISY: M is the noisy estimate -- `tiles` is its L plane (values as stored, raw = 2), the mirrored entry A_hat_ji comes
+// from the U plane (M_ji at (i, j)) and the diagonal is r_i^2 (1 + mdiag[i]) (mcgra_noise_stage)
+template <bool NOISY>
+__global__ void k_slab_ahat(const float* __restrict__ tiles, const float* __restrict__ Ut, const float* __restrict__ mdiag,
+                            int64_t n, int tr0, const float* mu, int raw, const float* __restrict__ r, int NB,
+                            float* __restrict__ slab) {
   const ParamView pv = load_view(mu, raw);
   const int I = tr0 + blockIdx.x;
-  const float* t = tiles + (tri((int64_t)I) - tri((int64_t)tr0)) * TILE_ELEMS;     // tile (I, 0)
+  const int64_t toff = (tri((int64_t)I) - tri((int64_t)tr0)) * TILE_ELEMS;          // tile (I, 0)
+  const float* t = tiles + toff;
   for (int e = threadIdx.x; e < TILE * NB; e += blockDim.x) {
     const int a = e / NB, b = e % NB;
     const int64_t i = (int64_t)I * TILE + a, j = b;
@@ -91,9 +96,10 @@ __global__ void k_slab_ahat(const float* __restrict__ tiles, int64_t n, int tr0,
     if (j < i) {
       const float v = r[i] * pv.adj(t[a * TILE + b]) * r[j];
       slab[i * NB + j] += v;
-      if (i < NB) slab[j * NB + i] += v;                          // mirrored entry (j, i), both < NB: tile (0, 0) only
+      if (i < NB)                                                 // mirrored entry (j, i), both < NB: tile (0, 0) only
+        slab[j * NB + i] += NOISY ? (r[j] * Ut[toff + a * TILE + b]) * r[i] : v;
     } else if (i == j) {
-      slab[i * NB + j] += r[i] * r[i];
+      slab[i * NB + j] += NOISY ? (r[i] * (1.f + mdiag[i])) * r[i] : r[i] * r[i];
     }
   }
 }
@@ -165,6 +171,66 @@ __global__ void k_softmax_rows(const float* __restrict__ em, const float* __rest
   for (int q = 0; q < c; ++q) p2[i * c + q] = z[q] / den;
 }
 
+// fp64 variant for two n x NB value slabs with the same bins (c1 / c2 on the noisy path): the kernel values are
+// recomputed in fp64 and the moments accumulated from fp64 products.  MI is there a difference of entropies ~1e6 times
+// larger than itself, and fp32 kernel values or fp32 products would already move it by ~1e-4 relative.
+constexpr double KDE_S64 = 2.0 * 0.4 * 0.4;              // utils.py:986, as the fp64 reference evaluates it
+constexpr int KR64 = 64;                                  // rows per CTA of k_kde_moments64
+__device__ __forceinline__ double kde_kv64(float v, int j, double bin) {
+  const double z = ((double)v - (double)j * bin) / KDE_S64;
+  return exp(-0.5 * z * z);
+}
+// mom [s1 (d) | s2 (d) | Sxy (d*d)] += wt * sums over the rows (caller zero-fills; the Syy block is left untouched)
+__global__ void __launch_bounds__(256)
+k_kde_moments64(const float* __restrict__ X, const float* __restrict__ Y, int d, int64_t m, double bin, double wt,
+                double* __restrict__ mom) {
+  __shared__ double kx[KR64 * KDE_MAXD], ky[KR64 * KDE_MAXD];
+  const int64_t i0 = (int64_t)blockIdx.x * KR64;
+  for (int e = threadIdx.x; e < KR64 * d; e += blockDim.x) {
+    const int64_t i = i0 + e / d;
+    const int j = e % d;
+    kx[e] = i < m ? kde_kv64(X[i * d + j], j, bin) : 0.0;
+    ky[e] = i < m ? kde_kv64(Y[i * d + j], j, bin) : 0.0;
+  }
+  __syncthreads();
+  for (int q = threadIdx.x; q < 2 * d + d * d; q += blockDim.x) {
+    double s = 0.0;
+    if (q < d) {
+      for (int r = 0; r < KR64; ++r) s += kx[r * d + q];
+    } else if (q < 2 * d) {
+      for (int r = 0; r < KR64; ++r) s += ky[r * d + q - d];
+    } else {
+      const int a = (q - 2 * d) / d, b = (q - 2 * d) % d;
+      for (int r = 0; r < KR64; ++r) s += kx[r * d + a] * ky[r * d + b];
+    }
+    if (s != 0.0) atomicAdd(mom + q, wt * s);
+  }
+}
+// backward through the moments and the kernel to the values: with g = d loss / d mom (mcgra_kde_scalars)
+//   gX[i][a] += wt (g_s1[a] + sum_b g_Sxy[a][b] kvy_b) kvx_a (-(x - bin_a) / s^2),  gY likewise with g_s2, g_Sxy^T
+__global__ void k_kde_chain64(const float* __restrict__ X, const float* __restrict__ Y, int d, int64_t m, double bin,
+                              double wt, const double* __restrict__ g, float* __restrict__ gX, float* __restrict__ gY) {
+  const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= m * d) return;
+  const int64_t i = e / d;
+  const int a = (int)(e % d);
+  const double* gJ = g + 2 * d;
+  double sx = g[a], sy = g[d + a];
+  for (int b = 0; b < d; ++b) {
+    sx += gJ[a * d + b] * kde_kv64(Y[i * d + b], b, bin);
+    sy += gJ[b * d + a] * kde_kv64(X[i * d + b], b, bin);
+  }
+  const double c = -wt / (KDE_S64 * KDE_S64);
+  if (gX != nullptr) {
+    const double zx = (double)X[e] - (double)a * bin;
+    gX[e] = (float)((double)gX[e] + sx * kde_kv64(X[e], a, bin) * zx * c);
+  }
+  if (gY != nullptr) {
+    const double zy = (double)Y[e] - (double)a * bin;
+    gY[e] = (float)((double)gY[e] + sy * kde_kv64(Y[e], a, bin) * zy * c);
+  }
+}
+
 }  // namespace
 
 extern "C" {
@@ -193,7 +259,35 @@ int mcgra_kde_scalars(const double* mom, int d, double m, double weight, double*
 int mcgra_slab_ahat(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* r, int NB,
                     float* slab, void* stream) {
   if (NB < 1 || NB > KDE_MAXD) return -1;
-  if (tr1 > tr0) k_slab_ahat<<<(unsigned)(tr1 - tr0), 256, 0, (cudaStream_t)stream>>>(tiles, n, tr0, tr1, mu, raw, r, NB, slab);
+  if (tr1 > tr0)
+    k_slab_ahat<false><<<(unsigned)(tr1 - tr0), 256, 0, (cudaStream_t)stream>>>(tiles, nullptr, nullptr, n, tr0, mu, raw,
+                                                                              r, NB, slab);
+  MCGRA_LAUNCH_CHECK();
+  return 0;
+}
+int mcgra_slab_ahat_noisy(const float* Lt, const float* Ut, const float* mdiag, int64_t n, int tr0, int tr1,
+                          const float* r, int NB, float* slab, void* stream) {
+  if (NB < 1 || NB > KDE_MAXD || Lt == nullptr || Ut == nullptr || mdiag == nullptr) return -1;
+  if (tr1 > tr0)
+    k_slab_ahat<true><<<(unsigned)(tr1 - tr0), 256, 0, (cudaStream_t)stream>>>(Lt, Ut, mdiag, n, tr0, nullptr, 2, r, NB,
+                                                                             slab);
+  MCGRA_LAUNCH_CHECK();
+  return 0;
+}
+int mcgra_kde_moments64(const float* X, const float* Y, int d, int64_t m, double bin_step, double wt, double* mom,
+                        void* stream) {
+  if (d < 1 || d > KDE_MAXD) return -1;
+  if (m <= 0) return 0;
+  k_kde_moments64<<<(unsigned)((m + KR64 - 1) / KR64), 256, 0, (cudaStream_t)stream>>>(X, Y, d, m, bin_step, wt, mom);
+  MCGRA_LAUNCH_CHECK();
+  return 0;
+}
+int mcgra_kde_chain64(const float* X, const float* Y, int d, int64_t m, double bin_step, double wt, const double* gmom,
+                      float* gX, float* gY, void* stream) {
+  if (d < 1 || d > KDE_MAXD) return -1;
+  if (m <= 0) return 0;
+  k_kde_chain64<<<(unsigned)((m * d + 255) / 256), 256, 0, (cudaStream_t)stream>>>(X, Y, d, m, bin_step, wt, gmom, gX,
+                                                                                 gY);
   MCGRA_LAUNCH_CHECK();
   return 0;
 }

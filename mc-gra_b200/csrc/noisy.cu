@@ -10,6 +10,8 @@
 //   k_noise_diag    M_ii and d_i = 1 + M_ii                         (before k_noise_stage adds the row sums)
 //   k_noisy_terms   c1 / c2 (MSELoss) and c6 over both orientations, degree-gradient row + column parts, dzhat of c2
 //   k_noisy_grad    dL/dx_ij = mask_ij dL/dM_ij + mask_ji dL/dM_ji into gradient tiles for mcgra_fold_adam (Gtiles)
+// Both also take an upstream gradient of the first nb columns of A_hat (gslab, --measure KDE): it only reaches tiles of
+// tile column 0, where it is added to e'_ij (column j < nb) and to e'_ji (row i < nb, i.e. tile (0, 0)).
 // All are exact fp32 (FFMA) one-tile-per-CTA kernels.  The sums p + N*eps are formed as the reference forms them -- one
 // rounded product, one rounded sum (no FMA) -- so the clamp masks agree with torch's on the same draw.
 #include "common.cuh"
@@ -122,6 +124,13 @@ __device__ __forceinline__ ElemOut elem_terms(const mcgra_noisy_args& a, float a
   return o;
 }
 
+// upstream dL/dA_hat of the first nb columns (slab [n x nb]) at the stored entry (i, j), i > j, of a tile of column 0:
+// A_hat_ij is slab entry (i, j) when j < nb, A_hat_ji is slab entry (j, i) when i < nb
+__device__ __forceinline__ void add_slab_grad(const mcgra_noisy_args& a, int64_t gi, int64_t gj, ElemOut& e) {
+  if (gj < a.nb) e.eij += a.gslab[gi * a.nb + gj];
+  if (gi < a.nb) e.eji += a.gslab[gj * a.nb + gi];
+}
+
 struct TermsSmem {
   float c[TILE][NT_LD];                  // dL/dS_ij of c2 (S = zhat zhat^T)
   float zI[TILE][HID + 1], zJ[TILE][HID + 1];
@@ -144,6 +153,7 @@ k_noisy_terms(mcgra_noisy_args na, int64_t t0) {
     sm.colacc[tid] = 0.f;
   }
   const bool c2 = na.k2 != 0.f;
+  const bool slab = J == 0 && na.gslab != nullptr;
   if (c2) {
     for (int e = tid; e < TILE * HID; e += 256) {
       const int r = e >> 4, q = e & 15;
@@ -175,7 +185,8 @@ k_noisy_terms(mcgra_noisy_args na, int64_t t0) {
 #pragma unroll
           for (int q = 0; q < HID; ++q) s = fmaf(sm.zI[a][q], sm.zJ[b][q], s);
         }
-        const ElemOut e = elem_terms<true>(na, (ri * L) * rj, (rj * U) * ri, fij, fji, s, v1, v2, v6);
+        ElemOut e = elem_terms<true>(na, (ri * L) * rj, (rj * U) * ri, fij, fji, s, v1, v2, v6);
+        if (slab) add_slab_grad(na, gi, gj, e);
         if (c2 && s > 0.f) cc = -2.f * na.k2 * ((((ri * L) * rj) - s) + (((rj * U) * ri) - s));
         const float t = e.eij * L + e.eji * U;         // row i: e'_ij M_ij r_j; row j: e'_ji M_ji r_i (+ column parts)
         rowp += t * rj;
@@ -252,6 +263,7 @@ k_noisy_grad(mcgra_noisy_args na, int64_t t0) {
   const int64_t n = na.n, np = na.npad, i0 = (int64_t)I * TILE, j0 = (int64_t)J * TILE;
   const int64_t base = (int64_t)blockIdx.x * TILE_ELEMS;
   const bool c2 = na.k2 != 0.f;
+  const bool slab = J == 0 && na.gslab != nullptr;
   if (tid < TILE) {
     const int64_t gi = i0 + tid, gj = j0 + tid;
     sm.rI[tid] = gi < n ? na.r[gi] : 0.f;
@@ -336,7 +348,8 @@ k_noisy_grad(mcgra_noisy_args na, int64_t t0) {
 #pragma unroll
             for (int q = 0; q < HID; ++q) s = fmaf(sm.zI[a][q], sm.zJ[b][q], s);
           }
-          const ElemOut e = elem_terms<false>(na, (ri * L) * rj, (rj * U) * ri, fl[k], fu[k], s, dummy, dummy, dummy);
+          ElemOut e = elem_terms<false>(na, (ri * L) * rj, (rj * U) * ri, fl[k], fu[k], s, dummy, dummy, dummy);
+          if (slab) add_slab_grad(na, gi, gj, e);
           const float gij = acc[0][p][cg * 4 + k] + ri * rj * e.eij + rhoi;
           const float gji = acc[1][p][cg * 4 + k] + ri * rj * e.eji + sm.rhoJ[b];
           g[k] = box_mask(vl) * gij + box_mask(vu) * gji;
@@ -349,7 +362,8 @@ k_noisy_grad(mcgra_noisy_args na, int64_t t0) {
 
 inline bool noisy_args_ok(const mcgra_noisy_args* a) {
   return a != nullptr && a->n > 0 && a->tiles != nullptr && a->noise != nullptr && a->r != nullptr &&
-         (a->k1 == 0.f || (a->FLt != nullptr && a->FUt != nullptr)) && (a->k2 == 0.f || a->zhat != nullptr);
+         (a->k1 == 0.f || (a->FLt != nullptr && a->FUt != nullptr)) && (a->k2 == 0.f || a->zhat != nullptr) &&
+         (a->gslab == nullptr || (a->nb >= 1 && a->nb <= TILE));
 }
 
 }  // namespace
@@ -382,7 +396,7 @@ int mcgra_diag_axpy(const float* mdiag, const float* B, int K, int64_t n, float*
 int mcgra_noisy_terms(const mcgra_noisy_args* a, void* stream) {
   if (!noisy_args_ok(a) || a->Lt == nullptr || a->Ut == nullptr) return -1;
   const int64_t nt = tri(a->tr1) - tri(a->tr0);
-  if (nt <= 0 || (a->k1 == 0.f && a->k2 == 0.f && a->k6 == 0.f)) return 0;
+  if (nt <= 0 || (a->k1 == 0.f && a->k2 == 0.f && a->k6 == 0.f && a->gslab == nullptr)) return 0;
   const size_t smem = sizeof(TermsSmem);
   cudaError_t e = cudaFuncSetAttribute(k_noisy_terms, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;

@@ -76,11 +76,15 @@ def output_band(n, rank, world):
     return min(n, rank * rb), min(n, (rank + 1) * rb)
 
 
+NOISE_MEASURES = ("MSELoss", "KDE")
+
+
 def check_noise_supported(measure, world, feature_adj, device):
-    """Scope of attack() with adjacency noise (--eps != 0): MSELoss on one CUDA device.  Raised before any device work."""
-    if measure != "MSELoss":
-        raise NotImplementedError(f"--eps != 0 is implemented for --measure MSELoss only (got {measure!r}): the other "
-                                  "measures' passes and closed forms assume a symmetric A_hat")
+    """Scope of attack() with adjacency noise (--eps != 0): MSELoss or KDE on one CUDA device.  Raised before any device
+    work."""
+    if measure not in NOISE_MEASURES:
+        raise NotImplementedError(f"--eps != 0 is implemented for --measure MSELoss and KDE only (got {measure!r}): the "
+                                  "other measures' passes and closed forms assume a symmetric A_hat")
     if world > 1 or isinstance(feature_adj, HostBands):
         raise NotImplementedError("--eps != 0 runs on one GPU: the sharded (world > 1) / row-band noisy path is not built")
     if torch.device(device).type != "cuda":
@@ -222,8 +226,10 @@ class PGDEngine:
             if isinstance(feature_adj, HostBands):
                 raise NotImplementedError("row-band feature_adj input is implemented for the element-wise measures (MSELoss, "
                                           "KL with w2 = 0); pass a full tensor for HSIC / CKA / DP / KL-c2")
-            self.Ft = torch.zeros(ntl, **f32)      # dL/dA_ij + dL/dA_ji
-            self.Ct = torch.zeros(ntl, **f32)      # dL/dM1_ij + dL/dM1_ji
+            # dL/dA_ij + dL/dA_ji and dL/dM1_ij + dL/dM1_ji.  The noisy path (KDE) hands the A_hat gradient to its own
+            # kernels as a column slab, and needs the M1 tiles only when c2 is on
+            self.Ft = torch.zeros(ntl, **f32) if self.eps == 0.0 else None
+            self.Ct = torch.zeros(ntl, **f32) if (self.eps == 0.0 or w2 != 0) else None
             self.Fdiag = torch.zeros(n, **f32)     # dL/dA_ii
             self.meas_nn = N.M_PRE
             self.sgn = sgn
@@ -245,7 +251,9 @@ class PGDEngine:
                                      gA=torch.zeros(n, nb, **f32), gM=torch.zeros(n, nb, **f32),
                                      mom=torch.zeros(2 * nb + 2 * nb * nb, dtype=torch.float64, device=dev),
                                      gmom=torch.zeros(2 * nb + 2 * nb * nb, dtype=torch.float64, device=dev))
-                if self.c1_active:
+                if self.c1_active and self.eps != 0.0:     # the noisy path's fp64 stage forms kernel values itself
+                    kd["slabF"] = fa[:, :nb].contiguous()
+                elif self.c1_active:
                     kd["kvF"] = torch.zeros(n, nb, **f32)
                     call("mcgra_kde_kv", ptr(fa), n, nb, n, kd["bin"], ptr(kd["kvF"]), N.stream_ptr())
             else:
@@ -553,9 +561,10 @@ class PGDEngine:
         call("mcgra_diag_axpy", ptr(self.mdiag), ptr(B), K, n, ptr(Y), st)
 
     def _iterate_noisy(self, t):
-        """One iteration with adjacency noise (--eps != 0, topology_attack.py:165, 474-478): single GPU, MSELoss.
-        noise stage -> node_pre -> M B1 -> node_mid -> M B2 -> node_head -> pairs (c7) -> noisy terms (c1, c2, c6)
-        -> node_bwd2 -> M^T B3 -> node_bwd1 -> M^T B4 -> node_rho_diag -> noisy gradient -> fold (Adam, clamp, sums)."""
+        """One iteration with adjacency noise (--eps != 0, topology_attack.py:165, 474-478): single GPU, MSELoss or KDE.
+        noise stage -> node_pre -> M B1 -> node_mid -> M B2 -> node_head -> [KDE: c1 / c2 slab stage, c9 / c10]
+        -> pairs (c7, KDE: c2's M1 gradient) -> noisy terms (c1, c2, c6; KDE: the A_hat slab gradient) -> node_bwd2
+        -> M^T B3 -> node_bwd1 -> M^T B4 -> node_rho_diag -> noisy gradient -> fold (Adam, clamp, sums)."""
         st = N.stream_ptr()
         n, tr0, tr1, mu, raw = self.n, self.tr0, self.tr1, ptr(self.mu), self.raw
         noise = self._noise_fn(t)
@@ -571,9 +580,16 @@ class PGDEngine:
         call("mcgra_node_mid", ap, st)
         self._propagate_noisy(self.B2, 32, self.Y2, False)
         call("mcgra_node_head", ap, st)
-        if self.k7 != 0.0:        # c7 is a function of the symmetric decode M1 only: the existing pass
-            call("mcgra_pairs", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.zhat), ptr(self.r), self.k7, 0.0, None, None,
-                 ptr(self.dzhat), ptr(self.eps_row), self._acc_row(t).data_ptr(), ptr(self.pairs_ws), st)
+        kde = self.nn_mode == "kde"
+        if kde:
+            self._kde_stage_noisy(t)
+        if self.measure == N.M_KDE and (self.w9 != 0.0 or self.w10 != 0.0):
+            self._kde_nd_stage(t)
+        # c7 and the M1 side of KDE's c2 are functions of the symmetric decode M1 only: the existing pass, with no A_hat
+        # tiles (EAt = NULL): the noisy kernels form A_hat's part of eps_row themselves
+        if self.k7 != 0.0 or self.Ct is not None:
+            call("mcgra_pairs", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.zhat), ptr(self.r), self.k7, 0.0, None,
+                 ptr(self.Ct), ptr(self.dzhat), ptr(self.eps_row), self._acc_row(t).data_ptr(), ptr(self.pairs_ws), st)
         na = N.NoisyArgs()
         na.n, na.npad, na.tr0, na.tr1 = n, self.npad, tr0, tr1
         na.tiles, na.mu, na.raw, na.noise, na.eps = ptr(self.xt), mu, raw, ptr(noise), self.eps
@@ -582,6 +598,8 @@ class PGDEngine:
         na.k1 = self.k1 if self.FLt is not None else 0.0
         na.k2, na.k6 = self.k2, self.k6
         na.acc, na.eps_row, na.dzhat, na.Gt = self._acc_row(t).data_ptr(), ptr(self.eps_row), ptr(self.dzhat), ptr(self.Gn)
+        if kde:
+            na.gslab, na.nb = ptr(self.kde["gA"]), self.kde["nb"]
         nap = C.byref(na)
         call("mcgra_noisy_terms", nap, st)
         call("mcgra_node_bwd2", ap, st)
@@ -762,6 +780,37 @@ class PGDEngine:
             call("mcgra_kde_chain", ptr(kd["slabM"]), nb, ptr(kd["kvM"]), ptr(kd["gkvM"]), nb, n, bin_, ptr(kd["gM"]), 0, st)
             call("mcgra_slab_to_tiles", ptr(kd["gM"]), n, self.tr0, self.tr1, nb, ptr(self.Ct), None, st)
         call("mcgra_slab_to_tiles", ptr(kd["gA"]), n, self.tr0, self.tr1, nb, ptr(self.Ft), None, st)
+        self.Fdiag.zero_()
+        self.Fdiag[:nb].copy_(kd["gA"][:nb, :nb].diagonal())
+
+    def _kde_stage_noisy(self, t):
+        """c1 / c2 under --measure KDE with adjacency noise (single GPU).  The draw decorrelates A_hat from feature_adj
+        and from M1, so each MI is ~1e-6 of the entropies it is the difference of: the kernel values and the moments are
+        formed in fp64 from the value slabs (mcgra_kde_moments64 / _chain64).  A_hat is gathered from the noisy
+        estimate's planes; its gradient stays the slab kd["gA"] (mcgra_noisy_terms / mcgra_noisy_grad read it as gslab),
+        its diagonal goes to Fdiag, M1's gradient to the tiles Ct."""
+        st = N.stream_ptr()
+        kd, n = self.kde, self.n
+        nb, bin_, wt = kd["nb"], float(n) / float(n - 1), 1.0 / n
+        acc = self._acc_row(t).data_ptr()
+        kd["slabA"].zero_()
+        call("mcgra_slab_ahat_noisy", ptr(self.Lt), ptr(self.Ut), ptr(self.mdiag), n, self.tr0, self.tr1, ptr(self.r), nb,
+             ptr(kd["slabA"]), st)
+        kd["gA"].zero_()
+        pairs = []
+        if self.c1_active:
+            pairs.append((kd["slabF"], kd["slabA"], kd["k1c"], ACC["C1D"], None, kd["gA"]))
+        if self.w2 != 0:
+            call("mcgra_slab_m1", ptr(self.zhat), n, nb, ptr(kd["slabM"]), st)
+            kd["gM"].zero_()
+            pairs.append((kd["slabA"], kd["slabM"], kd["k2c"], ACC["C2D"], kd["gA"], kd["gM"]))
+        for X, Y, weight, slot, gX, gY in pairs:
+            kd["mom"].zero_()
+            call("mcgra_kde_moments64", ptr(X), ptr(Y), nb, n, bin_, wt, ptr(kd["mom"]), st)
+            call("mcgra_kde_scalars", ptr(kd["mom"]), nb, float(n), weight, acc + 8 * slot, ptr(kd["gmom"]), st)
+            call("mcgra_kde_chain64", ptr(X), ptr(Y), nb, n, bin_, wt, ptr(kd["gmom"]), ptr(gX), ptr(gY), st)
+        if self.w2 != 0:
+            call("mcgra_slab_to_tiles", ptr(kd["gM"]), n, self.tr0, self.tr1, nb, ptr(self.Ct), None, st)
         self.Fdiag.zero_()
         self.Fdiag[:nb].copy_(kd["gA"][:nb, :nb].diagonal())
 

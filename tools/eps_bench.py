@@ -1,8 +1,9 @@
 """attack() with adjacency noise (--eps != 0) against the noise-free loop on one GPU: device-event it/s, peak device memory,
 per-kernel times of the noisy stages as fractions of the HBM peak, and a 3-iteration exact-FFMA vs default-engine
-comparison at the largest size with injected noise.  Profile A (README Cora weights), bench.py's synthetic inputs.
+comparison at the largest size with injected noise.  bench.py's synthetic inputs; --measure MSELoss runs Profile A (README
+Cora weights), --measure KDE the README's Cora K = {X, Y} KDE command (w1 = 1000, w6 = 0.01, lr = 1e-3).
 
-    python tools/eps_bench.py [--sizes cora,large] [--steps 10] [--out profiles/eps_bench.json]
+    python tools/eps_bench.py [--measure MSELoss|KDE] [--sizes cora,large] [--steps 10] [--out FILE]
 """
 import argparse
 import gc
@@ -19,6 +20,10 @@ sys.path.insert(0, ROOT)
 import bench  # noqa: E402  (the benchmark's problem builder and kernel timers)
 
 HBM_PEAK_GBS = 7700.0      # HGX B200 data sheet, one GPU
+# measure -> (weights w1..w10, lr exponent, description, default output)
+MEASURES = {"MSELoss": (bench.PROFILE_A, -2.0, bench.PROFILES["A"]["flags"], "eps_bench.json"),
+            "KDE": ((1000, 0, 0, 0, 0, 0.01, 0, 0, 0, 0), -3.0, "README Cora K={X,Y} KDE: w1=1000 w6=.01 lr=1e-3",
+                    "eps_kde_bench.json")}
 
 
 def card():
@@ -27,23 +32,28 @@ def card():
     return r.stdout.strip().splitlines()[0] if r.returncode == 0 and r.stdout.strip() else "unknown"
 
 
-def noisy_bytes(P):
+def noisy_bytes(P, n, feat, nb):
     """Compulsory HBM bytes per launch of each noisy stage (P = stored entries; a noise block is read twice: once per
-    orientation)."""
-    return {"mcgra_noise_stage": 20 * P, "propagate32_sel": 4 * P, "propagate16_sel": 4 * P, "mcgra_noisy_terms": 16 * P,
-            "mcgra_noisy_grad": 24 * P, "mcgra_fold_adam": 28 * P, "randn": 8 * P}
+    orientation; feat: the terms and gradient passes read both orientations of feature_adj (c1 under MSELoss); the KDE
+    gather reads nb columns of the L plane and updates an n x nb slab)."""
+    f = 8 * P if feat else 0
+    return {"mcgra_noise_stage": 20 * P, "propagate32_sel": 4 * P, "propagate16_sel": 4 * P, "mcgra_noisy_terms": 8 * P + f,
+            "mcgra_noisy_grad": 16 * P + f, "mcgra_fold_adam": 28 * P, "randn": 8 * P, "mcgra_slab_ahat_noisy": 12 * n * nb}
 
 
-def build(wl_name, eps, steps, noise=None):
+def build(wl_name, eps, steps, noise=None, measure="MSELoss"):
     from mcgra_b200 import _native as N
     dev = torch.device("cuda", 0)
     prob = bench.build_problem(bench.WORKLOADS[wl_name], dev)
+    weights, lr, _, _ = MEASURES[measure]
     args = bench.make_args("A")
-    args.eps = eps
+    args.eps, args.measure, args.lr = eps, measure, lr
+    for k, w in enumerate(weights, 1):
+        setattr(args, f"w{k}", w)
     atk, adj = bench.make_attack(prob, dev)
     n = prob["n"]
     kw = {} if noise is None else {"_noise": noise}
-    atk.attack(args, None, 10 ** args.lr, 0, 1.0, bench.PROFILE_A, prob["feature_adj"], 0, 0, 0, None, None, None, adj,
+    atk.attack(args, None, 10 ** args.lr, 0, 1.0, weights, prob["feature_adj"], 0, 0, 0, None, None, None, adj,
                prob["X"], torch.zeros(1), prob["labels"], prob["idx_attack"], int(1e7 * prob["nedges"]), 0, epochs=0,
                _engine_epochs=steps + 16, _skip_finalize=True, **kw)
     del prob
@@ -87,28 +97,32 @@ def kernels(atk, steps=3):
 
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument("--measure", default="MSELoss", choices=list(MEASURES))
     ap.add_argument("--sizes", default="cora,large")
     ap.add_argument("--steps", type=int, default=10)
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "eps_bench.json"))
+    ap.add_argument("--out", default=None, help="default: profiles/eps_bench.json (MSELoss), profiles/eps_kde_bench.json (KDE)")
     a = ap.parse_args()
+    if a.out is None:
+        a.out = os.path.join(ROOT, "profiles", MEASURES[a.measure][3])
     if not torch.cuda.is_available():
         raise SystemExit("eps_bench needs a CUDA device")
     from mcgra_b200 import _native as N
-    out = {"card": card(), "profile": bench.PROFILES["A"]["flags"], "hbm_peak_gbs_datasheet": HBM_PEAK_GBS, "sizes": {}}
+    out = {"card": card(), "profile": MEASURES[a.measure][2], "hbm_peak_gbs_datasheet": HBM_PEAK_GBS, "sizes": {}}
     print(out["card"], flush=True)
     for wl in a.sizes.split(","):
         rec = {}
         for eps in (0.0, 0.05):
             torch.cuda.empty_cache()
             torch.cuda.reset_peak_memory_stats()
-            atk = build(wl, eps, a.steps + 8)
+            atk = build(wl, eps, a.steps + 8, measure=a.measure)
             ms = time_loop(atk, 2, a.steps)
             r = {"ms_per_iter": ms, "it_s": 1000.0 / ms, "peak_mem_gb": torch.cuda.max_memory_allocated() / 1e9}
             if eps != 0.0:
                 n = atk.engine.n
                 P = n * (n - 1) // 2
                 kt, kc = kernels(atk)
-                by = noisy_bytes(P)
+                eng = atk.engine
+                by = noisy_bytes(P, n, getattr(eng, "FLt", None) is not None, eng.kde["nb"] if eng.nn_mode == "kde" else 0)
                 r["kernels"] = {k: {"ms": kt[k], "launches_per_iter": kc[k],
                                     **({"hbm_frac": by[k] / (kt[k] * 1e-3) / (HBM_PEAK_GBS * 1e9)} if k in by else {})}
                                 for k in kt}
@@ -135,7 +149,7 @@ def main():
             g.manual_seed(1000 + t)
             n = atk.engine.n
             return torch.randn((n, n), dtype=torch.float32, device=dev, generator=g)
-        atk = build(wl, 0.05, 3, noise=noise)
+        atk = build(wl, 0.05, 3, noise=noise, measure=a.measure)
         atk.engine.run(3)
         res.append((atk.engine.losses()["loss"], atk.engine.packed_parameter()[:1 << 22].cpu().numpy()))
         atk.engine = None
