@@ -546,6 +546,30 @@ int mcgra_auc_stage(int stage, const float* scores, const uint8_t* labels, int64
 int64_t mcgra_sort_workspace_bytes(int64_t N);
 int mcgra_argsort_desc(const float* scores, int64_t N, int64_t* order, void* ws, void* stream);
 
+/* ---- top-k recovered edges ----
+ * The k largest S[i, j] over the strict upper triangle (i < j) of a dense row-major n x n fp32 score matrix, or of the
+ * row band scores = rows [row0, row0 + rows) of it (leading dimension n), in row-major index order i * n + j.  Sorting
+ * the k values with the stable mcgra_argsort_desc then gives (score descending, index ascending).  fkey order: -0.0 ==
+ * +0.0, +-inf allowed; NaN candidates are counted and must be rejected by the caller.  1 <= k <= n (n - 1) / 2.
+ * Stages, in order 0 .. 7, each on every rank that holds a band:
+ *   0, 2, 4  histogram of level 0, 1, 2 (2^11, 2^11, 2^10 bins of key bits 31..21, 20..10, 9..0, over the candidates that
+ *            match the prefix selected so far): int64 hist[2049] at byte MCGRA_TOPK_HIST_OFFSET, the bins followed by
+ *            the number of NaN candidates (stage 0 only).  With row bands the caller sums hist over ranks (all-reduce)
+ *            before the next stage.
+ *   1, 3, 5  select the bin of the remaining-th largest key from hist; after stage 5, int64 at byte 0 = tau (the key of
+ *            the k-th largest candidate) and at byte 8 = t (candidates == tau still to take).  int64 at byte 32 is set to
+ *            1 when hist holds fewer than k candidates.
+ *   6        per-band counts: int64 at byte 16 = candidates > tau, at byte 24 = candidates == tau.
+ *   7        write the band's candidates > tau and the first tie_quota candidates == tau (in index order) to
+ *            out_idx / out_val [out_offset ...), as global indices i * n + j and raw scores.  One GPU: out_offset 0,
+ *            tie_quota = t.  Row bands in row order: rank r uses out_offset = sum over q < r of (gt_q + quota_q) and
+ *            quota_r = clamp(t - sum over q < r of eq_q, 0, eq_r).  Slots at or beyond k are never written.
+ * Workspace: O(rows * ceil(n / 8192) + 2049) int64, never O(n^2).                                                 */
+#define MCGRA_TOPK_HIST_OFFSET 256
+int64_t mcgra_topk_workspace_bytes(int64_t rows, int64_t n, int64_t k);
+int mcgra_topk_stage(int stage, const float* scores, int64_t row0, int64_t rows, int64_t n, int64_t k, void* ws,
+                     int64_t out_offset, int64_t tie_quota, int64_t* out_idx, float* out_val, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -188,7 +188,11 @@ _SIGS = {
     "mcgra_auc_stage": (C.c_int, [C.c_int, c_fp, c_fp, i64, i64, c_fp, c_fp, c_fp]),
     "mcgra_sort_workspace_bytes": (i64, [i64]),
     "mcgra_argsort_desc": (C.c_int, [c_fp, i64, c_fp, c_fp, c_fp]),
+    "mcgra_topk_workspace_bytes": (i64, [i64, i64, i64]),
+    "mcgra_topk_stage": (C.c_int, [C.c_int, c_fp, i64, i64, i64, i64, c_fp, i64, i64, c_fp, c_fp, c_fp]),
 }
+TOPK_HIST_OFFSET = 256       # MCGRA_TOPK_HIST_OFFSET
+TOPK_BINS = 2048
 
 _lib = None
 
@@ -247,7 +251,7 @@ LAUNCHES = {"count": 0, "kernels": 0}
 KERNELS_PER_CALL = {"mcgra_propagate": 3, "mcgra_propagate_sel": 3, "mcgra_noise_stage": 2, "mcgra_fold_adam": 2, "mcgra_auc_ap": 15, "mcgra_argsort_desc": 13,
                     "mcgra_version": 0, "mcgra_set_engine": 0, "mcgra_tiles_in_rows": 0, "mcgra_propagate_ws_bytes": 0,
                     "mcgra_fold_ws_bytes": 0, "mcgra_auc_workspace_bytes": 0, "mcgra_sort_workspace_bytes": 0,
-                    "mcgra_pairs_ws_bytes": 0, "mcgra_auc_hist_offset": 0, "mcgra_auc_stage": 5, "mcgra_nd_scratch_doubles": 0, "mcgra_nd_scratch_floats": 0, "mcgra_nd_measure": 5,
+                    "mcgra_pairs_ws_bytes": 0, "mcgra_auc_hist_offset": 0, "mcgra_topk_workspace_bytes": 0, "mcgra_auc_stage": 5, "mcgra_nd_scratch_doubles": 0, "mcgra_nd_scratch_floats": 0, "mcgra_nd_measure": 5,
                     "mcgra_image_from_dense": 2, "mcgra_smooth": 2, "mcgra_center_dense": 2, "mcgra_sym_to_tiles": 2}
 
 

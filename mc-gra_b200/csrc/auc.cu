@@ -13,12 +13,6 @@
 
 namespace {
 
-// order-preserving map float -> uint32 (ascending)
-__device__ __forceinline__ uint32_t fkey(float f) {
-  uint32_t u = __float_as_uint(f + 0.0f);          // -0.0 -> +0.0: they compare equal, so they must share a key
-  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
-}
-
 constexpr int CHUNK = 4096;   // elements per single-warp block
 
 __global__ void k_hist(const uint32_t* __restrict__ keys, int64_t N, int shift, uint32_t* __restrict__ hist /*[256][nb]*/,

@@ -74,6 +74,12 @@ __device__ __forceinline__ ParamView load_view(const float* mu, int raw) {
   return v;
 }
 
+// order-preserving map float -> uint32 (ascending); shared by the AUC ranking and the top-k selection
+__device__ __forceinline__ uint32_t fkey(float f) {
+  uint32_t u = __float_as_uint(f + 0.0f);          // -0.0 -> +0.0: they compare equal, so they must share a key
+  return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
+}
+
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);

@@ -15,7 +15,7 @@ import scipy.sparse as sp
 import torch
 
 from . import synth
-from .metrics import metric_pool
+from .metrics import metric_pool, precision_recall_at_k
 from .models.gcn import GCN, embedding_GCN
 from .topology_attack import PGDAttack
 
@@ -52,6 +52,9 @@ def build_parser():
     p.add_argument('--ensemble', action='store_true')
     p.add_argument('--add_noise', action='store_true')
     p.add_argument('--defense', action='store_true')
+    p.add_argument('--topk', type=int, default=0,
+                   help="K > 0: write the K highest-scoring pairs to results/<log_name>.topk.npz and log precision / "
+                        "recall against the true edges")
     return p
 
 
@@ -92,6 +95,9 @@ def dot_product_decode(Z, dataset):
 
 def main(argv=None):
     args = build_parser().parse_args(argv)
+    topk = vars(args).pop("topk")         # not part of the reference's parameter line in the log
+    if topk < 0:
+        raise ValueError(f"--topk {topk}: K must be >= 0 (0 = off)")
     if args.arch != "gcn" or args.mode != "evaluate":
         raise NotImplementedError("only --arch gcn --mode evaluate are on the B200 path (SURVEY.md 2)")
     device = torch.device("cuda:0")
@@ -140,6 +146,13 @@ def main(argv=None):
         f.write(f"current parameter: {args}\n")
         f.write(f"In attack graph: AUC={auc}\tIn train graph: AUC={auc_train}\tIn Whole Graph: AUC={auc_all}\n")
         f.write(f"current density: {float(inference_adj.mean())}\n")
+    if topk > 0:
+        rows, cols, scores = model.recovered_edges(topk)
+        precision, recall = precision_recall_at_k(rows, cols, adj, n)
+        np.savez(os.path.join("./results", args.log_name + ".topk.npz"), rows=rows.cpu().numpy(),
+                 cols=cols.cpu().numpy(), scores=scores.cpu().numpy())
+        with open(os.path.join("./results", args.log_name), "a") as f:
+            f.write(f"Top-K: precision={precision} recall={recall} k={topk}\n")
     return auc_all
 
 

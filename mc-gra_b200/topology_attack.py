@@ -422,6 +422,18 @@ class PGDAttack(BaseAttack):
         dist.all_gather_into_tensor(full, mine, group=eng.group)
         return full[:n]
 
+    def recovered_edges(self, k):
+        """The reconstructed graph: the k highest-scoring node pairs (i < j) of `modified_adj`, as (rows, cols, scores)
+        device tensors in (score desc, i * n + j asc) order (metrics.topk_pairs).  With world > 1 each rank passes its
+        row band and every rank returns the same result (metrics.topk_pairs_sharded)."""
+        if self.modified_adj is None:
+            raise RuntimeError("recovered_edges() needs the scores of attack(): call attack() first")
+        from .metrics import topk_pairs, topk_pairs_sharded
+        eng = self.engine
+        if eng is not None and eng.world > 1:
+            return topk_pairs_sharded(self.modified_adj, self.modified_adj_rows[0], self.nnodes, k, group=eng.group)
+        return topk_pairs(self.modified_adj, k)
+
     # ------------------------------------------------------------------------------------------------
     # stand-alone helpers of the reference class, same names and semantics
     def get_modified_adj(self, ori_adj=None):
