@@ -62,23 +62,21 @@ enum {
 };
 
 int mcgra_version(void);
-/* engine selection for A/B validation (values >= 100 are developer knobs -- grid caps for the tests, ablation / policy
- * bits -- and not for production use):
- *   which 0 = propagate:    0 exact fp32 FFMA (reference of the agreement tests), 5 both products on tcgen05 kind::f16 from
- *                           one fp16x2 image per tile [default]
+/* engine selection for A/B validation; the engines 0 are the exact references of the agreement tests:
+ *   which 0 = propagate:    0 exact fp32 FFMA, 5 both products on tcgen05 kind::f16 from one fp16x2 image per tile [default]
  *   which 1 = fold:         0 exact fp32 FFMA, 2 tcgen05 one tile per CTA (every parameter view / measure), 3 persistent
  *                           row runs with the A operand resident in tensor memory for the clamped and the lazily projected
- *                           view, engine 2 otherwise [default]
+ *                           view, engine 2 otherwise [default]; 100 + cap (0 <= cap < 900) caps the persistent grid at
+ *                           cap CTAs (0 = one per SM, the default)
  *   which 2 = pairs:        0 FFMA, 1 mma.sync 3xTF32, 2 tcgen05 for the entropy-only configuration + 1 otherwise [default]
- *   which 3 = mcgra_gemm_nt: 1 cta_group::1 (128 x 128 tiles), 2 cta_group::2 CTA pairs (256 x 256 tiles) [default]
  *   which 4 = element-wise pass: 0 one tile per CTA, 1 persistent bulk-staged kernel for MSE on the clamped / lazily
- *                           projected view, 0 otherwise [default]
+ *                           projected view, 0 otherwise [default]; 100 + cap as for which 1
  *   which 5 = mcgra_ensemble: 0 one CTA per 64 x 64 block, 1 one CTA per block PAIR (I, J) / (J, I) when the full matrix is
  *                           written (symmetric terms evaluated once), 0 for row bands [default]
  *   which 6 = mcgra_auc_ap: 0 1024-sample search table over the sorted positives, 1 the DISTINCT positive keys with their
  *                           start indices (and a CTA-private histogram while they fit) in up to 224 KB of shared memory,
  *                           sampled keys + one 32-byte block per segment beyond that [default]
- * Returns 0, or -1 for an unknown selector.                                                                            */
+ * Returns 0, or -1 (and changes nothing) for any other selector or value.                                              */
 int mcgra_set_engine(int which, int value);
 int64_t mcgra_tiles_in_rows(int tr0, int tr1);           /* number of tiles in tile rows [tr0,tr1) */
 
@@ -101,9 +99,23 @@ int mcgra_degree(const float* tiles, int64_t n, int tr0, int tr1, const float* m
 
 /* ---- propagation Y += M * B (GraphConvolution.forward's spmm, models/gcn.py:42, and its transpose
  *      in backward); M symmetric zero-diagonal from the tiles; B,Y row-major [n x K], K in {16,32}.
- *      Caller zero-fills Y.  Optional fused element-wise terms of the layer-1 pass (c1 MSE/KL against
- *      feature_adj, c6 entropy; topology_attack.py:212-232,44-47): values into acc[], the row sums
- *      eps_row[i] += sum_j (e'_ij+e'_ji) M_ij r_j needed by the degree gradient (SURVEY 8(a4)).     */
+ *      Caller zero-fills Y.                                                                          */
+/* ws (optional, may be NULL): device scratch of mcgra_propagate_ws_bytes(n, K) bytes; with it the tcgen05 engine
+ * pre-formats B once per call (tf32 hi/lo split, K-major core-matrix layout) instead of once per tile.          */
+int64_t mcgra_propagate_ws_bytes(int64_t n, int K);
+int mcgra_propagate(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw,
+                    const float* B, int K, float* Y, void* ws, void* stream);
+/* the same with a product selector: with L the stored strict lower triangle (entry (i,j), i > j, at tile (I,J)),
+ * DIRECT adds L*B, MIRRORED adds L^T*B, BOTH (= mcgra_propagate) their sum.  The noisy path (mcgra_noise_stage) keeps
+ * the two orientations of a non-symmetric M in two tile planes and forms M*B / M^T*B from one product of each.   */
+enum { MCGRA_PROD_DIRECT = 1, MCGRA_PROD_MIRRORED = 2, MCGRA_PROD_BOTH = 3 };
+int mcgra_propagate_sel(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw,
+                        const float* B, int K, float* Y, void* ws, int products, void* stream);
+
+/* ---- element-wise terms of the layer-1 pass (c1 MSE/KL against feature_adj, c6 entropy;
+ *      topology_attack.py:212-232,44-47) as a streaming pass over the shard (x and F tiles read once):
+ *      values into elem->acc, the row sums eps_row[i] += sum_j (e'_ij+e'_ji) M_ij r_j needed by the
+ *      degree gradient (SURVEY 8(a4)) into elem->eps_row.                                           */
 typedef struct {
   const float* r;         /* [n] D^-1/2                                                              */
   const float* Ftiles;    /* tiled feature_adj (same shard) or NULL                                  */
@@ -116,21 +128,6 @@ typedef struct {
   float* eps_row;         /* [n]                                                                      */
   const float* dlse;      /* [n] lseF - lseA evaluated in fp64 (KL value: log-ratio without cancellation)     */
 } mcgra_elem_args;
-/* ws (optional, may be NULL): device scratch of mcgra_propagate_ws_bytes(n, K) bytes; with it the tcgen05 engine
- * pre-formats B once per call (tf32 hi/lo split, K-major core-matrix layout) instead of once per tile.          */
-int64_t mcgra_propagate_ws_bytes(int64_t n, int K);
-int mcgra_propagate(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw,
-                    const float* B, int K, float* Y, const mcgra_elem_args* elem, void* ws, void* stream);
-/* the same with a product selector: with L the stored strict lower triangle (entry (i,j), i > j, at tile (I,J)),
- * DIRECT adds L*B, MIRRORED adds L^T*B, BOTH (= mcgra_propagate) their sum.  The noisy path (mcgra_noise_stage) keeps
- * the two orientations of a non-symmetric M in two tile planes and forms M*B / M^T*B from one product of each.
- * elem must be NULL unless products == MCGRA_PROD_BOTH.                                                          */
-enum { MCGRA_PROD_DIRECT = 1, MCGRA_PROD_MIRRORED = 2, MCGRA_PROD_BOTH = 3 };
-int mcgra_propagate_sel(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw,
-                        const float* B, int K, float* Y, const mcgra_elem_args* elem, void* ws, int products,
-                        void* stream);
-/* the same element-wise terms as a stand-alone streaming pass (x and F tiles read once): lets every propagation
- * use the plain tensor-core kernels; values into elem->acc, row sums into elem->eps_row.                        */
 int mcgra_elem_stats(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw,
                      const mcgra_elem_args* elem, void* stream);
 /* row log-sum-exp of A_hat over the shard: sumexp[i] += sum_{j != i} exp(r_i M_ij r_j) (KL measure) */

@@ -112,10 +112,9 @@ _SIGS = {
     "mcgra_tiles_to_dense": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, i64, c_fp]),
     "mcgra_degree": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, c_fp]),
     "mcgra_propagate_ws_bytes": (i64, [i64, C.c_int]),
-    "mcgra_propagate": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, C.c_int, c_fp,
-                                  C.POINTER(ElemArgs), c_fp, c_fp]),
-    "mcgra_propagate_sel": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, C.c_int, c_fp,
-                                      C.POINTER(ElemArgs), c_fp, C.c_int, c_fp]),
+    "mcgra_propagate": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, C.c_int, c_fp, c_fp, c_fp]),
+    "mcgra_propagate_sel": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, C.c_int, c_fp, c_fp, C.c_int,
+                                      c_fp]),
     "mcgra_noise_stage": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, C.c_float, c_fp, c_fp, c_fp, c_fp,
                                     c_fp]),
     "mcgra_diag_axpy": (C.c_int, [c_fp, c_fp, C.c_int, i64, c_fp, c_fp]),
@@ -218,7 +217,7 @@ def lib():
         # developer override for same-box A/B runs and profiling: MCGRA_ENGINES="0:5,1:2" (stage:engine, see mcgra.h)
         for item in filter(None, os.environ.get("MCGRA_ENGINES", "").split(",")):
             which, value = item.split(":")
-            L.mcgra_set_engine(int(which), int(value))
+            check(L.mcgra_set_engine(int(which), int(value)), f"MCGRA_ENGINES entry {item!r}")
     return _lib
 
 

@@ -178,7 +178,7 @@ k_rank_negatives(const float* __restrict__ scores, const uint8_t* __restrict__ l
 
 // Ranking against the DISTINCT positive keys, search table in dynamic shared memory.
 //
-// What bounds k_rank_negatives (measured, tools/auc_ab.py, 4.3e9 negatives): not the histogram updates (5 ms) but the
+// What bounds k_rank_negatives (measured, profiles/r02_auc_ablation.txt, 4.3e9 negatives): not the histogram updates (5 ms) but the
 // searches (87 of 119 ms) -- after its 1024-sample table every lane walks the sorted array in its own 128-byte line, and a
 // negative that ties with a positive is searched twice (lower and upper bound).  The scores of the reference's ensemble
 // (sums of sigmoids of clamped grams + integer label terms) are heavily tied: 2 055 distinct values among 294 878 positives at
@@ -264,7 +264,7 @@ __global__ void __launch_bounds__(1024, 1)
 k_rank_negatives_tab(const float* __restrict__ scores, const uint8_t* __restrict__ labels, int64_t N,
                      const uint32_t* __restrict__ U, const uint32_t* __restrict__ Cidx, const uint4* __restrict__ blocks,
                      const unsigned long long* __restrict__ counter, unsigned long long* __restrict__ hist /*[npos+1]*/,
-                     unsigned long long* __restrict__ sums /*[2]*/, int tab_cap, int dbg) {
+                     unsigned long long* __restrict__ sums /*[2]*/, int tab_cap) {
   uint32_t* tab = dyn_tab;
   const int npos = (int)counter[0];
   const int nU = (int)counter[3];
@@ -439,16 +439,14 @@ k_rank_negatives_tab(const float* __restrict__ scores, const uint8_t* __restrict
         tw32 += 2u * (unsigned)(npos - ub[e]) + (unsigned)(ub[e] - lb[e]);      // 12 npos < 2^32: npos < 2^28 checked by the host
         nneg += 1;
       }
-      if (!(dbg & 1)) {
-        const int sent = -1 - lane;         // unique sentinel so inactive lanes do not aggregate
-        if (hsm) {
-          // few distinct values = hot bins: global updates of the same ~nU addresses serialise in L2 (90 of 120 ms measured)
-          const unsigned peers = __match_any_sync(0xffffffffu, neg[e] ? vb[e] : sent);
-          if (neg[e] && lane == (__ffs(peers) - 1)) atomicAdd(Hs + vb[e], (unsigned)__popc(peers));
-        } else {
-          const unsigned peers = __match_any_sync(0xffffffffu, neg[e] ? ub[e] : sent);
-          if (neg[e] && lane == (__ffs(peers) - 1)) atomicAdd(hist + ub[e], (unsigned long long)__popc(peers));
-        }
+      const int sent = -1 - lane;         // unique sentinel so inactive lanes do not aggregate
+      if (hsm) {
+        // few distinct values = hot bins: global updates of the same ~nU addresses serialise in L2 (90 of 120 ms measured)
+        const unsigned peers = __match_any_sync(0xffffffffu, neg[e] ? vb[e] : sent);
+        if (neg[e] && lane == (__ffs(peers) - 1)) atomicAdd(Hs + vb[e], (unsigned)__popc(peers));
+      } else {
+        const unsigned peers = __match_any_sync(0xffffffffu, neg[e] ? ub[e] : sent);
+        if (neg[e] && lane == (__ffs(peers) - 1)) atomicAdd(hist + ub[e], (unsigned long long)__popc(peers));
       }
     }
     twice += (unsigned long long)tw32;
@@ -464,7 +462,7 @@ k_rank_negatives_tab(const float* __restrict__ scores, const uint8_t* __restrict
   }
   if (lane == 0) { r0[threadIdx.x >> 5] = twice; r1[threadIdx.x >> 5] = nneg; }
   __syncthreads();
-  if (hsm && !(dbg & 1)) {
+  if (hsm) {
     for (int t = threadIdx.x; t <= nU; t += blockDim.x) {
       const uint32_t c = Hs[t];
       if (c) atomicAdd(hist + Cs[t], (unsigned long long)c);
@@ -478,7 +476,6 @@ k_rank_negatives_tab(const float* __restrict__ scores, const uint8_t* __restrict
   }
 }
 
-int g_auc_dbg = 0;         // timing experiments only (mcgra_set_engine(6, 100 + bits)): 1 no histogram updates (AP invalid)
 int g_auc_engine = 1;      // mcgra_set_engine(6, v): 0 k_rank_negatives (1024-sample table), 1 k_rank_negatives_tab (default)
 constexpr int TAB_CAP_MAX = 57344;      // 224 KB of dynamic shared memory
 
@@ -583,7 +580,8 @@ int radix_sort(uint32_t* keys, PAY* pay, uint32_t* keys_tmp, PAY* pay_tmp, int64
 extern "C" {
 
 int mcgra_set_auc_engine_(int value) {
-  if (value >= 100) g_auc_dbg = value - 100; else g_auc_engine = value;
+  if (value != 0 && value != 1) return -1;
+  g_auc_engine = value;
   return 0;
 }
 
@@ -653,7 +651,7 @@ int mcgra_auc_stage(int stage, const float* scores, const uint8_t* labels, int64
       uint32_t* blocks = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(Cidx) + align256((npos_max + 2) * 4));
       if (want > cap) k_build_blocks<<<64, 256, 0, st>>>(pos_tmp, Cidx, counter, cap, blocks);
       k_rank_negatives_tab<<<148, 1024, smem, st>>>(scores, labels, N, pos_tmp, Cidx, reinterpret_cast<const uint4*>(blocks),
-                                                    counter, hist, sums, cap, g_auc_dbg);
+                                                    counter, hist, sums, cap);
     } else if (N > 0) {
       k_rank_negatives<<<148 * 8, 256, 0, st>>>(scores, labels, N, pos, counter, hist, sums);
     }

@@ -16,8 +16,7 @@
 // (128-byte rows, SWIZZLE_128B, K-major), hi and lo planes -> 64 KB per stage, ring of 3 stages filled by TMA
 // (cp.async.bulk.tensor.2d.cta_group::2, both CTAs signal the leader's mbarrier); warp 0 = TMA producer, warp 1 = MMA
 // issuer (leader CTA only, one thread) and TMEM owner, warps 2-9 = epilogue (tcgen05.ld -> scale -> rank-1 correction
-// -> reductions -> global).  A cta_group::1 instantiation (128 x 128 tile, no cluster) is kept for validation
-// (mcgra_set_engine(3, 1)).
+// -> reductions -> global).
 //
 // Accumulation: the tensor core adds every MMA into its fp32 TMEM accumulator with TRUNCATION -- measured here on
 // all-positive operands: a relative bias of -4.2e-8 per MMA, i.e. -1.3e-4 at K = 16 384 and -4.2e-4 at K = 65 536 when one
@@ -39,11 +38,10 @@ constexpr int G_PLANE = 128 * 128;             // bytes of one 128-row x 128-byt
 constexpr int G_STAGE = 4 * G_PLANE;           // A_hi | A_lo | B_hi | B_lo
 constexpr int G_STAGES = 3;
 constexpr int G_SMEM = G_STAGES * G_STAGE + 1024 /* alignment slack */ + 256 /* barriers */;
-int g_gemm_chunk = 16;                         // K-blocks per TMEM accumulation chunk (see header); mcgra_set_engine(3, 100 + c)
+constexpr int G_CHUNK = 16;                    // K-blocks per TMEM accumulation chunk (see header)
 constexpr int G_THREADS = 320;                 // producer warp, MMA warp, 8 epilogue warps
 constexpr int G_GROUP = 8;                     // tile rasterisation: sweep groups of 8 tile rows (L2 reuse)
-
-int g_gemm_cg = 2;
+constexpr int G_BT = 256;                      // tile edge of the CTA pair
 
 struct GemmParams {
   int64_t M, N, K;              // C is M x N (rows of A image x rows of B image), K = common column count
@@ -66,10 +64,9 @@ struct GemmParams {
   const float* inv_se;
   int64_t lde;
   int tiles_m, tiles_n;
-  int chunk;                    // K-blocks per accumulation chunk
 };
 
-// ---- PTX wrappers that depend on the CTA-group size ------------------------------------------------------------
+// ---- PTX wrappers (cluster, cta_group::2) ------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t cluster_ctarank() {
   uint32_t r;
   asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
@@ -91,72 +88,38 @@ __device__ __forceinline__ void fence_barrier_init() {
   asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
 
-template <int CG>
 __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t mbar) {
-  if constexpr (CG == 2) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::
-            "r"(dst), "l"((uint64_t)map), "r"(mbar), "r"(c0), "r"(c1)
-        : "memory");
-  } else {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::"r"(dst),
-        "l"((uint64_t)map), "r"(mbar), "r"(c0), "r"(c1)
-        : "memory");
-  }
+  asm volatile(
+      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::
+          "r"(dst), "l"((uint64_t)map), "r"(mbar), "r"(c0), "r"(c1)
+      : "memory");
 }
 
-template <int CG>
 __device__ __forceinline__ void mma_f16_cg(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  if constexpr (CG == 2) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-  } else {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-        "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-  }
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
 }
 
-// arrive on the mbarrier (same shared-memory offset in every CTA of the group) when all MMAs issued so far are complete
-template <int CG>
+// arrive on the mbarrier (same shared-memory offset in both CTAs of the pair) when all MMAs issued so far are complete
 __device__ __forceinline__ void mma_commit_cg(uint64_t* bar) {
-  if constexpr (CG == 2) {
-    asm volatile(
-        "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-            tc::smem_u32(bar)),
-        "h"((uint16_t)3)
-        : "memory");
-  } else {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(tc::smem_u32(bar))
-                 : "memory");
-  }
+  asm volatile(
+      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
+          tc::smem_u32(bar)),
+      "h"((uint16_t)3)
+      : "memory");
 }
 
-template <int CG>
 __device__ __forceinline__ void tmem_alloc_cg(uint32_t* smem_dst, uint32_t ncols) {
-  if constexpr (CG == 2) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tc::smem_u32(smem_dst)), "r"(ncols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  } else {
-    tc::tmem_alloc(smem_dst, ncols);
-  }
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tc::smem_u32(smem_dst)), "r"(ncols)
+               : "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
 }
-template <int CG>
 __device__ __forceinline__ void tmem_dealloc_cg(uint32_t taddr, uint32_t ncols) {
-  if constexpr (CG == 2) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-  } else {
-    tc::tmem_dealloc(taddr, ncols);
-  }
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
 
 // instruction descriptor: D = F32, A = B = F16, both K-major, dense
@@ -182,7 +145,6 @@ __device__ __forceinline__ void mbar_arrive_rank(uint64_t* bar, uint32_t rank, b
   }
 }
 
-template <int CG>
 __global__ void __launch_bounds__(G_THREADS, 1)
 k_gemm3(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUtensorMap mapAl,
         const __grid_constant__ CUtensorMap mapBh, const __grid_constant__ CUtensorMap mapBl, const GemmParams p) {
@@ -191,28 +153,26 @@ k_gemm3(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUten
   uint64_t* full = (uint64_t*)(smem + G_STAGES * G_STAGE);
   uint64_t* empty = full + G_STAGES;
   uint64_t* acc_full = empty + G_STAGES;       // [2] chunk accumulator b complete (MMA -> epilogue warps)
-  uint64_t* acc_empty = acc_full + 2;          // [2] chunk accumulator b drained (epilogue warps of the group -> MMA)
+  uint64_t* acc_empty = acc_full + 2;          // [2] chunk accumulator b drained (epilogue warps of the pair -> MMA)
   uint32_t* tmem_slot = (uint32_t*)(acc_empty + 2);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t cta_rank = (CG == 2) ? cluster_ctarank() : 0u;
-  constexpr int BT = 128 * CG;                 // tile edge of the CTA group
-  constexpr uint32_t NCOLS = 128 * CG;         // accumulator columns per CTA
+  const uint32_t cta_rank = cluster_ctarank();
+  constexpr uint32_t NCOLS = G_BT;             // accumulator columns per CTA
   constexpr int NPT = (int)NCOLS / 2;          // accumulator columns per epilogue thread
 
-  // grouped rasterisation of the group's tile
-  const int64_t tid = (int64_t)blockIdx.x / CG;
+  // grouped rasterisation of the pair's tile
+  const int64_t tid = (int64_t)blockIdx.x / 2;
   const int64_t per_group = (int64_t)G_GROUP * p.tiles_n;
   const int first_m = (int)(tid / per_group) * G_GROUP;
   const int gsz = min(p.tiles_m - first_m, G_GROUP);
   const int tm = first_m + (int)((tid % per_group) % gsz);
   const int tn = (int)((tid % per_group) / gsz);
 
-  const int64_t m_cta = p.row0 + (int64_t)tm * BT + (int64_t)cta_rank * 128;   // A rows / accumulator rows of this CTA
-  const int64_t nb_cta = (int64_t)tn * BT + (int64_t)cta_rank * 128;           // B rows this CTA stages
-  const int64_t n0 = (int64_t)tn * BT;                                         // first output column of the tile
+  const int64_t m_cta = p.row0 + (int64_t)tm * G_BT + (int64_t)cta_rank * 128;   // A rows / accumulator rows of this CTA
+  const int64_t nb_cta = (int64_t)tn * G_BT + (int64_t)cta_rank * 128;           // B rows this CTA stages
+  const int64_t n0 = (int64_t)tn * G_BT;                                         // first output column of the tile
   const int num_kb = (int)((p.K + G_BK - 1) / G_BK);
-  const int G_CHUNK = p.chunk;
   const int num_ch = (num_kb + G_CHUNK - 1) / G_CHUNK;
 
   if (warp == 0 && lane == 0) {
@@ -222,14 +182,14 @@ k_gemm3(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUten
     }
     for (int b = 0; b < 2; ++b) {
       tc::mbar_init(&acc_full[b], 1);
-      tc::mbar_init(&acc_empty[b], 8 * CG);    // one arrival per epilogue warp of every CTA of the group
+      tc::mbar_init(&acc_empty[b], 16);        // one arrival per epilogue warp of both CTAs of the pair
     }
     fence_barrier_init();
   }
-  if (warp == 1) tmem_alloc_cg<CG>(tmem_slot, 2 * NCOLS);
+  if (warp == 1) tmem_alloc_cg(tmem_slot, 2 * NCOLS);
   tc::fence_before();
   __syncthreads();                             // CTA-level order for tmem_slot / the barriers (and for racecheck, which
-  if constexpr (CG == 2) cluster_sync_all();   // does not model barrier.cluster); the pair then syncs across CTAs
+  cluster_sync_all();                          // does not model barrier.cluster); the pair then syncs across CTAs
   tc::fence_after();
   const uint32_t tmem = *tmem_slot;
 
@@ -240,20 +200,20 @@ k_gemm3(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUten
         const int s = kb % G_STAGES;
         const uint32_t ph = (uint32_t)(kb / G_STAGES) & 1u;
         tc::mbar_wait(&empty[s], ph ^ 1u);
-        if (cta_rank == 0) mbar_expect_tx(&full[s], (uint32_t)(CG * G_STAGE));
-        const uint32_t bar = (CG == 2) ? mapa_rank(tc::smem_u32(&full[s]), 0) : tc::smem_u32(&full[s]);
+        if (cta_rank == 0) mbar_expect_tx(&full[s], (uint32_t)(2 * G_STAGE));
+        const uint32_t bar = mapa_rank(tc::smem_u32(&full[s]), 0);
         const uint32_t base = tc::smem_u32(smem + s * G_STAGE);
         const int k0 = kb * G_BK;
-        tma_load_2d<CG>(base, &mapAh, k0, (int)m_cta, bar);
-        tma_load_2d<CG>(base + G_PLANE, &mapAl, k0, (int)m_cta, bar);
-        tma_load_2d<CG>(base + 2 * G_PLANE, &mapBh, k0, (int)nb_cta, bar);
-        tma_load_2d<CG>(base + 3 * G_PLANE, &mapBl, k0, (int)nb_cta, bar);
+        tma_load_2d(base, &mapAh, k0, (int)m_cta, bar);
+        tma_load_2d(base + G_PLANE, &mapAl, k0, (int)m_cta, bar);
+        tma_load_2d(base + 2 * G_PLANE, &mapBh, k0, (int)nb_cta, bar);
+        tma_load_2d(base + 3 * G_PLANE, &mapBl, k0, (int)nb_cta, bar);
       }
     }
   } else if (warp == 1) {
     // ===== MMA issuer (leader CTA, one thread) =====
     if (cta_rank == 0 && lane == 0) {
-      const uint32_t idesc = idesc_f16(BT, BT);
+      const uint32_t idesc = idesc_f16(G_BT, G_BT);
       for (int kb = 0; kb < num_kb; ++kb) {
         const int s = kb % G_STAGES;
         const uint32_t ph = (uint32_t)(kb / G_STAGES) & 1u;
@@ -270,12 +230,12 @@ k_gemm3(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUten
         for (int k = 0; k < G_BK / 16; ++k) {
           const uint64_t ah = desc_sw128(base + k * 32), al = desc_sw128(base + G_PLANE + k * 32);
           const uint64_t bh = desc_sw128(base + 2 * G_PLANE + k * 32), bl = desc_sw128(base + 3 * G_PLANE + k * 32);
-          mma_f16_cg<CG>(d, ah, bh, idesc, (kc | k) ? 1u : 0u);
-          mma_f16_cg<CG>(d, ah, bl, idesc, 1u);
-          mma_f16_cg<CG>(d, al, bh, idesc, 1u);
+          mma_f16_cg(d, ah, bh, idesc, (kc | k) ? 1u : 0u);
+          mma_f16_cg(d, ah, bl, idesc, 1u);
+          mma_f16_cg(d, al, bh, idesc, 1u);
         }
-        mma_commit_cg<CG>(&empty[s]);          // frees the stage in both CTAs once these MMAs have read it
-        if (kc == G_CHUNK - 1 || kb == num_kb - 1) mma_commit_cg<CG>(&acc_full[b]);   // chunk complete -> epilogue warps
+        mma_commit_cg(&empty[s]);          // frees the stage in both CTAs once these MMAs have read it
+        if (kc == G_CHUNK - 1 || kb == num_kb - 1) mma_commit_cg(&acc_full[b]);   // chunk complete -> epilogue warps
       }
     }
   } else {
@@ -301,7 +261,7 @@ k_gemm3(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUten
       }
       tc::fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive_rank(&acc_empty[b], 0, CG == 2 && cta_rank != 0);
+      if (lane == 0) mbar_arrive_rank(&acc_empty[b], 0, cta_rank != 0);
     }
     const int64_t row = m_cta + q * 32 + lane;
     const bool row_ok = row < p.row0 + p.rows && row < p.M;
@@ -350,8 +310,8 @@ k_gemm3(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUten
   }
 
   tc::fence_before();
-  if constexpr (CG == 2) cluster_sync_all(); else __syncthreads();
-  if (warp == 1) tmem_dealloc_cg<CG>(tmem, 2 * NCOLS);
+  cluster_sync_all();
+  if (warp == 1) tmem_dealloc_cg(tmem, 2 * NCOLS);
 }
 
 // ---- host side: tensor maps ------------------------------------------------------------------------------------
@@ -387,32 +347,30 @@ int make_map(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64
   return r == CUDA_SUCCESS ? 0 : -22;
 }
 
-template <int CG>
 int launch_gemm(const CUtensorMap* maps, GemmParams& p, cudaStream_t st) {
-  constexpr int BT = 128 * CG;
-  p.tiles_m = (int)((p.rows + BT - 1) / BT);
-  p.tiles_n = (int)((p.N + BT - 1) / BT);
+  p.tiles_m = (int)((p.rows + G_BT - 1) / G_BT);
+  p.tiles_n = (int)((p.N + G_BT - 1) / G_BT);
   const int64_t groups = (int64_t)p.tiles_m * p.tiles_n;
   if (groups <= 0) return 0;
   static bool attr_done = false;
   if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(k_gemm3<CG>, cudaFuncAttributeMaxDynamicSharedMemorySize, G_SMEM);
+    cudaError_t e = cudaFuncSetAttribute(k_gemm3, cudaFuncAttributeMaxDynamicSharedMemorySize, G_SMEM);
     if (e != cudaSuccess) return (int)e;
     attr_done = true;
   }
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)(groups * CG));
+  cfg.gridDim = dim3((unsigned)(groups * 2));
   cfg.blockDim = dim3(G_THREADS);
   cfg.dynamicSmemBytes = G_SMEM;
   cfg.stream = st;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = CG;
+  at[0].val.clusterDim.x = 2;
   at[0].val.clusterDim.y = 1;
   at[0].val.clusterDim.z = 1;
   cfg.attrs = at;
   cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, k_gemm3<CG>, maps[0], maps[1], maps[2], maps[3], p);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, k_gemm3, maps[0], maps[1], maps[2], maps[3], p);
   if (e != cudaSuccess) return (int)e;
   return 0;
 }
@@ -420,13 +378,6 @@ int launch_gemm(const CUtensorMap* maps, GemmParams& p, cudaStream_t st) {
 }  // namespace
 
 extern "C" {
-
-int mcgra_set_gemm_engine_(int value) {
-  if (value >= 100) { g_gemm_chunk = value - 100 > 0 ? value - 100 : 1; return 0; }
-  if (value != 1 && value != 2) return -1;
-  g_gemm_cg = value;
-  return 0;
-}
 
 int mcgra_gemm_nt(const mcgra_image* A, const mcgra_image* B, const mcgra_gemm_epilogue* e, void* stream) {
   if (A == nullptr || B == nullptr || e == nullptr) return -1;
@@ -449,7 +400,6 @@ int mcgra_gemm_nt(const mcgra_image* A, const mcgra_image* B, const mcgra_gemm_e
   p.u = e->u;
   p.v = e->v;
   p.coef = e->coef;
-  p.chunk = g_gemm_chunk;
   p.sumsq = e->sumsq;
   p.dot = e->dot;
   if (e->dot != nullptr) {
@@ -465,8 +415,7 @@ int mcgra_gemm_nt(const mcgra_image* A, const mcgra_image* B, const mcgra_gemm_e
   if ((rc = make_map(&maps[1], A->lo, A->rows, A->cols, A->ld)) != 0) return rc;
   if ((rc = make_map(&maps[2], B->hi, B->rows, B->cols, B->ld)) != 0) return rc;
   if ((rc = make_map(&maps[3], B->lo, B->rows, B->cols, B->ld)) != 0) return rc;
-  if (g_gemm_cg == 2) return launch_gemm<2>(maps, p, (cudaStream_t)stream);
-  return launch_gemm<1>(maps, p, (cudaStream_t)stream);
+  return launch_gemm(maps, p, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -102,7 +102,7 @@ __global__ void k_tiles_to_dense(const float* __restrict__ tiles, int64_t n, int
 
 extern "C" {
 
-int mcgra_version(void) { return 1; }
+int mcgra_version(void) { return 2; }
 
 int mcgra_history_push(const double* row, double* hist, int64_t max_rows, int* step, void* stream) {
   k_history_push<<<1, 32, 0, (cudaStream_t)stream>>>(row, hist, max_rows, step);

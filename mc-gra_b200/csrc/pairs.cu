@@ -878,8 +878,16 @@ int launch_pairs_mma(const float* tiles, int64_t n, int tr0, int64_t nt, const f
 
 extern "C" {
 
-int mcgra_set_pairs_engine_(int value) { g_pairs_engine = value; return 0; }
-int mcgra_set_ensemble_engine_(int value) { g_ensemble_engine = value; return 0; }
+int mcgra_set_pairs_engine_(int value) {
+  if (value < 0 || value > 2) return -1;
+  g_pairs_engine = value;
+  return 0;
+}
+int mcgra_set_ensemble_engine_(int value) {
+  if (value != 0 && value != 1) return -1;
+  g_ensemble_engine = value;
+  return 0;
+}
 
 int mcgra_pairs_tc_(int64_t n, int tr0, int tr1, const float* zhat, float k7, float* dzhat, double* acc, void* ws,
                     cudaStream_t st);

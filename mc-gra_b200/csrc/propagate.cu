@@ -3,7 +3,7 @@
 // Reference work replaced: GraphConvolution.forward's torch.spmm(adj, support) (MC-GRA/models/gcn.py:42) and its
 // transposed product in autograd, the row sums of utils.normalize_adj_tensor (MC-GRA/utils.py:224-225), and the
 // element-wise loss terms c1 (MSE/KL vs feature_adj) and c6 (Info_entropy) over A_hat
-// (MC-GRA/topology_attack.py:212-232, 44-47) which are fused into the first propagation pass.
+// (MC-GRA/topology_attack.py:212-232, 44-47), computed by a stand-alone streaming pass ahead of the first propagation.
 //
 // Tile-symmetric schedule: one CTA per 128x128 tile (I,J) of the lower triangle.  The tile is read from HBM once
 // and used twice:  Y[I rows] += T * B[J rows]  and  Y[J rows] += T^T * B[I rows].  The unnormalised / normalised
@@ -31,15 +31,12 @@ struct PropSmem {
   float xs[TILE][XS_LD];
   float bj[TILE][KC];
   float bi[TILE][KC];
-  float rI[TILE], rJ[TILE], lseAI[TILE], lseAJ[TILE], lseFI[TILE], lseFJ[TILE], dlI[TILE], dlJ[TILE];
-  float rowacc[TILE], colacc[TILE];
-  double red[32];
 };
 
-template <int KC, bool ELEM>
+template <int KC>
 __global__ void __launch_bounds__(128, 2)
 k_propagate(const float* __restrict__ tiles, int64_t n, int64_t t0, const float* mu, int raw,
-            const float* __restrict__ B, float* __restrict__ Y, mcgra_elem_args ea, int products) {
+            const float* __restrict__ B, float* __restrict__ Y, int products) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   PropSmem<KC>& sm = *reinterpret_cast<PropSmem<KC>*>(smem_raw);
   int I, J;
@@ -58,82 +55,18 @@ k_propagate(const float* __restrict__ tiles, int64_t n, int64_t t0, const float*
     reinterpret_cast<float4*>(&sm.bj[row][0])[c4] = vj;
     reinterpret_cast<float4*>(&sm.bi[row][0])[c4] = vi;
   }
-  if (ELEM) {
-    const int64_t gi = i0 + tid, gj = j0 + tid;
-    sm.rI[tid] = gi < n ? ea.r[gi] : 0.f;
-    sm.rJ[tid] = gj < n ? ea.r[gj] : 0.f;
-    if (ea.measure == MCGRA_M_KL) {
-      sm.lseAI[tid] = gi < n ? ea.lseA[gi] : 0.f;
-      sm.lseAJ[tid] = gj < n ? ea.lseA[gj] : 0.f;
-      sm.lseFI[tid] = gi < n ? ea.lseF[gi] : 0.f;
-      sm.lseFJ[tid] = gj < n ? ea.lseF[gj] : 0.f;
-      sm.dlI[tid] = gi < n ? ea.dlse[gi] : 0.f;
-      sm.dlJ[tid] = gj < n ? ea.dlse[gj] : 0.f;
-    }
-    sm.colacc[tid] = 0.f;
-    __syncthreads();
-  }
 
-  // ---- stage the tile (one warp = one 512 B row per step), fused element-wise terms -----------------------
-  float col_e[4] = {0.f, 0.f, 0.f, 0.f};
-  float v1 = 0.f, v6 = 0.f;
-  const float4* fsrc = (ELEM && ea.Ftiles != nullptr)
-                           ? reinterpret_cast<const float4*>(ea.Ftiles + (int64_t)blockIdx.x * TILE_ELEMS)
-                           : nullptr;
+  // ---- stage the tile (one warp = one 512 B row per step) ------------------------------------------------
 #pragma unroll 4
   for (int it = 0; it < 32; ++it) {
     const int row = it * 4 + warp;
-    const int idx = row * 32 + lane;
-    const float4 raw4 = src[idx];
+    const float4 raw4 = src[row * 32 + lane];
     const int64_t gi = i0 + row;
     const int64_t gj = j0 + lane * 4;
     float xv[4] = {raw4.x, raw4.y, raw4.z, raw4.w};
-    bool ok[4];
 #pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      ok[k] = (gj + k < gi) && (gi < n);
-      xv[k] = ok[k] ? pv.adj(xv[k]) : 0.f;
-    }
+    for (int k = 0; k < 4; ++k) xv[k] = ((gj + k < gi) && (gi < n)) ? pv.adj(xv[k]) : 0.f;
     *reinterpret_cast<float4*>(&sm.xs[row][lane * 4]) = make_float4(xv[0], xv[1], xv[2], xv[3]);
-    if (ELEM) {
-      float4 f4 = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (fsrc != nullptr) f4 = fsrc[idx];
-      const float fv[4] = {f4.x, f4.y, f4.z, f4.w};
-      const float ri = sm.rI[row];
-      float row_e = 0.f;
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        if (!ok[k]) continue;
-        const float rj = sm.rJ[lane * 4 + k];
-        const float ah = ri * xv[k] * rj;
-        float esym = 0.f;   // e'_ij + e'_ji
-        if (ea.measure == MCGRA_M_MSE) {
-          const float df = ah - fv[k];
-          v1 += 2.f * df * df;
-          esym += 4.f * ea.k1 * df;
-        } else if (ea.measure == MCGRA_M_KL) {
-          const float xij = __expf(fv[k] - sm.lseFI[row]);
-          const float xji = __expf(fv[k] - sm.lseFJ[lane * 4 + k]);
-          const float lij = ah - sm.lseAI[row];
-          const float lji = ah - sm.lseAJ[lane * 4 + k];
-          v1 += xij * ((fv[k] - ah) - sm.dlI[row]) + xji * ((fv[k] - ah) - sm.dlJ[lane * 4 + k]);
-          esym += ea.k1 * ((__expf(lij) - xij) + (__expf(lji) - xji));
-        }
-        if (ea.k6 != 0.f) {
-          v6 += 2.f * ent_val(ah);
-          esym += 2.f * ea.k6 * ent_grad(ah);
-        }
-        const float t = esym * xv[k];
-        row_e += t * rj;
-        col_e[k] += t * ri;
-      }
-      row_e = warp_sum(row_e);
-      if (lane == 0) sm.rowacc[row] = row_e;
-    }
-  }
-  if (ELEM) {
-#pragma unroll
-    for (int k = 0; k < 4; ++k) atomicAdd(&sm.colacc[lane * 4 + k], col_e[k]);
   }
   __syncthreads();
 
@@ -209,13 +142,6 @@ k_propagate(const float* __restrict__ tiles, int64_t n, int64_t t0, const float*
       for (int c4 = 0; c4 < KC / 4; ++c4)
         atomicAdd(dst + c4, make_float4(acc1[c4 * 4], acc1[c4 * 4 + 1], acc1[c4 * 4 + 2], acc1[c4 * 4 + 3]));
     }
-  }
-  if (ELEM) {
-    const int64_t gi = i0 + tid, gj = j0 + tid;
-    if (gi < n && sm.rowacc[tid] != 0.f) atomicAdd(ea.eps_row + gi, sm.rowacc[tid]);
-    if (gj < n && sm.colacc[tid] != 0.f) atomicAdd(ea.eps_row + gj, sm.colacc[tid]);
-    if (ea.measure != MCGRA_M_NONE) block_atomic_add_d((double)v1 * (double)ea.k1, ea.acc + MCGRA_ACC_C1, sm.red);
-    if (ea.k6 != 0.f) block_atomic_add_d((double)v6 * (double)ea.k6, ea.acc + MCGRA_ACC_C6, sm.red);
   }
 }
 
@@ -321,7 +247,6 @@ k_row_sumexp(const float* __restrict__ tiles, int64_t n, int64_t t0, const float
 // with setmaxnreg (converters keep two prefetched tiles in registers, everything else needs few).  TMEM columns: D1 (even tiles) [0, 3KC) | D1 (odd tiles) [96, 96+3KC) | D2[0] [192, 192+3KC) | D2[1] [288, 288+3KC).
 // ---------------------------------------------------------------------------------------------------------
 constexpr int H_RUN = 64;
-int g_prop_dbg = 0;                                // timing experiments only: mcgra_set_engine(0, 100 + bits)
 constexpr uint32_t H_SJ = 16 * 128 + 16;           // stride between 8-column groups of a plane (padded: conflict-free stores)
 constexpr uint32_t H_PLANE = 16 * H_SJ;
 
@@ -465,7 +390,7 @@ __device__ __forceinline__ void h_flush2(float* __restrict__ Y, int64_t n, int64
 template <int KC>
 __global__ void __launch_bounds__(H_THREADS, 1)
 k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* mu, int raw,
-              const unsigned char* __restrict__ Bk, const float* __restrict__ scale, float* __restrict__ Y, int dbg,
+              const unsigned char* __restrict__ Bk, const float* __restrict__ scale, float* __restrict__ Y,
               int products) {
   const int I = tr0 + (int)blockIdx.y;
   const int Jbeg = (int)blockIdx.x * H_RUN;
@@ -533,12 +458,12 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
         const int b = par, r = k % 3;
         tc::mbar_wait(&sm.bfull[r], (uint32_t)((k / 3) & 1));
         tc::mbar_wait(&sm.ready[b], (uint32_t)((k >> 1) & 1));
-        if (k >= 2 && !(dbg & 1)) tc::mbar_wait(&sm.flushed[b], (uint32_t)(((k - 2) >> 1) & 1));   // D2[b] of tile k-2 has been read
+        if (k >= 2) tc::mbar_wait(&sm.flushed[b], (uint32_t)(((k - 2) >> 1) & 1));   // D2[b] of tile k-2 has been read
         tc::fence_after();
         const uint32_t p0 = tc::smem_u32(sm.tile[b][0]), p1 = tc::smem_u32(sm.tile[b][1]);
         const uint64_t bJ0 = tc::make_desc(tc::smem_u32(sm.bkJ[r]), LBO_B, 128u);
 #pragma unroll 2
-        for (int ks = 0; ks < ((dbg & 2) ? 0 : TILE / 16); ++ks) {
+        for (int ks = 0; ks < TILE / 16; ++ks) {
           const uint64_t db = (uint64_t)((uint32_t)ks * ((2u * LBO_B) >> 4));
           const uint32_t acc1 = (k > par || ks > 0) ? 1u : 0u, acc2 = ks > 0 ? 1u : 0u;
           // direct: A K-major (M = row: SBO 128 between 8-row groups; K = column: LBO H_SJ between 8-column groups)
@@ -562,12 +487,11 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
     const int q = warp & 3;                              // TMEM lane quarter (= warp % 4)
     const int ltid = q * 32 + lane;
     const uint32_t tlane = tm + ((uint32_t)(q * 32) << 16);
-    const bool on = !(dbg & 1);
     for (int k = 0; k < nt; ++k) {
       const int b = k & 1;
       tc::mbar_wait(&sm.tile_done[b], (uint32_t)((k >> 1) & 1));
       tc::fence_after();
-      if (on && do_mir) {
+      if (do_mir) {
 #pragma unroll
         for (int cg = 0; cg < KC / 16; ++cg)
           h_flush<KC>(Y, n, (int64_t)tile_of(k) * TILE + ltid, tlane + COL_D2 + (uint32_t)b * 96u, cg * 16, sm.inv_s + cg * 16);
@@ -575,7 +499,7 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
       tc::fence_before();
       mbar_arrive(&sm.flushed[b]);
     }
-    if (on && do_dir) {                                  // the run's direct result (complete with the last tile_done)
+    if (do_dir) {                                        // the run's direct result (complete with the last tile_done)
 #pragma unroll
       for (int cg = 0; cg < KC / 16; ++cg) {
         if (nt >= 2) h_flush2<KC>(Y, n, i0 + ltid, tlane + COL_D1, tlane + COL_D1 + 96u, cg * 16, sm.inv_s + cg * 16);
@@ -660,14 +584,14 @@ int launch_prop_h(const float* tiles, int64_t n, int tr0, int tr1, const float* 
   if (e != cudaSuccess) return (int)e;
   if (tr1 - tr0 > 65535) return -3;
   dim3 grid((unsigned)((tr1 + H_RUN - 1) / H_RUN), (unsigned)(tr1 - tr0));
-  k_propagate_h<KC><<<grid, H_THREADS, smem, st>>>(tiles, n, tr0, mu, raw, Bk, scale, Y, g_prop_dbg, products);
+  k_propagate_h<KC><<<grid, H_THREADS, smem, st>>>(tiles, n, tr0, mu, raw, Bk, scale, Y, products);
   MCGRA_LAUNCH_CHECK();
   return 0;
 }
 
-// 0 = exact fp32 FFMA (reference of the engine-agreement tests; also runs the fused element-wise variant),
-// 5 = tcgen05 kind::f16 on the fp16x2 image (default).  (Engines 1-4 of rounds 1-2 -- mma.sync 3xTF32, the tcgen05 tf32
-// hybrids -- are gone; their measurements are in profiles/history and profiles/r01_umma_rate.txt.)
+// 0 = exact fp32 FFMA (reference of the engine-agreement tests), 5 = tcgen05 kind::f16 on the fp16x2 image (default).
+// (Engines 1-4 of rounds 1-2 -- mma.sync 3xTF32, the tcgen05 tf32 hybrids -- are gone; their measurements are in
+// profiles/history and profiles/r01_umma_rate.txt.)
 int g_prop_engine = 5;
 int g_elem_engine = 1;     // mcgra_set_engine(4, v): 0 = k_elem_stats everywhere, 1 = bulk-staged persistent k_elem_rs for the steady state
 int g_elem_grid = 0;       // test knob: cap on the persistent grid (mcgra_set_engine(4, 100 + cap); 0 = one CTA per SM)
@@ -676,7 +600,7 @@ int g_elem_grid = 0;       // test knob: cap on the persistent grid (mcgra_set_e
 // ---------------------------------------------------------------------------------------------------------
 // Stand-alone element-wise pass (c1 MSE/KL against feature_adj, c6 entropy; values + degree-gradient row sums).
 // A pure streaming kernel (x and F tiles read once, 8 bytes per entry) that runs at full occupancy; the propagation
-// passes then all use the plain tensor-core kernels.  Same arithmetic as the fused variants above.
+// passes then all use the plain tensor-core kernels.
 // ---------------------------------------------------------------------------------------------------------
 // Streaming structure: a warp owns rows warp, warp + 8, ...; the loads of EIGHT rows (x and F: 16 LDG.128 per thread)
 // are issued before any arithmetic, and the per-row degree-gradient sums go to shared memory instead of one global
@@ -978,15 +902,13 @@ k_elem_rs(const float* __restrict__ tiles, int64_t n, int tr0, int64_t ntiles, c
   }
 }
 
-template <int KC, bool ELEM>
+template <int KC>
 int launch_prop(const float* tiles, int64_t n, int64_t t0, int64_t nt, const float* mu, int raw, const float* B,
-                float* Y, const mcgra_elem_args* elem, cudaStream_t st, int products) {
+                float* Y, cudaStream_t st, int products) {
   const size_t smem = sizeof(PropSmem<KC>);
-  cudaError_t e = cudaFuncSetAttribute(k_propagate<KC, ELEM>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  cudaError_t e = cudaFuncSetAttribute(k_propagate<KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  mcgra_elem_args ea = {};
-  if (ELEM) ea = *elem;
-  k_propagate<KC, ELEM><<<(unsigned)nt, 128, smem, st>>>(tiles, n, t0, mu, raw, B, Y, ea, products);
+  k_propagate<KC><<<(unsigned)nt, 128, smem, st>>>(tiles, n, t0, mu, raw, B, Y, products);
   MCGRA_LAUNCH_CHECK();
   return 0;
 }
@@ -997,23 +919,25 @@ extern "C" {
 
 int mcgra_set_fold_engine_(int value);
 int mcgra_set_pairs_engine_(int value);
-int mcgra_set_gemm_engine_(int value);
 int mcgra_set_ensemble_engine_(int value);
 int mcgra_set_auc_engine_(int value);
 int mcgra_set_engine(int which, int value) {
-  if (which == 5) return mcgra_set_ensemble_engine_(value);
-  if (which == 6) return mcgra_set_auc_engine_(value);
-  if (which == 3) return mcgra_set_gemm_engine_(value);
-  if (which == 4) {
-    if (value >= 100) g_elem_grid = value - 100;
-    else g_elem_engine = value;
-    return 0;
+  switch (which) {
+    case 0:
+      if (value != 0 && value != 5) return -1;
+      g_prop_engine = value;
+      return 0;
+    case 1: return mcgra_set_fold_engine_(value);
+    case 2: return mcgra_set_pairs_engine_(value);
+    case 4:
+      if (value >= 100 && value < 1000) g_elem_grid = value - 100;
+      else if (value == 0 || value == 1) g_elem_engine = value;
+      else return -1;
+      return 0;
+    case 5: return mcgra_set_ensemble_engine_(value);
+    case 6: return mcgra_set_auc_engine_(value);
+    default: return -1;
   }
-  if (which == 0 && value >= 100) { g_prop_dbg = value - 100; return 0; }
-  if (which == 0) { g_prop_engine = value; return 0; }
-  if (which == 1) return mcgra_set_fold_engine_(value);
-  if (which == 2) return mcgra_set_pairs_engine_(value);
-  return -1;
 }
 
 int mcgra_degree(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, float* d, void* stream) {
@@ -1071,32 +995,25 @@ int64_t mcgra_propagate_ws_bytes(int64_t n, int K) {
 }
 
 int mcgra_propagate_sel(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* B, int K,
-                        float* Y, const mcgra_elem_args* elem, void* ws, int products, void* stream) {
+                        float* Y, void* ws, int products, void* stream) {
   const int64_t nt = tri(tr1) - tri(tr0);
   if (products < MCGRA_PROD_DIRECT || products > MCGRA_PROD_BOTH) return -1;
-  if (elem != nullptr && products != MCGRA_PROD_BOTH) return -1;     // the fused terms cover both orientations
   if (nt <= 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t t0 = tri(tr0);
-  if (ws != nullptr && g_prop_engine == 5 && elem == nullptr) {
+  if (ws != nullptr && g_prop_engine == 5) {
     if (K == 32) return launch_prop_h<32>(tiles, n, tr0, tr1, mu, raw, B, Y, ws, st, products);
     if (K == 16) return launch_prop_h<16>(tiles, n, tr0, tr1, mu, raw, B, Y, ws, st, products);
     return -1;
   }
-  if (K == 32) {
-    return elem ? launch_prop<32, true>(tiles, n, t0, nt, mu, raw, B, Y, elem, st, products)
-                : launch_prop<32, false>(tiles, n, t0, nt, mu, raw, B, Y, nullptr, st, products);
-  }
-  if (K == 16) {
-    return elem ? launch_prop<16, true>(tiles, n, t0, nt, mu, raw, B, Y, elem, st, products)
-                : launch_prop<16, false>(tiles, n, t0, nt, mu, raw, B, Y, nullptr, st, products);
-  }
+  if (K == 32) return launch_prop<32>(tiles, n, t0, nt, mu, raw, B, Y, st, products);
+  if (K == 16) return launch_prop<16>(tiles, n, t0, nt, mu, raw, B, Y, st, products);
   return -1;
 }
 
 int mcgra_propagate(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* B, int K,
-                    float* Y, const mcgra_elem_args* elem, void* ws, void* stream) {
-  return mcgra_propagate_sel(tiles, n, tr0, tr1, mu, raw, B, K, Y, elem, ws, MCGRA_PROD_BOTH, stream);
+                    float* Y, void* ws, void* stream) {
+  return mcgra_propagate_sel(tiles, n, tr0, tr1, mu, raw, B, K, Y, ws, MCGRA_PROD_BOTH, stream);
 }
 
 }  // extern "C"

@@ -367,7 +367,6 @@ class PGDEngine:
             #  after attack() drops the engine)
             self._noise_fn = noise if noise is not None else (
                 lambda t, n=n, dev=dev: torch.randn((n, n), dtype=torch.float32, device=dev))
-        self.split_elem = True     # element-wise c1/c6 terms as a separate streaming pass (faster than fused, see DESIGN)
         self.set_parameter(x0)
         _tick("set_parameter")
 
@@ -449,7 +448,6 @@ class PGDEngine:
             lseA64 = torch.log(self.sumexp.double() + torch.exp((self.r * self.r).double()))   # + diagonal r_i^2
             self.lseA.copy_(lseA64)
             self.dlse.copy_(self.lseF64 - lseA64)
-        ea = None
         c1_native = self.c1_active and self.nn_mode == "native"
         if c1_native or self.k6 != 0.0:
             e = N.ElemArgs()
@@ -458,16 +456,12 @@ class PGDEngine:
             e.k1, e.k6 = (self.k1 if c1_native else 0.0), self.k6
             e.acc, e.eps_row = self._acc_row(t).data_ptr(), ptr(self.eps_row)
             e.dlse = ptr(self.dlse)
-            ea = C.byref(e)
-        if ea is not None and self.split_elem:
-            # element-wise terms as their own streaming pass; the propagation then runs on the plain tcgen05 kernel
-            call("mcgra_elem_stats", ptr(self.xt), n, tr0, tr1, mu, raw, ea, st, tag="elem_stats")
-            ea = None
-        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B1), 32, ptr(self.Y1), ea, ptr(self.prop_ws), st,
-             tag="propagate32" if ea is None else "propagate32_elem")
+            call("mcgra_elem_stats", ptr(self.xt), n, tr0, tr1, mu, raw, C.byref(e), st, tag="elem_stats")
+        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B1), 32, ptr(self.Y1), ptr(self.prop_ws), st,
+             tag="propagate32")
         self._allreduce(self.Y1)
         call("mcgra_node_mid", ap, st)
-        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B2), 32, ptr(self.Y2), None, ptr(self.prop_ws), st, tag="propagate32")
+        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B2), 32, ptr(self.Y2), ptr(self.prop_ws), st, tag="propagate32")
         self._allreduce(self.Y2)
         call("mcgra_node_head", ap, st)
         return a
@@ -503,10 +497,10 @@ class PGDEngine:
                 N.LAUNCHES["kernels"] += 2      # tcgen05 engine: operand prep (2 kernels) + k_pairs_tc
             self._allreduce(self.dzhat)
         call("mcgra_node_bwd2", ap, st)
-        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B3), 32, ptr(self.Y3), None, ptr(self.prop_ws), st, tag="propagate32")
+        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B3), 32, ptr(self.Y3), ptr(self.prop_ws), st, tag="propagate32")
         self._allreduce(self.Y3)
         call("mcgra_node_bwd1", ap, st)
-        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B4), 16, ptr(self.Y4), None, ptr(self.prop_ws), st, tag="propagate16")
+        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B4), 16, ptr(self.Y4), ptr(self.prop_ws), st, tag="propagate16")
         self._allreduce(self.Y4e)          # Y4 and eps_row in one collective
         call("mcgra_node_rho", ap, st)
         if self.smooth is not None and self.smooth_on:
@@ -556,8 +550,8 @@ class PGDEngine:
         st, n = N.stream_ptr(), self.n
         first, second = (self.Ut, self.Lt) if transpose else (self.Lt, self.Ut)
         for plane, sel in ((first, N.PROD_DIRECT), (second, N.PROD_MIRRORED)):
-            call("mcgra_propagate_sel", ptr(plane), n, self.tr0, self.tr1, None, 2, ptr(B), K, ptr(Y), None,
-                 ptr(self.prop_ws), sel, st, tag=f"propagate{K}_sel")
+            call("mcgra_propagate_sel", ptr(plane), n, self.tr0, self.tr1, None, 2, ptr(B), K, ptr(Y), ptr(self.prop_ws),
+                 sel, st, tag=f"propagate{K}_sel")
         call("mcgra_diag_axpy", ptr(self.mdiag), ptr(B), K, n, ptr(Y), st)
 
     def _iterate_noisy(self, t):

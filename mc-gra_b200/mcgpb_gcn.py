@@ -62,7 +62,7 @@ class TiledAdjacency:
         if K not in (16, 32):
             raise NotImplementedError("native propagation handles 16- or 32-wide operands (nhid = 16 in the reference)")
         Y = torch.zeros_like(B)
-        call("mcgra_propagate", ptr(self.tiles), self.n, 0, self.T, None, 2, ptr(B), K, ptr(Y), None, ptr(self.ws),
+        call("mcgra_propagate", ptr(self.tiles), self.n, 0, self.T, None, 2, ptr(B), K, ptr(Y), ptr(self.ws),
              N.stream_ptr())
         return Y + self.diag[:, None] * B
 

@@ -282,11 +282,11 @@ class PGDAttack(BaseAttack):
         self.adj_changes.data = packed                                   # :301
         # embeddings / victim output on the raw decoded adjacency (:304-308): two propagations over xf
         Y = torch.zeros(n, HID, dtype=torch.float32, device=dev)
-        call("mcgra_propagate", ptr(xf), n, 0, T, None, 1, ptr(eng.S1), HID, ptr(Y), None, ptr(eng.prop_ws), st)
+        call("mcgra_propagate", ptr(xf), n, 0, T, None, 1, ptr(eng.S1), HID, ptr(Y), ptr(eng.prop_ws), st)
         H1 = torch.relu(Y + b1)
         T2 = (H1 @ W2).contiguous()
         Y2 = torch.zeros(n, HID, dtype=torch.float32, device=dev)
-        call("mcgra_propagate", ptr(xf), n, 0, T, None, 1, ptr(T2), HID, ptr(Y2), None, ptr(eng.prop_ws), st)
+        call("mcgra_propagate", ptr(xf), n, 0, T, None, 1, ptr(T2), HID, ptr(Y2), ptr(eng.prop_ws), st)
         H2 = torch.relu(Y2 + b2)
         YA2 = F.log_softmax(H2 @ Wl.t() + bl, dim=1)
         # cur_adj = modified_adj (:302) + H_A1 + H_A2 + feature_adj + Y_A2 (+ ori_HA) (+ ori_YA) (+ label_adj), summed in
@@ -350,12 +350,12 @@ class PGDAttack(BaseAttack):
             dist.all_reduce(packed, group=eng.group)
             self.adj_changes.data = packed
         Y = torch.zeros(n, HID, dtype=torch.float32, device=dev)
-        call("mcgra_propagate", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(eng.S1), HID, ptr(Y), None, ptr(eng.prop_ws), st)
+        call("mcgra_propagate", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(eng.S1), HID, ptr(Y), ptr(eng.prop_ws), st)
         dist.all_reduce(Y, group=eng.group)
         H1 = torch.relu(Y + b1)
         T2 = (H1 @ W2).contiguous()
         Y2 = torch.zeros(n, HID, dtype=torch.float32, device=dev)
-        call("mcgra_propagate", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(T2), HID, ptr(Y2), None, ptr(eng.prop_ws), st)
+        call("mcgra_propagate", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(T2), HID, ptr(Y2), ptr(eng.prop_ws), st)
         dist.all_reduce(Y2, group=eng.group)
         del xf
         H2 = torch.relu(Y2 + b2)

@@ -39,6 +39,26 @@ def test_version_and_tile_count(native):
     assert L.mcgra_tiles_in_rows(2, 4) == 7
 
 
+DEFAULT_ENGINES = {0: 5, 1: 3, 2: 2, 4: 1, 5: 1, 6: 1}
+
+
+def test_set_engine_accepts_only_known_values(native):
+    L = native.lib()
+    accepted = {0: [0, 5], 1: [0, 2, 3, 100, 101, 999], 2: [0, 1, 2], 4: [0, 1, 100, 101, 999], 5: [0, 1], 6: [0, 1]}
+    rejected = [(3, 1), (3, 2), (3, 116), (0, 3), (0, 1), (0, 101), (1, 1), (1, 4), (1, 1007), (1, 1000), (1, -1),
+                (2, 3), (2, -1), (4, 2), (4, 1000), (5, 2), (6, 2), (6, 101), (7, 0), (-1, 0)]
+    try:
+        for which, values in accepted.items():
+            for value in values:
+                assert L.mcgra_set_engine(which, value) == 0, (which, value)
+        for which, value in rejected:
+            assert L.mcgra_set_engine(which, value) == -1, (which, value)
+    finally:
+        for which, value in DEFAULT_ENGINES.items():
+            assert L.mcgra_set_engine(which, value) == 0
+        assert L.mcgra_set_engine(1, 100) == 0 and L.mcgra_set_engine(4, 100) == 0     # grid caps off
+
+
 def test_struct_sizes_match_c(native):
     # the C structs are passed by pointer; their size must match what nvcc laid out (probe via a tiny C check)
     import subprocess, tempfile, textwrap

@@ -1,4 +1,4 @@
-"""GPU parity of the dense contraction K6 (csrc/gemm.cu: TMA-fed tcgen05 kind::f16 x3, cta_group::1 and ::2) and of its
+"""GPU parity of the dense contraction K6 (csrc/gemm.cu: TMA-fed tcgen05 kind::f16 x3 on CTA pairs) and of its
 O(n^2) helpers (csrc/dense.cu) against fp64 torch, through the C ABI."""
 import ctypes as C
 
@@ -54,9 +54,10 @@ def test_image_from_dense(transpose):
     assert float((img.hi[:, :ocols].float() * 1.0).abs().max()) <= 16384.0
 
 
-@pytest.mark.parametrize("cg", [1, 2])
-@pytest.mark.parametrize("shape", [(256, 256, 64), (300, 200, 150), (1000, 700, 513), (130, 5, 37), (640, 1290, 2050)])
-def test_gemm_nt(cg, shape):
+# the last five shapes put the end of K on and next to the boundaries of the 16-K-block accumulation chunks
+@pytest.mark.parametrize("shape", [(256, 256, 64), (300, 200, 150), (1000, 700, 513), (130, 5, 37), (640, 1290, 2050),
+                                   (256, 256, 1024), (300, 260, 1088), (257, 511, 2048), (200, 520, 3136), (512, 384, 4160)])
+def test_gemm_nt(shape):
     N = _N()
     dev = torch.device("cuda:0")
     M, Nn, K = shape
@@ -64,44 +65,40 @@ def test_gemm_nt(cg, shape):
     A = (torch.randn(M, K, generator=g) * torch.exp(torch.randn(M, 1, generator=g))).to(dev)
     B = torch.rand(Nn, K, generator=g).to(dev)
     ia, ib = _image_of(N, A), _image_of(N, B)
-    assert N.lib().mcgra_set_engine(3, cg) == 0
-    try:
-        ldc = (Nn + 63) // 64 * 64
-        Cbuf = torch.full((M, ldc), 7.0, dtype=torch.float32, device=dev)
-        u, v = torch.randn(M, device=dev), torch.randn(Nn, device=dev)
-        red = torch.zeros(2, dtype=torch.float64, device=dev)
-        alpha_dev = torch.tensor([0.5], device=dev)
-        e = N.GemmEpilogue()
-        e.C, e.ldc, e.alpha, e.beta = N.ptr(Cbuf), ldc, 2.0, 0.25
-        e.alpha_dev = N.ptr(alpha_dev)
-        e.u, e.v, e.coef = N.ptr(u), N.ptr(v), 1.5
-        e.sumsq = red.data_ptr()
-        N.call("mcgra_gemm_nt", ia.ref, ib.ref, C.byref(e), N.stream_ptr())
-        torch.cuda.synchronize()
-        ref = A.double() @ B.double().t() - 1.5 * torch.outer(u.double(), v.double())
-        scale = (A.double().abs() @ B.double().abs().t()) + 1.5 * torch.outer(u.double().abs(), v.double().abs())
-        got = Cbuf[:, :Nn].double()
-        want = 0.25 * 7.0 + 2.0 * 0.5 * ref
-        err = float(((got - want).abs() / (scale + 1.0)).max())
-        assert err < 2e-6, f"cg={cg} shape={shape}: max scaled err {err:.3e}"
-        assert torch.all(Cbuf[:, Nn:] == 7.0), "padding columns must stay untouched"
-        ssq = float(red[0])
-        # (tensor-core fp32 accumulation truncates: a small systematic bias, see test_gemm_large_k)
-        assert abs(ssq - float((ref ** 2).sum())) <= 2e-5 * float((ref ** 2).sum())
-        # row panel: only rows [row0, row1) are written
-        C2 = torch.zeros(M, ldc, dtype=torch.float32, device=dev)
-        e2 = N.GemmEpilogue()
-        e2.C, e2.ldc, e2.alpha, e2.beta = N.ptr(C2), ldc, 1.0, 0.0
-        e2.row0, e2.row1 = M // 3, M // 3 + max(1, M // 2)
-        N.call("mcgra_gemm_nt", ia.ref, ib.ref, C.byref(e2), N.stream_ptr())
-        torch.cuda.synchronize()
-        full = A.double() @ B.double().t()
-        r0, r1 = e2.row0, e2.row1
-        sc = A.double().abs() @ B.double().abs().t() + 1.0
-        assert float(((C2[r0:r1, :Nn].double() - full[r0:r1]).abs() / sc[r0:r1]).max()) < 2e-6
-        assert torch.all(C2[:r0] == 0) and torch.all(C2[r1:] == 0)
-    finally:
-        N.lib().mcgra_set_engine(3, 2)
+    ldc = (Nn + 63) // 64 * 64
+    Cbuf = torch.full((M, ldc), 7.0, dtype=torch.float32, device=dev)
+    u, v = torch.randn(M, device=dev), torch.randn(Nn, device=dev)
+    red = torch.zeros(2, dtype=torch.float64, device=dev)
+    alpha_dev = torch.tensor([0.5], device=dev)
+    e = N.GemmEpilogue()
+    e.C, e.ldc, e.alpha, e.beta = N.ptr(Cbuf), ldc, 2.0, 0.25
+    e.alpha_dev = N.ptr(alpha_dev)
+    e.u, e.v, e.coef = N.ptr(u), N.ptr(v), 1.5
+    e.sumsq = red.data_ptr()
+    N.call("mcgra_gemm_nt", ia.ref, ib.ref, C.byref(e), N.stream_ptr())
+    torch.cuda.synchronize()
+    ref = A.double() @ B.double().t() - 1.5 * torch.outer(u.double(), v.double())
+    scale = (A.double().abs() @ B.double().abs().t()) + 1.5 * torch.outer(u.double().abs(), v.double().abs())
+    got = Cbuf[:, :Nn].double()
+    want = 0.25 * 7.0 + 2.0 * 0.5 * ref
+    err = float(((got - want).abs() / (scale + 1.0)).max())
+    assert err < 2e-6, f"shape={shape}: max scaled err {err:.3e}"
+    assert torch.all(Cbuf[:, Nn:] == 7.0), "padding columns must stay untouched"
+    ssq = float(red[0])
+    # (tensor-core fp32 accumulation truncates: a small systematic bias, see test_gemm_large_k)
+    assert abs(ssq - float((ref ** 2).sum())) <= 2e-5 * float((ref ** 2).sum())
+    # row panel: only rows [row0, row1) are written
+    C2 = torch.zeros(M, ldc, dtype=torch.float32, device=dev)
+    e2 = N.GemmEpilogue()
+    e2.C, e2.ldc, e2.alpha, e2.beta = N.ptr(C2), ldc, 1.0, 0.0
+    e2.row0, e2.row1 = M // 3, M // 3 + max(1, M // 2)
+    N.call("mcgra_gemm_nt", ia.ref, ib.ref, C.byref(e2), N.stream_ptr())
+    torch.cuda.synchronize()
+    full = A.double() @ B.double().t()
+    r0, r1 = e2.row0, e2.row1
+    sc = A.double().abs() @ B.double().abs().t() + 1.0
+    assert float(((C2[r0:r1, :Nn].double() - full[r0:r1]).abs() / sc[r0:r1]).max()) < 2e-6
+    assert torch.all(C2[:r0] == 0) and torch.all(C2[r1:] == 0)
 
 
 @pytest.mark.parametrize("K", [16384, 65536])
