@@ -432,7 +432,7 @@ int mcgra_nd_measure(const mcgra_nd_args* a, void* stream);
  * M <- clamp(M + eps * noise, 0, 1) (PGDAttack.adding_noise, topology_attack.py:474-478; noise = the caller's N(0,1) draw) */
 int mcgra_noise_clamp(float* M, const float* noise, float eps, int64_t count, void* stream);
 
-/* ---- attack() with adjacency noise (--eps != 0, topology_attack.py:165, 474-478), single GPU, MSELoss ----
+/* ---- attack() with adjacency noise (--eps != 0, topology_attack.py:165, 474-478), MSELoss / KDE ----
  * Per iteration M = clamp(p + N*eps, 0, 1) with a fresh dense n x n N (row-major fp32) and p the parameter view of
  * the tiles (off the diagonal; the diagonal is clamp(N_ii*eps, 0, 1)).  M is not symmetric: its two orientations are
  * kept as tile planes Lt (M_ij at (i,j), i > j) and Ut (M_ji at (i,j)), read by mcgra_propagate_sel with raw = 2:
@@ -440,6 +440,13 @@ int mcgra_noise_clamp(float* M, const float* noise, float eps, int64_t count, vo
  * The clamp masks are not stored: the gradient pass recomputes p + N*eps with the same two roundings.             */
 int mcgra_noise_stage(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* noise,
                       float eps, float* Lt, float* Ut, float* mdiag, float* d, void* stream);   /* d = 1 + row sums of M */
+/* The same stage split for tile-row shards (world > 1), where d must be all-reduced between the two halves:
+ *   mcgra_noise_tiles: Lt, Ut of tile rows [tr0, tr1) and d += this shard's part of the row sums (d is not initialised);
+ *   mcgra_noise_diag:  mdiag = M_ii and d += 1 + M_ii, once, after the all-reduce of d.
+ * mcgra_noise_stage = k_noise_diag (d = 1 + M_ii) + mcgra_noise_tiles. */
+int mcgra_noise_tiles(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* noise,
+                      float eps, float* Lt, float* Ut, float* d, void* stream);
+int mcgra_noise_diag(int64_t n, const float* noise, float eps, float* mdiag, float* d, void* stream);
 /* Y[i, :] += mdiag[i] * B[i, :]  (B, Y row-major [n x K]) */
 int mcgra_diag_axpy(const float* mdiag, const float* B, int K, int64_t n, float* Y, void* stream);
 typedef struct {

@@ -117,6 +117,8 @@ _SIGS = {
                                       c_fp]),
     "mcgra_noise_stage": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, C.c_float, c_fp, c_fp, c_fp, c_fp,
                                     c_fp]),
+    "mcgra_noise_tiles": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, C.c_float, c_fp, c_fp, c_fp, c_fp]),
+    "mcgra_noise_diag": (C.c_int, [i64, c_fp, C.c_float, c_fp, c_fp, c_fp]),
     "mcgra_diag_axpy": (C.c_int, [c_fp, c_fp, C.c_int, i64, c_fp, c_fp]),
     "mcgra_noisy_terms": (C.c_int, [C.POINTER(NoisyArgs), c_fp]),
     "mcgra_noisy_grad": (C.c_int, [C.POINTER(NoisyArgs), c_fp]),

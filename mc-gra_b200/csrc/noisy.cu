@@ -7,7 +7,7 @@
 // node kernels see M*B and M^T*B exactly where the symmetric path sees M*B, so only the degree gradient's diagonal changes
 // (mcgra_node_rho_diag).  This file holds the stages whose algebra differs from the symmetric path:
 //   k_noise_stage   x view + N -> Lt, Ut, degree row sums          (one CTA per stored tile)
-//   k_noise_diag    M_ii and d_i = 1 + M_ii                         (before k_noise_stage adds the row sums)
+//   k_noise_diag    M_ii and d_i = 1 + M_ii (ADD: d_i += 1 + M_ii)  (around k_noise_stage's row sums, see below)
 //   k_noisy_terms   c1 / c2 (MSELoss) and c6 over both orientations, degree-gradient row + column parts, dzhat of c2
 //   k_noisy_grad    dL/dx_ij = mask_ij dL/dM_ij + mask_ji dL/dM_ji into gradient tiles for mcgra_fold_adam (Gtiles)
 // Both also take an upstream gradient of the first nb columns of A_hat (gslab, --measure KDE): it only reaches tiles of
@@ -33,13 +33,16 @@ __device__ __forceinline__ void stage_noise_t(float* nt, const float* __restrict
   }
 }
 
+// ADD = false: d = 1 + M_ii before k_noise_stage adds one GPU's row sums; ADD = true: d += 1 + M_ii after the row sums of
+// every shard were all-reduced (the diagonal is then counted once, not once per rank)
+template <bool ADD>
 __global__ void k_noise_diag(int64_t n, const float* __restrict__ noise, float eps, float* __restrict__ mdiag,
                              float* __restrict__ d) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
   const float m = clamp01(__fmul_rn(noise[i * n + i], eps));     // 0 + N_ii * eps
   mdiag[i] = m;
-  d[i] = 1.f + m;
+  d[i] = ADD ? d[i] + (1.f + m) : 1.f + m;
 }
 
 __global__ void __launch_bounds__(256)
@@ -372,16 +375,28 @@ extern "C" {
 
 int mcgra_noise_stage(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* noise,
                       float eps, float* Lt, float* Ut, float* mdiag, float* d, void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
   if (n <= 0 || noise == nullptr) return -1;
-  k_noise_diag<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(n, noise, eps, mdiag, d);
+  k_noise_diag<false><<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n, noise, eps, mdiag, d);
   MCGRA_LAUNCH_CHECK();
+  return mcgra_noise_tiles(tiles, n, tr0, tr1, mu, raw, noise, eps, Lt, Ut, d, stream);
+}
+
+int mcgra_noise_tiles(const float* tiles, int64_t n, int tr0, int tr1, const float* mu, int raw, const float* noise,
+                      float eps, float* Lt, float* Ut, float* d, void* stream) {
+  if (n <= 0 || noise == nullptr) return -1;
   const int64_t nt = tri(tr1) - tri(tr0);
   if (nt <= 0) return 0;
   const size_t smem = (size_t)TILE * NT_LD * sizeof(float);
   cudaError_t e = cudaFuncSetAttribute(k_noise_stage, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  k_noise_stage<<<(unsigned)nt, 256, smem, st>>>(tiles, n, tri(tr0), mu, raw, noise, eps, Lt, Ut, d);
+  k_noise_stage<<<(unsigned)nt, 256, smem, (cudaStream_t)stream>>>(tiles, n, tri(tr0), mu, raw, noise, eps, Lt, Ut, d);
+  MCGRA_LAUNCH_CHECK();
+  return 0;
+}
+
+int mcgra_noise_diag(int64_t n, const float* noise, float eps, float* mdiag, float* d, void* stream) {
+  if (n <= 0 || noise == nullptr) return -1;
+  k_noise_diag<true><<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n, noise, eps, mdiag, d);
   MCGRA_LAUNCH_CHECK();
   return 0;
 }

@@ -80,13 +80,16 @@ NOISE_MEASURES = ("MSELoss", "KDE")
 
 
 def check_noise_supported(measure, world, feature_adj, device):
-    """Scope of attack() with adjacency noise (--eps != 0): MSELoss or KDE on one CUDA device.  Raised before any device
-    work."""
+    """Scope of attack() with adjacency noise (--eps != 0): MSELoss or KDE on one CUDA device, MSELoss on tile-row shards
+    (world > 1), feature_adj as a full tensor.  Raised before any device work."""
     if measure not in NOISE_MEASURES:
         raise NotImplementedError(f"--eps != 0 is implemented for --measure MSELoss and KDE only (got {measure!r}): the "
                                   "other measures' passes and closed forms assume a symmetric A_hat")
-    if world > 1 or isinstance(feature_adj, HostBands):
-        raise NotImplementedError("--eps != 0 runs on one GPU: the sharded (world > 1) / row-band noisy path is not built")
+    if isinstance(feature_adj, HostBands):
+        raise NotImplementedError("--eps != 0 needs feature_adj as a full tensor: the row-band noisy path is not built")
+    if world > 1 and measure != "MSELoss":
+        raise NotImplementedError(f"--eps != 0 with world > 1 is implemented for --measure MSELoss only (got {measure!r}): "
+                                  "the sharded noisy KDE path is not built")
     if torch.device(device).type != "cuda":
         raise NotImplementedError(f"--eps != 0 needs a CUDA device (got {device!r}); there is no CPU fallback")
 
@@ -198,14 +201,19 @@ class PGDEngine:
                      0 if isinstance(feature_adj, HostBands) else 1, ptr(self.Ft), ptr(self.Fdiag), N.stream_ptr())
                 if self.eps != 0.0:
                     # the noisy A_hat is not symmetric: c1 pairs A_hat_ij with F_ij and A_hat_ji with F_ji, so both
-                    # orientations of feature_adj are tiled as they are (F, then F^T)
-                    fdg = torch.zeros(n, **f32)
+                    # orientations of feature_adj are tiled as they are (F, then F^T).  Only the rows of this rank's tile
+                    # rows are read, so F^T is formed for that band alone (columns [r0, r1) of F): n x (r1 - r0) floats
+                    # instead of n x n, with the pointer shifted as for row-band input
                     self.FLt = torch.zeros(ntl, **f32)
-                    call("mcgra_dense_to_tiles", ptr(fa), n, n, 0, self.T, 0, ptr(self.FLt), ptr(fdg), N.stream_ptr())
-                    faT = fa.t().contiguous()
                     self.FUt = torch.zeros(ntl, **f32)
-                    call("mcgra_dense_to_tiles", ptr(faT), n, n, 0, self.T, 0, ptr(self.FUt), ptr(fdg), N.stream_ptr())
-                    del faT, fdg
+                    r0, r1 = self.tr0 * TILE, min(n, self.tr1 * TILE)
+                    if r1 > r0:
+                        call("mcgra_dense_to_tiles", ptr(fa), n, n, self.tr0, self.tr1, 0, ptr(self.FLt), None,
+                             N.stream_ptr())
+                        faT = fa[:, r0:r1].t().contiguous()
+                        call("mcgra_dense_to_tiles", faT.data_ptr() - r0 * n * 4, n, n, self.tr0, self.tr1, 0,
+                             ptr(self.FUt), None, N.stream_ptr())
+                        del faT
                 if world > 1:     # each rank wrote the diagonal of its own tile rows only
                     self._allreduce(self.Fdiag)
                 self.meas_nn = self.measure
@@ -367,6 +375,10 @@ class PGDEngine:
             #  after attack() drops the engine)
             self._noise_fn = noise if noise is not None else (
                 lambda t, n=n, dev=dev: torch.randn((n, n), dtype=torch.float32, device=dev))
+            # world > 1: every rank draws the whole matrix and reads its tiles' blocks of it, so the ranks must draw
+            # alike.  Per iteration, the fp64 sums of row 0 and of the diagonal (f) go through one MAX all-reduce as
+            # (f, -f); the ranks agreed iff max f == min f (check_noise_agreement, once, after the loop)
+            self.noise_fp = torch.zeros(max_epochs, 4, dtype=torch.float64, device=dev) if world > 1 else None
         self.set_parameter(x0)
         _tick("set_parameter")
 
@@ -545,28 +557,61 @@ class PGDEngine:
                  ptr(self.step_dev), st)
         self.step = t + 1
 
-    def _propagate_noisy(self, B, K, Y, transpose):
-        """Y += M B (transpose=False) or M^T B from the two orientation planes and the diagonal (mcgra.h)."""
+    def _propagate_noisy(self, B, K, Y, transpose, reduce=None):
+        """Y += M B (transpose=False) or M^T B from the two orientation planes and the diagonal (mcgra.h).  With world > 1
+        the shards' products are all-reduced (`reduce`: a buffer that holds Y, default Y itself) before the diagonal is
+        added, once, on every rank."""
         st, n = N.stream_ptr(), self.n
         first, second = (self.Ut, self.Lt) if transpose else (self.Lt, self.Ut)
         for plane, sel in ((first, N.PROD_DIRECT), (second, N.PROD_MIRRORED)):
             call("mcgra_propagate_sel", ptr(plane), n, self.tr0, self.tr1, None, 2, ptr(B), K, ptr(Y), ptr(self.prop_ws),
                  sel, st, tag=f"propagate{K}_sel")
+        self._allreduce(Y if reduce is None else reduce)
         call("mcgra_diag_axpy", ptr(self.mdiag), ptr(B), K, n, ptr(Y), st)
 
+    def _record_noise(self, noise, t):
+        """Fingerprint of this rank's draw, reduced across ranks without a host synchronisation (world > 1)."""
+        import torch.distributed as dist
+        f = torch.stack((noise[0].double().sum(), noise.diagonal().double().sum()))
+        row = self.noise_fp[t]
+        row[:2], row[2:] = f, -f
+        self._allreduce(row, dist.ReduceOp.MAX)
+
+    def check_noise_agreement(self):
+        """Raise if the ranks drew different noise in any iteration so far (world > 1, --eps != 0).  One host read."""
+        if self.eps == 0.0 or self.world == 1 or self.step == 0:
+            return
+        rec = self.noise_fp[:self.step].cpu()
+        bad = torch.nonzero(rec[:, :2] != -rec[:, 2:])
+        if bad.numel():
+            raise RuntimeError(f"--eps != 0 with world = {self.world}: the ranks drew different noise (first in iteration "
+                               f"{int(bad[0, 0])}).  Every rank draws the full n x n matrix from its default CUDA generator: "
+                               "seed all ranks alike (torch.cuda.manual_seed) before attack()")
+
     def _iterate_noisy(self, t):
-        """One iteration with adjacency noise (--eps != 0, topology_attack.py:165, 474-478): single GPU, MSELoss or KDE.
+        """One iteration with adjacency noise (--eps != 0, topology_attack.py:165, 474-478): MSELoss or KDE on one GPU,
+        MSELoss on tile-row shards.
         noise stage -> node_pre -> M B1 -> node_mid -> M B2 -> node_head -> [KDE: c1 / c2 slab stage, c9 / c10]
         -> pairs (c7, KDE: c2's M1 gradient) -> noisy terms (c1, c2, c6; KDE: the A_hat slab gradient) -> node_bwd2
-        -> M^T B3 -> node_bwd1 -> M^T B4 -> node_rho_diag -> noisy gradient -> fold (Adam, clamp, sums)."""
+        -> M^T B3 -> node_bwd1 -> M^T B4 -> node_rho_diag -> noisy gradient -> fold (Adam, clamp, sums).
+        world > 1 adds the collectives of DESIGN.md 3.7: the draw's fingerprint, d between the two noise stages, each
+        product before its diagonal, dzhat, Y4 with eps_row, and after the fold the statistics and the bracket."""
         st = N.stream_ptr()
         n, tr0, tr1, mu, raw = self.n, self.tr0, self.tr1, ptr(self.mu), self.raw
         noise = self._noise_fn(t)
         if tuple(noise.shape) != (n, n):
             raise ValueError(f"noise draw of shape {tuple(noise.shape)}, expected ({n}, {n})")
         noise = noise.to(device=self.dev, dtype=torch.float32).contiguous()
-        call("mcgra_noise_stage", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(noise), self.eps, ptr(self.Lt), ptr(self.Ut),
-             ptr(self.mdiag), ptr(self.d), st)
+        if self.world == 1:
+            call("mcgra_noise_stage", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(noise), self.eps, ptr(self.Lt),
+                 ptr(self.Ut), ptr(self.mdiag), ptr(self.d), st)
+        else:
+            self._record_noise(noise, t)
+            self.d.zero_()
+            call("mcgra_noise_tiles", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(noise), self.eps, ptr(self.Lt),
+                 ptr(self.Ut), ptr(self.d), st)
+            self._allreduce(self.d)
+            call("mcgra_noise_diag", n, ptr(noise), self.eps, ptr(self.mdiag), ptr(self.d), st)
         a = self._node_args(t)
         ap = C.byref(a)
         call("mcgra_node_pre", ap, st)
@@ -596,10 +641,11 @@ class PGDEngine:
             na.gslab, na.nb = ptr(self.kde["gA"]), self.kde["nb"]
         nap = C.byref(na)
         call("mcgra_noisy_terms", nap, st)
+        self._allreduce(self.dzhat)
         call("mcgra_node_bwd2", ap, st)
         self._propagate_noisy(self.B3, 32, self.Y3, True)
         call("mcgra_node_bwd1", ap, st)
-        self._propagate_noisy(self.B4, 16, self.Y4, True)
+        self._propagate_noisy(self.B4, 16, self.Y4, True, reduce=self.Y4e)      # Y4 and eps_row in one collective
         call("mcgra_node_rho_diag", ap, ptr(self.mdiag), st)
         call("mcgra_noisy_grad", nap, st)
 
@@ -623,6 +669,12 @@ class PGDEngine:
              ptr(self.minmax), st)
         self.raw = 0 if self.proj_possible else 2
         self.mu.zero_()
+        if self.world > 1:
+            import torch.distributed as dist
+            self._allreduce(self._acc_row(t + 1)[:16])
+            if self.proj_possible:
+                self._allreduce(self.minmax[0:1], dist.ReduceOp.MIN)
+                self._allreduce(self.minmax[1:2], dist.ReduceOp.MAX)
         if self.proj_possible:
             self._project(t)
         self.step = t + 1     # (the degree of the next iteration comes from its own noise stage)

@@ -208,6 +208,7 @@ class PGDAttack(BaseAttack):
         # `_noise`: callable(t) -> n x n draw of iteration t for --eps != 0 (default: torch.randn on the attack's device)
         on_iter = (lambda: self._trace.append(eng.packed_parameter())) if kwargs.get("_trace") else None
         eng.run(int(epochs), on_iter=on_iter, use_graph=kwargs.get("_graph", "auto"))
+        eng.check_noise_agreement()        # world > 1 with noise: raises if the ranks drew differently
         if kwargs.get("_skip_finalize"):         # bench hook: engine is driven by the caller
             return 0, 0, 0, 0
         if int(epochs) == 0:
