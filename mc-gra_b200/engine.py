@@ -3,9 +3,14 @@
 One PGD iteration of the reference (MC-GRA/topology_attack.py:161-283, SURVEY.md 3.2 steps 1-17) becomes a
 fixed sequence of C-ABI calls on the current CUDA stream, with no host synchronisation:
 
-    node_pre -> [row_sumexp] -> propagate#1(+element-wise c1/c6) -> node_mid -> propagate#2 -> node_head
-    -> pairs(c7,c2) -> node_bwd2 -> propagate#3 -> node_bwd1 -> propagate#4 -> node_rho -> fold_adam
-    -> [bisection passes]
+    node_pre -> [row_sumexp] -> elem_stats (c1/c6) -> propagate#1 -> node_mid -> propagate#2 -> node_head
+    -> [n x n stage: HSIC/CKA/DP, KL-c2, KDE] -> [n x d stage: c9/c10] -> pairs (c7, c2) -> node_bwd2 -> propagate#3
+    -> node_bwd1 -> propagate#4 -> node_rho -> [smoothing] -> fold_adam -> [bisection passes]
+
+With adjacency noise (--eps != 0, topology_attack.py:165, 474-478) a noise stage forms the noisy estimate M first; the
+four products run on M's two orientation planes plus its diagonal (M^T for #3 and #4); row_sumexp and elem_stats are
+skipped and a noisy-terms pass before node_bwd2 carries c1/c2/c6 instead; KDE's n x n stage works on M's slabs; pairs
+keeps c7 and KDE's M1 gradient only; node_rho_diag and a noisy-gradient pass replace node_rho.
 
 The adjacency estimate lives only as the tiled lower triangle (x', Adam m, v); n x n matrices are never
 materialised.  With world_size > 1 every rank owns a contiguous range of tile rows (equal tile counts) and the
@@ -446,14 +451,15 @@ class PGDEngine:
         a.dlse = ptr(self.dlse)
         return a
 
-    def forward_stages(self, t):
-        """Forward half of an iteration (through node_head); returns the node-args struct."""
+    def forward_stages(self, t, noisy=False):
+        """Forward half of an iteration (through node_head) on the noise-free operator, or on the noisy one (`noisy`: the
+        noise stage of iteration t has run; its terms pass carries c1 / c6); returns the node-args struct."""
         st = N.stream_ptr()
         n, tr0, tr1, mu, raw = self.n, self.tr0, self.tr1, ptr(self.mu), self.raw
         a = self._node_args(t)
         ap = C.byref(a)
         call("mcgra_node_pre", ap, st)
-        if self.meas_nn == N.M_KL and self.nn_mode == "native":
+        if not noisy and self.meas_nn == N.M_KL and self.nn_mode == "native":
             self.sumexp.zero_()
             call("mcgra_row_sumexp", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.r), ptr(self.sumexp), st)
             self._allreduce(self.sumexp)
@@ -461,7 +467,7 @@ class PGDEngine:
             self.lseA.copy_(lseA64)
             self.dlse.copy_(self.lseF64 - lseA64)
         c1_native = self.c1_active and self.nn_mode == "native"
-        if c1_native or self.k6 != 0.0:
+        if not noisy and (c1_native or self.k6 != 0.0):
             e = N.ElemArgs()
             e.r, e.Ftiles, e.lseA, e.lseF = ptr(self.r), (ptr(self.Ft) if c1_native else None), ptr(self.lseA), ptr(self.lseF)
             e.measure = self.meas_nn if c1_native else N.M_NONE
@@ -469,25 +475,41 @@ class PGDEngine:
             e.acc, e.eps_row = self._acc_row(t).data_ptr(), ptr(self.eps_row)
             e.dlse = ptr(self.dlse)
             call("mcgra_elem_stats", ptr(self.xt), n, tr0, tr1, mu, raw, C.byref(e), st, tag="elem_stats")
-        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B1), 32, ptr(self.Y1), ptr(self.prop_ws), st,
-             tag="propagate32")
-        self._allreduce(self.Y1)
+        self._product(self.B1, 32, self.Y1, False, noisy)
         call("mcgra_node_mid", ap, st)
-        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B2), 32, ptr(self.Y2), ptr(self.prop_ws), st, tag="propagate32")
-        self._allreduce(self.Y2)
+        self._product(self.B2, 32, self.Y2, False, noisy)
         call("mcgra_node_head", ap, st)
         return a
 
+    def _product(self, B, K, Y, transpose, noisy, reduce=None):
+        """Y += A_hat B, or A_hat^T B (`transpose`), for the n x K operand B.  Noise-free: one pass over the symmetric x'.
+        Noisy: the two orientation planes of M, then the diagonal (mcgra.h).  With world > 1 the shards' products are
+        all-reduced (`reduce`: a buffer that holds Y, default Y itself) before the diagonal is added, once, on every rank."""
+        st, n = N.stream_ptr(), self.n
+        if noisy:
+            first, second = (self.Ut, self.Lt) if transpose else (self.Lt, self.Ut)
+            for plane, sel in ((first, N.PROD_DIRECT), (second, N.PROD_MIRRORED)):
+                call("mcgra_propagate_sel", ptr(plane), n, self.tr0, self.tr1, None, 2, ptr(B), K, ptr(Y),
+                     ptr(self.prop_ws), sel, st, tag=f"propagate{K}_sel")
+        else:
+            call("mcgra_propagate", ptr(self.xt), n, self.tr0, self.tr1, ptr(self.mu), self.raw, ptr(B), K, ptr(Y),
+                 ptr(self.prop_ws), st, tag=f"propagate{K}")
+        self._allreduce(Y if reduce is None else reduce)
+        if noisy:
+            call("mcgra_diag_axpy", ptr(self.mdiag), ptr(B), K, n, ptr(Y), st)
+
     def iterate(self):
-        """One full PGD iteration (forward, backward, Adam, projection); no host synchronisation."""
+        """One full PGD iteration (forward, backward, Adam, projection): the stage list of the module docstring, with its
+        noisy variants when eps != 0.  No host synchronisation.  With world > 1 the n x K products, dzhat, and the fold's
+        sums and bracket are all-reduced; under noise also d and the draw's fingerprint (DESIGN.md 3.7)."""
         t = self.step
         if t >= self.max_epochs:
             raise RuntimeError("acc history exhausted; construct the engine with a larger max_epochs")
-        if self.eps != 0.0:
-            return self._iterate_noisy(t)
         st = N.stream_ptr()
         n, tr0, tr1, mu, raw = self.n, self.tr0, self.tr1, ptr(self.mu), self.raw
-        a = self.forward_stages(t)
+        noisy = self.eps != 0.0
+        noise = self._noise_stage(t) if noisy else None
+        a = self.forward_stages(t, noisy)
         ap = C.byref(a)
         dense = self.nn_mode in ("dense", "kl2", "kde")      # gradient tiles handed over as MCGRA_M_PRE
         if self.nn_mode == "dense":
@@ -495,50 +517,49 @@ class PGDEngine:
         elif self.nn_mode == "kl2":
             self._kl2_stage(t)
         elif self.nn_mode == "kde":
-            self._kde_stage(t)
+            (self._kde_stage_noisy if noisy else self._kde_stage)(t)
         if self.measure == N.M_KDE:
             if self.w9 != 0.0 or self.w10 != 0.0:
                 self._kde_nd_stage(t)
         elif not self.nd_native and (self.w9 != 0.0 or self.w10 != 0.0):
             self._nd_stage(t)
-        if self.k7 != 0.0 or self.k2 != 0.0 or dense:
-            call("mcgra_pairs", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.zhat), ptr(self.r),
-                 self.k7, self.k2, (ptr(self.Ft) if dense else None), (ptr(self.Ct) if dense else None),
-                 ptr(self.dzhat), ptr(self.eps_row), self._acc_row(t).data_ptr(), ptr(self.pairs_ws), st)
-            if self.k7 != 0.0 and self.k2 == 0.0 and not dense:
+        # under noise c7 and the M1 side of KDE's c2 are functions of the symmetric decode M1 only: no A_hat tiles exist
+        # (Ft = None), the noisy kernels form A_hat's part of eps_row themselves
+        EAt, Ct = (self.Ft, self.Ct) if dense else (None, None)
+        k2 = 0.0 if noisy else self.k2
+        pairs = self.k7 != 0.0 or k2 != 0.0 or EAt is not None or Ct is not None
+        if pairs:
+            call("mcgra_pairs", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.zhat), ptr(self.r), self.k7, k2, ptr(EAt),
+                 ptr(Ct), ptr(self.dzhat), ptr(self.eps_row), self._acc_row(t).data_ptr(), ptr(self.pairs_ws), st)
+            if self.k7 != 0.0 and k2 == 0.0 and EAt is None and Ct is None:
                 N.LAUNCHES["kernels"] += 2      # tcgen05 engine: operand prep (2 kernels) + k_pairs_tc
+        if noisy:
+            na = N.NoisyArgs()
+            na.n, na.npad, na.tr0, na.tr1 = n, self.npad, tr0, tr1
+            na.tiles, na.mu, na.raw, na.noise, na.eps = ptr(self.xt), mu, raw, ptr(noise), self.eps
+            na.Lt, na.Ut, na.FLt, na.FUt = ptr(self.Lt), ptr(self.Ut), ptr(self.FLt), ptr(self.FUt)
+            na.zhat, na.r, na.rho, na.Wt = ptr(self.zhat), ptr(self.r), ptr(self.rho), ptr(self.Wt)
+            na.k1 = self.k1 if self.FLt is not None else 0.0
+            na.k2, na.k6 = self.k2, self.k6
+            na.acc, na.eps_row, na.dzhat, na.Gt = self._acc_row(t).data_ptr(), ptr(self.eps_row), ptr(self.dzhat), ptr(self.Gn)
+            if self.nn_mode == "kde":
+                na.gslab, na.nb = ptr(self.kde["gA"]), self.kde["nb"]
+            nap = C.byref(na)
+            call("mcgra_noisy_terms", nap, st)
+        if pairs or noisy:
             self._allreduce(self.dzhat)
         call("mcgra_node_bwd2", ap, st)
-        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B3), 32, ptr(self.Y3), ptr(self.prop_ws), st, tag="propagate32")
-        self._allreduce(self.Y3)
+        self._product(self.B3, 32, self.Y3, True, noisy)
         call("mcgra_node_bwd1", ap, st)
-        call("mcgra_propagate", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.B4), 16, ptr(self.Y4), ptr(self.prop_ws), st, tag="propagate16")
-        self._allreduce(self.Y4e)          # Y4 and eps_row in one collective
-        call("mcgra_node_rho", ap, st)
-        if self.smooth is not None and self.smooth_on:
-            self._smooth_stage(t)
-
-        f = N.FoldArgs()
-        f.n, f.npad, f.Wt, f.r, f.rho = n, self.npad, ptr(self.Wt), ptr(self.r), ptr(self.rho)
-        use_f = dense or (self.c1_active and self.nn_mode == "native")
-        f.Ftiles = ptr(self.Ft) if use_f else None
-        f.lseA, f.lseF = ptr(self.lseA), ptr(self.lseF)
-        f.zhat = ptr(self.zhat)
-        f.measure = self.meas_nn if use_f else N.M_NONE
-        f.k1, f.k6, f.k2 = (self.k1 if use_f else 0.0), self.k6, self.k2
-        f.norm_coef = self.weight_sup * 0.001
-        f.lr, f.beta1, f.beta2, f.adam_eps = self.lr, 0.9, 0.999, 1e-8
-        f.step = t + 1
-        f.acc_prev = self._acc_row(t).data_ptr()
-        f.acc_next = self._acc_row(t + 1).data_ptr()
-        f.step_ptr = ptr(self.step_dev) if self.ring_mode else None
-        f.d_next = ptr(self.d_next)
-        f.store_clamped = 0 if self.proj_possible else 1
-        f.Wk = ptr(self.fold_ws)
-        f.plain_gd = 1 if self.plain_gd else 0
-        f.Gtiles = ptr(self.Gt) if (self.smooth is not None and self.smooth_on) else None
-        call("mcgra_fold_adam", ptr(self.xt), ptr(self.mt), ptr(self.vt), tr0, tr1, mu, raw, C.byref(f),
-             ptr(self.minmax), st)
+        self._product(self.B4, 16, self.Y4, True, noisy, reduce=self.Y4e)      # Y4 and eps_row in one collective
+        if noisy:
+            call("mcgra_node_rho_diag", ap, ptr(self.mdiag), st)
+            call("mcgra_noisy_grad", nap, st)
+        else:
+            call("mcgra_node_rho", ap, st)
+            if self.smooth is not None and self.smooth_on:
+                self._smooth_stage(t)
+        self._fold(t, noisy)
         # the buffer now holds the un-projected Adam output x' (mu = 0), or the clamped parameter itself
         self.raw = 0 if self.proj_possible else 2
         self.mu.zero_()
@@ -550,24 +571,63 @@ class PGDEngine:
                 self._allreduce(self.minmax[1:2], dist.ReduceOp.MAX)
         if self.proj_possible:
             self._project(t)
-        self._allreduce(self.d_next)
-        self.d, self.d_next = self.d_next, self.d
-        if self.ring_mode:       # hist[step_dev] = finished row; step_dev += 1
-            call("mcgra_history_push", self._acc_row(t).data_ptr(), ptr(self.acc_hist), self.acc_hist.shape[0],
-                 ptr(self.step_dev), st)
+        if not noisy:      # (under noise the degree of the next iteration comes from its own noise stage)
+            self._allreduce(self.d_next)
+            self.d, self.d_next = self.d_next, self.d
+            if self.ring_mode:       # hist[step_dev] = finished row; step_dev += 1
+                call("mcgra_history_push", self._acc_row(t).data_ptr(), ptr(self.acc_hist), self.acc_hist.shape[0],
+                     ptr(self.step_dev), st)
         self.step = t + 1
 
-    def _propagate_noisy(self, B, K, Y, transpose, reduce=None):
-        """Y += M B (transpose=False) or M^T B from the two orientation planes and the diagonal (mcgra.h).  With world > 1
-        the shards' products are all-reduced (`reduce`: a buffer that holds Y, default Y itself) before the diagonal is
-        added, once, on every rank."""
+    def _fold(self, t, noisy):
+        """Adam step, clamp and the next iteration's sums (mcgra_fold_adam).  Under noise the product and degree terms
+        are already inside the gradient tiles Gn: zero factors and rho, no n x n term."""
+        f = N.FoldArgs()
+        f.n, f.npad, f.r = self.n, self.npad, ptr(self.r)
+        f.norm_coef = self.weight_sup * 0.001
+        f.lr, f.beta1, f.beta2, f.adam_eps = self.lr, 0.9, 0.999, 1e-8
+        f.step = t + 1
+        f.acc_prev = self._acc_row(t).data_ptr()
+        f.acc_next = self._acc_row(t + 1).data_ptr()
+        f.d_next = ptr(self.d_next)
+        f.store_clamped = 0 if self.proj_possible else 1
+        f.Wk = ptr(self.fold_ws)
+        if noisy:
+            f.Wt, f.rho = ptr(self.Wt0), ptr(self.rho0)
+            f.measure = N.M_NONE
+            f.Gtiles = ptr(self.Gn)
+        else:
+            use_f = self.nn_mode in ("dense", "kl2", "kde") or (self.c1_active and self.nn_mode == "native")
+            f.Wt, f.rho = ptr(self.Wt), ptr(self.rho)
+            f.Ftiles = ptr(self.Ft) if use_f else None
+            f.lseA, f.lseF = ptr(self.lseA), ptr(self.lseF)
+            f.zhat = ptr(self.zhat)
+            f.measure = self.meas_nn if use_f else N.M_NONE
+            f.k1, f.k6, f.k2 = (self.k1 if use_f else 0.0), self.k6, self.k2
+            f.step_ptr = ptr(self.step_dev) if self.ring_mode else None
+            f.plain_gd = 1 if self.plain_gd else 0
+            f.Gtiles = ptr(self.Gt) if (self.smooth is not None and self.smooth_on) else None
+        call("mcgra_fold_adam", ptr(self.xt), ptr(self.mt), ptr(self.vt), self.tr0, self.tr1, ptr(self.mu), self.raw,
+             C.byref(f), ptr(self.minmax), N.stream_ptr())
+
+    def _noise_stage(self, t):
+        """Draw iteration t's noise and form M's two orientation planes, its diagonal and the degree d; returns the draw.
+        With world > 1 the draw is fingerprinted and d is all-reduced before the diagonal is added, once."""
         st, n = N.stream_ptr(), self.n
-        first, second = (self.Ut, self.Lt) if transpose else (self.Lt, self.Ut)
-        for plane, sel in ((first, N.PROD_DIRECT), (second, N.PROD_MIRRORED)):
-            call("mcgra_propagate_sel", ptr(plane), n, self.tr0, self.tr1, None, 2, ptr(B), K, ptr(Y), ptr(self.prop_ws),
-                 sel, st, tag=f"propagate{K}_sel")
-        self._allreduce(Y if reduce is None else reduce)
-        call("mcgra_diag_axpy", ptr(self.mdiag), ptr(B), K, n, ptr(Y), st)
+        noise = self._noise_fn(t)
+        if tuple(noise.shape) != (n, n):
+            raise ValueError(f"noise draw of shape {tuple(noise.shape)}, expected ({n}, {n})")
+        noise = noise.to(device=self.dev, dtype=torch.float32).contiguous()
+        args = (ptr(self.xt), n, self.tr0, self.tr1, ptr(self.mu), self.raw, ptr(noise), self.eps, ptr(self.Lt), ptr(self.Ut))
+        if self.world == 1:
+            call("mcgra_noise_stage", *args, ptr(self.mdiag), ptr(self.d), st)
+        else:
+            self._record_noise(noise, t)
+            self.d.zero_()
+            call("mcgra_noise_tiles", *args, ptr(self.d), st)
+            self._allreduce(self.d)
+            call("mcgra_noise_diag", n, ptr(noise), self.eps, ptr(self.mdiag), ptr(self.d), st)
+        return noise
 
     def _record_noise(self, noise, t):
         """Fingerprint of this rank's draw, reduced across ranks without a host synchronisation (world > 1)."""
@@ -587,97 +647,6 @@ class PGDEngine:
             raise RuntimeError(f"--eps != 0 with world = {self.world}: the ranks drew different noise (first in iteration "
                                f"{int(bad[0, 0])}).  Every rank draws the full n x n matrix from its default CUDA generator: "
                                "seed all ranks alike (torch.cuda.manual_seed) before attack()")
-
-    def _iterate_noisy(self, t):
-        """One iteration with adjacency noise (--eps != 0, topology_attack.py:165, 474-478): MSELoss or KDE on one GPU,
-        MSELoss on tile-row shards.
-        noise stage -> node_pre -> M B1 -> node_mid -> M B2 -> node_head -> [KDE: c1 / c2 slab stage, c9 / c10]
-        -> pairs (c7, KDE: c2's M1 gradient) -> noisy terms (c1, c2, c6; KDE: the A_hat slab gradient) -> node_bwd2
-        -> M^T B3 -> node_bwd1 -> M^T B4 -> node_rho_diag -> noisy gradient -> fold (Adam, clamp, sums).
-        world > 1 adds the collectives of DESIGN.md 3.7: the draw's fingerprint, d between the two noise stages, each
-        product before its diagonal, dzhat, Y4 with eps_row, and after the fold the statistics and the bracket."""
-        st = N.stream_ptr()
-        n, tr0, tr1, mu, raw = self.n, self.tr0, self.tr1, ptr(self.mu), self.raw
-        noise = self._noise_fn(t)
-        if tuple(noise.shape) != (n, n):
-            raise ValueError(f"noise draw of shape {tuple(noise.shape)}, expected ({n}, {n})")
-        noise = noise.to(device=self.dev, dtype=torch.float32).contiguous()
-        if self.world == 1:
-            call("mcgra_noise_stage", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(noise), self.eps, ptr(self.Lt),
-                 ptr(self.Ut), ptr(self.mdiag), ptr(self.d), st)
-        else:
-            self._record_noise(noise, t)
-            self.d.zero_()
-            call("mcgra_noise_tiles", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(noise), self.eps, ptr(self.Lt),
-                 ptr(self.Ut), ptr(self.d), st)
-            self._allreduce(self.d)
-            call("mcgra_noise_diag", n, ptr(noise), self.eps, ptr(self.mdiag), ptr(self.d), st)
-        a = self._node_args(t)
-        ap = C.byref(a)
-        call("mcgra_node_pre", ap, st)
-        self._propagate_noisy(self.B1, 32, self.Y1, False)
-        call("mcgra_node_mid", ap, st)
-        self._propagate_noisy(self.B2, 32, self.Y2, False)
-        call("mcgra_node_head", ap, st)
-        kde = self.nn_mode == "kde"
-        if kde:
-            self._kde_stage_noisy(t)
-        if self.measure == N.M_KDE and (self.w9 != 0.0 or self.w10 != 0.0):
-            self._kde_nd_stage(t)
-        # c7 and the M1 side of KDE's c2 are functions of the symmetric decode M1 only: the existing pass, with no A_hat
-        # tiles (EAt = NULL): the noisy kernels form A_hat's part of eps_row themselves
-        if self.k7 != 0.0 or self.Ct is not None:
-            call("mcgra_pairs", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.zhat), ptr(self.r), self.k7, 0.0, None,
-                 ptr(self.Ct), ptr(self.dzhat), ptr(self.eps_row), self._acc_row(t).data_ptr(), ptr(self.pairs_ws), st)
-        na = N.NoisyArgs()
-        na.n, na.npad, na.tr0, na.tr1 = n, self.npad, tr0, tr1
-        na.tiles, na.mu, na.raw, na.noise, na.eps = ptr(self.xt), mu, raw, ptr(noise), self.eps
-        na.Lt, na.Ut, na.FLt, na.FUt = ptr(self.Lt), ptr(self.Ut), ptr(self.FLt), ptr(self.FUt)
-        na.zhat, na.r, na.rho, na.Wt = ptr(self.zhat), ptr(self.r), ptr(self.rho), ptr(self.Wt)
-        na.k1 = self.k1 if self.FLt is not None else 0.0
-        na.k2, na.k6 = self.k2, self.k6
-        na.acc, na.eps_row, na.dzhat, na.Gt = self._acc_row(t).data_ptr(), ptr(self.eps_row), ptr(self.dzhat), ptr(self.Gn)
-        if kde:
-            na.gslab, na.nb = ptr(self.kde["gA"]), self.kde["nb"]
-        nap = C.byref(na)
-        call("mcgra_noisy_terms", nap, st)
-        self._allreduce(self.dzhat)
-        call("mcgra_node_bwd2", ap, st)
-        self._propagate_noisy(self.B3, 32, self.Y3, True)
-        call("mcgra_node_bwd1", ap, st)
-        self._propagate_noisy(self.B4, 16, self.Y4, True, reduce=self.Y4e)      # Y4 and eps_row in one collective
-        call("mcgra_node_rho_diag", ap, ptr(self.mdiag), st)
-        call("mcgra_noisy_grad", nap, st)
-
-        f = N.FoldArgs()
-        f.n, f.npad, f.Wt, f.r, f.rho = n, self.npad, ptr(self.Wt0), ptr(self.r), ptr(self.rho0)
-        f.Ftiles, f.lseA, f.lseF, f.zhat = None, None, None, None
-        f.measure = N.M_NONE
-        f.k1, f.k6, f.k2 = 0.0, 0.0, 0.0
-        f.norm_coef = self.weight_sup * 0.001
-        f.lr, f.beta1, f.beta2, f.adam_eps = self.lr, 0.9, 0.999, 1e-8
-        f.step = t + 1
-        f.acc_prev = self._acc_row(t).data_ptr()
-        f.acc_next = self._acc_row(t + 1).data_ptr()
-        f.step_ptr = None
-        f.d_next = ptr(self.d_next)
-        f.store_clamped = 0 if self.proj_possible else 1
-        f.Wk = ptr(self.fold_ws)
-        f.plain_gd = 0
-        f.Gtiles = ptr(self.Gn)
-        call("mcgra_fold_adam", ptr(self.xt), ptr(self.mt), ptr(self.vt), tr0, tr1, mu, raw, C.byref(f),
-             ptr(self.minmax), st)
-        self.raw = 0 if self.proj_possible else 2
-        self.mu.zero_()
-        if self.world > 1:
-            import torch.distributed as dist
-            self._allreduce(self._acc_row(t + 1)[:16])
-            if self.proj_possible:
-                self._allreduce(self.minmax[0:1], dist.ReduceOp.MIN)
-                self._allreduce(self.minmax[1:2], dist.ReduceOp.MAX)
-        if self.proj_possible:
-            self._project(t)
-        self.step = t + 1     # (the degree of the next iteration comes from its own noise stage)
 
     def run(self, epochs, on_iter=None, use_graph="auto"):
         """`epochs` iterations.  In ring mode (small graphs) two consecutive iterations are captured once as a CUDA graph

@@ -218,10 +218,7 @@ class PGDAttack(BaseAttack):
             eng.dense = None
         if fa is None:
             fa = feature_adj.to(dev) if torch.is_tensor(feature_adj) else _dense(feature_adj, dev)
-        if world > 1:
-            self._finalize_sharded(eng, args, fa, labels_t, W2, b1, b2, Wl, bl, gather_x=kwargs.get("_gather_x", True))
-        else:
-            self._finalize(eng, args, fa, labels_t, W2, b1, b2, Wl, bl)
+        self._finalize(eng, args, fa, labels_t, W2, b1, b2, Wl, bl, gather_x=kwargs.get("_gather_x", True))
         _mark("finalize")
         return 0, 0, 0, 0
 
@@ -266,52 +263,67 @@ class PGDAttack(BaseAttack):
         n, d = Zp.shape
         call("mcgra_gram_accumulate", ptr(Zp), d, n, variant, ptr(rown), ptr(out), n, 0, n, N.stream_ptr())
 
-    def _finalize(self, eng, args, fa, labels_t, W2, b1, b2, Wl, bl):
-        """topology_attack.py:300-322."""
+    def _finalize(self, eng, args, fa, labels_t, W2, b1, b2, Wl, bl, gather_x=True):
+        """topology_attack.py:300-322.  The decoded parameter stays sharded by tile rows like the loop's (its two
+        propagations are all-reduced), and every rank evaluates the ensemble for ITS ROW BAND of the n x n result only
+        (`self.modified_adj` = rows [b0, b1), `self.modified_adj_rows`); with world > 1 `gather_modified_adj()` assembles
+        the full matrix and `metrics.auc_ap_from_edges_sharded` scores the bands in place.  One GPU owns all rows."""
+        import ctypes as _C
         st = N.stream_ptr()
-        n, T = eng.n, eng.T
-        dev = eng.dev
+        n, dev, world = eng.n, eng.dev, eng.world
         # em = embedding(X, adj_norm of the last iteration) == hidden state H2 of the normalised branch
         zf = torch.empty_like(eng.H2)
         call("mcgra_row_normalize", ptr(eng.H2), n, HID, 2.0, ptr(zf), st)
-        ntl = T * (T + 1) // 2
-        xf = torch.empty(ntl * N.TILE * N.TILE, dtype=torch.float32, device=dev)
-        call("mcgra_decode_to_tiles", ptr(zf), n, 0, T, ptr(xf), st)
-        P = n * (n - 1) // 2
-        packed = torch.empty(P, dtype=torch.float32, device=dev)
-        call("mcgra_tiles_to_tril", ptr(xf), n, 0, T, None, 1, ptr(packed), st)
-        self.adj_changes.data = packed                                   # :301
+        xf = torch.empty(max(eng.ntiles, 1) * N.TILE * N.TILE, dtype=torch.float32, device=dev)
+        call("mcgra_decode_to_tiles", ptr(zf), n, eng.tr0, eng.tr1, ptr(xf), st)
+        if gather_x or world == 1:      # the reference leaves the full packed vector in adj_changes.data (:301)
+            # (with world > 1 every rank writes its tile rows' entries and the shards are summed)
+            packed = (torch.empty if world == 1 else torch.zeros)(n * (n - 1) // 2, dtype=torch.float32, device=dev)
+            call("mcgra_tiles_to_tril", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(packed), st)
+            eng._allreduce(packed)
+            self.adj_changes.data = packed
         # embeddings / victim output on the raw decoded adjacency (:304-308): two propagations over xf
         Y = torch.zeros(n, HID, dtype=torch.float32, device=dev)
-        call("mcgra_propagate", ptr(xf), n, 0, T, None, 1, ptr(eng.S1), HID, ptr(Y), ptr(eng.prop_ws), st)
+        call("mcgra_propagate", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(eng.S1), HID, ptr(Y), ptr(eng.prop_ws), st)
+        eng._allreduce(Y)
         H1 = torch.relu(Y + b1)
         T2 = (H1 @ W2).contiguous()
         Y2 = torch.zeros(n, HID, dtype=torch.float32, device=dev)
-        call("mcgra_propagate", ptr(xf), n, 0, T, None, 1, ptr(T2), HID, ptr(Y2), ptr(eng.prop_ws), st)
+        call("mcgra_propagate", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(T2), HID, ptr(Y2), ptr(eng.prop_ws), st)
+        eng._allreduce(Y2)
         H2 = torch.relu(Y2 + b2)
         YA2 = F.log_softmax(H2 @ Wl.t() + bl, dim=1)
         # cur_adj = modified_adj (:302) + H_A1 + H_A2 + feature_adj + Y_A2 (+ ori_HA) (+ ori_YA) (+ label_adj), summed in
-        # this order in ONE pass over the n x n result (mcgra_ensemble)
+        # this order in ONE pass over the result band (mcgra_ensemble)
+        b0, b1_ = output_band(n, eng.rank, world)
         ea = N.EnsembleArgs()
         keep = []                                   # operands must outlive the launch
 
-        def gram(Z):
-            Zp, variant, rown = self._decode2_spec(Z.to(torch.float32))
+        def gram(Z, variant=None):
+            if variant is None:
+                Zp, variant, rown = self._decode2_spec(Z.to(torch.float32))
+            else:
+                Zp, rown = Z.to(torch.float32).contiguous(), None
             keep.append((Zp, rown))
             t = ea.t[ea.nterms]
             t.kind, t.d, t.variant, t.Z, t.rownorm = N.TERM_GRAM, int(Zp.shape[1]), variant, ptr(Zp), ptr(rown)
             ea.nterms += 1
 
-        def dense(M):
-            M = M.to(torch.float32).contiguous()
-            keep.append(M)
+        def dense(band):            # rows [b0, b1) of an n x n operand: the global row index lands in the band
+            band = band.to(device=dev, dtype=torch.float32).contiguous()
+            keep.append(band)
             t = ea.t[ea.nterms]
-            t.kind, t.dense = N.TERM_DENSE, ptr(M)
+            t.kind, t.dense = N.TERM_DENSE, band.data_ptr() - b0 * n * 4
             ea.nterms += 1
 
+        # modified_adj: one GPU reads the decoded tiles (clamped to [0, 1] in the kernel); the row bands of several
+        # GPUs need tiles of other ranks, so they re-expand relu(zf zf^T) with zero diagonal instead and free theirs
+        if world > 1:
+            xf = None
+            gram(zf, 4)
         gram(H1)
         gram(H2)
-        dense(fa)
+        dense(HostBands.of(fa).rows(b0, b1_, dev))
         gram(YA2)
         if args.useH_A:
             gram(self.H_A.detach().to(dev))
@@ -321,96 +333,22 @@ class PGDAttack(BaseAttack):
             path = "./saved_data/" + args.dataset + ".npy"
             lab = np.load(path, mmap_mode="r") if os.path.exists(path) else None                # :133-134
             if lab is not None and lab.shape == (n, n):      # (a stale file of another graph size is ignored)
-                dense(torch.from_numpy(np.ascontiguousarray(lab)).to(dev))
+                dense(torch.from_numpy(np.ascontiguousarray(lab[b0:b1_])))
             else:    # same matrix built from the labels (main.prepare, main.py:440-450)
                 t = ea.t[ea.nterms]
                 t.kind, t.labels = N.TERM_LABEL, ptr(labels_t)
                 ea.nterms += 1
-        out = torch.empty(n, n, dtype=torch.float32, device=dev)
-        import ctypes as _C
-        call("mcgra_ensemble", ptr(xf), n, _C.byref(ea), ptr(out), n, 0, n, st)
-        del xf, keep
-        self.modified_adj = out.detach()
-
-    def _finalize_sharded(self, eng, args, fa, labels_t, W2, b1, b2, Wl, bl, gather_x=True):
-        """topology_attack.py:300-322 with world > 1: the decoded parameter stays sharded by tile rows (its two
-        propagations are reduced across ranks like the loop's), and every rank evaluates the ensemble for ITS ROW BAND of
-        the n x n result only (`self.modified_adj` = rows [b0, b1), `self.modified_adj_rows`); `gather_modified_adj()`
-        assembles the full matrix, `metrics.auc_ap_from_edges_sharded` scores the bands in place."""
-        import ctypes as _C
-        import torch.distributed as dist
-        st = N.stream_ptr()
-        n, dev = eng.n, eng.dev
-        zf = torch.empty_like(eng.H2)
-        call("mcgra_row_normalize", ptr(eng.H2), n, HID, 2.0, ptr(zf), st)
-        xf = torch.zeros(max(eng.ntiles, 1) * N.TILE * N.TILE, dtype=torch.float32, device=dev)
-        call("mcgra_decode_to_tiles", ptr(zf), n, eng.tr0, eng.tr1, ptr(xf), st)
-        if gather_x:          # the reference leaves the full packed vector in adj_changes.data (:301)
-            packed = torch.zeros(n * (n - 1) // 2, dtype=torch.float32, device=dev)
-            call("mcgra_tiles_to_tril", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(packed), st)
-            dist.all_reduce(packed, group=eng.group)
-            self.adj_changes.data = packed
-        Y = torch.zeros(n, HID, dtype=torch.float32, device=dev)
-        call("mcgra_propagate", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(eng.S1), HID, ptr(Y), ptr(eng.prop_ws), st)
-        dist.all_reduce(Y, group=eng.group)
-        H1 = torch.relu(Y + b1)
-        T2 = (H1 @ W2).contiguous()
-        Y2 = torch.zeros(n, HID, dtype=torch.float32, device=dev)
-        call("mcgra_propagate", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(T2), HID, ptr(Y2), ptr(eng.prop_ws), st)
-        dist.all_reduce(Y2, group=eng.group)
-        del xf
-        H2 = torch.relu(Y2 + b2)
-        YA2 = F.log_softmax(H2 @ Wl.t() + bl, dim=1)
-        b0, b1_ = output_band(n, eng.rank, eng.world)
-        ea = N.EnsembleArgs()
-        keep = []
-
-        def gram(Z, variant_override=None):
-            if variant_override is None:
-                Zp, variant, rown = self._decode2_spec(Z.to(torch.float32))
-            else:
-                Zp, variant, rown = Z.to(torch.float32).contiguous(), variant_override, None
-            keep.append((Zp, rown))
-            t = ea.t[ea.nterms]
-            t.kind, t.d, t.variant, t.Z, t.rownorm = N.TERM_GRAM, int(Zp.shape[1]), variant, ptr(Zp), ptr(rown)
-            ea.nterms += 1
-
-        gram(zf, 4)                    # modified_adj = symmetric expansion of relu(zf zf^T), zero diagonal (:302)
-        gram(H1)
-        gram(H2)
-        fa_band = HostBands.of(fa).rows(b0, b1_, dev) if b1_ > b0 else torch.zeros(0, n, device=dev)
-        keep.append(fa_band)
-        t = ea.t[ea.nterms]
-        t.kind, t.dense = N.TERM_DENSE, fa_band.data_ptr() - b0 * n * 4        # global row index lands in the band
-        ea.nterms += 1
-        gram(YA2)
-        if args.useH_A:
-            gram(self.H_A.detach().to(dev))
-        if args.useY_A:
-            gram(self.Y_A.detach().to(dev))
-        if args.useY:
-            path = "./saved_data/" + args.dataset + ".npy"
-            lab_dense = None
-            if os.path.exists(path):
-                arr = np.load(path, mmap_mode="r")
-                if arr.shape == (n, n):
-                    lab_dense = torch.from_numpy(np.ascontiguousarray(arr[b0:b1_])).to(dev, torch.float32)
-            t = ea.t[ea.nterms]
-            if lab_dense is not None:
-                keep.append(lab_dense)
-                t.kind, t.dense = N.TERM_DENSE, lab_dense.data_ptr() - b0 * n * 4
-            else:
-                t.kind, t.labels = N.TERM_LABEL, ptr(labels_t)
-            ea.nterms += 1
         out = torch.empty(max(b1_ - b0, 0), n, dtype=torch.float32, device=dev)
         if b1_ > b0:
-            call("mcgra_ensemble", None, n, _C.byref(ea), out.data_ptr() - b0 * n * 4, n, b0, b1_, st)
-        torch.cuda.current_stream().synchronize()       # `keep` holds the operands until the launch has consumed them
+            call("mcgra_ensemble", ptr(xf), n, _C.byref(ea), out.data_ptr() - b0 * n * 4, n, b0, b1_, st)
+        if world > 1:
+            torch.cuda.current_stream().synchronize()       # `keep` holds the operands until the launch has consumed them
+        del xf, keep
         self.modified_adj = out.detach()
         self.modified_adj_rows = (b0, b1_)
 
     def gather_modified_adj(self):
-        """Full n x n result on every rank from the row bands of `_finalize_sharded` (world > 1); identity otherwise."""
+        """Full n x n result on every rank from the row bands of `_finalize` (world > 1); identity otherwise."""
         eng = self.engine
         if eng is None or eng.world == 1:
             return self.modified_adj

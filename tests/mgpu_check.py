@@ -1,4 +1,7 @@
-"""Run under torchrun with N >= 2 GPUs: the sharded attack must reproduce the single-GPU golden fixtures."""
+"""Run under torchrun: the sharded attack must reproduce the single-GPU golden fixtures.
+
+One rank per GPU over NCCL; with --gloo every rank runs on cuda:0 over gloo (the same code path and collectives on a
+one-GPU box)."""
 import os
 import sys
 
@@ -13,16 +16,17 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 
 
 def main():
-    local = int(os.environ.get("LOCAL_RANK", 0))
-    torch.cuda.set_device(local)
-    dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+    gloo = "--gloo" in sys.argv
+    dev = torch.device("cuda", 0 if gloo else int(os.environ.get("LOCAL_RANK", 0)))
+    torch.cuda.set_device(dev)
+    dist.init_process_group("gloo" if gloo else "nccl", **({} if gloo else {"device_id": dev}))
     import pgd_oracle as O
     from helpers import run_native_case, synthetic_case
     rank = dist.get_rank()
     ok = True
     for case in ["mse_A_n150", "mse_all_n150", "mse_budget_n150"]:
         d = np.load(os.path.join(ROOT, "tests", "golden", f"attack_{case}.npz"))
-        got = run_native_case(d, device=f"cuda:{local}")
+        got = run_native_case(d, device=dev)
         e_loss = float(np.max(np.abs(got["loss"] - d["loss"]) / np.abs(d["loss"])))
         e_x = float(np.max(np.abs(np.stack(got["x_iters"]) - d["x_iters"])))
         e_adj = float(np.max(np.abs(got["modified_adj"] - d["modified_adj"])))
@@ -34,7 +38,7 @@ def main():
     # sharded loss against the single-GPU golden, robust x comparison as in tests/test_gpu_attack.py
     for case in ["hsic_B_n150", "hsic_all_n90", "cka_n90", "dp_n90", "kl_all_n90", "kl_C_n150", "kde_n90", "kde_readme_n150"]:
         d = np.load(os.path.join(ROOT, "tests", "golden", f"attack_{case}.npz"))
-        got = run_native_case(d, device=f"cuda:{local}")
+        got = run_native_case(d, device=dev)
         e_loss = float(np.max(np.abs(got["loss"] - d["loss"]) / np.abs(d["loss"])))
         if case.startswith("kde"):
             # the reference's fp32 MutualInformation is itself 1e-4 .. 1e-3 from its fp64 value (tests/test_oracle_golden.py::
@@ -77,7 +81,7 @@ def main():
     hb = HostBands(n, bands)
     torch.from_numpy = lambda a: hb if a is d_b["feature_adj"] else torch_from(a)
     try:
-        got = run_native_case(d_b, device=f"cuda:{local}")
+        got = run_native_case(d_b, device=dev)
     finally:
         torch.from_numpy = torch_from
     e_loss = float(np.max(np.abs(got["loss"] - d["loss"]) / np.abs(d["loss"])))
@@ -96,7 +100,7 @@ def main():
                        mean_deg=8.0)
     prob, cfg = O.problem_from_npz(d)
     ref = O.attack(prob, cfg, 3, x0=torch.from_numpy(d["x0"]))
-    got = run_native_case(d, device=f"cuda:{local}")
+    got = run_native_case(d, device=dev)
     e_loss = float(np.max(np.abs(got["loss"] - np.array(ref["loss"])) / np.abs(np.array(ref["loss"]))))
     e_x = max(float(np.max(np.abs(a - b.numpy()))) for a, b in zip(got["x_iters"], ref["x_iters"]))
     if rank == 0:

@@ -254,23 +254,32 @@ def test_tcgen05_propagate_multi_tile(eng):
     assert np.max(np.abs(np.stack(a["x_iters"]) - np.stack(b["x_iters"]))) < 5e-5
 
 
-def test_two_gpu_sharded_attack_matches_golden():
-    """Tile-row sharding over 2 ranks (NCCL): same trajectories as the single-GPU golden fixtures (tests/mgpu_check.py
-    under torchrun).  Skipped on a 1-GPU box; `gpurun --gpus 2` runs it."""
+def _torchrun_mgpu_check(nproc, *extra):
     import socket
     import subprocess
     import sys
-    import torch
-    if torch.cuda.device_count() < 2:
-        pytest.skip("needs 2 GPUs")
     with socket.socket() as s:
         s.bind(("127.0.0.1", 0))
         port = s.getsockname()[1]
     here = os.path.dirname(os.path.abspath(__file__))
-    out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
-                          "--master-addr", "127.0.0.1", "--master-port", str(port), os.path.join(here, "mgpu_check.py")],
-                         capture_output=True, text=True, timeout=600)
+    out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(nproc),
+                          "--master-addr", "127.0.0.1", "--master-port", str(port), os.path.join(here, "mgpu_check.py"),
+                          *extra], capture_output=True, text=True, timeout=900)
+    print(out.stdout[-4000:])
     assert out.returncode == 0 and "MGPU_OK" in out.stdout, out.stdout[-2000:] + out.stderr[-2000:]
+
+
+def test_two_gpu_sharded_attack_matches_golden():
+    """Tile-row sharding over 2 ranks (NCCL): same trajectories as the single-GPU golden fixtures (tests/mgpu_check.py
+    under torchrun).  Skipped on a 1-GPU box."""
+    if torch.cuda.device_count() < 2:
+        pytest.skip("needs 2 GPUs")
+    _torchrun_mgpu_check(2)
+
+
+def test_sharded_attack_gloo_one_gpu():
+    """The same checks with 3 ranks sharing cuda:0 over gloo (noise-free sharded iteration and row-band finalisation)."""
+    _torchrun_mgpu_check(3, "--gloo")
 
 
 @pytest.mark.parametrize("case,epochs", [("mse_all_n150", 13), ("mse_budget_n150", 12)])
