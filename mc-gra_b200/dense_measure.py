@@ -13,7 +13,7 @@ With A = A_hat and M = M1 (both symmetric), Hc = H (HSIC, CKA) or I (DP), a = A 
     HSIC: c = k S;  DP: c = k sqrt(S);  CKA: c = k S / sqrt(h_xx h_yy)   (scalars on device: mcgra_dense_scalars).
 
 The dense gradients GA = dL/dA_hat and GM = dL/dM1 are handed to the tiled pipeline as tiles of G_ij + G_ji
-(`engine.Ft`, `engine.Ct`, measure code MCGRA_M_PRE) and the diagonal dL/dA_ii (`engine.Fdiag`).
+(`Ftiles`, `Ct`, measure code MCGRA_M_PRE) and the diagonal dL/dA_ii (`Fdiag`): terms.NNTerms.
 
 Multi-GPU: every GEMM is computed by row panels (rank g owns rows [g*rp, (g+1)*rp)) and the panels are all-gathered
 (NCCL); the operand images are rebuilt redundantly on every rank from the all-reduced tile triangle (O(n^2)).
@@ -24,6 +24,7 @@ import torch
 
 from . import _native as N
 from ._native import ACC, call, ptr
+from .terms import NNTerms
 
 TILE = N.TILE
 
@@ -47,19 +48,19 @@ class _Img:
         return C.byref(self.c)
 
 
-class DenseMeasure:
+class DenseMeasure(NNTerms):
     def __init__(self, eng, feature_adj, measure, k1c, k2c, sign):
-        """eng: PGDEngine (n, dev, rank, world, tiles, r, zhat, Ft/Ct/Fdiag); feature_adj: dense fp32 device tensor or
-        None (c1 inactive); k1c / k2c: fully scaled term weights (0 = off); sign: -1 for HSIC (:215-229)."""
-        self.eng = eng
-        self.n, self.dev = eng.n, eng.dev
-        self.measure = measure
+        """eng: PGDEngine (n, dev, rank, world, group, tile rows); feature_adj: dense fp32 device tensor or None (c1
+        inactive); k1c / k2c: fully scaled term weights (0 = off); sign: -1 for HSIC (:215-229)."""
+        self._gradient_tiles(eng, k2c != 0.0)
+        self.n, self.dev, self.rank, self.world, self.group = eng.n, eng.dev, eng.rank, eng.world, eng.group
+        self.kind = measure
         self.k1c, self.k2c, self.sign = float(k1c), float(k2c), float(sign)
         self.c1 = feature_adj is not None and k1c != 0.0
         self.c2 = k2c != 0.0
         self.cka = measure == N.M_CKA
         self.cen = 0.0 if measure == N.M_DP else 1.0
-        n, dev, world = self.n, self.dev, eng.world
+        n, dev, world = self.n, self.dev, self.world
         self.ld = _rup(n, 64)
         self.rp = (n + world - 1) // world                  # rows per rank panel
         self.row0 = min(n, eng.rank * self.rp)
@@ -106,10 +107,10 @@ class DenseMeasure:
         e.row0, e.row1 = self.row0, self.row1
         if self.row1 > self.row0:
             call("mcgra_gemm_nt", A.ref, B.ref, C.byref(e), N.stream_ptr(), tag=tag)
-        if self.eng.world > 1 and Cbuf is not None:
+        if self.world > 1 and Cbuf is not None:
             import torch.distributed as dist
-            panel = Cbuf[self.eng.rank * self.rp:(self.eng.rank + 1) * self.rp]
-            dist.all_gather_into_tensor(Cbuf, panel, group=self.eng.group)
+            panel = Cbuf[self.rank * self.rp:(self.rank + 1) * self.rp]
+            dist.all_gather_into_tensor(Cbuf, panel, group=self.group)
 
     def _image(self, src, img, transpose=0):
         call("mcgra_image_from_dense", ptr(src), self.n, self.n, self.ld, transpose, img.ref, ptr(self.ws), N.stream_ptr())
@@ -138,8 +139,7 @@ class DenseMeasure:
         self.imgK = _Img(n, n, self.dev)
         self._image(self.GA, self.imgK)
 
-    def _full_tiles(self):
-        eng = self.eng
+    def _full_tiles(self, eng):
         if eng.world == 1:
             return eng.xt
         import torch.distributed as dist
@@ -156,11 +156,11 @@ class DenseMeasure:
         call("mcgra_d2f", ptr(self.vd), self.n, 1.0, ptr(out32), st)
 
     # ------------------------------------------------------------------------------------------------
-    def step(self, t):
-        """Evaluate c1 / c2 and their gradients at the current parameter; fills eng.Ft / eng.Fdiag / eng.Ct."""
-        eng, n, st = self.eng, self.n, N.stream_ptr()
+    def step(self, eng, t, noisy):
+        """Evaluate c1 / c2 and their gradients at the current parameter; fills Ftiles / Fdiag / Ct."""
+        n, st = self.n, N.stream_ptr()
         cen = self.cen
-        tiles = self._full_tiles()
+        tiles = self._full_tiles(eng)
         self.scal.zero_()
         self.rsA.zero_()
         call("mcgra_image_ahat", ptr(tiles), n, ptr(eng.mu), eng.raw, ptr(eng.r), self.imgA.ref, ptr(self.rsA), st)
@@ -199,7 +199,7 @@ class DenseMeasure:
             dist.all_reduce(self.scal[:4], group=eng.group)
         if self.cka and self.c1:
             self.scal[4:5].copy_(self.hFF)
-        call("mcgra_dense_scalars", self.measure, ptr(self.scal), self.k1c if self.c1 else 0.0, self.k2c, self.sign,
+        call("mcgra_dense_scalars", self.kind, ptr(self.scal), self.k1c if self.c1 else 0.0, self.k2c, self.sign,
              eng._acc_row(t).data_ptr(), ptr(self.alpha), st)
 
         # ---- gradients: GA = dL/dA_hat, GM = dL/dM1 ----
@@ -227,9 +227,9 @@ class DenseMeasure:
                 self._gemm(self.imgM, self.imgSM, self.GM, alpha=1.0, alpha_dev=self._aptr(4), beta=1.0,
                            v=self.v4 if cen else None, coef=cen, tag="gemm_grad")
         call("mcgra_sym_to_tiles", ptr(self.GA), self.ld, n, eng.tr0, eng.tr1, 1.0,
-             self._aptr(0) if ga == "raw" else None, ptr(eng.Ft), ptr(eng.Fdiag), st)
+             self._aptr(0) if ga == "raw" else None, ptr(self.Ftiles), ptr(self.Fdiag), st)
         if gm:
-            call("mcgra_sym_to_tiles", ptr(self.GM), self.ld, n, eng.tr0, eng.tr1, 1.0, None, ptr(eng.Ct), None, st)
+            call("mcgra_sym_to_tiles", ptr(self.GM), self.ld, n, eng.tr0, eng.tr1, 1.0, None, ptr(self.Ct), None, st)
 
 
 def cross_frobenius(X, Y, center):

@@ -12,6 +12,8 @@ four products run on M's two orientation planes plus its diagonal (M^T for #3 an
 skipped and a noisy-terms pass before node_bwd2 carries c1/c2/c6 instead; KDE's n x n stage works on M's slabs; pairs
 keeps c7 and KDE's M1 gradient only; node_rho_diag and a noisy-gradient pass replace node_rho.
 
+The measure-specific stages and their buffers are the engine's terms objects `nn` (c1 / c2) and `nd` (c9 / c10).
+
 The adjacency estimate lives only as the tiled lower triangle (x', Adam m, v); n x n matrices are never
 materialised.  With world_size > 1 every rank owns a contiguous range of tile rows (equal tile counts) and the
 n x K partial results are summed with torch.distributed.all_reduce (NCCL over NVLink) between stages.
@@ -25,11 +27,12 @@ import torch
 
 from . import _native as N
 from ._native import ACC, call, ptr
+from .dense_measure import DenseMeasure
+from .terms import ElementwiseTerms, Kl2Terms, KdeNdTerms, KdeTerms, MomentNdTerms, NNTerms
 
 HID = N.HID
 TILE = N.TILE
 MEASURES = {"MSELoss": N.M_MSE, "KL": N.M_KL, "HSIC": N.M_HSIC, "CKA": N.M_CKA, "DP": N.M_DP, "KDE": N.M_KDE}
-KDE_NB = 8      # columns of an n x n operand that reach utils.MutualInformation's kernel (bin_j ~ j, values in [0, 1]; csrc/kde.cu)
 ALIGN = {"c1": 100, "c2": 1000, "c6": 10, "c7": 10, "c9": 1, "c10": 1}      # MC-GRA/utils.py:1100-1111
 
 
@@ -119,7 +122,6 @@ class PGDEngine:
                 now = _t.perf_counter()
                 print(f"[engine-setup rank {rank}] {name}: {now - _t0[0]:.3f}s", flush=True)
                 _t0[0] = now
-        self._tick = _tick
         dev = torch.device(device)
         self.dev, self.n, self.rank, self.world, self.group = dev, int(n), rank, world, group
         n = self.n
@@ -151,147 +153,46 @@ class PGDEngine:
             raise NotImplementedError(f"measure {measure!r}")
         self.measure = MEASURES[measure]
         w1, w2, _, _, _, w6, w7, _w8, w9, w10 = [float(w) for w in weights]
-        self.w = (w1, w2, w6, w7, w9, w10)
         self.weight_sup = float(weight_sup)
         self.lr = float(lr)
         nn2 = float(n) * float(n)
         sgn = -1.0 if measure == "HSIC" else 1.0
-        self.c1_active = False
-        self.Ft = self.Fdiag = self.lseF = self.Ct = None
-        self.k1 = self.k2 = 0.0
-        self.meas_nn = N.M_NONE       # measure code used by the element-wise n x n kernels
         self.idx = idx
-        fa = None
-        fa_row0 = 0           # first global row held by `fa` (row-band input: only this rank's tile rows are resident)
+        fa = None             # feature_adj on the device when c1 is on (topology_attack.py:212: off when it is constant)
+        banded = isinstance(feature_adj, HostBands)
+        fa_row0 = self.tr0 * TILE if banded else 0    # first global row held by `fa` (row-band input: this rank's rows)
         if w1 != 0 and feature_adj is not None:
-            if isinstance(feature_adj, HostBands):
-                fa_row0 = self.tr0 * TILE
+            if banded:
                 fa = feature_adj.rows(fa_row0, min(n, self.tr1 * TILE), dev)
                 mm = torch.stack([fa.max() if fa.numel() else torch.tensor(-math.inf, device=dev),
                                   -(fa.min() if fa.numel() else torch.tensor(math.inf, device=dev))])
-                if world > 1:
-                    import torch.distributed as dist
-                    dist.all_reduce(mm, op=dist.ReduceOp.MAX, group=group)
-                self.c1_active = bool(mm[0] != -mm[1])
+                self._allreduce(mm, torch.distributed.ReduceOp.MAX)
+                fa = fa if bool(mm[0] != -mm[1]) else None
             else:
                 fa = feature_adj.to(dev)
-                # topology_attack.py:212: the term is skipped when feature_adj is constant
-                if bool(fa.max() != fa.min()):
-                    self.c1_active = True
-                    fa = fa.to(torch.float32).contiguous()
+                fa = fa.to(torch.float32).contiguous() if bool(fa.max() != fa.min()) else None
+        c1 = fa is not None
         _tick("node constants + feature_adj rows on device")
-        native_nn = (self.measure == N.M_MSE) or (self.measure == N.M_KL and w2 == 0)
-        # Which engine evaluates the n x n terms c1 / c2:
-        #   "native": fused element-wise kernels (MSELoss; KL when only c1 is on)
-        #   "kl2"   : KL with c2 on -- row-softmax statistics of A_hat AND of the decode gram M1: three tile passes
-        #             (csrc/kl2.cu) that hand the element-wise gradient tiles to the pipeline (MCGRA_M_PRE)
-        #   "dense" : HSIC / CKA / DP -- n^3 contractions on tcgen05 (dense_measure.DenseMeasure, csrc/gemm.cu), gradient
-        #             tiles handed over the same way
-        #   "kde"   : utils.MutualInformation -- kernel-value slabs of the first KDE_NB columns, weighted second moments
-        #             and their closed-form gradient (csrc/kde.cu), gradient tiles handed over the same way
-        self.nn_mode = "native" if native_nn else ("kl2" if self.measure == N.M_KL else
-                                                   "kde" if self.measure == N.M_KDE else "dense")
-        if not (self.c1_active or w2 != 0):
-            self.nn_mode = "off"
-        self.w1, self.w2 = w1, w2
-        self.dense = None
-        ntl = max(self.ntiles, 1) * TILE * TILE
-        if self.nn_mode == "native":
-            if self.c1_active:
-                self.Ft = torch.zeros(ntl, **f32)
-                self.Fdiag = torch.zeros(n, **f32)
-                # (row-band input: the pointer is shifted so that the kernel's global row index lands in the band; the
-                #  mirrored entries live on other ranks, so the band is taken as is instead of (F_ij + F_ji) / 2)
-                call("mcgra_dense_to_tiles", fa.data_ptr() - fa_row0 * n * 4, n, n, self.tr0, self.tr1,
-                     0 if isinstance(feature_adj, HostBands) else 1, ptr(self.Ft), ptr(self.Fdiag), N.stream_ptr())
-                if self.eps != 0.0:
-                    # the noisy A_hat is not symmetric: c1 pairs A_hat_ij with F_ij and A_hat_ji with F_ji, so both
-                    # orientations of feature_adj are tiled as they are (F, then F^T).  Only the rows of this rank's tile
-                    # rows are read, so F^T is formed for that band alone (columns [r0, r1) of F): n x (r1 - r0) floats
-                    # instead of n x n, with the pointer shifted as for row-band input
-                    self.FLt = torch.zeros(ntl, **f32)
-                    self.FUt = torch.zeros(ntl, **f32)
-                    r0, r1 = self.tr0 * TILE, min(n, self.tr1 * TILE)
-                    if r1 > r0:
-                        call("mcgra_dense_to_tiles", ptr(fa), n, n, self.tr0, self.tr1, 0, ptr(self.FLt), None,
-                             N.stream_ptr())
-                        faT = fa[:, r0:r1].t().contiguous()
-                        call("mcgra_dense_to_tiles", faT.data_ptr() - r0 * n * 4, n, n, self.tr0, self.tr1, 0,
-                             ptr(self.FUt), None, N.stream_ptr())
-                        del faT
-                if world > 1:     # each rank wrote the diagonal of its own tile rows only
-                    self._allreduce(self.Fdiag)
-                self.meas_nn = self.measure
-                if self.measure == N.M_MSE:
-                    self.k1 = w1 * 1000 * ALIGN["c1"] / nn2
-                else:
-                    self.k1 = w1 * 1000 * ALIGN["c1"] / float(n)
-                    if isinstance(feature_adj, HostBands):
-                        self.lseF64 = torch.zeros(n, dtype=torch.float64, device=dev)
-                        self.lseF64[fa_row0:fa_row0 + fa.shape[0]] = torch.logsumexp(fa.double(), dim=1)
-                        self._allreduce(self.lseF64)
-                    else:
-                        self.lseF64 = torch.logsumexp(fa.double(), dim=1)
-                    self.lseF = self.lseF64.float().contiguous()
-            if w2 != 0:
-                self.k2 = w2 * 100 * ALIGN["c2"] / nn2
-        elif self.nn_mode in ("kl2", "dense", "kde"):
-            if isinstance(feature_adj, HostBands):
+        # c1 / c2: element-wise (MSELoss; KL with c2 off) or a stage handing over gradient tiles (terms.py)
+        k1c = w1 * 1000 * ALIGN["c1"] if c1 else 0.0
+        k2c = w2 * 100 * ALIGN["c2"]
+        self.k2 = k2c / nn2 if self.measure == N.M_MSE else 0.0      # MSELoss's c2: element-wise in pairs / node kernels
+        self.nn = NNTerms()
+        if self.measure == N.M_MSE or (self.measure == N.M_KL and w2 == 0):
+            if c1:
+                self.nn = ElementwiseTerms(self, fa, fa_row0, banded, self.measure, k1c)
+        elif c1 or w2 != 0:
+            if banded:
                 raise NotImplementedError("row-band feature_adj input is implemented for the element-wise measures (MSELoss, "
                                           "KL with w2 = 0); pass a full tensor for HSIC / CKA / DP / KL-c2")
-            # dL/dA_ij + dL/dA_ji and dL/dM1_ij + dL/dM1_ji.  The noisy path (KDE) hands the A_hat gradient to its own
-            # kernels as a column slab, and needs the M1 tiles only when c2 is on
-            self.Ft = torch.zeros(ntl, **f32) if self.eps == 0.0 else None
-            self.Ct = torch.zeros(ntl, **f32) if (self.eps == 0.0 or w2 != 0) else None
-            self.Fdiag = torch.zeros(n, **f32)     # dL/dA_ii
-            self.meas_nn = N.M_PRE
-            self.sgn = sgn
-            k1c = w1 * 1000 * ALIGN["c1"] if self.c1_active else 0.0
-            k2c = w2 * 100 * ALIGN["c2"]
-            if self.nn_mode == "dense":
-                from .dense_measure import DenseMeasure
-                self.dense = DenseMeasure(self, fa if self.c1_active else None, self.measure, k1c, k2c, sgn)
-            elif self.nn_mode == "kde":
-                nb = min(KDE_NB, n)
-                hi = max(float(fa.max()), 1.0) if self.c1_active else 1.0
-                if hi > 3.0:      # column j >= KDE_NB would no longer underflow: exp(-0.5 ((v - j) / 0.32)^2) > fp32 min
-                    raise NotImplementedError("KDE: feature_adj values above 3 reach bins beyond the kept columns")
-                self.kde = kd = dict(nb=nb, k1c=k1c, k2c=k2c, bin=float(n) / float(n - 1),
-                                     w=torch.full((n,), 1.0 / n, **f32),
-                                     slabA=torch.zeros(n, nb, **f32), slabM=torch.zeros(n, nb, **f32),
-                                     kvA=torch.zeros(n, nb, **f32), kvM=torch.zeros(n, nb, **f32),
-                                     gkvA=torch.zeros(n, nb, **f32), gkvM=torch.zeros(n, nb, **f32),
-                                     gA=torch.zeros(n, nb, **f32), gM=torch.zeros(n, nb, **f32),
-                                     mom=torch.zeros(2 * nb + 2 * nb * nb, dtype=torch.float64, device=dev),
-                                     gmom=torch.zeros(2 * nb + 2 * nb * nb, dtype=torch.float64, device=dev))
-                if self.c1_active and self.eps != 0.0:     # the noisy path's fp64 stage forms kernel values itself
-                    kd["slabF"] = fa[:, :nb].contiguous()
-                elif self.c1_active:
-                    kd["kvF"] = torch.zeros(n, nb, **f32)
-                    call("mcgra_kde_kv", ptr(fa), n, nb, n, kd["bin"], ptr(kd["kvF"]), N.stream_ptr())
+            if self.measure in (N.M_KL, N.M_KDE):
+                self.nn = (Kl2Terms if self.measure == N.M_KL else KdeTerms)(self, fa, k1c, k2c)
             else:
-                self.kl2 = k = N.Kl2Args()
-                self._kl2_keep = keep = {}
-                for name in ("seA", "seM", "lseA", "lseM", "klrow", "c1row"):
-                    keep[name] = torch.zeros(n, **f32)
-                    setattr(k, name, ptr(keep[name]))
-                if self.c1_active:
-                    keep["Ffeat"] = torch.zeros(ntl, **f32)
-                    keep["Fdiag_feat"] = torch.zeros(n, **f32)
-                    call("mcgra_dense_to_tiles", ptr(fa), n, n, self.tr0, self.tr1, 1, ptr(keep["Ffeat"]),
-                         ptr(keep["Fdiag_feat"]), N.stream_ptr())
-                    if world > 1:
-                        self._allreduce(keep["Fdiag_feat"])
-                    keep["lseF"] = torch.logsumexp(fa.double(), dim=1).float().contiguous()
-                    k.Ftiles, k.Fdiag_feat, k.lseF = ptr(keep["Ffeat"]), ptr(keep["Fdiag_feat"]), ptr(keep["lseF"])
-                k.tr0, k.tr1, k.n = self.tr0, self.tr1, n
-                k.EAt, k.Ct = ptr(self.Ft), ptr(self.Ct)
-                k.k1c, k.k2c = k1c, k2c
+                self.nn = DenseMeasure(self, fa, self.measure, k1c, k2c, sgn)
         del fa
         _tick("feature tiles / measure setup")
         self.k6 = -w6 * 100 * ALIGN["c6"] / nn2
         self.k7 = -w7 * ALIGN["c7"] / nn2
-        self.nd_native = self.measure in (N.M_MSE, N.M_KL)
         self.w9 = sgn * w9 * ALIGN["c9"]
         self.w10 = sgn * w10 * ALIGN["c10"]
         self.plain_gd = bool(plain_gd)
@@ -315,8 +216,9 @@ class PGDEngine:
         # counter and a tiny kernel appends the finished row to acc_hist, so that no launch carries a per-iteration host
         # scalar and two consecutive iterations can be replayed as ONE CUDA graph (run()).  Large graphs keep the direct
         # history rows: launch overhead is < 1 % there and per-kernel CUDA-event timing stays possible.
-        self.ring_mode = (GRAPH_MAX_N > 0 and n <= GRAPH_MAX_N and world == 1 and self.nn_mode in ("native", "off")
-                          and self.measure == N.M_MSE and self.eps == 0.0)
+        # (MSELoss has element-wise n x n terms or none)
+        self.ring_mode = (GRAPH_MAX_N > 0 and n <= GRAPH_MAX_N and world == 1 and self.measure == N.M_MSE
+                          and self.eps == 0.0)
         self.acc_ring = torch.zeros(2, N.ACC_N, dtype=torch.float64, device=dev)
         self.step_dev = torch.zeros(1, dtype=torch.int32, device=dev)
         self._graph = None
@@ -343,30 +245,9 @@ class PGDEngine:
         self.fold_ws = torch.empty(int(N.lib().mcgra_fold_ws_bytes(n)), dtype=torch.uint8, device=dev)
         self.prop_ws = torch.empty(int(N.lib().mcgra_propagate_ws_bytes(n, 32)), dtype=torch.uint8, device=dev)
         self.pairs_ws = torch.empty(int(N.lib().mcgra_pairs_ws_bytes(n)), dtype=torch.uint8, device=dev)
-        kl_native = self.meas_nn == N.M_KL and self.nn_mode == "native"
-        self.sumexp = z(n) if kl_native else None
-        self.lseA = z(n) if kl_native else None
-        self.dlse = z(n) if kl_native else None
-
-        if self.measure == N.M_KDE and (self.w9 != 0.0 or self.w10 != 0.0):
-            c = self.nclass
-            md = max(HID, c)
-            self.kde_nd = nd = dict(kvE=z(n, md), gkv=z(n, md), gV=z(n, md), p2=z(n, c),
-                                    mom=torch.zeros(2 * md + 2 * md * md, dtype=torch.float64, device=dev),
-                                    gmom=torch.zeros(2 * md + 2 * md * md, dtype=torch.float64, device=dev),
-                                    m=float(idx.numel()))
-            if self.w9 != 0.0:        # bins = linspace(0, 16, 16) (topology_attack.py:246-248)
-                nd["kvH"] = z(n, HID)
-                call("mcgra_kde_kv", ptr(self.HA), HID, HID, n, HID / (HID - 1.0), ptr(nd["kvH"]), N.stream_ptr())
-            if self.w10 != 0.0:       # bins = linspace(0, c, c) (:261-263)
-                nd["kvY"] = z(n, c)
-                nd["binc"] = c / (c - 1.0) if c > 1 else 0.0
-                call("mcgra_kde_kv", ptr(self.YA), c, c, n, nd["binc"], ptr(nd["kvY"]), N.stream_ptr())
-        elif not self.nd_native and (self.w9 != 0.0 or self.w10 != 0.0):
-            self.nd_p2 = z(n, self.nclass)
-            self.nd_mom = torch.zeros(int(N.lib().mcgra_nd_scratch_doubles(self.nclass)), dtype=torch.float64, device=dev)
-            self.nd_coef = z(int(N.lib().mcgra_nd_scratch_floats(self.nclass)))
-            self.nd_m = float(idx.numel())
+        self.nd = None         # c9 / c10 outside the node kernels (HSIC / CKA / DP, KDE)
+        if (self.w9 != 0.0 or self.w10 != 0.0) and self.measure not in (N.M_MSE, N.M_KL):
+            self.nd = KdeNdTerms(self) if self.measure == N.M_KDE else MomentNdTerms(self)
         _tick("state + node buffers")
         if self.eps != 0.0:
             # noisy path: the two orientations of M, its diagonal, the gradient tiles handed to the fold, and zero
@@ -374,8 +255,6 @@ class PGDEngine:
             self.Lt, self.Ut, self.Gn = (torch.zeros(nel, **f32) for _ in range(3))
             self.mdiag = z(n)
             self.Wt0, self.rho0 = z(128, self.npad), z(n)
-            if not self.c1_active or self.nn_mode != "native":
-                self.FLt = self.FUt = None
             # (the default draw captures no reference to the engine: a cycle would keep its device memory alive
             #  after attack() drops the engine)
             self._noise_fn = noise if noise is not None else (
@@ -392,6 +271,15 @@ class PGDEngine:
         if self.world > 1:
             import torch.distributed as dist
             dist.all_reduce(t, op=op or dist.ReduceOp.SUM, group=self.group)
+
+    def _dense_tiles(self, dense, symmetrize, row0=0):
+        """Tiles of this rank's tile rows of a dense n x n matrix (`row0`: first row of a band), all-reduced diagonal."""
+        tiles = torch.zeros(max(self.ntiles, 1) * TILE * TILE, dtype=torch.float32, device=self.dev)
+        diag = torch.zeros(self.n, dtype=torch.float32, device=self.dev)
+        call("mcgra_dense_to_tiles", dense.data_ptr() - row0 * self.n * 4, self.n, self.n, self.tr0, self.tr1, symmetrize,
+             ptr(tiles), ptr(diag), N.stream_ptr())
+        self._allreduce(diag)
+        return tiles, diag
 
     def set_parameter(self, x_packed):
         """Load a packed parameter vector (reference layout) -- zeros when None (topology_attack.py:77-78)."""
@@ -434,21 +322,19 @@ class PGDEngine:
         a.dQ2, a.demd, a.zhat, a.dzhat = ptr(self.dQ2), ptr(self.demd), ptr(self.zhat), ptr(self.dzhat)
         a.inv_norm, a.masks, a.masks2 = ptr(self.inv_norm), ptr(self.masks), ptr(self.masks2)
         a.eps_row, a.rho, a.Wt = ptr(self.eps_row), ptr(self.rho), ptr(self.Wt)
-        a.Fdiag = ptr(self.Fdiag)
+        a.Fdiag = ptr(self.nn.Fdiag)
         a.acc = self._acc_row(t).data_ptr()
         a.measure = self.measure                      # n x d terms c9 / c10 (node kernel handles MSE / KL)
-        a.measure_nn = self.meas_nn                   # n x n terms: diagonal part in node_rho
+        a.measure_nn = self.nn.measure                # n x n terms: diagonal part in node_rho
         a.weight_sup = self.weight_sup
-        a.k1 = self.k1 if (self.c1_active and self.nn_mode == "native") else 0.0
-        a.k2, a.k6, a.k7 = self.k2, self.k6, self.k7
-        a.w9, a.w10 = (self.w9, self.w10) if self.nd_native else (0.0, 0.0)
+        a.k1, a.k2, a.k6, a.k7 = self.nn.k1, self.k2, self.k6, self.k7
+        a.w9, a.w10 = (0.0, 0.0) if self.nd is not None else (self.w9, self.w10)
         a.npad = self.npad
         a.d_next, a.d_fill = ptr(self.d_next), (1.0 if self.rank == 0 else 0.0)
         a.acc_next = self._acc_row(t + 1).data_ptr()
         a.minmax = ptr(self.minmax)
-        a.lseA, a.lseF = ptr(self.lseA), ptr(self.lseF)
+        a.lseA, a.lseF, a.dlse = ptr(self.nn.lseA), ptr(self.nn.lseF), ptr(self.nn.dlse)
         a.em = ptr(self.em)
-        a.dlse = ptr(self.dlse)
         return a
 
     def forward_stages(self, t, noisy=False):
@@ -459,21 +345,15 @@ class PGDEngine:
         a = self._node_args(t)
         ap = C.byref(a)
         call("mcgra_node_pre", ap, st)
-        if not noisy and self.meas_nn == N.M_KL and self.nn_mode == "native":
-            self.sumexp.zero_()
-            call("mcgra_row_sumexp", ptr(self.xt), n, tr0, tr1, mu, raw, ptr(self.r), ptr(self.sumexp), st)
-            self._allreduce(self.sumexp)
-            lseA64 = torch.log(self.sumexp.double() + torch.exp((self.r * self.r).double()))   # + diagonal r_i^2
-            self.lseA.copy_(lseA64)
-            self.dlse.copy_(self.lseF64 - lseA64)
-        c1_native = self.c1_active and self.nn_mode == "native"
-        if not noisy and (c1_native or self.k6 != 0.0):
+        nn = self.nn
+        elem = nn.measure in (N.M_MSE, N.M_KL)       # c1 evaluated element-wise
+        if elem:
+            nn.step(self, t, noisy)
+        if not noisy and (elem or self.k6 != 0.0):
             e = N.ElemArgs()
-            e.r, e.Ftiles, e.lseA, e.lseF = ptr(self.r), (ptr(self.Ft) if c1_native else None), ptr(self.lseA), ptr(self.lseF)
-            e.measure = self.meas_nn if c1_native else N.M_NONE
-            e.k1, e.k6 = (self.k1 if c1_native else 0.0), self.k6
-            e.acc, e.eps_row = self._acc_row(t).data_ptr(), ptr(self.eps_row)
-            e.dlse = ptr(self.dlse)
+            e.r, e.lseA, e.lseF, e.dlse = ptr(self.r), ptr(nn.lseA), ptr(nn.lseF), ptr(nn.dlse)
+            e.Ftiles, e.measure, e.k1 = (ptr(nn.Ftiles), nn.measure, nn.k1) if elem else (None, N.M_NONE, 0.0)
+            e.k6, e.acc, e.eps_row = self.k6, self._acc_row(t).data_ptr(), ptr(self.eps_row)
             call("mcgra_elem_stats", ptr(self.xt), n, tr0, tr1, mu, raw, C.byref(e), st, tag="elem_stats")
         self._product(self.B1, 32, self.Y1, False, noisy)
         call("mcgra_node_mid", ap, st)
@@ -511,21 +391,15 @@ class PGDEngine:
         noise = self._noise_stage(t) if noisy else None
         a = self.forward_stages(t, noisy)
         ap = C.byref(a)
-        dense = self.nn_mode in ("dense", "kl2", "kde")      # gradient tiles handed over as MCGRA_M_PRE
-        if self.nn_mode == "dense":
-            self.dense.step(t)
-        elif self.nn_mode == "kl2":
-            self._kl2_stage(t)
-        elif self.nn_mode == "kde":
-            (self._kde_stage_noisy if noisy else self._kde_stage)(t)
-        if self.measure == N.M_KDE:
-            if self.w9 != 0.0 or self.w10 != 0.0:
-                self._kde_nd_stage(t)
-        elif not self.nd_native and (self.w9 != 0.0 or self.w10 != 0.0):
-            self._nd_stage(t)
+        nn = self.nn
+        pre = nn.measure == N.M_PRE          # gradient tiles handed over by the measure's own stage
+        if pre:
+            nn.step(self, t, noisy)
+        if self.nd is not None:
+            self.nd.step(self, t)
         # under noise c7 and the M1 side of KDE's c2 are functions of the symmetric decode M1 only: no A_hat tiles exist
-        # (Ft = None), the noisy kernels form A_hat's part of eps_row themselves
-        EAt, Ct = (self.Ft, self.Ct) if dense else (None, None)
+        # (Ftiles = None), the noisy kernels form A_hat's part of eps_row themselves
+        EAt, Ct = (nn.Ftiles, nn.Ct) if pre else (None, None)
         k2 = 0.0 if noisy else self.k2
         pairs = self.k7 != 0.0 or k2 != 0.0 or EAt is not None or Ct is not None
         if pairs:
@@ -537,13 +411,11 @@ class PGDEngine:
             na = N.NoisyArgs()
             na.n, na.npad, na.tr0, na.tr1 = n, self.npad, tr0, tr1
             na.tiles, na.mu, na.raw, na.noise, na.eps = ptr(self.xt), mu, raw, ptr(noise), self.eps
-            na.Lt, na.Ut, na.FLt, na.FUt = ptr(self.Lt), ptr(self.Ut), ptr(self.FLt), ptr(self.FUt)
+            na.Lt, na.Ut, na.FLt, na.FUt = ptr(self.Lt), ptr(self.Ut), ptr(nn.FLt), ptr(nn.FUt)
             na.zhat, na.r, na.rho, na.Wt = ptr(self.zhat), ptr(self.r), ptr(self.rho), ptr(self.Wt)
-            na.k1 = self.k1 if self.FLt is not None else 0.0
-            na.k2, na.k6 = self.k2, self.k6
+            na.k1, na.k2, na.k6 = nn.k1, self.k2, self.k6
             na.acc, na.eps_row, na.dzhat, na.Gt = self._acc_row(t).data_ptr(), ptr(self.eps_row), ptr(self.dzhat), ptr(self.Gn)
-            if self.nn_mode == "kde":
-                na.gslab, na.nb = ptr(self.kde["gA"]), self.kde["nb"]
+            na.gslab, na.nb = ptr(nn.gslab), nn.nb
             nap = C.byref(na)
             call("mcgra_noisy_terms", nap, st)
         if pairs or noisy:
@@ -597,13 +469,11 @@ class PGDEngine:
             f.measure = N.M_NONE
             f.Gtiles = ptr(self.Gn)
         else:
-            use_f = self.nn_mode in ("dense", "kl2", "kde") or (self.c1_active and self.nn_mode == "native")
             f.Wt, f.rho = ptr(self.Wt), ptr(self.rho)
-            f.Ftiles = ptr(self.Ft) if use_f else None
-            f.lseA, f.lseF = ptr(self.lseA), ptr(self.lseF)
+            f.Ftiles, f.measure = ptr(self.nn.Ftiles), self.nn.measure
+            f.lseA, f.lseF = ptr(self.nn.lseA), ptr(self.nn.lseF)
             f.zhat = ptr(self.zhat)
-            f.measure = self.meas_nn if use_f else N.M_NONE
-            f.k1, f.k6, f.k2 = (self.k1 if use_f else 0.0), self.k6, self.k2
+            f.k1, f.k6, f.k2 = self.nn.k1, self.k6, self.k2
             f.step_ptr = ptr(self.step_dev) if self.ring_mode else None
             f.plain_gd = 1 if self.plain_gd else 0
             f.Gtiles = ptr(self.Gt) if (self.smooth is not None and self.smooth_on) else None
@@ -719,13 +589,9 @@ class PGDEngine:
         X = X.detach().to(dev, torch.float32).contiguous()
         G = torch.zeros(n, n, **f32)
         call("mcgra_gram_accumulate", ptr(X), X.shape[1], n, 3, None, ptr(G), n, 0, n, st) if X.shape[1] <= 32 else G.copy_(X @ X.t())
-        ntl = max(self.ntiles, 1) * TILE * TILE
-        Gfeat = torch.zeros(ntl, **f32)
-        gdiag = torch.zeros(n, **f32)
-        call("mcgra_dense_to_tiles", ptr(G), n, n, self.tr0, self.tr1, 1, ptr(Gfeat), ptr(gdiag), st)
-        gdiag.copy_(G.diagonal())
+        Gfeat, gdiag = self._dense_tiles(G, 1)
         del G
-        self.Gt = torch.zeros(ntl, **f32)
+        self.Gt = torch.zeros(max(self.ntiles, 1) * TILE * TILE, **f32)
         self.smooth = dict(Gfeat=Gfeat, gdiag=gdiag, rt=torch.zeros(n, **f32), trow=torch.zeros(n, **f32), coef=float(coef))
 
     def _smooth_stage(self, t):
@@ -735,132 +601,6 @@ class PGDEngine:
         self._allreduce(sm["trow"])
         call("mcgra_smooth_node", self.n, ptr(self.d), ptr(sm["rt"]), ptr(sm["trow"]), ptr(sm["gdiag"]), sm["coef"],
              ptr(self.rho), self._acc_row(t).data_ptr() + 8 * ACC["C1D"], st)
-
-    def _kl2_stage(self, t):
-        """c1 / c2 under --measure KL with c2 on (topology_attack.py:212-229, 483-487): three tile passes, row
-        statistics all-reduced across ranks in between (csrc/kl2.cu)."""
-        st = N.stream_ptr()
-        k, keep = self.kl2, self._kl2_keep
-        k.tiles, k.mu, k.raw = ptr(self.xt), ptr(self.mu), self.raw
-        k.zhat, k.r = ptr(self.zhat), ptr(self.r)
-        kp = C.byref(k)
-        for name in ("seA", "seM", "klrow", "c1row"):
-            keep[name].zero_()
-        call("mcgra_kl2_pass", 0, kp, st)
-        self._allreduce(keep["seA"])
-        self._allreduce(keep["seM"])
-        call("mcgra_kl2_node", 0, kp, None, None, st)
-        call("mcgra_kl2_pass", 1, kp, st)
-        self._allreduce(keep["klrow"])
-        self._allreduce(keep["c1row"])
-        call("mcgra_kl2_node", 1, kp, ptr(self.Fdiag), self._acc_row(t).data_ptr(), st)
-        call("mcgra_kl2_pass", 2, kp, st)
-
-    def _kde_mi(self, X, dx, Y, dy, w, m, weight, slot, mom, gmom, gX, gY):
-        """weight * MutualInformation(X, Y) from the kernel-value matrices X [n x d], Y [n x d] (d = dx = dy): moments,
-        entropies + d/d moments, gradient w.r.t. the kernel values (gX / gY may be None)."""
-        st = N.stream_ptr()
-        n = self.n
-        mom.zero_()
-        call("mcgra_cross_moments", ptr(X), dx, ptr(Y), dy, ptr(w), n, ptr(mom), st)
-        call("mcgra_kde_scalars", ptr(mom), dx, m, weight, slot, ptr(gmom), st)
-        call("mcgra_cross_moments_bwd", ptr(X), dx, ptr(Y), dy, ptr(w), n, ptr(gmom), ptr(gX), ptr(gY), st)
-
-    def _kde_stage(self, t):
-        """c1 / c2 under --measure KDE (topology_attack.py:199-201, 212-229; utils.py:980-1053): only the first KDE_NB
-        columns of A_hat / M1 / feature_adj reach the Gaussian bins, so the n x n x n joint pdf is an NB x NB weighted
-        second moment.  Slabs are assembled from every rank's tile rows (one all-reduce), the scalar work is replicated."""
-        st = N.stream_ptr()
-        kd, n = self.kde, self.n
-        nb, bin_ = kd["nb"], kd["bin"]
-        acc = self._acc_row(t).data_ptr()
-        kd["slabA"].zero_()
-        call("mcgra_slab_ahat", ptr(self.xt), n, self.tr0, self.tr1, ptr(self.mu), self.raw, ptr(self.r), nb,
-             ptr(kd["slabA"]), st)
-        self._allreduce(kd["slabA"])
-        call("mcgra_kde_kv", ptr(kd["slabA"]), nb, nb, n, bin_, ptr(kd["kvA"]), st)
-        first = True
-        if self.c1_active:
-            self._kde_mi(kd["kvF"], nb, kd["kvA"], nb, kd["w"], float(n), kd["k1c"], acc + 8 * ACC["C1D"], kd["mom"],
-                         kd["gmom"], None, kd["gkvA"])
-            call("mcgra_kde_chain", ptr(kd["slabA"]), nb, ptr(kd["kvA"]), ptr(kd["gkvA"]), nb, n, bin_, ptr(kd["gA"]), 0, st)
-            first = False
-        if self.w2 != 0:
-            call("mcgra_slab_m1", ptr(self.zhat), n, nb, ptr(kd["slabM"]), st)
-            call("mcgra_kde_kv", ptr(kd["slabM"]), nb, nb, n, bin_, ptr(kd["kvM"]), st)
-            self._kde_mi(kd["kvA"], nb, kd["kvM"], nb, kd["w"], float(n), kd["k2c"], acc + 8 * ACC["C2D"], kd["mom"],
-                         kd["gmom"], kd["gkvA"], kd["gkvM"])
-            call("mcgra_kde_chain", ptr(kd["slabA"]), nb, ptr(kd["kvA"]), ptr(kd["gkvA"]), nb, n, bin_, ptr(kd["gA"]),
-                 0 if first else 1, st)
-            call("mcgra_kde_chain", ptr(kd["slabM"]), nb, ptr(kd["kvM"]), ptr(kd["gkvM"]), nb, n, bin_, ptr(kd["gM"]), 0, st)
-            call("mcgra_slab_to_tiles", ptr(kd["gM"]), n, self.tr0, self.tr1, nb, ptr(self.Ct), None, st)
-        call("mcgra_slab_to_tiles", ptr(kd["gA"]), n, self.tr0, self.tr1, nb, ptr(self.Ft), None, st)
-        self.Fdiag.zero_()
-        self.Fdiag[:nb].copy_(kd["gA"][:nb, :nb].diagonal())
-
-    def _kde_stage_noisy(self, t):
-        """c1 / c2 under --measure KDE with adjacency noise (single GPU).  The draw decorrelates A_hat from feature_adj
-        and from M1, so each MI is ~1e-6 of the entropies it is the difference of: the kernel values and the moments are
-        formed in fp64 from the value slabs (mcgra_kde_moments64 / _chain64).  A_hat is gathered from the noisy
-        estimate's planes; its gradient stays the slab kd["gA"] (mcgra_noisy_terms / mcgra_noisy_grad read it as gslab),
-        its diagonal goes to Fdiag, M1's gradient to the tiles Ct."""
-        st = N.stream_ptr()
-        kd, n = self.kde, self.n
-        nb, bin_, wt = kd["nb"], float(n) / float(n - 1), 1.0 / n
-        acc = self._acc_row(t).data_ptr()
-        kd["slabA"].zero_()
-        call("mcgra_slab_ahat_noisy", ptr(self.Lt), ptr(self.Ut), ptr(self.mdiag), n, self.tr0, self.tr1, ptr(self.r), nb,
-             ptr(kd["slabA"]), st)
-        kd["gA"].zero_()
-        pairs = []
-        if self.c1_active:
-            pairs.append((kd["slabF"], kd["slabA"], kd["k1c"], ACC["C1D"], None, kd["gA"]))
-        if self.w2 != 0:
-            call("mcgra_slab_m1", ptr(self.zhat), n, nb, ptr(kd["slabM"]), st)
-            kd["gM"].zero_()
-            pairs.append((kd["slabA"], kd["slabM"], kd["k2c"], ACC["C2D"], kd["gA"], kd["gM"]))
-        for X, Y, weight, slot, gX, gY in pairs:
-            kd["mom"].zero_()
-            call("mcgra_kde_moments64", ptr(X), ptr(Y), nb, n, bin_, wt, ptr(kd["mom"]), st)
-            call("mcgra_kde_scalars", ptr(kd["mom"]), nb, float(n), weight, acc + 8 * slot, ptr(kd["gmom"]), st)
-            call("mcgra_kde_chain64", ptr(X), ptr(Y), nb, n, bin_, wt, ptr(kd["gmom"]), ptr(gX), ptr(gY), st)
-        if self.w2 != 0:
-            call("mcgra_slab_to_tiles", ptr(kd["gM"]), n, self.tr0, self.tr1, nb, ptr(self.Ct), None, st)
-        self.Fdiag.zero_()
-        self.Fdiag[:nb].copy_(kd["gA"][:nb, :nb].diagonal())
-
-    def _kde_nd_stage(self, t):
-        """c9 / c10 under --measure KDE (topology_attack.py:246-269): bins = 16 / nclass; gradient added to demd."""
-        st = N.stream_ptr()
-        nd, n, c = self.kde_nd, self.n, self.nclass
-        acc = self._acc_row(t).data_ptr()
-        if self.w9 != 0.0:
-            b16 = HID / (HID - 1.0)
-            kv, gkv, gV = (nd[k].view(-1)[: n * HID].view(n, HID) for k in ("kvE", "gkv", "gV"))
-            call("mcgra_kde_kv", ptr(self.em), HID, HID, n, b16, ptr(kv), st)
-            self._kde_mi(nd["kvH"], HID, kv, HID, self.wmult, nd["m"], self.w9, acc + 8 * ACC["C9"], nd["mom"], nd["gmom"],
-                         None, gkv)
-            call("mcgra_kde_chain", ptr(self.em), HID, ptr(kv), ptr(gkv), HID, n, b16, ptr(gV), 0, st)
-            self.demd.add_(gV)
-        if self.w10 != 0.0:
-            kv, gkv, gV = (nd[k].view(-1)[: n * c].view(n, c) for k in ("kvE", "gkv", "gV"))
-            call("mcgra_softmax_rows", ptr(self.em), ptr(self.Wl), ptr(self.bl), n, c, ptr(nd["p2"]), st)
-            call("mcgra_kde_kv", ptr(nd["p2"]), c, c, n, nd["binc"], ptr(kv), st)
-            self._kde_mi(nd["kvY"], c, kv, c, self.wmult, nd["m"], self.w10, acc + 8 * ACC["C10"], nd["mom"], nd["gmom"],
-                         None, gkv)
-            call("mcgra_kde_chain", ptr(nd["p2"]), c, ptr(kv), ptr(gkv), c, n, nd["binc"], ptr(gV), 0, st)
-            call("mcgra_softmax_chain", ptr(gV), ptr(nd["p2"]), ptr(self.Wl), n, c, ptr(self.demd), st)
-
-    def _nd_stage(self, t):
-        """c9 / c10 under HSIC / CKA / DP (n x 16 and n x c operands): weighted second moments + closed-form gradient,
-        O(n d^2) (csrc/ndmeasure.cu); the gradient is added to the node-level demd buffer."""
-        a = N.NdArgs()
-        a.n, a.nclass, a.measure = self.n, self.nclass, self.measure
-        a.em, a.HA, a.YA, a.Wl, a.bl, a.wmult = (ptr(x) for x in (self.em, self.HA, self.YA, self.Wl, self.bl, self.wmult))
-        a.m, a.w9, a.w10 = self.nd_m, self.w9, self.w10
-        a.p2, a.mom, a.coef, a.demd = ptr(self.nd_p2), ptr(self.nd_mom), ptr(self.nd_coef), ptr(self.demd)
-        a.acc = self._acc_row(t).data_ptr()
-        call("mcgra_nd_measure", C.byref(a), N.stream_ptr())
 
     # ------------------------------------------------------------------------------------------------
     def losses(self):

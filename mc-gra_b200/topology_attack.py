@@ -22,6 +22,7 @@ from torch.nn.parameter import Parameter
 from . import _native as N
 from ._native import call, ptr
 from .base_attack import BaseAttack
+from .dense_measure import DenseMeasure
 from .engine import HID, HostBands, PGDEngine, check_noise_supported, output_band
 
 Align_Parameter_Cora = {"c1": 100, "c2": 1000, "c3": 100, "c4": 10, "c5": 10, "c6": 10, "c7": 10, "c8": 0.01,
@@ -199,7 +200,7 @@ class PGDAttack(BaseAttack):
                                 eps=eps, noise=kwargs.get("_noise"))
         eng = self.engine
         fa_on_host = not isinstance(feature_adj, HostBands) and not (torch.is_tensor(feature_adj) and feature_adj.is_cuda)
-        if eng.nn_mode == "dense" and fa_on_host:
+        if isinstance(eng.nn, DenseMeasure) and fa_on_host:
             fa = None          # the contraction stage keeps its own constant image; the dense copy returns for the ensemble
         _mark("engine_setup")
         self._trace = []
@@ -214,8 +215,8 @@ class PGDAttack(BaseAttack):
         if int(epochs) == 0:
             eng.forward_stages(0)
         _mark("iterations")
-        if eng.dense is not None:          # n x n operand images / gradient buffers are not needed past the loop
-            eng.dense = None
+        if isinstance(eng.nn, DenseMeasure):     # n x n operand images / gradient buffers are not needed past the loop
+            eng.nn = None
         if fa is None:
             fa = feature_adj.to(dev) if torch.is_tensor(feature_adj) else _dense(feature_adj, dev)
         self._finalize(eng, args, fa, labels_t, W2, b1, b2, Wl, bl, gather_x=kwargs.get("_gather_x", True))

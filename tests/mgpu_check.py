@@ -59,31 +59,29 @@ def main():
     # single-process values of the full matrix
     from mcgra_b200 import metrics
     from mcgra_b200.engine import HostBands, TILE, output_band, shard_tile_rows
-    import helpers
+    world = dist.get_world_size()
+
+    def run_row_bands(d):
+        n = int(d["labels"].shape[0])
+        T = (n + TILE - 1) // TILE
+        tr0, tr1 = shard_tile_rows(T, world)[rank]
+        fa_full = torch.from_numpy(d["feature_adj"])
+        bands = {}
+        for r0, r1 in {(tr0 * TILE, min(n, tr1 * TILE)), output_band(n, rank, world)}:
+            if r1 > r0:
+                bands[(r0, r1)] = fa_full[r0:r1].clone().pin_memory()
+        # run_native_case does torch.from_numpy(d["feature_adj"]): hand it the band object instead
+        hb = HostBands(n, bands)
+        torch_from = torch.from_numpy
+        torch.from_numpy = lambda a: hb if a is d["feature_adj"] else torch_from(a)
+        try:
+            return run_native_case(d, device=dev)
+        finally:
+            torch.from_numpy = torch_from
+
     d = dict(np.load(os.path.join(ROOT, "tests", "golden", "attack_mse_all_n150.npz")))
     n = int(d["labels"].shape[0])
-    world = dist.get_world_size()
-    T = (n + TILE - 1) // TILE
-    tr0, tr1 = shard_tile_rows(T, world)[rank]
-    fa_full = torch.from_numpy(d["feature_adj"])
-    bands = {}
-    for r0, r1 in {(tr0 * TILE, min(n, tr1 * TILE)), output_band(n, rank, world)}:
-        if r1 > r0:
-            bands[(r0, r1)] = fa_full[r0:r1].clone().pin_memory()
-    orig_from_numpy = torch.from_numpy
-    d_b = dict(d)
-    d_b["feature_adj"] = d["feature_adj"]
-    _rn = helpers.run_native_case
-
-    class _FA:       # run_native_case does torch.from_numpy(d["feature_adj"]): hand it the band object instead
-        pass
-    torch_from = torch.from_numpy
-    hb = HostBands(n, bands)
-    torch.from_numpy = lambda a: hb if a is d_b["feature_adj"] else torch_from(a)
-    try:
-        got = run_native_case(d_b, device=dev)
-    finally:
-        torch.from_numpy = torch_from
+    got = run_row_bands(d)
     e_loss = float(np.max(np.abs(got["loss"] - d["loss"]) / np.abs(d["loss"])))
     e_adj = float(np.max(np.abs(got["modified_adj"] - d["modified_adj"])))
     mdl = got["model"]
@@ -105,6 +103,18 @@ def main():
     e_x = max(float(np.max(np.abs(a - b.numpy()))) for a, b in zip(got["x_iters"], ref["x_iters"]))
     if rank == 0:
         print(f"[mgpu] n=900 budget-active vs oracle: rel loss err {e_loss:.2e} max|dx| {e_x:.2e}")
+    ok &= e_loss < 1e-4 and e_x < 2e-4
+    # KL with c2 off on row-band feature_adj against the oracle: the element-wise KL path, whose row log-sum-exp of
+    # feature_adj is assembled from the rank's band and all-reduced
+    d = synthetic_case(900, 40, 5, measure="KL", weights={1: 0.5, 6: 2.0, 7: 3.0, 9: 1.5, 10: 50.0}, epochs=3,
+                       mean_deg=8.0)
+    prob, cfg = O.problem_from_npz(d)
+    ref = O.attack(prob, cfg, 3, x0=torch.from_numpy(d["x0"]))
+    got = run_row_bands(d)
+    e_loss = float(np.max(np.abs(got["loss"] - np.array(ref["loss"])) / np.abs(np.array(ref["loss"]))))
+    e_x = max(float(np.max(np.abs(a - b.numpy()))) for a, b in zip(got["x_iters"], ref["x_iters"]))
+    if rank == 0:
+        print(f"[mgpu] n=900 KL c1-only, row-band feature_adj, vs oracle: rel loss err {e_loss:.2e} max|dx| {e_x:.2e}")
     ok &= e_loss < 1e-4 and e_x < 2e-4
     dist.barrier()
     dist.destroy_process_group()

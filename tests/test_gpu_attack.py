@@ -91,13 +91,14 @@ def test_ranking_of_tie_free_scores(case):
     assert np.array_equal(order[tie_free], ref_order[tie_free])
 
 
-@pytest.mark.parametrize("n,weights,density", [
-    (700, {1: 0.01, 6: 10, 7: 10, 9: 10, 10: 1000}, 1e7),           # Profile A, 6 tile rows, J-runs of 4 + 2
-    (1100, {1: 0.5, 2: 0.3, 6: 2.0, 7: 3.0, 9: 1.5, 10: 50.0}, 1.0),  # all MSE terms, budget binds (bisection)
+@pytest.mark.parametrize("n,measure,weights,density", [
+    (700, "MSELoss", {1: 0.01, 6: 10, 7: 10, 9: 10, 10: 1000}, 1e7),           # Profile A, 6 tile rows, J-runs of 4 + 2
+    (1100, "MSELoss", {1: 0.5, 2: 0.3, 6: 2.0, 7: 3.0, 9: 1.5, 10: 50.0}, 1.0),  # all MSE terms, budget binds (bisection)
+    (700, "KL", {1: 0.5, 6: 2.0, 7: 3.0, 9: 1.5, 10: 50.0}, 1e7),             # element-wise KL (c2 off)
 ])
-def test_multi_tile_matches_oracle(n, weights, density):
+def test_multi_tile_matches_oracle(n, measure, weights, density):
     from helpers import synthetic_case
-    d = synthetic_case(n, 40, 5, weights=weights, epochs=3, density=density, mean_deg=8.0)
+    d = synthetic_case(n, 40, 5, measure=measure, weights=weights, epochs=3, density=density, mean_deg=8.0)
     prob, cfg = O.problem_from_npz(d)
     ref = O.attack(prob, cfg, 3, x0=torch.from_numpy(d["x0"]))
     got = run_native_case(d)

@@ -122,7 +122,7 @@ def main():
                 P = n * (n - 1) // 2
                 kt, kc = kernels(atk)
                 eng = atk.engine
-                by = noisy_bytes(P, n, getattr(eng, "FLt", None) is not None, eng.kde["nb"] if eng.nn_mode == "kde" else 0)
+                by = noisy_bytes(P, n, eng.nn.FLt is not None, eng.nn.nb)
                 r["kernels"] = {k: {"ms": kt[k], "launches_per_iter": kc[k],
                                     **({"hbm_frac": by[k] / (kt[k] * 1e-3) / (HBM_PEAK_GBS * 1e9)} if k in by else {})}
                                 for k in kt}
