@@ -161,16 +161,19 @@ class PGDEngine:
         fa = None             # feature_adj on the device when c1 is on (topology_attack.py:212: off when it is constant)
         banded = isinstance(feature_adj, HostBands)
         fa_row0 = self.tr0 * TILE if banded else 0    # first global row held by `fa` (row-band input: this rank's rows)
+        fmax = None           # max of all of feature_adj (KDE's range check)
         if w1 != 0 and feature_adj is not None:
             if banded:
                 fa = feature_adj.rows(fa_row0, min(n, self.tr1 * TILE), dev)
                 mm = torch.stack([fa.max() if fa.numel() else torch.tensor(-math.inf, device=dev),
                                   -(fa.min() if fa.numel() else torch.tensor(math.inf, device=dev))])
                 self._allreduce(mm, torch.distributed.ReduceOp.MAX)
+                fmax = mm[0]
                 fa = fa if bool(mm[0] != -mm[1]) else None
             else:
                 fa = feature_adj.to(dev)
-                fa = fa.to(torch.float32).contiguous() if bool(fa.max() != fa.min()) else None
+                fmax = fa.max()
+                fa = fa.to(torch.float32).contiguous() if bool(fmax != fa.min()) else None
         c1 = fa is not None
         _tick("node constants + feature_adj rows on device")
         # c1 / c2: element-wise (MSELoss; KL with c2 off) or a stage handing over gradient tiles (terms.py)
@@ -182,13 +185,12 @@ class PGDEngine:
             if c1:
                 self.nn = ElementwiseTerms(self, fa, fa_row0, banded, self.measure, k1c)
         elif c1 or w2 != 0:
-            if banded:
-                raise NotImplementedError("row-band feature_adj input is implemented for the element-wise measures (MSELoss, "
-                                          "KL with w2 = 0); pass a full tensor for HSIC / CKA / DP / KL-c2")
-            if self.measure in (N.M_KL, N.M_KDE):
-                self.nn = (Kl2Terms if self.measure == N.M_KL else KdeTerms)(self, fa, k1c, k2c)
-            else:
-                self.nn = DenseMeasure(self, fa, self.measure, k1c, k2c, sgn)
+            if self.measure == N.M_KL:
+                self.nn = Kl2Terms(self, fa, fa_row0, banded, k1c, k2c)
+            elif self.measure == N.M_KDE:
+                self.nn = KdeTerms(self, fa, fa_row0, banded, fmax, k1c, k2c)
+            else:       # Kf = Hc F F^T Hc needs all of F: row bands are assembled on the device for the setup only
+                self.nn = DenseMeasure(self, self._full_rows(fa, fa_row0, banded), self.measure, k1c, k2c, sgn)
         del fa
         _tick("feature tiles / measure setup")
         self.k6 = -w6 * 100 * ALIGN["c6"] / nn2
@@ -280,6 +282,18 @@ class PGDEngine:
              ptr(tiles), ptr(diag), N.stream_ptr())
         self._allreduce(diag)
         return tiles, diag
+
+    def _full_rows(self, fa, row0, banded, cols=None):
+        """Columns [0, cols) of all n rows of feature_adj (None: c1 off).  Full input: a view of `fa`.  Row bands (`fa`:
+        rows [row0, ...) of disjoint bands that cover [0, n)): placed in a zero-filled buffer summed across the ranks,
+        which is exact because every entry has exactly one non-zero contributor."""
+        if fa is None or not banded:
+            return fa if fa is None else fa[:, :cols]
+        cols = self.n if cols is None else cols
+        full = torch.zeros(self.n, cols, dtype=torch.float32, device=self.dev)
+        full[row0:row0 + fa.shape[0]] = fa[:, :cols]
+        self._allreduce(full)
+        return full
 
     def set_parameter(self, x_packed):
         """Load a packed parameter vector (reference layout) -- zeros when None (topology_attack.py:77-78)."""

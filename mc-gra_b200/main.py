@@ -4,7 +4,10 @@
            --useH_A --useY_A --useY --measure=MSELoss            (MC-GRA/README.md:29)
 
 Data: `./dataset/<name>.npz` in the reference's npz layout (adj_data/indices/indptr/shape, attr_*, labels), or
-`--dataset synthetic:<n>:<f>:<c>`.  Only `--mode evaluate` and `--arch gcn` are on the north-star path."""
+`--dataset synthetic:<n>:<f>:<c>`.  Only `--mode evaluate` and `--arch gcn` are on the north-star path.
+
+Several GPUs: `torchrun --nproc-per-node N -m mcgra_b200.main ...` (WORLD_SIZE > 1) joins a process group and runs the
+tile-row sharded attack; every rank forms only the row bands of feature_adj it touches and of the result it owns."""
 import argparse
 import os
 import random
@@ -15,7 +18,8 @@ import scipy.sparse as sp
 import torch
 
 from . import synth
-from .metrics import metric_pool, precision_recall_at_k
+from .engine import TILE, HostBands, output_band, shard_tile_rows
+from .metrics import metric_pool, metric_pool_sharded, precision_recall_at_k
 from .models.gcn import GCN, embedding_GCN
 from .topology_attack import PGDAttack
 
@@ -55,6 +59,9 @@ def build_parser():
     p.add_argument('--topk', type=int, default=0,
                    help="K > 0: write the K highest-scoring pairs to results/<log_name>.topk.npz and log precision / "
                         "recall against the true edges")
+    p.add_argument("--dist_backend", type=str, default="nccl", choices=["nccl", "gloo"],
+                   help="process-group backend under torchrun (WORLD_SIZE > 1): nccl, one GPU per rank (LOCAL_RANK); "
+                        "gloo, every rank on cuda:0")
     return p
 
 
@@ -84,23 +91,73 @@ def load_graph(name, root='./dataset'):
     return adj.astype(np.float32), feats, labels
 
 
-def dot_product_decode(Z, dataset):
-    """main.dot_product_decode (main.py:44-55) -> feature_adj."""
-    eye = torch.eye(Z.shape[0], device=Z.device)
+def eye_rows(n, r0, r1, device=None):
+    """Rows [r0, r1) of the n x n identity."""
+    e = torch.zeros(r1 - r0, n, device=device)
+    i = torch.arange(r1 - r0, device=device)
+    e[i, r0 + i] = 1.0
+    return e
+
+
+def dot_product_decode(Z, dataset, rows=None):
+    """main.dot_product_decode (main.py:44-55) -> feature_adj, or only its rows [r0, r1) (`rows`), formed from Z alone."""
+    n = Z.shape[0]
+    r0, r1 = rows if rows is not None else (0, n)
+    eye = eye_rows(n, r0, r1, Z.device)
     if dataset in ('cora', 'citeseer', 'AIDS') or dataset.startswith("synthetic"):
-        return torch.sigmoid(torch.relu(Z @ Z.t() - eye))
+        return torch.sigmoid(torch.relu(Z[r0:r1] @ Z.t() - eye))
     Zn = torch.nn.functional.normalize(Z, p=2, dim=1)
-    return torch.relu(Zn @ Zn.t() - eye)
+    return torch.relu(Zn[r0:r1] @ Zn.t() - eye)
+
+
+def feature_adj_bands(Z, dataset, rank, world, nofeature=False):
+    """feature_adj as the row bands one rank of `world` touches -- its tile-row shard (engine.shard_tile_rows) for the
+    loop and its band of the result (engine.output_band) for the ensemble -- each formed on Z's device from Z alone
+    (identity rows with --nofeature): no rank holds the n x n matrix."""
+    n = Z.shape[0]
+    tr0, tr1 = shard_tile_rows((n + TILE - 1) // TILE, world)[rank]
+    bands = {}
+    for r0, r1 in {(tr0 * TILE, min(n, tr1 * TILE)), output_band(n, rank, world)}:
+        if r1 > r0:
+            bands[(r0, r1)] = eye_rows(n, r0, r1, Z.device) if nofeature else dot_product_decode(Z, dataset, (r0, r1))
+    return HostBands(n, bands)
+
+
+def _share_victim(victim, device):
+    """Rank 0's trained victim and random-number state on every rank, so that all ranks attack the same victim and
+    continue the same random streams (the draws of --eps) whatever the run-to-run variation of training."""
+    import torch.distributed as dist
+    with torch.no_grad():
+        for t in victim.state_dict().values():
+            dist.broadcast(t, 0)
+    for get, put in ((torch.get_rng_state, torch.set_rng_state), (torch.cuda.get_rng_state, torch.cuda.set_rng_state)):
+        state = get().to(device)
+        dist.broadcast(state, 0)
+        put(state.cpu())
 
 
 def main(argv=None):
     args = build_parser().parse_args(argv)
     topk = vars(args).pop("topk")         # not part of the reference's parameter line in the log
+    backend = vars(args).pop("dist_backend")
     if topk < 0:
         raise ValueError(f"--topk {topk}: K must be >= 0 (0 = off)")
     if args.arch != "gcn" or args.mode != "evaluate":
         raise NotImplementedError("only --arch gcn --mode evaluate are on the B200 path (SURVEY.md 2)")
-    device = torch.device("cuda:0")
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    if world == 1:
+        return _run(args, topk, torch.device("cuda:0"), 0, 1)
+    import torch.distributed as dist
+    device = torch.device("cuda", 0 if backend == "gloo" else int(os.environ.get("LOCAL_RANK", "0")))
+    torch.cuda.set_device(device)
+    dist.init_process_group(backend, **({"device_id": device} if backend == "nccl" else {}))
+    try:
+        return _run(args, topk, device, dist.get_rank(), dist.get_world_size())
+    finally:
+        dist.destroy_process_group()
+
+
+def _run(args, topk, device, rank, world):
     np.random.seed(args.seed); random.seed(args.seed); torch.manual_seed(args.seed); torch.cuda.manual_seed(args.seed)
     adj_sp, feats, labels = load_graph(args.dataset)
     if args.dataset.startswith("synthetic"):
@@ -119,14 +176,20 @@ def main(argv=None):
                                   torch.from_numpy(coo.data.astype(np.float32)), (n, n)).coalesce().to(device)
     features = torch.from_numpy(feats)
     labels_t = torch.from_numpy(labels)
-    feature_adj = dot_product_decode(features.to(device), args.dataset)
-    if args.nofeature:
-        feature_adj = torch.eye(n, device=device)
+    if world > 1 and args.eps == 0:
+        feature_adj = feature_adj_bands(features.to(device), args.dataset, rank, world, args.nofeature)
+    else:       # (--eps != 0 needs feature_adj as a full tensor, also on several GPUs)
+        feature_adj = dot_product_decode(features.to(device), args.dataset)
+        if args.nofeature:
+            feature_adj = torch.eye(n, device=device)
     victim = GCN(nfeat=features.shape[1], nclass=int(labels.max()) + 1, nhid=16, nlayer=args.nlayers, dropout=0.5,
                  weight_decay=5e-4, device=device).to(device)
     for layer in victim.gc:
         layer.to(device)
-    victim.fit(features, adj, labels_t, idx_train, idx_val)
+    if rank == 0:
+        victim.fit(features, adj, labels_t, idx_train, idx_val)
+    if world > 1:
+        _share_victim(victim, device)
     embedding = embedding_GCN(nfeat=features.shape[1], nhid=16, nlayer=args.nlayers, device=device)
     embedding.gc = deepcopy(victim.gc)
     victim.eval(); embedding.eval()
@@ -138,16 +201,31 @@ def main(argv=None):
     model.attack(args, None, 10 ** args.lr, 0, args.weight_sup, weight_param, feature_adj, 0, 0, 0, idx_train, idx_val,
                  idx_test, adj, features, torch.zeros(1), labels_t, idx_attack, num_edges, 0, epochs=args.epochs)
     inference_adj = model.modified_adj
-    auc = metric_pool(adj, inference_adj, idx_attack, None)
-    auc_train = metric_pool(adj, inference_adj, idx_train, None)
-    auc_all = metric_pool(adj, inference_adj, np.arange(n), None, True)
-    os.makedirs("./results/", exist_ok=True)
-    with open(os.path.join("./results", args.log_name), "a") as f:
-        f.write(f"current parameter: {args}\n")
-        f.write(f"In attack graph: AUC={auc}\tIn train graph: AUC={auc_train}\tIn Whole Graph: AUC={auc_all}\n")
-        f.write(f"current density: {float(inference_adj.mean())}\n")
+    if world == 1:
+        auc = metric_pool(adj, inference_adj, idx_attack, None)
+        auc_train = metric_pool(adj, inference_adj, idx_train, None)
+        auc_all = metric_pool(adj, inference_adj, np.arange(n), None, True)
+        density = float(inference_adj.mean())
+    else:       # every rank holds its row band of the result (model.modified_adj_rows)
+        import torch.distributed as dist
+        row0 = model.modified_adj_rows[0]
+        auc, auc_train, auc_all = (metric_pool_sharded(adj, inference_adj, row0, n, ix)
+                                   for ix in (idx_attack, idx_train, np.arange(n)))
+        total = inference_adj.double().sum().reshape(1)
+        dist.all_reduce(total)
+        density = float(total.item()) / float(n) ** 2
+        if rank == 0:
+            print(f"current auc={auc_all}")
+    if rank == 0:
+        os.makedirs("./results/", exist_ok=True)
+        with open(os.path.join("./results", args.log_name), "a") as f:
+            f.write(f"current parameter: {args}\n")
+            f.write(f"In attack graph: AUC={auc}\tIn train graph: AUC={auc_train}\tIn Whole Graph: AUC={auc_all}\n")
+            f.write(f"current density: {density}\n")
     if topk > 0:
-        rows, cols, scores = model.recovered_edges(topk)
+        rows, cols, scores = model.recovered_edges(topk)      # (world > 1: the same pairs on every rank)
+        if rank != 0:
+            return auc_all
         precision, recall = precision_recall_at_k(rows, cols, adj, n)
         np.savez(os.path.join("./results", args.log_name + ".topk.npz"), rows=rows.cpu().numpy(),
                  cols=cols.cpu().numpy(), scores=scores.cpu().numpy())

@@ -75,18 +75,47 @@ def auc_ap_from_edges_sharded(scores_band, row0, n, edges, group=None):
     """metric_pool semantics (all n^2 ordered pairs) when every rank holds a ROW BAND of the scores (rows row0 ...): the
     positives' keys are all-gathered, every rank ranks its own negatives against the global positives (mcgra_auc_stage),
     the integer counts are all-reduced and every rank finishes with the same AUC / AP."""
-    import torch.distributed as dist
     dev = scores_band.device
     rows = scores_band.shape[0]
-    world = dist.get_world_size(group)
     e = torch.as_tensor(edges, device=dev).long()
     lab = torch.zeros(rows, n, dtype=torch.uint8, device=dev)
     for a, b in ((e[:, 0], e[:, 1]), (e[:, 1], e[:, 0])):
         m = (a >= row0) & (a < row0 + rows)
         lab[a[m] - row0, b[m]] = 1
-    npos_max = max(2 * int(e.shape[0]), 1)
-    s = scores_band.detach().reshape(-1).to(torch.float32).contiguous()
-    lab = lab.reshape(-1)
+    return _auc_ap_sharded(scores_band, lab, max(2 * int(e.shape[0]), 1), group)
+
+
+def metric_pool_sharded(ori_adj, scores_band, row0, n, idx, group=None):
+    """metric_pool(ori_adj, gathered scores, idx) when every rank holds a ROW BAND of the n x n scores (rows row0 ...):
+    ROC-AUC over adj[idx][:, idx], the same value on every rank.  Each rank scores the rows of idx that fall in its band
+    (all columns idx) and reads their labels from ori_adj (sparse COO or dense) by index, never as an n x n matrix.
+    Bands may be empty; together they must cover each row once."""
+    import torch.distributed as dist
+    dev = scores_band.device
+    rows, row0 = int(scores_band.shape[0]), int(row0)
+    if scores_band.dim() != 2 or scores_band.shape[1] != n or row0 < 0 or row0 + rows > n:
+        raise ValueError(f"rows [{row0}, {row0 + rows}) of an n = {n} score matrix expected, got shape "
+                         f"{tuple(scores_band.shape)}")
+    idx_t = torch.as_tensor(np.asarray(idx), device=dev).long()
+    mine = idx_t[(idx_t >= row0) & (idx_t < row0 + rows)]
+    pred = scores_band[mine - row0][:, idx_t]
+    a = ori_adj.to(dev)
+    real = (a.coalesce() if a.is_sparse else a).index_select(0, mine).index_select(1, idx_t)
+    lab = ((real.to_dense() if real.is_sparse else real) != 0).to(torch.uint8)
+    npos = lab.sum(dtype=torch.int64).reshape(1)
+    dist.all_reduce(npos, group=group)
+    return _auc_ap_sharded(pred, lab, max(int(npos.item()), 1), group)[0]
+
+
+def _auc_ap_sharded(scores, lab, npos_max, group):
+    """AUC / AP of the union of every rank's (scores, labels): the positives' keys are all-gathered, every rank ranks its
+    own negatives against the global positives (mcgra_auc_stage), the integer counts are all-reduced and every rank
+    finishes with the same values.  `npos_max`: a bound on the positives of all ranks together, the same on every rank."""
+    import torch.distributed as dist
+    dev = scores.device
+    world = dist.get_world_size(group)
+    s = scores.detach().reshape(-1).to(torch.float32).contiguous()
+    lab = lab.reshape(-1).contiguous()
     total = s.numel()
     ws = torch.zeros(N.lib().mcgra_auc_workspace_bytes(max(total, 1), npos_max), dtype=torch.uint8, device=dev)
     out = torch.zeros(4, dtype=torch.float64, device=dev)

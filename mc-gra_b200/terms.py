@@ -85,9 +85,10 @@ class ElementwiseTerms(NNTerms):
 
 
 class Kl2Terms(NNTerms):
-    """c1 / c2 under --measure KL with c2 on (topology_attack.py:212-229, 483-487): three tile passes (csrc/kl2.cu)."""
+    """c1 / c2 under --measure KL with c2 on (topology_attack.py:212-229, 483-487): three tile passes (csrc/kl2.cu).
+    `fa` holds rows [row0, ...) of feature_adj (`banded`: only this rank's tile rows, tiled as they are)."""
 
-    def __init__(self, eng, fa, k1c, k2c):
+    def __init__(self, eng, fa, row0, banded, k1c, k2c):
         self._gradient_tiles(eng, True)
         self.args = k = N.Kl2Args()
         self.bufs = b = {}
@@ -95,8 +96,8 @@ class Kl2Terms(NNTerms):
             b[name] = torch.zeros(eng.n, dtype=torch.float32, device=eng.dev)
             setattr(k, name, ptr(b[name]))
         if fa is not None:
-            b["Ffeat"], b["Fdiag_feat"] = eng._dense_tiles(fa, 1)
-            b["lseF"] = feature_lse(eng, fa).float().contiguous()
+            b["Ffeat"], b["Fdiag_feat"] = eng._dense_tiles(fa, 0 if banded else 1, row0)
+            b["lseF"] = feature_lse(eng, fa, row0, banded).float().contiguous()
             k.Ftiles, k.Fdiag_feat, k.lseF = ptr(b["Ffeat"]), ptr(b["Fdiag_feat"]), ptr(b["lseF"])
         k.tr0, k.tr1, k.n = eng.tr0, eng.tr1, eng.n
         k.EAt, k.Ct = ptr(self.Ftiles), ptr(self.Ct)
@@ -131,13 +132,14 @@ def _kde_mi(n, X, dx, Y, dy, w, m, weight, slot, mom, gmom, gX, gY):
 
 class KdeTerms(NNTerms):
     """c1 / c2 under --measure KDE (utils.py:980-1053): only the first KDE_NB columns of A_hat / M1 / feature_adj reach
-    the Gaussian bins, so the joint pdf is an NB x NB weighted second moment."""
+    the Gaussian bins, so the joint pdf is an NB x NB weighted second moment.  `fa` holds rows [row0, ...) of
+    feature_adj (`banded`: only this rank's tile rows); `fmax`: the maximum of all of feature_adj."""
 
-    def __init__(self, eng, fa, k1c, k2c):
+    def __init__(self, eng, fa, row0, banded, fmax, k1c, k2c):
         n, f32 = eng.n, dict(dtype=torch.float32, device=eng.dev)
         self._gradient_tiles(eng, k2c != 0.0)
         self.nb = nb = min(KDE_NB, n)
-        hi = max(float(fa.max()), 1.0) if fa is not None else 1.0
+        hi = max(float(fmax), 1.0) if fa is not None else 1.0
         if hi > 3.0:      # column j >= KDE_NB would no longer underflow: exp(-0.5 ((v - j) / 0.32)^2) > fp32 min
             raise NotImplementedError("KDE: feature_adj values above 3 reach bins beyond the kept columns")
         self.c1, self.c2 = fa is not None, k2c != 0.0
@@ -147,11 +149,12 @@ class KdeTerms(NNTerms):
             torch.zeros(n, nb, **f32) for _ in range(8))
         self.mom, self.gmom = (torch.zeros(2 * nb + 2 * nb * nb, dtype=torch.float64, device=eng.dev) for _ in range(2))
         self.gslab = self.gA
+        slabF = eng._full_rows(fa, row0, banded, nb).contiguous() if self.c1 else None      # F[:, :NB]
         if self.c1 and eng.eps != 0.0:     # the noisy path's fp64 stage forms kernel values itself
-            self.slabF = fa[:, :nb].contiguous()
+            self.slabF = slabF
         elif self.c1:
             self.kvF = torch.zeros(n, nb, **f32)
-            call("mcgra_kde_kv", ptr(fa), n, nb, n, self.bin, ptr(self.kvF), N.stream_ptr())
+            call("mcgra_kde_kv", ptr(slabF), nb, nb, n, self.bin, ptr(self.kvF), N.stream_ptr())
 
     def step(self, eng, t, noisy):
         """Under noise each MI is ~1e-6 of the entropies it is the difference of: kernel values and moments are formed
