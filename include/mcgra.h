@@ -253,6 +253,11 @@ int mcgra_history_push(const double* row, double* hist, int64_t max_rows, int* s
 /* ---- finalisation (topology_attack.py:300-322) ---- */
 /* x_final tiles = relu(zf_i . zf_j) for j<i (dot_product_decode of the last embedding)              */
 int mcgra_decode_to_tiles(const float* zhat, int64_t n, int tr0, int tr1, float* tiles, void* stream);
+/* rows [b0, b1) of the expanded decode, written (not accumulated) row-major: out[(i - b0) * ld + j] = relu(z_i . z_j) for
+ * j != i and 0 for j == i, z n x 16 as given (row-normalised or raw).  Every entry is bit-equal to what
+ * mcgra_decode_to_tiles followed by mcgra_tiles_to_dense (raw = 1) produce: same 16-term fmaf order, no clamp.
+ * The GraphMI attacks' modified_adj on a row band (baseline.py, mcgpb_attack.py with world > 1). 0 <= b0, b1 <= n <= ld. */
+int mcgra_decode_band(const float* zhat, int64_t n, int64_t b0, int64_t b1, float* out, int64_t ld, void* stream);
 /* one gram term of the ensemble: out[i,j] (+)= f(Z_i . Z_j) with the dataset's decode2 variant
  * (dot_product_decode2, :421-467): variant 0 sigmoid(relu(g - I)), 1 relu(g - I),
  * 2 relu(g/rownorm_i - I) (rownorm = ||row i of ZZ^T||, given), 3 plain g (gcn_parameterized.py:406-416),

@@ -142,6 +142,7 @@ _SIGS = {
     "mcgra_bisect_update": (C.c_int, [C.c_double, C.c_float, c_fp, c_fp, c_fp, c_fp]),
     "mcgra_bisect_finish": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, c_fp, c_fp, c_fp, C.c_int, c_fp]),
     "mcgra_decode_to_tiles": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, c_fp]),
+    "mcgra_decode_band": (C.c_int, [c_fp, i64, i64, i64, c_fp, i64, c_fp]),
     "mcgra_gram_accumulate": (C.c_int, [c_fp, C.c_int, i64, C.c_int, c_fp, c_fp, i64, i64, i64, c_fp]),
     "mcgra_label_accumulate": (C.c_int, [c_fp, i64, c_fp, i64, i64, i64, c_fp]),
     "mcgra_dense_add": (C.c_int, [c_fp, c_fp, i64, c_fp]),

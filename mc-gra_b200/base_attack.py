@@ -53,3 +53,35 @@ class BaseAttack(Module):
         if type(modified_features) is torch.Tensor:
             modified_features = sp.csr_matrix(modified_features.detach().cpu().numpy())
         sp.save_npz(osp.join(root, name), modified_features)
+
+
+class RowBandResult:
+    """The n x n result of the native attacks on several GPUs: with world > 1 every rank holds only its row band
+    `modified_adj` = rows [b0, b1) (`modified_adj_rows`, engine.output_band) of its PGDEngine `self.engine`."""
+
+    def gather_modified_adj(self):
+        """Full n x n result on every rank from the row bands (world > 1); identity otherwise."""
+        eng = self.engine
+        if eng is None or eng.world == 1:
+            return self.modified_adj
+        import torch.distributed as dist
+        from .engine import output_band
+        n = eng.n
+        rb = output_band(n, 0, eng.world)[1]
+        mine = torch.zeros(rb, n, dtype=torch.float32, device=eng.dev)
+        mine[:self.modified_adj.shape[0]] = self.modified_adj
+        full = torch.empty(eng.world * rb, n, dtype=torch.float32, device=eng.dev)
+        dist.all_gather_into_tensor(full, mine, group=eng.group)
+        return full[:n]
+
+    def recovered_edges(self, k):
+        """The reconstructed graph: the k highest-scoring node pairs (i < j) of `modified_adj`, as (rows, cols, scores)
+        device tensors in (score desc, i * n + j asc) order (metrics.topk_pairs).  With world > 1 each rank passes its
+        row band and every rank returns the same result (metrics.topk_pairs_sharded)."""
+        if self.modified_adj is None:
+            raise RuntimeError("recovered_edges() needs the scores of attack(): call attack() first")
+        from .metrics import topk_pairs, topk_pairs_sharded
+        eng = self.engine
+        if eng is not None and eng.world > 1:
+            return topk_pairs_sharded(self.modified_adj, self.modified_adj_rows[0], self.nnodes, k, group=eng.group)
+        return topk_pairs(self.modified_adj, k)

@@ -14,12 +14,12 @@ from torch.nn.parameter import Parameter
 
 from . import _native as N
 from ._native import call, ptr
-from .base_attack import BaseAttack
-from .engine import HID, PGDEngine
+from .base_attack import BaseAttack, RowBandResult
+from .engine import HID, PGDEngine, output_band
 from .topology_attack import PGDAttack as _MCGRA, _dense
 
 
-class PGDAttack(BaseAttack):
+class PGDAttack(RowBandResult, BaseAttack):
 
     def __init__(self, model=None, embedding=None, nnodes=None, loss_type='CE', feature_shape=None,
                  attack_structure=True, attack_features=False, device='cpu'):
@@ -50,7 +50,7 @@ class PGDAttack(BaseAttack):
     decode_normalised = True    # ... and decodes without row normalisation
 
     def _run(self, lr, weight_sup, ori_features, ori_adj, labels, idx_attack, num_edges, epochs, trace=False,
-             setup=None, pre_iter=None):
+             setup=None, pre_iter=None, gather_x=True):
         if self.loss_type != 'CE':
             raise NotImplementedError("native path implements loss_type='CE' (the reference driver's choice)")
         dev = torch.device(self.device)
@@ -95,23 +95,48 @@ class PGDAttack(BaseAttack):
                 self._trace.append(eng.packed_parameter())
         if int(epochs) == 0:
             eng.forward_stages(0)
+        self._finalize(eng, gather_x)
+        return F.log_softmax(eng.H2 @ Wl.t() + bl, dim=1).detach()       # victim output of the last iteration
+
+    def _finalize(self, eng, gather_x=True):
+        """Final decode: adj_changes.data = tril(relu(zf zf^T)), modified_adj its symmetric expansion.  One GPU
+        holds all of both; with world > 1 a rank decodes only its tile rows and keeps only its row band of modified_adj
+        (`modified_adj_rows`, engine.output_band), `gather_modified_adj()` assembles the full matrix."""
         st = N.stream_ptr()
+        n, dev = eng.n, eng.dev
         # em = embedding(features, adj_norm of the last iteration) = hidden state of the normalised branch (:80-82)
         zf = torch.empty_like(eng.H2)
         if self.decode_normalised:
             call("mcgra_row_normalize", ptr(eng.H2), n, HID, 2.0, ptr(zf), st)
         else:
             zf.copy_(eng.H2)
-        T = eng.T
-        xf = torch.empty(T * (T + 1) // 2 * N.TILE * N.TILE, dtype=torch.float32, device=dev)
-        call("mcgra_decode_to_tiles", ptr(zf), n, 0, T, ptr(xf), st)
-        packed = torch.empty(n * (n - 1) // 2, dtype=torch.float32, device=dev)
-        call("mcgra_tiles_to_tril", ptr(xf), n, 0, T, None, 1, ptr(packed), st)
-        self.adj_changes.data = packed
-        out = torch.zeros(n, n, dtype=torch.float32, device=dev)
-        call("mcgra_tiles_to_dense", ptr(xf), n, 0, T, None, 1, ptr(out), n, st)
+        if eng.world == 1:
+            T = eng.T
+            xf = torch.empty(T * (T + 1) // 2 * N.TILE * N.TILE, dtype=torch.float32, device=dev)
+            call("mcgra_decode_to_tiles", ptr(zf), n, 0, T, ptr(xf), st)
+            packed = torch.empty(n * (n - 1) // 2, dtype=torch.float32, device=dev)
+            call("mcgra_tiles_to_tril", ptr(xf), n, 0, T, None, 1, ptr(packed), st)
+            self.adj_changes.data = packed
+            out = torch.zeros(n, n, dtype=torch.float32, device=dev)
+            call("mcgra_tiles_to_dense", ptr(xf), n, 0, T, None, 1, ptr(out), n, st)
+            self.modified_adj = out.detach()
+            self.modified_adj_rows = (0, n)
+            return
+        # every value below equals the single-GPU one bit for bit (mcgra_decode_band is the tiles' symmetric expansion)
+        if gather_x:        # the reference leaves the full packed vector in adj_changes.data (`_gather_x=False`: skip it)
+            # every rank writes its tile rows' entries into a zeroed vector and the vectors are summed
+            xf = torch.empty(max(eng.ntiles, 1) * N.TILE * N.TILE, dtype=torch.float32, device=dev)
+            call("mcgra_decode_to_tiles", ptr(zf), n, eng.tr0, eng.tr1, ptr(xf), st)
+            packed = torch.zeros(n * (n - 1) // 2, dtype=torch.float32, device=dev)
+            call("mcgra_tiles_to_tril", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(packed), st)
+            del xf
+            eng._allreduce(packed)
+            self.adj_changes.data = packed
+        b0, b1 = output_band(n, eng.rank, eng.world)
+        out = torch.empty(max(b1 - b0, 0), n, dtype=torch.float32, device=dev)
+        call("mcgra_decode_band", ptr(zf), n, b0, b1, ptr(out), n, st)
         self.modified_adj = out.detach()
-        return F.log_softmax(eng.H2 @ Wl.t() + bl, dim=1).detach()       # victim output of the last iteration
+        self.modified_adj_rows = (b0, b1)
 
     def attack(self, index_delete, lr_ori, weight_aux, weight_supervised, weight_param, feature_adj,
                aux_adj, aux_feature, aux_num_edges, idx_train, idx_val, idx_test, adj,
@@ -119,7 +144,7 @@ class PGDAttack(BaseAttack):
                dropout_rate, epochs=200, sample=False, **kwargs):
         """baseline.py:36-86.  (`sample=True` only changes an unused local `lr` in the reference, :72-74.)"""
         return self._run(lr_ori, 1.0, ori_features, ori_adj, labels, idx_attack, num_edges, epochs,
-                         trace=bool(kwargs.get("_trace")))
+                         trace=bool(kwargs.get("_trace")), gather_x=kwargs.get("_gather_x", True))
 
     def get_modified_adj(self, ori_adj=None):
         return self._expand(self.adj_changes.data, ori_adj)

@@ -4,7 +4,8 @@
            --useH_A --useY_A --useY --measure=MSELoss            (MC-GRA/README.md:29)
 
 Data: `./dataset/<name>.npz` in the reference's npz layout (adj_data/indices/indptr/shape, attr_*, labels), or
-`--dataset synthetic:<n>:<f>:<c>`.  Only `--mode evaluate` and `--arch gcn` are on the north-star path.
+`--dataset synthetic:<n>:<f>:<c>`.  `--arch gcn` with `--mode evaluate` (the MC-GRA attack, topology_attack.py) or
+`--mode baseline` (the GraphMI attack it is compared against, baseline.py; no adjacency noise) run natively.
 
 Several GPUs: `torchrun --nproc-per-node N -m mcgra_b200.main ...` (WORLD_SIZE > 1) joins a process group and runs the
 tile-row sharded attack; every rank forms only the row bands of feature_adj it touches and of the result it owns."""
@@ -18,6 +19,7 @@ import scipy.sparse as sp
 import torch
 
 from . import synth
+from .baseline import PGDAttack as GraphMI
 from .engine import TILE, HostBands, output_band, shard_tile_rows
 from .metrics import metric_pool, metric_pool_sharded, precision_recall_at_k
 from .models.gcn import GCN, embedding_GCN
@@ -142,8 +144,11 @@ def main(argv=None):
     backend = vars(args).pop("dist_backend")
     if topk < 0:
         raise ValueError(f"--topk {topk}: K must be >= 0 (0 = off)")
-    if args.arch != "gcn" or args.mode != "evaluate":
-        raise NotImplementedError("only --arch gcn --mode evaluate are on the B200 path (SURVEY.md 2)")
+    if args.arch != "gcn" or args.mode not in ("evaluate", "baseline"):
+        raise NotImplementedError("only --arch gcn with --mode evaluate or --mode baseline are on the B200 path "
+                                  "(SURVEY.md 2)")
+    if args.mode == "baseline" and args.eps != 0:
+        raise NotImplementedError("--mode baseline with --eps != 0: the GraphMI baseline attack has no adjacency noise")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world == 1:
         return _run(args, topk, torch.device("cuda:0"), 0, 1)
@@ -176,7 +181,9 @@ def _run(args, topk, device, rank, world):
                                   torch.from_numpy(coo.data.astype(np.float32)), (n, n)).coalesce().to(device)
     features = torch.from_numpy(feats)
     labels_t = torch.from_numpy(labels)
-    if world > 1 and args.eps == 0:
+    if args.mode == "baseline":
+        feature_adj = None      # GraphMI never reads it
+    elif world > 1 and args.eps == 0:
         feature_adj = feature_adj_bands(features.to(device), args.dataset, rank, world, args.nofeature)
     else:       # (--eps != 0 needs feature_adj as a full tensor, also on several GPUs)
         feature_adj = dot_product_decode(features.to(device), args.dataset)
@@ -193,13 +200,19 @@ def _run(args, topk, device, rank, world):
     embedding = embedding_GCN(nfeat=features.shape[1], nhid=16, nlayer=args.nlayers, device=device)
     embedding.gc = deepcopy(victim.gc)
     victim.eval(); embedding.eval()
-    with torch.no_grad():
-        H_A2 = embedding(features.to(device), adj.to(device))
-        Y_A = victim(features.to(device), adj.to(device))
-    model = PGDAttack(model=victim, embedding=embedding, H_A=H_A2, Y_A=Y_A, nnodes=n, loss_type='CE', device=device)
     weight_param = tuple(getattr(args, f"w{k}") for k in range(1, 11))
-    model.attack(args, None, 10 ** args.lr, 0, args.weight_sup, weight_param, feature_adj, 0, 0, 0, idx_train, idx_val,
-                 idx_test, adj, features, torch.zeros(1), labels_t, idx_attack, num_edges, 0, epochs=args.epochs)
+    if args.mode == "baseline":
+        model = GraphMI(model=victim, embedding=embedding, nnodes=n, loss_type='CE', device=device)
+        model.attack(None, 10 ** args.lr, 0, args.weight_sup, weight_param, feature_adj, 0, 0, 0, idx_train, idx_val,
+                     idx_test, adj, features, torch.zeros(1), labels_t, idx_attack, num_edges, 0, epochs=args.epochs)
+    else:
+        with torch.no_grad():
+            H_A2 = embedding(features.to(device), adj.to(device))
+            Y_A = victim(features.to(device), adj.to(device))
+        model = PGDAttack(model=victim, embedding=embedding, H_A=H_A2, Y_A=Y_A, nnodes=n, loss_type='CE', device=device)
+        model.attack(args, None, 10 ** args.lr, 0, args.weight_sup, weight_param, feature_adj, 0, 0, 0, idx_train,
+                     idx_val, idx_test, adj, features, torch.zeros(1), labels_t, idx_attack, num_edges, 0,
+                     epochs=args.epochs)
     inference_adj = model.modified_adj
     if world == 1:
         auc = metric_pool(adj, inference_adj, idx_attack, None)

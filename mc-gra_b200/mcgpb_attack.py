@@ -27,7 +27,8 @@ class PGDAttack(_Baseline):
             eng.smooth_on = t >= 50                                   # :51-61
             eng.lr = 200.0 / np.sqrt(t + 1) if sample else 0.1        # :66-69
         return self._run(0.1, 1.0, ori_features, ori_adj, labels, idx_attack, num_edges, epochs,
-                         trace=bool(kwargs.get("_trace")), setup=setup if int(epochs) > 50 or kwargs.get("_smooth_from") is not None else None,
+                         trace=bool(kwargs.get("_trace")), gather_x=kwargs.get("_gather_x", True),
+                         setup=setup if int(epochs) > 50 or kwargs.get("_smooth_from") is not None else None,
                          pre_iter=pre_iter if kwargs.get("_smooth_from") is None else
                          (lambda eng, t: (setattr(eng, "smooth_on", t >= kwargs["_smooth_from"]),
                                           setattr(eng, "lr", 0.1))))

@@ -21,7 +21,7 @@ from torch.nn.parameter import Parameter
 
 from . import _native as N
 from ._native import call, ptr
-from .base_attack import BaseAttack
+from .base_attack import BaseAttack, RowBandResult
 from .dense_measure import DenseMeasure
 from .engine import HID, HostBands, PGDEngine, check_noise_supported, output_band
 
@@ -53,7 +53,7 @@ def _dense(t, device):
     return t.to(device=device, dtype=torch.float32)
 
 
-class PGDAttack(BaseAttack):
+class PGDAttack(RowBandResult, BaseAttack):
 
     def __init__(self, model=None, embedding=None, H_A=None, Y_A=None, nnodes=None, loss_type='CE', feature_shape=None,
                  attack_structure=True, attack_features=False, device='cpu'):
@@ -347,32 +347,6 @@ class PGDAttack(BaseAttack):
         del xf, keep
         self.modified_adj = out.detach()
         self.modified_adj_rows = (b0, b1_)
-
-    def gather_modified_adj(self):
-        """Full n x n result on every rank from the row bands of `_finalize` (world > 1); identity otherwise."""
-        eng = self.engine
-        if eng is None or eng.world == 1:
-            return self.modified_adj
-        import torch.distributed as dist
-        n = eng.n
-        rb = output_band(n, 0, eng.world)[1]
-        mine = torch.zeros(rb, n, dtype=torch.float32, device=eng.dev)
-        mine[:self.modified_adj.shape[0]] = self.modified_adj
-        full = torch.empty(eng.world * rb, n, dtype=torch.float32, device=eng.dev)
-        dist.all_gather_into_tensor(full, mine, group=eng.group)
-        return full[:n]
-
-    def recovered_edges(self, k):
-        """The reconstructed graph: the k highest-scoring node pairs (i < j) of `modified_adj`, as (rows, cols, scores)
-        device tensors in (score desc, i * n + j asc) order (metrics.topk_pairs).  With world > 1 each rank passes its
-        row band and every rank returns the same result (metrics.topk_pairs_sharded)."""
-        if self.modified_adj is None:
-            raise RuntimeError("recovered_edges() needs the scores of attack(): call attack() first")
-        from .metrics import topk_pairs, topk_pairs_sharded
-        eng = self.engine
-        if eng is not None and eng.world > 1:
-            return topk_pairs_sharded(self.modified_adj, self.modified_adj_rows[0], self.nnodes, k, group=eng.group)
-        return topk_pairs(self.modified_adj, k)
 
     # ------------------------------------------------------------------------------------------------
     # stand-alone helpers of the reference class, same names and semantics
