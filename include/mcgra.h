@@ -222,7 +222,7 @@ typedef struct {
   const int* step_ptr;    /* optional: device counter of completed iterations; Adam step = *step_ptr + 1 (overrides
                              `step`) so that the launch carries no per-iteration host scalar (CUDA-graph replay) */
   int plain_gd;           /* != 0: x <- x - lr * g instead of Adam (MC-GPB/topology_attack.py:66-70: adj_changes +=
-                             lr * (-grad), lr = 0.1); m, v are carried through unchanged                          */
+                             lr * (-grad), lr = 0.1); m, v still receive Adam's moment update, which the step ignores */
   const float* Gtiles;    /* optional tiles of dL/dM_ij + dL/dM_ji computed upstream (feature smoothing of the GraphMI
                              attack, MC-GPB/topology_attack.py:57-61), added to the gradient as is; NULL = none      */
 } mcgra_fold_args;

@@ -177,7 +177,7 @@ k_fold_adam(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restri
         const float mn = fa.beta1 * ms[k] + omb1 * g;
         const float vn = fa.beta2 * vs[k] + omb2 * g * g;
         const float denom = sqrtf(vn) / sqrt_bc2 + fa.adam_eps;
-        const float xn = p_ - step_size * (mn / denom);
+        const float xn = fa.plain_gd ? p_ - fa.lr * g : p_ - step_size * (mn / denom);
         const float c = fminf(fmaxf(xn, 0.f), 1.f);
         xo[k] = valid ? (fa.store_clamped ? c : xn) : 0.f;
         mo[k] = valid ? mn : 0.f;
