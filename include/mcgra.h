@@ -551,9 +551,30 @@ int mcgra_auc_ap(const float* scores, const uint8_t* labels, int64_t N, int64_t 
 int64_t mcgra_auc_hist_offset(int64_t npos_max);
 int mcgra_auc_stage(int stage, const float* scores, const uint8_t* labels, int64_t N, int64_t npos_max, void* ws,
                     double* out, void* stream);
+/* mcgra_auc_stage for the link AUROC of the defended training (calculate_AUC, MC-GPB/models/gcn.py:348-357) without
+ * an n x n object: the scores are s_ij = relu(z_i . z_j - [i == j]) of Z [n x d] (1 <= d <= 32), computed with the
+ * fp32 operation order of mcgra_gram_accumulate variant 1, so every key equals that of the dense score matrix; the
+ * positives are the entries of the CSR (rowptr int64 [n + 1], cols int32, sorted within each row) of the true
+ * adjacency.  The pairs are those of rows [row0, row1) and all n columns.  Stage 0 keys the band's positives from the
+ * CSR, stage 1 sorts them and ranks the band's negatives, generated row by row by merging the column walk with the
+ * row's neighbour list, stage 2 writes out[4] = {auc, ap, npos, nneg}.  The workspace has the layout of mcgra_auc_stage
+ * (count at byte 0, keys from byte 256, sums at byte 8, hist at mcgra_auc_hist_offset(npos_max)), so row bands combine
+ * as they do there.  npos_max >= the band's CSR entries (>= all bands' after an all-gather), < 2^28.  Stage 0 stores
+ * the band's true entry count even when it exceeds npos_max (only npos_max keys are kept); out[2] then reports it, and
+ * a caller must reject out[2] > npos_max, as metrics.roc_auc_ap does for mcgra_auc_ap.                             */
+int64_t mcgra_gram_auc_workspace_bytes(int64_t npos_max);
+int mcgra_gram_auc_stage(int stage, const float* Z, int d, int64_t n, const int64_t* rowptr, const int32_t* cols,
+                         int64_t row0, int64_t row1, int64_t npos_max, void* ws, double* out, void* stream);
 /* stable descending arg-sort (LSD radix sort, key = score, payload = index): the recovered-edge ranking */
 int64_t mcgra_sort_workspace_bytes(int64_t N);
 int mcgra_argsort_desc(const float* scores, int64_t N, int64_t* order, void* ws, void* stream);
+
+/* ---- sparse propagation (GraphConvolution of the defended training on a CSR adjacency) ----
+ * Y = A B, A n x n in CSR (rowptr int64 [n + 1], cols int32, vals fp32; a self-loop is an ordinary entry), B and Y
+ * n x K row-major, K 16 or 32, 16-byte aligned; Y is overwritten.  Each row is summed in a fixed order without atomics
+ * (bit-identical reruns).  For a symmetric A the backward product is the same call.                                  */
+int mcgra_spmm_csr(const int64_t* rowptr, const int32_t* cols, const float* vals, int64_t n, const float* B, int K,
+                   float* Y, void* stream);
 
 /* ---- top-k recovered edges ----
  * The k largest S[i, j] over the strict upper triangle (i < j) of a dense row-major n x n fp32 score matrix, or of the

@@ -192,6 +192,9 @@ _SIGS = {
     "mcgra_argsort_desc": (C.c_int, [c_fp, i64, c_fp, c_fp, c_fp]),
     "mcgra_topk_workspace_bytes": (i64, [i64, i64, i64]),
     "mcgra_topk_stage": (C.c_int, [C.c_int, c_fp, i64, i64, i64, i64, c_fp, i64, i64, c_fp, c_fp, c_fp]),
+    "mcgra_gram_auc_workspace_bytes": (i64, [i64]),
+    "mcgra_gram_auc_stage": (C.c_int, [C.c_int, c_fp, C.c_int, i64, c_fp, c_fp, i64, i64, i64, c_fp, c_fp, c_fp]),
+    "mcgra_spmm_csr": (C.c_int, [c_fp, c_fp, c_fp, i64, c_fp, C.c_int, c_fp, c_fp]),
 }
 TOPK_HIST_OFFSET = 256       # MCGRA_TOPK_HIST_OFFSET
 TOPK_BINS = 2048
@@ -253,17 +256,33 @@ LAUNCHES = {"count": 0, "kernels": 0}
 KERNELS_PER_CALL = {"mcgra_propagate": 3, "mcgra_propagate_sel": 3, "mcgra_noise_stage": 2, "mcgra_fold_adam": 2, "mcgra_auc_ap": 15, "mcgra_argsort_desc": 13,
                     "mcgra_version": 0, "mcgra_set_engine": 0, "mcgra_tiles_in_rows": 0, "mcgra_propagate_ws_bytes": 0,
                     "mcgra_fold_ws_bytes": 0, "mcgra_auc_workspace_bytes": 0, "mcgra_sort_workspace_bytes": 0,
-                    "mcgra_pairs_ws_bytes": 0, "mcgra_auc_hist_offset": 0, "mcgra_topk_workspace_bytes": 0, "mcgra_auc_stage": 5, "mcgra_nd_scratch_doubles": 0, "mcgra_nd_scratch_floats": 0, "mcgra_nd_measure": 5,
+                    "mcgra_pairs_ws_bytes": 0, "mcgra_auc_hist_offset": 0, "mcgra_topk_workspace_bytes": 0, "mcgra_auc_stage": 5, "mcgra_gram_auc_workspace_bytes": 0, "mcgra_nd_scratch_doubles": 0, "mcgra_nd_scratch_floats": 0, "mcgra_nd_measure": 5,
                     "mcgra_image_from_dense": 2, "mcgra_smooth": 2, "mcgra_center_dense": 2, "mcgra_sym_to_tiles": 2}
 
 
 TIMERS = {"on": None}     # when a dict: name -> list of (start, end) CUDA events around each call
 
 
+
+
+def _gram_auc_kernels(stage, Z, d, n, rowptr, cols, row0, row1, npos_max, *rest):
+    """Kernels one mcgra_gram_auc_stage call launches: stage 0 k_gram_pos; stage 1 the radix sort (4 x 3), then for a
+    non-empty band k_unique_pos, k_build_blocks when the distinct keys may exceed the shared-memory table, and the
+    ranker; stage 2 k_ap_finish."""
+    band = row1 > row0
+    if stage == 1:
+        return 12 + (2 + (3 * npos_max + 2 > 57344) if band else 0)
+    return int(band) if stage == 0 else 1
+
+
+KERNELS_BY_ARGS = {"mcgra_gram_auc_stage": _gram_auc_kernels}       # entries whose launch count depends on the arguments
+
+
 def call(name, *args, tag=None):
     """Call a C-ABI entry point, check its return code, count the launch (bench.py's gpu_launches)."""
     LAUNCHES["count"] += 1
-    LAUNCHES["kernels"] += KERNELS_PER_CALL.get(name, 1)
+    by_args = KERNELS_BY_ARGS.get(name)
+    LAUNCHES["kernels"] += by_args(*args) if by_args is not None else KERNELS_PER_CALL.get(name, 1)
     tm = TIMERS["on"]
     if tm is not None:
         import torch

@@ -260,11 +260,153 @@ __global__ void k_build_blocks(const uint32_t* __restrict__ U, const uint32_t* _
 }
 
 constexpr int RK_E = 4;       // pairs per thread and round
+
+// Sources of the negatives' scores for k_rank_negatives_tab.  `run(rank)` calls rank(sc, neg) on groups of RK_E scores
+// (neg[e]: score e is a negative) with a trip count that is uniform over the warp: the ranker's bin updates are
+// warp-collective.
+struct DenseNegatives {       // scores[N] with labels[N] (non-zero = positive)
+  const float* __restrict__ scores;
+  const uint8_t* __restrict__ labels;
+  int64_t N;
+
+  template <class Rank>
+  __device__ __forceinline__ void run(Rank& rank) const {
+    const bool vec = ((reinterpret_cast<uintptr_t>(scores) & 15) == 0) && ((reinterpret_cast<uintptr_t>(labels) & 3) == 0);
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x * RK_E;
+    const int64_t nround = (N + stride - 1) / stride;
+    const int lane = threadIdx.x & 31;
+
+    auto load = [&](int64_t g, float (&sc)[RK_E], bool (&neg)[RK_E]) {
+      if (vec && g + RK_E <= N) {
+        const float4 s4 = *reinterpret_cast<const float4*>(scores + g);
+        const uchar4 l4 = *reinterpret_cast<const uchar4*>(labels + g);
+        sc[0] = s4.x; sc[1] = s4.y; sc[2] = s4.z; sc[3] = s4.w;
+        neg[0] = !l4.x; neg[1] = !l4.y; neg[2] = !l4.z; neg[3] = !l4.w;
+      } else {
+#pragma unroll
+        for (int e = 0; e < RK_E; ++e) {
+          const bool in = g + e < N;
+          neg[e] = in && !labels[in ? g + e : 0];
+          sc[e] = in ? scores[g + e] : 0.f;
+        }
+      }
+    };
+
+    int64_t g = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * RK_E;
+    float sc[RK_E], scn[RK_E];
+    bool neg[RK_E], negn[RK_E];
+#pragma unroll
+    for (int e = 0; e < RK_E; ++e) { sc[e] = scn[e] = 0.f; neg[e] = negn[e] = false; }
+    if (g < N) load(g, sc, neg);
+    for (int64_t rd = 0; rd < nround; ++rd) {
+      const int64_t gn = g + stride;
+#pragma unroll
+      for (int e = 0; e < RK_E; ++e) negn[e] = false;
+      if (rd + 1 < nround && gn < N) load(gn, scn, negn);
+      {                                                   // rounds further ahead: into L2 (no registers)
+        const int64_t gp = g + 4 * stride;
+        if (gp + RK_E <= N) {
+          asm volatile("prefetch.global.L2 [%0];" ::"l"(scores + gp));
+          if ((lane & 3) == 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(labels + gp));
+        }
+      }
+      rank(sc, neg);
+      g = gn;
+#pragma unroll
+      for (int e = 0; e < RK_E; ++e) { sc[e] = scn[e]; neg[e] = negn[e]; }
+    }
+  }
+};
+
+// Pairs (i, j), i in [row0, row1), j in [0, n), scored s_ij = relu(z_i . z_j - [i == j]) with k_gram_accumulate's
+// variant-1 arithmetic (fmaf chain over k = 0 .. d - 1, then the diagonal term and the relu), so every key equals the
+// key of the dense score matrix.  Positives: (i, j) in the CSR (rowptr, cols), columns sorted within each row.  One
+// warp per row; lane L scores columns j0 + RK_E L .. j0 + RK_E L + RK_E - 1 of the current 32 RK_E-column chunk and
+// reads their membership from a 128-bit mask that the warp merges from the row's column list (one cursor per row).
+struct GramNegatives {
+  const float* __restrict__ Z;
+  int d;
+  int64_t n;
+  const int64_t* __restrict__ rowptr;
+  const int32_t* __restrict__ cols;
+  int64_t row0, row1;
+
+  template <class Rank>
+  __device__ __forceinline__ void run(Rank& rank) const {
+    constexpr int W = 32 * RK_E;         // columns per chunk
+    const int lane = threadIdx.x & 31;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    const bool vec = (d & 3) == 0 && (reinterpret_cast<uintptr_t>(Z) & 15) == 0;
+    for (int64_t i = row0 + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5); i < row1; i += nwarps) {
+      const float zi = lane < d ? Z[i * d + lane] : 0.f;       // z_i[k] is broadcast from lane k
+      int64_t p = rowptr[i];
+      const int64_t pe = rowptr[i + 1];
+      for (int64_t j0 = 0; j0 < n; j0 += W) {
+        const int64_t j1 = j0 + W;
+        uint32_t m0 = 0, m1 = 0, m2 = 0, m3 = 0;               // bit o of m(o / 32): column j0 + o is a neighbour
+        while (p < pe && cols[p] < j1) {
+          const int64_t q = p + lane;
+          const int64_t c = q < pe ? (int64_t)cols[q] : j1;
+          const bool in = c < j1;
+          const uint32_t o = in ? (uint32_t)(c - j0) : 0u;
+          const uint32_t bit = in ? 1u << (o & 31) : 0u;
+          m0 |= __reduce_or_sync(0xffffffffu, (o >> 5) == 0 ? bit : 0u);
+          m1 |= __reduce_or_sync(0xffffffffu, (o >> 5) == 1 ? bit : 0u);
+          m2 |= __reduce_or_sync(0xffffffffu, (o >> 5) == 2 ? bit : 0u);
+          m3 |= __reduce_or_sync(0xffffffffu, (o >> 5) == 3 ? bit : 0u);
+          p += __popc(__ballot_sync(0xffffffffu, in));
+        }
+        const int w = lane >> 3;
+        const uint32_t mw = w == 0 ? m0 : w == 1 ? m1 : w == 2 ? m2 : m3;
+        const uint32_t mine = (mw >> ((lane & 7) * RK_E)) & ((1u << RK_E) - 1u);
+        const int64_t jb = j0 + (int64_t)lane * RK_E;
+        float s[RK_E];
+#pragma unroll
+        for (int e = 0; e < RK_E; ++e) s[e] = 0.f;
+        // rows jb .. jb + RK_E - 1 of Z are contiguous: lane's operand starts at zj (clamped into Z for the last chunk)
+        const float* zj = Z + (jb < n ? jb : n - 1) * d;
+        const int last = (int)(n - 1 - (jb < n ? jb : n - 1));   // rows beyond it are clamped to row n - 1
+        if (vec) {
+#pragma unroll 1
+          for (int k = 0; k < d; k += 4) {
+            const float a0 = __shfl_sync(0xffffffffu, zi, k), a1 = __shfl_sync(0xffffffffu, zi, k + 1);
+            const float a2 = __shfl_sync(0xffffffffu, zi, k + 2), a3 = __shfl_sync(0xffffffffu, zi, k + 3);
+#pragma unroll
+            for (int e = 0; e < RK_E; ++e) {
+              const float4 b = __ldg(reinterpret_cast<const float4*>(zj + (e < last ? e : last) * d + k));
+              s[e] = fmaf(a0, b.x, s[e]);
+              s[e] = fmaf(a1, b.y, s[e]);
+              s[e] = fmaf(a2, b.z, s[e]);
+              s[e] = fmaf(a3, b.w, s[e]);
+            }
+          }
+        } else {
+#pragma unroll 1
+          for (int k = 0; k < d; ++k) {
+            const float a = __shfl_sync(0xffffffffu, zi, k);
+#pragma unroll
+            for (int e = 0; e < RK_E; ++e) s[e] = fmaf(a, __ldg(zj + (e < last ? e : last) * d + k), s[e]);
+          }
+        }
+        float sc[RK_E];
+        bool neg[RK_E];
+#pragma unroll
+        for (int e = 0; e < RK_E; ++e) {
+          sc[e] = fmaxf(s[e] - (jb + e == i ? 1.f : 0.f), 0.f);
+          neg[e] = jb + e < n && !((mine >> e) & 1u);
+        }
+        rank(sc, neg);
+      }
+    }
+  }
+};
+
+template <class Src>
 __global__ void __launch_bounds__(1024, 1)
-k_rank_negatives_tab(const float* __restrict__ scores, const uint8_t* __restrict__ labels, int64_t N,
-                     const uint32_t* __restrict__ U, const uint32_t* __restrict__ Cidx, const uint4* __restrict__ blocks,
-                     const unsigned long long* __restrict__ counter, unsigned long long* __restrict__ hist /*[npos+1]*/,
-                     unsigned long long* __restrict__ sums /*[2]*/, int tab_cap) {
+k_rank_negatives_tab(const Src src, const uint32_t* __restrict__ U, const uint32_t* __restrict__ Cidx,
+                     const uint4* __restrict__ blocks, const unsigned long long* __restrict__ counter,
+                     unsigned long long* __restrict__ hist /*[npos+1]*/, unsigned long long* __restrict__ sums /*[2]*/,
+                     int tab_cap) {
   uint32_t* tab = dyn_tab;
   const int npos = (int)counter[0];
   const int nU = (int)counter[3];
@@ -282,46 +424,10 @@ k_rank_negatives_tab(const float* __restrict__ scores, const uint8_t* __restrict
   if (hsm)
     for (int t = threadIdx.x; t <= nU; t += blockDim.x) Hs[t] = 0u;
   __syncthreads();
-  const bool vec = ((reinterpret_cast<uintptr_t>(scores) & 15) == 0) && ((reinterpret_cast<uintptr_t>(labels) & 3) == 0);
-  const int64_t stride = (int64_t)gridDim.x * blockDim.x * RK_E;
-  const int64_t nround = (N + stride - 1) / stride;
   const int lane = threadIdx.x & 31;
   unsigned long long twice = 0, nneg = 0;
 
-  auto load = [&](int64_t g, float (&sc)[RK_E], bool (&neg)[RK_E]) {
-    if (vec && g + RK_E <= N) {
-      const float4 s4 = *reinterpret_cast<const float4*>(scores + g);
-      const uchar4 l4 = *reinterpret_cast<const uchar4*>(labels + g);
-      sc[0] = s4.x; sc[1] = s4.y; sc[2] = s4.z; sc[3] = s4.w;
-      neg[0] = !l4.x; neg[1] = !l4.y; neg[2] = !l4.z; neg[3] = !l4.w;
-    } else {
-#pragma unroll
-      for (int e = 0; e < RK_E; ++e) {
-        const bool in = g + e < N;
-        neg[e] = in && !labels[in ? g + e : 0];
-        sc[e] = in ? scores[g + e] : 0.f;
-      }
-    }
-  };
-
-  int64_t g = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * RK_E;
-  float sc[RK_E], scn[RK_E];
-  bool neg[RK_E], negn[RK_E];
-#pragma unroll
-  for (int e = 0; e < RK_E; ++e) { sc[e] = scn[e] = 0.f; neg[e] = negn[e] = false; }
-  if (g < N) load(g, sc, neg);
-  for (int64_t rd = 0; rd < nround; ++rd) {
-    const int64_t gn = g + stride;
-#pragma unroll
-    for (int e = 0; e < RK_E; ++e) negn[e] = false;
-    if (rd + 1 < nround && gn < N) load(gn, scn, negn);
-    {                                                   // rounds further ahead: into L2 (no registers)
-      const int64_t gp = g + 4 * stride;
-      if (gp + RK_E <= N) {
-        asm volatile("prefetch.global.L2 [%0];" ::"l"(scores + gp));
-        if ((lane & 3) == 0) asm volatile("prefetch.global.L2 [%0];" ::"l"(labels + gp));
-      }
-    }
+  auto rank = [&](const float (&sc)[RK_E], const bool (&neg)[RK_E]) {
     uint32_t k[RK_E];
     int u[RK_E];
     int lb[RK_E], ub[RK_E], vb[RK_E];     // vb: ub in the space of distinct keys (ub = C[vb])
@@ -450,10 +556,8 @@ k_rank_negatives_tab(const float* __restrict__ scores, const uint8_t* __restrict
       }
     }
     twice += (unsigned long long)tw32;
-    g = gn;
-#pragma unroll
-    for (int e = 0; e < RK_E; ++e) { sc[e] = scn[e]; neg[e] = negn[e]; }
-  }
+  };
+  src.run(rank);
   __shared__ unsigned long long r0[32], r1[32];
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
@@ -575,6 +679,51 @@ int radix_sort(uint32_t* keys, PAY* pay, uint32_t* keys_tmp, PAY* pay_tmp, int64
   return 0;   // after 4 passes the result is back in `keys` / `pay`
 }
 
+// the sorted positives pos[0 .. npos) -> their distinct keys (into the free sort buffer pos_tmp) and start indices (behind
+// the histogram); then every negative of `src` is ranked against them (k_rank_negatives_tab)
+template <class Src>
+int rank_tab(const Src& src, const uint32_t* pos, uint32_t* pos_tmp, unsigned long long* counter,
+             unsigned long long* hist, unsigned long long* sums, int64_t npos_max, cudaStream_t st) {
+  uint32_t* Cidx = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(hist) + align256((npos_max + 2) * 8));
+  k_unique_pos<<<1, 1024, 0, st>>>(pos, counter, npos_max, pos_tmp, Cidx);
+  // table capacity (32-bit words): keys + start indices + private histogram of all distinct values when they fit, else
+  // what fits of them (the kernel decides from the number of distinct keys), at least the largest sample
+  const int64_t want = 3 * npos_max + 2;
+  const int cap = (int)(want < TAB_CAP_MAX ? (want > 1024 ? want : 1024) : TAB_CAP_MAX);
+  const size_t smem = (size_t)cap * 4;
+  static bool attr_set = false;          // one per source type: the attribute belongs to each instantiation
+  if (!attr_set) {
+    cudaError_t e = cudaFuncSetAttribute(k_rank_negatives_tab<Src>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         TAB_CAP_MAX * 4);
+    if (e != cudaSuccess) return (int)e;
+    attr_set = true;
+  }
+  uint32_t* blocks = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(Cidx) + align256((npos_max + 2) * 4));
+  if (want > cap) k_build_blocks<<<64, 256, 0, st>>>(pos_tmp, Cidx, counter, cap, blocks);
+  k_rank_negatives_tab<Src><<<148, 1024, smem, st>>>(src, pos_tmp, Cidx, reinterpret_cast<const uint4*>(blocks), counter,
+                                                     hist, sums, cap);
+  MCGRA_LAUNCH_CHECK();
+  return 0;
+}
+
+// keys of the positives of rows [row0, row1): entry p of the CSR -> pos[p - rowptr[row0]] (CSR order; stage 1 sorts
+// them), scored as GramNegatives scores the negatives.  One warp per row.
+__global__ void __launch_bounds__(256)
+k_gram_pos(const float* __restrict__ Z, int d, const int64_t* __restrict__ rowptr, const int32_t* __restrict__ cols,
+           int64_t row0, int64_t row1, uint32_t* __restrict__ poskeys, int64_t cap, unsigned long long* __restrict__ counter) {
+  const int64_t i = row0 + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+  const int lane = threadIdx.x & 31;
+  const int64_t base = rowptr[row0];
+  if (blockIdx.x == 0 && threadIdx.x == 0) *counter = (unsigned long long)(rowptr[row1] - base);
+  if (i >= row1) return;
+  for (int64_t p = rowptr[i] + lane; p < rowptr[i + 1]; p += 32) {
+    const int64_t j = cols[p];
+    float s = 0.f;
+    for (int k = 0; k < d; ++k) s = fmaf(Z[i * d + k], Z[j * d + k], s);
+    if (p - base < cap) poskeys[p - base] = fkey(fmaxf(s - (j == i ? 1.f : 0.f), 0.f));
+  }
+}
+
 }  // namespace
 
 extern "C" {
@@ -633,25 +782,7 @@ int mcgra_auc_stage(int stage, const float* scores, const uint8_t* labels, int64
     int rc = radix_sort<uint32_t>(pos, nullptr, pos_tmp, nullptr, npos_max, hs, offs, st);
     if (rc) return rc;
     if (N > 0 && g_auc_engine == 1 && npos_max < (1LL << 28)) {      // (per-round 32-bit partial sums: 12 npos < 2^32)
-      // distinct keys into the (now free) sort buffer, start indices behind the histogram
-      uint32_t* Cidx = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(hist) + align256((npos_max + 2) * 8));
-      k_unique_pos<<<1, 1024, 0, st>>>(pos, counter, npos_max, pos_tmp, Cidx);
-      // table capacity (32-bit words): keys + start indices + private histogram of all distinct values when they fit, else
-      // what fits of them (the kernel decides from the number of distinct keys), at least the largest sample
-      const int64_t want = 3 * npos_max + 2;
-      const int cap = (int)(want < TAB_CAP_MAX ? (want > 1024 ? want : 1024) : TAB_CAP_MAX);
-      const size_t smem = (size_t)cap * 4;
-      static bool attr_set = false;
-      if (!attr_set) {
-        cudaError_t e = cudaFuncSetAttribute(k_rank_negatives_tab, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             TAB_CAP_MAX * 4);
-        if (e != cudaSuccess) return (int)e;
-        attr_set = true;
-      }
-      uint32_t* blocks = reinterpret_cast<uint32_t*>(reinterpret_cast<char*>(Cidx) + align256((npos_max + 2) * 4));
-      if (want > cap) k_build_blocks<<<64, 256, 0, st>>>(pos_tmp, Cidx, counter, cap, blocks);
-      k_rank_negatives_tab<<<148, 1024, smem, st>>>(scores, labels, N, pos_tmp, Cidx, reinterpret_cast<const uint4*>(blocks),
-                                                    counter, hist, sums, cap);
+      return rank_tab(DenseNegatives{scores, labels, N}, pos, pos_tmp, counter, hist, sums, npos_max, st);
     } else if (N > 0) {
       k_rank_negatives<<<148 * 8, 256, 0, st>>>(scores, labels, N, pos, counter, hist, sums);
     }
@@ -690,6 +821,47 @@ int mcgra_argsort_desc(const float* scores, int64_t N, int64_t* order, void* ws,
   int64_t* offs = (int64_t*)p;
   k_make_keys_desc<<<148 * 8, 256, 0, st>>>(scores, N, keys, order);
   return radix_sort<int64_t>(keys, order, keys_tmp, idx_tmp, N, hs, offs, st);
+}
+
+// mcgra_auc_stage over the n x n gram scores relu(z_i . z_j - [i == j]) of rows [row0, row1), with the labels given by
+// the CSR of the true adjacency: no score or label array.  Same workspace layout (counter, keys, hist) as
+// mcgra_auc_stage with npos_max, so row bands combine in the same way.
+int64_t mcgra_gram_auc_workspace_bytes(int64_t npos_max) { return mcgra_auc_workspace_bytes(0, npos_max); }
+
+int mcgra_gram_auc_stage(int stage, const float* Z, int d, int64_t n, const int64_t* rowptr, const int32_t* cols,
+                         int64_t row0, int64_t row1, int64_t npos_max, void* ws, double* out, void* stream) {
+  cudaStream_t st = (cudaStream_t)stream;
+  if (stage < 0 || stage > 2 || d < 1 || d > 32 || row0 < 0 || row1 < row0 || row1 > n) return -1;
+  if (npos_max <= 0 || npos_max >= (1LL << 28)) return -1;    // (k_rank_negatives_tab: 12 npos < 2^32)
+  char* p = (char*)ws;
+  unsigned long long* counter = (unsigned long long*)p;
+  unsigned long long* sums = counter + 1;
+  p += 256;
+  uint32_t* pos = (uint32_t*)p; p += align256(npos_max * 4);
+  uint32_t* pos_tmp = (uint32_t*)p; p += align256(npos_max * 4);
+  const int64_t nb = (npos_max + CHUNK - 1) / CHUNK + 1;
+  uint32_t* hs = (uint32_t*)p; p += align256(nb * 256 * 4);
+  int64_t* offs = (int64_t*)p; p += align256(nb * 256 * 8);
+  unsigned long long* hist = (unsigned long long*)p;
+  const int64_t rows = row1 - row0;
+  if (stage == 0) {
+    cudaError_t e = cudaMemsetAsync(ws, 0, 256, st);
+    if (e != cudaSuccess) return (int)e;
+    e = cudaMemsetAsync(hist, 0, (npos_max + 2) * 8, st);
+    if (e != cudaSuccess) return (int)e;
+    e = cudaMemsetAsync(pos, 0xff, npos_max * 4, st);
+    if (e != cudaSuccess) return (int)e;
+    if (rows > 0) k_gram_pos<<<(unsigned)((rows + 7) / 8), 256, 0, st>>>(Z, d, rowptr, cols, row0, row1, pos, npos_max, counter);
+  } else if (stage == 1) {
+    int rc = radix_sort<uint32_t>(pos, nullptr, pos_tmp, nullptr, npos_max, hs, offs, st);
+    if (rc) return rc;
+    if (rows > 0) return rank_tab(GramNegatives{Z, d, n, rowptr, cols, row0, row1}, pos, pos_tmp, counter, hist, sums,
+                                  npos_max, st);
+  } else {
+    k_ap_finish<<<1, 1024, 0, st>>>(pos, counter, hist, sums, out);
+  }
+  MCGRA_LAUNCH_CHECK();
+  return 0;
 }
 
 }  // extern "C"

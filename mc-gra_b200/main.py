@@ -26,6 +26,28 @@ from .models.gcn import GCN, embedding_GCN
 from .topology_attack import PGDAttack
 
 
+DEFENSE_MI_TYPES = ("linear_HSIC", "linear_CKA", "DP")
+DEFENSE_BETA_KEYS = ("layer-0", "layer-1", "layer-2", "layer_inter-0", "layer_inter-1")
+# test accuracy of the plain GCN per dataset, the defended training's model-selection reference (MC-GPB/main.py:290-299)
+PLAIN_ACC = {"cora": 0.757, "citeseer": 0.6303, "polblogs": 0.8386, "usair": 0.4703, "brazil": 0.7308, "AIDS": 0.6682,
+             "enzyme": 0.6461, "ogb_arxiv": 0.376}
+
+
+def parse_beta(text):
+    """--beta "b0,b1,b2,i0,i1" -> the beta dict of mcgpb_gcn.GCN.fit (keys DEFENSE_BETA_KEYS)."""
+    parts = [] if text is None else text.split(",")
+    if len(parts) != len(DEFENSE_BETA_KEYS):
+        raise ValueError(f"--beta {text!r}: --defense needs {len(DEFENSE_BETA_KEYS)} comma-separated values for "
+                         + ", ".join(DEFENSE_BETA_KEYS))
+    try:
+        vals = [float(v) for v in parts]
+    except ValueError:
+        raise ValueError(f"--beta {text!r}: the values must be numbers") from None
+    if not all(np.isfinite(vals)):
+        raise ValueError(f"--beta {text!r}: the values must be finite")
+    return dict(zip(DEFENSE_BETA_KEYS, vals))
+
+
 def build_parser():
     p = argparse.ArgumentParser()
     p.add_argument('--seed', type=int, default=15)
@@ -57,7 +79,12 @@ def build_parser():
     p.add_argument('--useY', action='store_true')
     p.add_argument('--ensemble', action='store_true')
     p.add_argument('--add_noise', action='store_true')
-    p.add_argument('--defense', action='store_true')
+    p.add_argument('--defense', action='store_true',
+                   help="attack a victim trained with MC-GPB's defence (mcgpb_gcn.GCN.fit with --beta and --MI_type)")
+    p.add_argument('--MI_type', type=str, default='linear_HSIC', choices=DEFENSE_MI_TYPES,
+                   help="--defense: the information-bottleneck penalty of the defended training")
+    p.add_argument('--beta', type=str, default=None,
+                   help="--defense: five comma-separated penalty weights for " + ", ".join(DEFENSE_BETA_KEYS))
     p.add_argument('--topk', type=int, default=0,
                    help="K > 0: write the K highest-scoring pairs to results/<log_name>.topk.npz and log precision / "
                         "recall against the true edges")
@@ -138,6 +165,33 @@ def _share_victim(victim, device):
         put(state.cpu())
 
 
+def _defend(victim, args, dataset, features, adj, labels, idx_train, idx_val, idx_test, device):
+    """Train MC-GPB's defended GCN (mcgpb_gcn.GCN.fit with args.beta / args.MI_type) on the sparse adjacency and copy its
+    weights (gc1.*, gc2.*, linear1.*) into `victim`.  The model selection compares against the reference's plain
+    accuracy of the dataset, or else the test accuracy of the plain `victim` as trained."""
+    from . import mcgpb_gcn, utils
+    if dataset in PLAIN_ACC:
+        plain_acc = PLAIN_ACC[dataset]
+    else:
+        with torch.no_grad():
+            plain_acc = float(utils.accuracy(victim.predict()[idx_test], victim.labels[idx_test]))
+    model = mcgpb_gcn.GCN(nfeat=features.shape[1], nhid=16, nclass=int(labels.max()) + 1, nlayer=args.nlayers,
+                          dropout=0.5, weight_decay=5e-4, device=device).to(device)
+    for layer in model.gc:
+        layer.to(device)
+    model.fit(features, adj, labels, idx_train, idx_val, idx_test, beta=args.beta, MI_type=args.MI_type,
+              plain_acc=plain_acc)
+    # the link AUROC of every layer of the weights fit selected, in eval mode (fit's own final_layer_aucs are of a
+    # training-mode forward, and None when no epoch passed its selection test)
+    model.eval()
+    with torch.no_grad():
+        layer_aucs = [mcgpb_gcn.link_auc(e, model.origin_csr) for e in model(model.features, model.adj_norm)[1]]
+    victim.load_state_dict(model.state_dict())
+    with torch.no_grad():
+        acc = float(utils.accuracy(victim.predict()[idx_test], victim.labels[idx_test]))
+    return {"acc_test": acc, "plain_acc": plain_acc, "final_layer_aucs": layer_aucs}
+
+
 def main(argv=None):
     args = build_parser().parse_args(argv)
     topk = vars(args).pop("topk")         # not part of the reference's parameter line in the log
@@ -149,6 +203,8 @@ def main(argv=None):
                                   "(SURVEY.md 2)")
     if args.mode == "baseline" and args.eps != 0:
         raise NotImplementedError("--mode baseline with --eps != 0: the GraphMI baseline attack has no adjacency noise")
+    if args.defense:
+        args.beta = parse_beta(args.beta)
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world == 1:
         return _run(args, topk, torch.device("cuda:0"), 0, 1)
@@ -165,6 +221,7 @@ def main(argv=None):
 def _run(args, topk, device, rank, world):
     np.random.seed(args.seed); random.seed(args.seed); torch.manual_seed(args.seed); torch.cuda.manual_seed(args.seed)
     adj_sp, feats, labels = load_graph(args.dataset)
+    dataset = args.dataset
     if args.dataset.startswith("synthetic"):
         # the reference's dataset-keyed tables (feature similarity main.py:44-55, dot_product_decode2
         # topology_attack.py:421-467) have no synthetic entry: synthetic graphs use the Cora branches
@@ -193,8 +250,11 @@ def _run(args, topk, device, rank, world):
                  weight_decay=5e-4, device=device).to(device)
     for layer in victim.gc:
         layer.to(device)
+    defended = None
     if rank == 0:
         victim.fit(features, adj, labels_t, idx_train, idx_val)
+        if args.defense:
+            defended = _defend(victim, args, dataset, features, adj, labels_t, idx_train, idx_val, idx_test, device)
     if world > 1:
         _share_victim(victim, device)
     embedding = embedding_GCN(nfeat=features.shape[1], nhid=16, nlayer=args.nlayers, device=device)
@@ -233,6 +293,9 @@ def _run(args, topk, device, rank, world):
         os.makedirs("./results/", exist_ok=True)
         with open(os.path.join("./results", args.log_name), "a") as f:
             f.write(f"current parameter: {args}\n")
+            if defended is not None:
+                f.write(f"Defended victim: test accuracy={defended['acc_test']}\tplain accuracy={defended['plain_acc']}\n")
+                f.write(f"Defended victim: final layer AUROCs={defended['final_layer_aucs']}\n")
             f.write(f"In attack graph: AUC={auc}\tIn train graph: AUC={auc_train}\tIn Whole Graph: AUC={auc_all}\n")
             f.write(f"current density: {density}\n")
     if topk > 0:

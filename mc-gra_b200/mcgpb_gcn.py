@@ -17,6 +17,8 @@ What runs natively (C ABI, include/mcgra.h):
         DP(N N^T, Z)          = ||Z Z^T N N^T||_F = sqrt(tr(Gs (N^T Z) (Z^T Z) (Z^T N)))
     (the d x d algebra on the moment matrices is a handful of torch ops on 16 x 16 tensors);
   * the link AUROCs: `mcgra_gram_accumulate` (relu(Z Z^T - I)) + `mcgra_auc_ap` (exact sklearn semantics, on device).
+A sparse adjacency takes the CSR path instead, which holds no n x n object: `mcgra_spmm_csr` propagates, and
+`mcgra_gram_auc_stage` ranks the gram scores against the CSR labels as it generates them (bit-equal AUCs).
 PyTorch keeps the parameter tensors, autograd's tape between the native ops, the small dense X W products and Adam.
 There is no CPU path: the model must live on a CUDA device.
 """
@@ -65,6 +67,59 @@ class TiledAdjacency:
         call("mcgra_propagate", ptr(self.tiles), self.n, 0, self.T, None, 2, ptr(B), K, ptr(Y), ptr(self.ws),
              N.stream_ptr())
         return Y + self.diag[:, None] * B
+
+
+class SparseAdjacency:
+    """Fixed symmetric adjacency in CSR form (int64 row pointers, int32 sorted columns, fp32 values, the self-loop an
+    ordinary entry): the operand of mcgra_spmm_csr, with the matmul interface of TiledAdjacency.  Holds O(n + |E|)."""
+
+    def __init__(self, rowptr, cols, vals):
+        if not vals.is_cuda:
+            raise N.NativeError("mcgpb_gcn needs a CUDA device (no CPU fallback)")
+        self.rowptr, self.cols, self.vals = rowptr.contiguous(), cols.contiguous(), vals.contiguous()
+        self.n = rowptr.numel() - 1
+
+    def matmul(self, B):
+        B = B.contiguous()
+        K = B.shape[1]
+        if K not in (16, 32):
+            raise NotImplementedError("native propagation handles 16- or 32-wide operands (nhid = 16 in the reference)")
+        Y = torch.empty_like(B)
+        call("mcgra_spmm_csr", ptr(self.rowptr), ptr(self.cols), ptr(self.vals), self.n, ptr(B), K, ptr(Y),
+             N.stream_ptr())
+        return Y
+
+
+class Csr:
+    """CSR of a sparse n x n matrix without explicit zeros: rowptr (int64, n + 1), rows / cols of the entries in row-major
+    order (int64 / int32), vals (float32)."""
+
+    def __init__(self, a):
+        n = a.shape[0]
+        if a.layout != torch.sparse_coo:
+            a = a.to_sparse_coo()
+        a = a.coalesce()                     # row-major, columns sorted within a row
+        keep = a.values() != 0
+        self.rows, cols = a.indices()[0][keep], a.indices()[1][keep]
+        self.cols, self.vals = cols.to(torch.int32).contiguous(), a.values()[keep].to(torch.float32).contiguous()
+        self.rowptr = torch.zeros(n + 1, dtype=torch.int64, device=a.device)
+        self.rowptr[1:] = torch.cumsum(torch.bincount(self.rows, minlength=n), 0)
+        self.n = n
+
+    def coo(self):
+        return torch.sparse_coo_tensor(torch.stack([self.rows, self.cols.long()]), self.vals, (self.n, self.n))
+
+
+def normalize_csr(a):
+    """utils.normalize_adj_tensor on a Csr: D^-1/2 (A + I) D^-1/2 with the same value order (r_i * m_ij) * r_j, where
+    r = rowsum(A + I)^-1/2 (0 where the row sum is 0)."""
+    n, dev = a.n, a.vals.device
+    ar = torch.arange(n, device=dev)
+    mx = Csr(torch.sparse_coo_tensor(torch.stack([torch.cat([a.rows, ar]), torch.cat([a.cols.long(), ar])]),
+                                     torch.cat([a.vals, torch.ones(n, device=dev)]), (n, n)))
+    r_inv = torch.segment_reduce(mx.vals, "sum", offsets=mx.rowptr).pow(-1 / 2)
+    r_inv = torch.where(torch.isinf(r_inv), torch.zeros_like(r_inv), r_inv)
+    return SparseAdjacency(mx.rowptr, mx.cols, (r_inv[mx.rows] * mx.vals) * r_inv[mx.cols.long()])
 
 
 class _Propagate(torch.autograd.Function):
@@ -144,12 +199,24 @@ MI_FUNCS = {"linear_HSIC": linear_HSIC, "linear_CKA": linear_CKA, "DP": DP}
 
 def link_auc(Z, adj_labels):
     """calculate_AUC (MC-GPB/models/gcn.py:348-357): AUROC of relu(Z Z^T - I) against the true adjacency over all n^2
-    ordered pairs, on the device."""
+    ordered pairs, on the device.  `adj_labels`: the n x n uint8 label matrix, or the Csr of the true adjacency (then
+    mcgra_gram_auc_stage forms neither scores nor labels; the same AUC bit for bit)."""
     from .metrics import roc_auc_ap
     Zc = Z.detach().to(torch.float32).contiguous()
     n, d = Zc.shape
     if d > 32:
         raise NotImplementedError("embedding width > 32")
+    if isinstance(adj_labels, Csr):
+        npos = max(int(adj_labels.cols.numel()), 1)
+        ws = torch.empty(N.lib().mcgra_gram_auc_workspace_bytes(npos), dtype=torch.uint8, device=Zc.device)
+        out = torch.zeros(4, dtype=torch.float64, device=Zc.device)
+        for stage in range(3):
+            call("mcgra_gram_auc_stage", stage, ptr(Zc), d, n, ptr(adj_labels.rowptr), ptr(adj_labels.cols), 0, n, npos,
+                 ptr(ws), ptr(out), N.stream_ptr())
+        o = out.cpu().numpy()
+        if int(o[2]) > npos:
+            raise N.NativeError(f"positives {int(o[2])} exceed npos_max {npos}")
+        return float(o[0])
     S = torch.zeros(n, n, dtype=torch.float32, device=Zc.device)
     call("mcgra_gram_accumulate", ptr(Zc), d, n, 1, None, ptr(S), n, 0, n, N.stream_ptr())
     return roc_auc_ap(S, adj_labels)[0]
@@ -176,7 +243,7 @@ class GraphConvolution(Module):
 
     def forward(self, input, adj):
         support = torch.mm(input, self.weight)
-        if isinstance(adj, TiledAdjacency):
+        if isinstance(adj, (TiledAdjacency, SparseAdjacency)):
             output = _Propagate.apply(support, adj)
         else:
             output = torch.spmm(adj, support)
@@ -219,6 +286,7 @@ class GCN(nn.Module):
         self.weight_decay = weight_decay if with_relu else 0
         self.with_relu, self.with_bias = with_relu, with_bias
         self.output = self.best_model = self.best_output = self.adj_norm = self.features = self.origin_adj = None
+        self.origin_csr = None
         self.initialize()
 
     def forward(self, x, adj):
@@ -241,7 +309,11 @@ class GCN(nn.Module):
             verbose=False, normalize=True, patience=500, beta=None, MI_type='linear_HSIC', stochastic=0, con=0, aug_pe=0.1,
             plain_acc=0.7, pair_draws=None, **kwargs):
         """models/gcn.py:184-277.  `pair_draws` (test hook): the node-pair index draws of every epoch instead of
-        np.random.choice, so that a run can be replayed against a reference fixture."""
+        np.random.choice, so that a run can be replayed against a reference fixture.
+
+        A sparse `adj` (torch sparse tensor or scipy matrix) is never densified: the normalised adjacency, the labels of
+        the link AUROCs and the node pairs are held in CSR form (O(n + |E|) device memory), with the same node-pair and
+        edge-drop draws as a dense `adj`.  A dense `adj` takes the tiled dense path."""
         self.device = self.gc1.weight.device
         if self.device.type != "cuda":
             raise N.NativeError("mcgpb_gcn needs a CUDA device (no CPU fallback)")
@@ -249,8 +321,30 @@ class GCN(nn.Module):
             features, adj, labels = utils.to_tensor(features, adj, labels, device=self.device)
         else:
             features, adj, labels = features.to(self.device), adj.to(self.device), labels.to(self.device)
-        if adj.is_sparse:
-            adj = adj.to_dense()
+        if adj.layout != torch.strided:
+            self._set_sparse_adj(adj, stochastic, aug_pe, normalize)
+        else:
+            self._set_dense_adj(adj, stochastic, aug_pe, normalize)
+        self.features, self.labels = features, labels
+        if con:
+            raise NotImplementedError("contrastive training (con=1) is not on the MC-GPB README path")
+        if beta is None:
+            return self._train_with_val(labels, idx_train, idx_val, train_iters, verbose)
+        return self._train_with_MI_constrain(labels, idx_train, idx_val, idx_test, train_iters, beta, MI_type, plain_acc,
+                                             verbose, pair_draws)
+
+    def _set_sparse_adj(self, adj, stochastic, aug_pe, normalize):
+        a = Csr(adj)
+        if stochastic:        # the dense path's edge drop: one draw per upper-triangle entry, in row-major order
+            up = a.cols.long() > a.rows
+            keep = torch.rand(int(up.sum()), device=self.device) >= aug_pe
+            i, j = a.rows[up][keep], a.cols.long()[up][keep]
+            a = Csr(torch.sparse_coo_tensor(torch.stack([torch.cat([i, j]), torch.cat([j, i])]),
+                                            torch.ones(2 * i.numel(), device=self.device), (a.n, a.n)))
+        self.adj_norm = normalize_csr(a) if normalize else SparseAdjacency(a.rowptr, a.cols, a.vals)
+        self.origin_adj, self.origin_csr = a.coo(), a
+
+    def _set_dense_adj(self, adj, stochastic, aug_pe, normalize):
         if stochastic:        # utils.stochastic (PyGCL EdgeRemoving, MC-GPB/utils.py:799-805): drop each undirected edge with prob. pe
             iu = torch.triu(adj, 1).nonzero()
             keep = torch.rand(iu.shape[0], device=self.device) >= aug_pe
@@ -259,13 +353,7 @@ class GCN(nn.Module):
             adj = new + new.t()
         adj_norm = utils.normalize_adj_tensor(adj) if normalize else adj
         self.adj_norm = TiledAdjacency(adj_norm)
-        self.features, self.labels, self.origin_adj = features, labels, adj
-        if con:
-            raise NotImplementedError("contrastive training (con=1) is not on the MC-GPB README path")
-        if beta is None:
-            return self._train_with_val(labels, idx_train, idx_val, train_iters, verbose)
-        return self._train_with_MI_constrain(labels, idx_train, idx_val, idx_test, train_iters, beta, MI_type, plain_acc,
-                                             verbose, pair_draws)
+        self.origin_adj, self.origin_csr = adj, None
 
     def _train_with_val(self, labels, idx_train, idx_val, train_iters, verbose):
         """models/gcn.py:279-319."""
@@ -300,9 +388,13 @@ class GCN(nn.Module):
         IAZ = torch.zeros((train_iters, self.nlayer + 1))
         IYZ = torch.zeros((train_iters, self.nlayer + 1))
         full_losses = [[] for _ in range(4)]
-        edge_index = self.origin_adj.nonzero()
+        if self.origin_csr is not None:          # row-major, as origin_adj.nonzero() lists them
+            edge_index = torch.stack([self.origin_csr.rows, self.origin_csr.cols.long()], 1)
+            adj_labels = self.origin_csr
+        else:
+            edge_index = self.origin_adj.nonzero()
+            adj_labels = (self.origin_adj != 0).to(torch.uint8).contiguous()
         sample_size = min(1000, edge_index.size(0))
-        adj_labels = (self.origin_adj != 0).to(torch.uint8).contiguous()
         best_layer_AUC, weights, final_layer_aucs, best_acc_test = 1e10, None, 1000, 0
         weights2 = final_layer_aucs_2 = None
         for epoch in range(train_iters):
