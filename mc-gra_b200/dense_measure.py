@@ -26,8 +26,6 @@ from . import _native as N
 from ._native import ACC, call, ptr
 from .terms import NNTerms
 
-TILE = N.TILE
-
 
 def _rup(x, m):
     return (x + m - 1) // m * m
@@ -90,8 +88,8 @@ class DenseMeasure(NNTerms):
         self.imgSM = _Img(n, n, dev) if (self.cka and self.c2) else None
         self.tiles_full = None
         if world > 1:
-            T = eng.T
-            self.tiles_full = torch.zeros((T * (T + 1) // 2) * TILE * TILE, **f32)
+            from .engine import tile_buffer      # (engine imports this module)
+            self.tiles_full = tile_buffer(0, eng.T, dev)
 
     # ------------------------------------------------------------------------------------------------
     def _gemm(self, A, B, Cbuf=None, alpha=1.0, beta=0.0, alpha_dev=None, beta_dev=None, u=None, v=None, coef=0.0,
@@ -143,9 +141,10 @@ class DenseMeasure(NNTerms):
         if eng.world == 1:
             return eng.xt
         import torch.distributed as dist
+        from .engine import tile_offset
         self.tiles_full.zero_()
-        o = (eng.tr0 * (eng.tr0 + 1) // 2) * TILE * TILE
-        self.tiles_full[o:o + eng.ntiles * TILE * TILE].copy_(eng.xt[:eng.ntiles * TILE * TILE])
+        o, m = tile_offset(eng.tr0), tile_offset(eng.tr1) - tile_offset(eng.tr0)
+        self.tiles_full[o:o + m].copy_(eng.xt[:m])
         dist.all_reduce(self.tiles_full, group=eng.group)
         return self.tiles_full
 

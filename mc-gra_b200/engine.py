@@ -36,13 +36,57 @@ MEASURES = {"MSELoss": N.M_MSE, "KL": N.M_KL, "HSIC": N.M_HSIC, "CKA": N.M_CKA, 
 ALIGN = {"c1": 100, "c2": 1000, "c6": 10, "c7": 10, "c9": 1, "c10": 1}      # MC-GRA/utils.py:1100-1111
 
 
-# largest n for which the iteration is replayed as a CUDA graph (0 disables); env override for A/B runs
+# 10 passes x 3 halvings: brackets up to ~10^4 wide at eps = 1e-5; finished passes read nothing
 BISECT_PASSES = 10
+# largest n for which the iteration is replayed as a CUDA graph (0 disables); env override for A/B runs
 GRAPH_MAX_N = int(os.environ.get("MCGRA_GRAPH_MAX_N", "8192"))
 
 
 def tri(i):
     return i * (i + 1) // 2
+
+
+def tile_offset(tr):
+    """Elements of the packed tile triangle before tile row `tr`."""
+    return tri(tr) * TILE * TILE
+
+
+def tile_buffer(tr0, tr1, device, zero=True):
+    """fp32 buffer for the tiles of tile rows [tr0, tr1) of the lower triangle; at least one tile (a rank without rows
+    still hands the kernels an address)."""
+    return (torch.zeros if zero else torch.empty)(max(tri(tr1) - tri(tr0), 1) * TILE * TILE, dtype=torch.float32,
+                                                  device=device)
+
+
+def packed_to_tiles(packed, n, tr0, tr1, out=None):
+    """Tiles of rows [tr0, tr1) from a packed parameter vector (reference layout, fp32 on the device)."""
+    out = tile_buffer(tr0, tr1, packed.device, zero=False) if out is None else out
+    call("mcgra_tril_to_tiles", ptr(packed), n, tr0, tr1, ptr(out), N.stream_ptr())
+    return out
+
+
+def tiles_to_packed(tiles, n, tr0, tr1, mu, raw, reduce=None):
+    """The packed parameter vector of the tiles of rows [tr0, tr1) under the parameter view (mu, raw).  A rank that
+    holds only part of the rows writes its entries into zeros and `reduce` (an all-reduce) sums the ranks' vectors."""
+    T = (n + TILE - 1) // TILE
+    out = (torch.empty if (tr0, tr1) == (0, T) else torch.zeros)(n * (n - 1) // 2, dtype=torch.float32,
+                                                                 device=tiles.device)
+    call("mcgra_tiles_to_tril", ptr(tiles), n, tr0, tr1, ptr(mu), raw, ptr(out), N.stream_ptr())
+    if reduce is not None:
+        reduce(out)
+    return out
+
+
+def bisect(tiles, n, tr0, tr1, budget, eps, passes, bstate, cand, mu, reduce=None):
+    """`passes` passes of the device bisection for sum(clamp(x - mu, 0, 1)) = budget, each three halvings of the bracket
+    in `bstate` over the tiles of rows [tr0, tr1); `reduce` sums the ranks' candidate sums `cand`.  Allocates nothing and
+    reads nothing back (it runs inside a captured CUDA graph)."""
+    st = N.stream_ptr()
+    for _ in range(passes):
+        call("mcgra_bisect_pass", ptr(tiles), n, tr0, tr1, eps, ptr(bstate), ptr(cand), st)
+        if reduce is not None:
+            reduce(cand)
+        call("mcgra_bisect_update", budget, eps, ptr(bstate), ptr(cand), ptr(mu), st)
 
 
 def shard_tile_rows(T, world):
@@ -128,7 +172,6 @@ class PGDEngine:
         self.T = (n + TILE - 1) // TILE
         self.npad = self.T * TILE
         self.tr0, self.tr1 = shard_tile_rows(self.T, world)[rank]
-        self.ntiles = tri(self.tr1) - tri(self.tr0)
         self.P = n * (n - 1) // 2
         f32 = dict(dtype=torch.float32, device=dev)
 
@@ -205,10 +248,7 @@ class PGDEngine:
         self.proj_possible = self.budget < float(self.P)
 
         # ---- state: tiled triangle of x', m, v ----
-        nel = max(self.ntiles, 1) * TILE * TILE
-        self.xt = torch.zeros(nel, **f32)
-        self.mt = torch.zeros(nel, **f32)
-        self.vt = torch.zeros(nel, **f32)
+        self.xt, self.mt, self.vt = (tile_buffer(self.tr0, self.tr1, dev) for _ in range(3))
         self.mu = torch.zeros(1, **f32)
         self.raw = 0
         self.step = 0
@@ -254,7 +294,7 @@ class PGDEngine:
         if self.eps != 0.0:
             # noisy path: the two orientations of M, its diagonal, the gradient tiles handed to the fold, and zero
             # factors / rho for that fold (its own product and degree terms are already inside the gradient tiles)
-            self.Lt, self.Ut, self.Gn = (torch.zeros(nel, **f32) for _ in range(3))
+            self.Lt, self.Ut, self.Gn = (tile_buffer(self.tr0, self.tr1, dev) for _ in range(3))
             self.mdiag = z(n)
             self.Wt0, self.rho0 = z(128, self.npad), z(n)
             # (the default draw captures no reference to the engine: a cycle would keep its device memory alive
@@ -276,7 +316,7 @@ class PGDEngine:
 
     def _dense_tiles(self, dense, symmetrize, row0=0):
         """Tiles of this rank's tile rows of a dense n x n matrix (`row0`: first row of a band), all-reduced diagonal."""
-        tiles = torch.zeros(max(self.ntiles, 1) * TILE * TILE, dtype=torch.float32, device=self.dev)
+        tiles = tile_buffer(self.tr0, self.tr1, self.dev)
         diag = torch.zeros(self.n, dtype=torch.float32, device=self.dev)
         call("mcgra_dense_to_tiles", dense.data_ptr() - row0 * self.n * 4, self.n, self.n, self.tr0, self.tr1, symmetrize,
              ptr(tiles), ptr(diag), N.stream_ptr())
@@ -312,7 +352,7 @@ class PGDEngine:
         else:
             xp = x_packed.detach().to(device=self.dev, dtype=torch.float32).contiguous()
             assert xp.numel() == self.P
-            call("mcgra_tril_to_tiles", ptr(xp), self.n, self.tr0, self.tr1, ptr(self.xt), st)
+            packed_to_tiles(xp, self.n, self.tr0, self.tr1, out=self.xt)
             self.raw = 1
             sumsq = float((xp.double() ** 2).sum())
         self._acc_row(0)[ACC["SUMSQ"]] = sumsq
@@ -577,10 +617,7 @@ class PGDEngine:
         acc_next = self._acc_row(t + 1).data_ptr()
         self.cand.zero_()
         call("mcgra_bisect_init", acc_next, ptr(self.minmax), self.budget, ptr(self.bstate), ptr(self.mu), st)
-        for _ in range(BISECT_PASSES):   # 10 passes x 3 halvings: brackets up to ~10^4 wide at eps = 1e-5; finished passes read nothing
-            call("mcgra_bisect_pass", ptr(self.xt), n, tr0, tr1, 1e-5, ptr(self.bstate), ptr(self.cand), st)
-            self._allreduce(self.cand)
-            call("mcgra_bisect_update", self.budget, 1e-5, ptr(self.bstate), ptr(self.cand), ptr(self.mu), st)
+        bisect(self.xt, n, tr0, tr1, self.budget, 1e-5, BISECT_PASSES, self.bstate, self.cand, self.mu, self._allreduce)
         call("mcgra_bisect_finish", ptr(self.xt), n, tr0, tr1, ptr(self.bstate), ptr(self.mu), acc_next,
              ptr(self.d_next), 1, st)
         # (with world > 1 the reset writes d_next = 1 on every rank; keep rank 0's only)
@@ -605,7 +642,7 @@ class PGDEngine:
         call("mcgra_gram_accumulate", ptr(X), X.shape[1], n, 3, None, ptr(G), n, 0, n, st) if X.shape[1] <= 32 else G.copy_(X @ X.t())
         Gfeat, gdiag = self._dense_tiles(G, 1)
         del G
-        self.Gt = torch.zeros(max(self.ntiles, 1) * TILE * TILE, **f32)
+        self.Gt = tile_buffer(self.tr0, self.tr1, dev)
         self.smooth = dict(Gfeat=Gfeat, gdiag=gdiag, rt=torch.zeros(n, **f32), trow=torch.zeros(n, **f32), coef=float(coef))
 
     def _smooth_stage(self, t):
@@ -638,8 +675,4 @@ class PGDEngine:
 
     def packed_parameter(self):
         """The optimised parameter in the reference's packed layout (all ranks' shards summed)."""
-        out = torch.zeros(self.P, dtype=torch.float32, device=self.dev)
-        call("mcgra_tiles_to_tril", ptr(self.xt), self.n, self.tr0, self.tr1, ptr(self.mu), self.raw, ptr(out),
-             N.stream_ptr())
-        self._allreduce(out)
-        return out
+        return tiles_to_packed(self.xt, self.n, self.tr0, self.tr1, self.mu, self.raw, self._allreduce)

@@ -36,8 +36,7 @@ from torch.nn.parameter import Parameter
 from . import _native as N
 from . import utils
 from ._native import call, ptr
-
-TILE = N.TILE
+from .engine import TILE, tile_buffer
 
 
 # ----------------------------------------------------------------------------------------------------------------
@@ -53,7 +52,7 @@ class TiledAdjacency:
         A = (A.to_dense() if A.is_sparse else A).to(torch.float32).contiguous()
         n = A.shape[0]
         self.n, self.T = n, (n + TILE - 1) // TILE
-        self.tiles = torch.zeros(self.T * (self.T + 1) // 2 * TILE * TILE, dtype=torch.float32, device=A.device)
+        self.tiles = tile_buffer(0, self.T, A.device)
         self.diag = torch.zeros(n, dtype=torch.float32, device=A.device)
         call("mcgra_dense_to_tiles", ptr(A), n, n, 0, self.T, 1, ptr(self.tiles), ptr(self.diag), N.stream_ptr())
         self.ws = torch.empty(int(N.lib().mcgra_propagate_ws_bytes(n, 32)), dtype=torch.uint8, device=A.device)

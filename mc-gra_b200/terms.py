@@ -23,10 +23,11 @@ class NNTerms:
 
     def _gradient_tiles(self, eng, c2):
         """Gradient tiles (MCGRA_M_PRE); under noise A_hat's gradient is a slab and M1's tiles exist only with c2."""
-        ntl, noisy = max(eng.ntiles, 1) * TILE * TILE, eng.eps != 0.0
+        from .engine import tile_buffer      # (engine imports this module)
+        noisy = eng.eps != 0.0
         self.measure = N.M_PRE
-        self.Ftiles = None if noisy else torch.zeros(ntl, dtype=torch.float32, device=eng.dev)
-        self.Ct = torch.zeros(ntl, dtype=torch.float32, device=eng.dev) if (not noisy or c2) else None
+        self.Ftiles = None if noisy else tile_buffer(eng.tr0, eng.tr1, eng.dev)
+        self.Ct = tile_buffer(eng.tr0, eng.tr1, eng.dev) if (not noisy or c2) else None
         self.Fdiag = torch.zeros(eng.n, dtype=torch.float32, device=eng.dev)     # dL/dA_ii
 
 
@@ -53,8 +54,9 @@ class ElementwiseTerms(NNTerms):
         else:
             # the noisy A_hat is not symmetric: F and F^T are tiled as they are (on the diagonal F equals its
             # symmetrisation).  F^T is formed for this rank's rows alone (columns [r0, r1) of F), pointer shifted
-            ntl = max(eng.ntiles, 1) * TILE * TILE
-            self.FLt, self.FUt, self.Fdiag = torch.zeros(ntl, **f32), torch.zeros(ntl, **f32), torch.zeros(n, **f32)
+            from .engine import tile_buffer
+            self.FLt, self.FUt = tile_buffer(eng.tr0, eng.tr1, eng.dev), tile_buffer(eng.tr0, eng.tr1, eng.dev)
+            self.Fdiag = torch.zeros(n, **f32)
             r0, r1 = eng.tr0 * TILE, min(n, eng.tr1 * TILE)
             if r1 > r0:
                 call("mcgra_dense_to_tiles", ptr(fa), n, n, eng.tr0, eng.tr1, 0, ptr(self.FLt), ptr(self.Fdiag),

@@ -14,14 +14,12 @@ Deliberately hoisted / dropped (results unchanged, SURVEY.md Appendix C):
 import os
 
 import numpy as np
-import scipy.sparse as sp
 import torch
 from torch.nn import functional as F
-from torch.nn.parameter import Parameter
 
 from . import _native as N
 from ._native import call, ptr
-from .base_attack import BaseAttack, RowBandResult
+from .base_attack import RowBandResult, _dense, _rank_world
 from .dense_measure import DenseMeasure
 from .engine import HID, HostBands, PGDEngine, check_noise_supported, output_band
 
@@ -43,39 +41,16 @@ def _ident(t):
     return (id(t), getattr(t, "shape", None))
 
 
-def _dense(t, device):
-    if sp.issparse(t):
-        t = np.asarray(t.todense())
-    if isinstance(t, np.ndarray):
-        t = torch.from_numpy(np.ascontiguousarray(t))
-    if t.is_sparse:
-        t = t.to_dense()
-    return t.to(device=device, dtype=torch.float32)
-
-
-class PGDAttack(RowBandResult, BaseAttack):
+class PGDAttack(RowBandResult):
 
     def __init__(self, model=None, embedding=None, H_A=None, Y_A=None, nnodes=None, loss_type='CE', feature_shape=None,
                  attack_structure=True, attack_features=False, device='cpu'):
-        super(PGDAttack, self).__init__(model, nnodes, attack_structure, attack_features, device)
-        assert attack_features or attack_structure, 'attack_features or attack_structure cannot be both False'
-        self.loss_type = loss_type
-        self.modified_adj = None
-        self.modified_features = None
-        self.edge_select = None
-        self.complementary = None
+        super().__init__(model, embedding, nnodes, loss_type, feature_shape, attack_structure, attack_features, device)
         self.complementary_after = None
-        self.embedding = embedding
         self.H_A = H_A
         self.Y_A = Y_A
         self._adj_changes_after = None
-        self.engine = None
         self._const_cache = {}
-        if attack_structure:
-            assert nnodes is not None, 'Please give nnodes='
-            self.adj_changes = Parameter(torch.zeros(int(nnodes * (nnodes - 1) / 2)))
-        if attack_features:
-            assert True, 'Topology Attack does not support attack feature'
 
     # the reference allocates a second P-vector eagerly on the host (:73-74); it is materialised on demand here
     @property
@@ -89,26 +64,6 @@ class PGDAttack(RowBandResult, BaseAttack):
         self._adj_changes_after = v
 
     # ------------------------------------------------------------------------------------------------
-    def _victim_weights(self):
-        victim, emb = self.surrogate, self.embedding
-        if len(victim.gc) != 2:
-            raise NotImplementedError("native path is built for the 2-layer GCN victim (main.py --nlayers 2)")
-        W1, b1 = victim.gc[0].weight, victim.gc[0].bias
-        W2, b2 = victim.gc[1].weight, victim.gc[1].bias
-        Wl, bl = victim.linear1.weight, victim.linear1.bias
-        if W1.shape[1] != HID or W2.shape != (HID, HID):
-            raise NotImplementedError("native path is built for nhid=16 (hard-coded in the reference, main.py:175)")
-        if b1 is None or b2 is None or bl is None:
-            raise NotImplementedError("with_bias=False victims are not supported")
-        if not getattr(victim, "with_relu", True):
-            raise NotImplementedError("with_relu=False victims are not supported (the native path hard-codes the relu)")
-        if emb is not None:
-            for k in range(2):   # embedding.gc = deepcopy(victim.gc) in the reference driver (main.py:185-190)
-                if not (torch.equal(emb.gc[k].weight.detach().cpu(), victim.gc[k].weight.detach().cpu())
-                        and torch.equal(emb.gc[k].bias.detach().cpu(), victim.gc[k].bias.detach().cpu())):
-                    raise NotImplementedError("embedding.gc must share the victim's GC weights (main.py:185-190)")
-        return [t.detach().to(self.device, torch.float32).contiguous() for t in (W1, b1, W2, b2, Wl, bl)]
-
     @staticmethod
     def _mm_adj(adj, S):
         return torch.sparse.mm(adj, S) if adj.is_sparse else adj @ S
@@ -121,13 +76,9 @@ class PGDAttack(RowBandResult, BaseAttack):
         if args.max_eval == 1:
             lr_ori = 10 ** args.lr
         self.args = args
-        if self.loss_type != 'CE':
-            raise NotImplementedError("native path implements loss_type='CE' (the reference driver's choice)")
         eps = float(getattr(args, "eps", 0) or 0)
         if eps != 0.0:        # scope of the noisy path, checked before any device work
-            world_ = (torch.distributed.get_world_size()
-                      if torch.distributed.is_available() and torch.distributed.is_initialized() else 1)
-            check_noise_supported(args.measure, world_, feature_adj, self.device)
+            check_noise_supported(args.measure, _rank_world()[1], feature_adj, self.device)
         dev = torch.device(self.device)
         n = self.nnodes
         timing = {} if kwargs.get("_timing") else None      # bench hook: phase wall-clock (adds synchronisations)
@@ -142,23 +93,7 @@ class PGDAttack(RowBandResult, BaseAttack):
                 timing[name] = timing.get(name, 0.0) + now - _t[0]
             _t[0] = now
         _mark("start")
-        # release the previous call's device state first: the allocator can then recycle its blocks instead of growing
-        # (x', m, v, F tiles and the n x n result are tens of GB at n = 65 536; cudaMalloc of such blocks costs ~0.1 s each)
-        self.engine = None
-        self.modified_adj = None
-        victim_model = self.surrogate
-        victim_model.eval()
-        if self.embedding is not None:
-            self.embedding.eval()
-        W1, b1, W2, b2, Wl, bl = self._victim_weights()
-        X = _dense(ori_features, dev)
-        labels_t = torch.as_tensor(np.asarray(labels) if not torch.is_tensor(labels) else labels).long().to(dev)
-        if torch.is_tensor(ori_adj):
-            assert not bool(ori_adj.any()), "reference driver passes init_adj = 0 (dataset.py:433-437)"
-        elif sp.issparse(ori_adj):
-            assert ori_adj.nnz == 0, "reference driver passes init_adj = 0"
-        else:
-            assert not np.any(ori_adj), "reference driver passes init_adj = 0"
+        (W1, b1, W2, b2, Wl, bl), X, labels_t, (rank, world), x0 = self._prepare(ori_features, ori_adj, labels)
         adj_d = adj.to(dev) if torch.is_tensor(adj) else _dense(adj, dev)
         if not adj_d.is_sparse:
             adj_d = adj_d.to(torch.float32)
@@ -188,11 +123,6 @@ class PGDAttack(RowBandResult, BaseAttack):
             fa = feature_adj.to(dev) if torch.is_tensor(feature_adj) else _dense(feature_adj, dev)
         _mark("feature_adj_h2d")
 
-        rank, world = 0, 1
-        if torch.distributed.is_available() and torch.distributed.is_initialized():
-            rank, world = torch.distributed.get_rank(), torch.distributed.get_world_size()
-        x0 = self.adj_changes.data
-        x0 = x0 if bool((x0 != 0).any()) else None
         self.engine = PGDEngine(n, S1, W2, b1, b2, Wl, bl, labels_t, idx_attack, HA_loop, YA_loop, fa,
                                 args.measure, weights, lr_ori, weight_sup=weight_supervised, num_edges=num_edges,
                                 x0=x0, device=dev, rank=rank, world=world,
@@ -272,17 +202,7 @@ class PGDAttack(RowBandResult, BaseAttack):
         import ctypes as _C
         st = N.stream_ptr()
         n, dev, world = eng.n, eng.dev, eng.world
-        # em = embedding(X, adj_norm of the last iteration) == hidden state H2 of the normalised branch
-        zf = torch.empty_like(eng.H2)
-        call("mcgra_row_normalize", ptr(eng.H2), n, HID, 2.0, ptr(zf), st)
-        xf = torch.empty(max(eng.ntiles, 1) * N.TILE * N.TILE, dtype=torch.float32, device=dev)
-        call("mcgra_decode_to_tiles", ptr(zf), n, eng.tr0, eng.tr1, ptr(xf), st)
-        if gather_x or world == 1:      # the reference leaves the full packed vector in adj_changes.data (:301)
-            # (with world > 1 every rank writes its tile rows' entries and the shards are summed)
-            packed = (torch.empty if world == 1 else torch.zeros)(n * (n - 1) // 2, dtype=torch.float32, device=dev)
-            call("mcgra_tiles_to_tril", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(packed), st)
-            eng._allreduce(packed)
-            self.adj_changes.data = packed
+        zf, xf = self._decode_last(eng, gather_x)        # adj_changes.data (:301)
         # embeddings / victim output on the raw decoded adjacency (:304-308): two propagations over xf
         Y = torch.zeros(n, HID, dtype=torch.float32, device=dev)
         call("mcgra_propagate", ptr(xf), n, eng.tr0, eng.tr1, None, 1, ptr(eng.S1), HID, ptr(Y), ptr(eng.prop_ws), st)
@@ -349,96 +269,18 @@ class PGDAttack(RowBandResult, BaseAttack):
         self.modified_adj_rows = (b0, b1_)
 
     # ------------------------------------------------------------------------------------------------
-    # stand-alone helpers of the reference class, same names and semantics
-    def get_modified_adj(self, ori_adj=None):
-        """Symmetric zero-diagonal expansion of adj_changes (+ ori_adj) (topology_attack.py:365-379)."""
-        return self._expand(self.adj_changes.data, ori_adj)
-
+    # stand-alone helpers of the reference class, same names and semantics (more in base_attack.RowBandResult)
     def get_modified_adj2(self, ori_adj, adj_changes):
         return self._expand(adj_changes, ori_adj)
 
     def get_modified_adj_after(self, ori_adj=None):
         return self._expand(self.adj_changes_after, ori_adj)
 
-    def _expand(self, packed, ori_adj=None):
-        dev = torch.device(self.device)
-        n = self.nnodes
-        T = (n + N.TILE - 1) // N.TILE
-        st = N.stream_ptr()
-        xp = packed.detach().to(dev, torch.float32).contiguous()
-        tiles = torch.empty(T * (T + 1) // 2 * N.TILE * N.TILE, dtype=torch.float32, device=dev)
-        call("mcgra_tril_to_tiles", ptr(xp), n, 0, T, ptr(tiles), st)
-        out = torch.zeros(n, n, dtype=torch.float32, device=dev)
-        call("mcgra_tiles_to_dense", ptr(tiles), n, 0, T, None, 1, ptr(out), n, st)
-        if ori_adj is not None and torch.is_tensor(ori_adj) and bool(ori_adj.any()):
-            out = out + ori_adj.to(dev)
-        return out
-
-    def dot_product_decode(self, Z):
-        """tril(relu(Zn Zn^T)), Zn = F.normalize(Z) (topology_attack.py:414-419) -> packed P-vector."""
-        dev = torch.device(self.device)
-        n = Z.shape[0]
-        if Z.shape[1] != HID:
-            raise NotImplementedError("native decode is built for 16-wide embeddings")
-        T = (n + N.TILE - 1) // N.TILE
-        st = N.stream_ptr()
-        Zc = Z.detach().to(dev, torch.float32).contiguous()
-        zn = torch.empty_like(Zc)
-        call("mcgra_row_normalize", ptr(Zc), n, HID, 2.0, ptr(zn), st)
-        tiles = torch.empty(T * (T + 1) // 2 * N.TILE * N.TILE, dtype=torch.float32, device=dev)
-        call("mcgra_decode_to_tiles", ptr(zn), n, 0, T, ptr(tiles), st)
-        packed = torch.empty(n * (n - 1) // 2, dtype=torch.float32, device=dev)
-        call("mcgra_tiles_to_tril", ptr(tiles), n, 0, T, None, 1, ptr(packed), st)
-        return packed
-
     def dot_product_decode2(self, Z):
         n = Z.shape[0]
         out = torch.zeros(n, n, dtype=torch.float32, device=torch.device(self.device))
         self._gram_add(out, Z.detach().to(self.device))
         return out
-
-    def projection(self, num_edges):
-        """Stand-alone projection of adj_changes (topology_attack.py:338-347) on the device bisection."""
-        dev = torch.device(self.device)
-        n = self.nnodes
-        T = (n + N.TILE - 1) // N.TILE
-        st = N.stream_ptr()
-        x = self.adj_changes.data.detach().to(dev, torch.float32).contiguous()
-        tiles = torch.empty(T * (T + 1) // 2 * N.TILE * N.TILE, dtype=torch.float32, device=dev)
-        call("mcgra_tril_to_tiles", ptr(x), n, 0, T, ptr(tiles), st)
-        acc = torch.zeros(N.ACC_N, dtype=torch.float64, device=dev)
-        acc[N.ACC["SUMCLAMP"]] = torch.clamp(x, 0, 1).double().sum()
-        minmax = torch.stack([x.min(), x.max()]).contiguous()
-        state = torch.zeros(8, dtype=torch.float32, device=dev)
-        mu = torch.zeros(1, dtype=torch.float32, device=dev)
-        cand = torch.zeros(8, dtype=torch.float64, device=dev)
-        call("mcgra_bisect_init", ptr(acc), ptr(minmax), float(num_edges), ptr(state), ptr(mu), st)
-        for _ in range(10):
-            call("mcgra_bisect_pass", ptr(tiles), n, 0, T, 1e-5, ptr(state), ptr(cand), st)
-            call("mcgra_bisect_update", float(num_edges), 1e-5, ptr(state), ptr(cand), ptr(mu), st)
-        out = torch.empty_like(x)
-        call("mcgra_tiles_to_tril", ptr(tiles), n, 0, T, ptr(mu), 0, ptr(out), st)
-        self.adj_changes.data.copy_(out)
-
-    def bisection(self, a, b, num_edges, epsilon):
-        """Root of sum(clamp(adj_changes - mu, 0, 1)) = num_edges on [a, b] (topology_attack.py:397-412) on the device
-        bisection kernels (same fp32 midpoints as the scalar loop, three halvings per pass over the parameter)."""
-        dev = torch.device(self.device)
-        n = self.nnodes
-        T = (n + N.TILE - 1) // N.TILE
-        st = N.stream_ptr()
-        x = self.adj_changes.data.detach().to(dev, torch.float32).contiguous()
-        tiles = torch.empty(T * (T + 1) // 2 * N.TILE * N.TILE, dtype=torch.float32, device=dev)
-        call("mcgra_tril_to_tiles", ptr(x), n, 0, T, ptr(tiles), st)
-        a, b = float(a), float(b)
-        state = torch.tensor([a, b, a, 0.0, 1.0, 0.0, 0.0, 0.0], dtype=torch.float32, device=dev)
-        mu = torch.full((1,), a, dtype=torch.float32, device=dev)
-        cand = torch.zeros(8, dtype=torch.float64, device=dev)
-        passes = max(1, int(np.ceil(np.log2(max(b - a, epsilon) / epsilon) / 3.0)) + 1)
-        for _ in range(passes):
-            call("mcgra_bisect_pass", ptr(tiles), n, 0, T, float(epsilon), ptr(state), ptr(cand), st)
-            call("mcgra_bisect_update", float(num_edges), float(epsilon), ptr(state), ptr(cand), ptr(mu), st)
-        return mu[0]
 
     def adding_noise(self, modified_adj, eps=0):
         """clamp(M + eps * N(0,1), 0, 1) in place on M (topology_attack.py:474-478).  The draw comes from torch's CUDA
@@ -478,14 +320,3 @@ class PGDAttack(RowBandResult, BaseAttack):
         adj_norm = utils.normalize_adj_tensor(adj)
         output = victim_model(features, adj_norm)
         return utils.accuracy(output[idx_test], labels[idx_test]).item()
-
-    def _loss(self, output, labels):
-        if self.loss_type == "CE":
-            return F.nll_loss(output, labels)
-        if self.loss_type == "CW":       # topology_attack.py:329-335 (stand-alone helper; the loop uses CE)
-            onehot = torch.eye(int(labels.max()) + 1, device=output.device)[labels]
-            best_second_class = (output - 1000 * onehot).argmax(1)
-            ar = torch.arange(len(output), device=output.device)
-            margin = output[ar, labels] - output[ar, best_second_class]
-            return -torch.clamp(margin, min=0).mean()
-        raise ValueError(self.loss_type)
