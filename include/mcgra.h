@@ -78,6 +78,8 @@ int mcgra_version(void);
  *                           sampled keys + one 32-byte block per segment beyond that [default]
  * Returns 0, or -1 (and changes nothing) for any other selector or value.                                              */
 int mcgra_set_engine(int which, int value);
+/* the current engine of stage `which` (0, 1, 2, 4, 5 or 6; not the grid caps), -1 for any other selector */
+int mcgra_get_engine(int which);
 int64_t mcgra_tiles_in_rows(int tr0, int tr1);           /* number of tiles in tile rows [tr0,tr1) */
 
 /* ---- layout (replaces torch.tril_indices + index_put + m+m.t(), topology_attack.py:365-379) ---- */

@@ -105,6 +105,7 @@ class EnsembleArgs(C.Structure):
 _SIGS = {
     "mcgra_version": (C.c_int, []),
     "mcgra_set_engine": (C.c_int, [C.c_int, C.c_int]),
+    "mcgra_get_engine": (C.c_int, [C.c_int]),
     "mcgra_tiles_in_rows": (i64, [C.c_int, C.c_int]),
     "mcgra_tril_to_tiles": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, c_fp]),
     "mcgra_tiles_to_tril": (C.c_int, [c_fp, i64, C.c_int, C.c_int, c_fp, C.c_int, c_fp, c_fp]),
@@ -220,10 +221,6 @@ def lib():
             fn.restype = res
             fn.argtypes = args
         _lib = L
-        # developer override for same-box A/B runs and profiling: MCGRA_ENGINES="0:5,1:2" (stage:engine, see mcgra.h)
-        for item in filter(None, os.environ.get("MCGRA_ENGINES", "").split(",")):
-            which, value = item.split(":")
-            check(L.mcgra_set_engine(int(which), int(value)), f"MCGRA_ENGINES entry {item!r}")
     return _lib
 
 
@@ -254,7 +251,7 @@ LAUNCHES = {"count": 0, "kernels": 0}
 # propagate = k_colmax + k_prep_b16 + k_propagate_h; fold_adam = k_prep_w + k_fold_tc; auc_ap = compact + 4 x (hist, scan,
 # scatter) + rank + finish; argsort_desc = make_keys + 4 x 3
 KERNELS_PER_CALL = {"mcgra_propagate": 3, "mcgra_propagate_sel": 3, "mcgra_noise_stage": 2, "mcgra_fold_adam": 2, "mcgra_auc_ap": 15, "mcgra_argsort_desc": 13,
-                    "mcgra_version": 0, "mcgra_set_engine": 0, "mcgra_tiles_in_rows": 0, "mcgra_propagate_ws_bytes": 0,
+                    "mcgra_version": 0, "mcgra_set_engine": 0, "mcgra_get_engine": 0, "mcgra_tiles_in_rows": 0, "mcgra_propagate_ws_bytes": 0,
                     "mcgra_fold_ws_bytes": 0, "mcgra_auc_workspace_bytes": 0, "mcgra_sort_workspace_bytes": 0,
                     "mcgra_pairs_ws_bytes": 0, "mcgra_auc_hist_offset": 0, "mcgra_topk_workspace_bytes": 0, "mcgra_auc_stage": 5, "mcgra_gram_auc_workspace_bytes": 0, "mcgra_nd_scratch_doubles": 0, "mcgra_nd_scratch_floats": 0, "mcgra_nd_measure": 5,
                     "mcgra_image_from_dense": 2, "mcgra_smooth": 2, "mcgra_center_dense": 2, "mcgra_sym_to_tiles": 2}

@@ -580,7 +580,6 @@ k_rank_negatives_tab(const Src src, const uint32_t* __restrict__ U, const uint32
   }
 }
 
-int g_auc_engine = 1;      // mcgra_set_engine(6, v): 0 k_rank_negatives (1024-sample table), 1 k_rank_negatives_tab (default)
 constexpr int TAB_CAP_MAX = 57344;      // 224 KB of dynamic shared memory
 
 // suffix sums of hist -> fp(>= pos[t]) = sum_{j > t} hist[j]; AP over distinct positive values.  Single block.
@@ -728,12 +727,6 @@ k_gram_pos(const float* __restrict__ Z, int d, const int64_t* __restrict__ rowpt
 
 extern "C" {
 
-int mcgra_set_auc_engine_(int value) {
-  if (value != 0 && value != 1) return -1;
-  g_auc_engine = value;
-  return 0;
-}
-
 // workspace layout (bytes): [counter+sums 256][poskeys cap*4][poskeys_tmp cap*4][hist_sort][offs_sort][hist cap+1 u64]
 // [start indices of the distinct keys cap+1 u32][segment blocks 57 344 x 32 B]   (counter block: [0] npos, [1..2] sums, [3] number of distinct keys)
 int64_t mcgra_auc_workspace_bytes(int64_t N, int64_t npos_max) {
@@ -781,7 +774,7 @@ int mcgra_auc_stage(int stage, const float* scores, const uint8_t* labels, int64
   } else if (stage == 1) {
     int rc = radix_sort<uint32_t>(pos, nullptr, pos_tmp, nullptr, npos_max, hs, offs, st);
     if (rc) return rc;
-    if (N > 0 && g_auc_engine == 1 && npos_max < (1LL << 28)) {      // (per-round 32-bit partial sums: 12 npos < 2^32)
+    if (N > 0 && g_engines.auc == 1 && npos_max < (1LL << 28)) {      // (per-round 32-bit partial sums: 12 npos < 2^32)
       return rank_tab(DenseNegatives{scores, labels, N}, pos, pos_tmp, counter, hist, sums, npos_max, st);
     } else if (N > 0) {
       k_rank_negatives<<<148 * 8, 256, 0, st>>>(scores, labels, N, pos, counter, hist, sums);

@@ -16,6 +16,31 @@
     if (e__ != cudaSuccess) return (int)e__;         \
   } while (0)
 
+// The kernel engine of each stage that has more than one (mcgra_set_engine / mcgra_get_engine, include/mcgra.h; the
+// table and its defaults are in propagate.cu).  Engine 0 of every stage is the exact reference of the agreement tests.
+struct EngineTable {
+  int propagate;   // stage 0: mcgra_propagate_sel
+  int fold;        // stage 1: mcgra_fold_adam
+  int fold_grid;   //          cap on fold engine 3's persistent grid (0 = one CTA per SM)
+  int pairs;       // stage 2: mcgra_pairs
+  int elem;        // stage 4: mcgra_elem_stats
+  int elem_grid;   //          cap on element-wise engine 1's persistent grid (0 = one CTA per SM)
+  int ensemble;    // stage 5: mcgra_ensemble
+  int auc;         // stage 6: stage 1 of mcgra_auc_stage
+};
+extern EngineTable g_engines;
+
+// number of SMs of the current device, queried on the first call
+inline int sm_count() {
+  static int sms = 0;
+  if (sms == 0) {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  }
+  return sms;
+}
+
 __host__ __device__ __forceinline__ int64_t tri(int64_t I) { return I * (I + 1) / 2; }
 
 // linear (global) tile index -> (I, J), J <= I

@@ -948,9 +948,6 @@ k_fold_rs(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restrict
   if (warp == 2) tc::tmem_dealloc(tm, 512);
 }
 
-int g_fold_engine = 3;     // 0 = exact fp32 FFMA (reference of the agreement tests), 2 = tcgen05 one tile per CTA (k_fold_tc: every
-                           // parameter view / measure), 3 = persistent row-run tcgen05 (k_fold_rs) for fast launches, k_fold_tc otherwise
-
 // ---------------------------------------------------------------------------------------------------------
 // Bisection on device.  state: [0]=a [1]=b [2]=mu(last midpoint) [3]=done [4]=active
 // One pass evaluates the 7 midpoints of a depth-3 bisection tree rooted at (a,b); the update walks the tree
@@ -1121,14 +1118,6 @@ __global__ void k_bisect_reset(int64_t n, const float* state, double* acc_next, 
 
 extern "C" {
 
-int g_fold_ws_grid = 0;     // test knob: cap on the persistent grid (0 = one CTA per SM), mcgra_set_engine(1, 100 + cap)
-int mcgra_set_fold_engine_(int value) {
-  if (value >= 100 && value < 1000) g_fold_ws_grid = value - 100;
-  else if (value == 0 || value == 2 || value == 3) g_fold_engine = value;
-  else return -1;
-  return 0;
-}
-
 int64_t mcgra_fold_ws_bytes(int64_t n) { return ((n + TILE - 1) / TILE) * (int64_t)WBLOCK + 256; }
 
 int mcgra_fold_adam(float* tiles, float* m, float* v, int tr0, int tr1, const float* mu, int raw,
@@ -1138,16 +1127,10 @@ int mcgra_fold_adam(float* tiles, float* m, float* v, int tr0, int tr1, const fl
   const bool lazy = raw == 0 && !a->store_clamped;        // un-projected buffer + mu (the budget may bind)
   const bool fastable = ((raw == 2 && a->store_clamped) || lazy) && a->k2 == 0.f && a->measure != MCGRA_M_KL && !a->plain_gd &&
                         a->Gtiles == nullptr && !(a->measure != MCGRA_M_NONE && a->Ftiles == nullptr);
-  if (g_fold_engine == 3 && a->Wk != nullptr && fastable) {
+  if (g_engines.fold == 3 && a->Wk != nullptr && fastable) {
     const int64_t np = a->npad;
     k_prep_w<<<(unsigned)((np * 128 + 255) / 256), 256, 0, (cudaStream_t)stream>>>(a->Wt, np, (unsigned char*)a->Wk);
-    static int sms = 0;
-    if (sms == 0) {
-      int dev = 0;
-      cudaGetDevice(&dev);
-      cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    }
-    const int cap = g_fold_ws_grid > 0 ? g_fold_ws_grid : sms;
+    const int cap = g_engines.fold_grid > 0 ? g_engines.fold_grid : sm_count();
     const unsigned grid = (unsigned)(nt < cap ? nt : cap);
     const size_t smem4 = sizeof(FoldRsSmem) + 1024;
     const unsigned char* wk = (const unsigned char*)a->Wk;
@@ -1170,7 +1153,7 @@ int mcgra_fold_adam(float* tiles, float* m, float* v, int tr0, int tr1, const fl
     MCGRA_LAUNCH_CHECK();
     return 0;
   }
-  if (g_fold_engine >= 2 && a->Wk != nullptr) {
+  if (g_engines.fold >= 2 && a->Wk != nullptr) {
     const int64_t np = a->npad;
     k_prep_w<<<(unsigned)((np * 128 + 255) / 256), 256, 0, (cudaStream_t)stream>>>(a->Wt, np, (unsigned char*)a->Wk);
     const size_t smem3 = sizeof(FoldTcSmem) + 1024;

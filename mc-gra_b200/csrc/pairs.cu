@@ -424,9 +424,6 @@ k_pairs_mma(const float* __restrict__ tiles, int64_t n, int64_t t0, const float*
   if (k2 != 0.f) block_atomic_add_d((double)v2 * (double)k2, acc + MCGRA_ACC_C2, sm.red);
 }
 
-int g_ensemble_engine = 1;  // mcgra_set_engine(5, v): 0 one CTA per 64 x 64 block, 1 one CTA per block PAIR for the full matrix (default)
-int g_pairs_engine = 2;     // 0 fp32 FFMA (exact), 1 mma.sync 3xTF32, 2 tcgen05 for the entropy-only configuration (else 1)
-
 // x_final tiles = relu(z_i . z_j), j < i < n  (dot_product_decode of the last embedding, :300-301)
 // Register-tiled: thread (tx, ty) owns rows 8 ty .. + 7 and columns 8 tx .. + 7 of the tile; factors staged transposed
 // ([k][row], pitch 132) so that one k step is four 16-byte shared loads for 64 FMAs (the scalar form was LDS-bound:
@@ -945,17 +942,6 @@ int launch_pairs_mma(const float* tiles, int64_t n, int tr0, int64_t nt, const f
 
 extern "C" {
 
-int mcgra_set_pairs_engine_(int value) {
-  if (value < 0 || value > 2) return -1;
-  g_pairs_engine = value;
-  return 0;
-}
-int mcgra_set_ensemble_engine_(int value) {
-  if (value != 0 && value != 1) return -1;
-  g_ensemble_engine = value;
-  return 0;
-}
-
 int mcgra_pairs_tc_(int64_t n, int tr0, int tr1, const float* zhat, float k7, float* dzhat, double* acc, void* ws,
                     cudaStream_t st);
 
@@ -965,9 +951,9 @@ int mcgra_pairs(const float* tiles, int64_t n, int tr0, int tr1, const float* mu
   const int64_t nt = tri(tr1) - tri(tr0);
   if (nt <= 0) return 0;
   // engine 2: the entropy-only configuration (README Cora profile) entirely on tcgen05, no HBM stream (pairs_tc.cu)
-  if (g_pairs_engine == 2 && ws != nullptr && k7 != 0.f && k2 == 0.f && EAt == nullptr && Ct == nullptr)
+  if (g_engines.pairs == 2 && ws != nullptr && k7 != 0.f && k2 == 0.f && EAt == nullptr && Ct == nullptr)
     return mcgra_pairs_tc_(n, tr0, tr1, zhat, k7, dzhat, acc, ws, (cudaStream_t)stream);
-  if (g_pairs_engine >= 1) {
+  if (g_engines.pairs >= 1) {
     const bool f7 = k7 != 0.f, f2 = k2 != 0.f, fd = (EAt != nullptr) || (Ct != nullptr);
 #define MCGRA_PAIRS_CASE(A, B, D)                                                                                  \
     if (f7 == A && f2 == B && fd == D)                                                                             \
@@ -1025,7 +1011,7 @@ int mcgra_ensemble(const float* tiles, int64_t n, const mcgra_ensemble_args* arg
   for (int t = 0; t < args->nterms; ++t)
     if (args->t[t].kind == MCGRA_TERM_GRAM && (args->t[t].d < 1 || args->t[t].d > 32)) return -1;
   if (row1 <= row0) return 0;
-  if (g_ensemble_engine == 1 && row0 == 0 && row1 >= n) {       // full matrix: block pairs (I >= J), both orientations per CTA
+  if (g_engines.ensemble == 1 && row0 == 0 && row1 >= n) {       // full matrix: block pairs (I >= J), both orientations per CTA
     const int64_t nb = (n + EB - 1) / EB, pairs = nb * (nb + 1) / 2;
     if (pairs > 2147483647LL) return -3;
     k_ensemble_sym<<<(unsigned)pairs, 256, 0, (cudaStream_t)stream>>>(tiles, n, *args, out, ld);

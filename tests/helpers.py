@@ -1,4 +1,5 @@
-"""Shared helpers for the GPU parity tests: run the native attack on a golden fixture."""
+"""Shared helpers for the GPU parity tests: run the native attack on a golden fixture, switch kernel engines."""
+import contextlib
 import os
 import tempfile
 from copy import deepcopy
@@ -9,6 +10,27 @@ import torch
 
 class Args:
     pass
+
+
+@contextlib.contextmanager
+def engines(values, caps=None):
+    """Run the block with the kernel engines `values` ({stage: engine}, mcgra_set_engine in include/mcgra.h) and the
+    persistent-grid caps `caps` ({stage: CTAs} for stages 1 and 4).  On exit, even on failure, every stage in `values`
+    gets its previous engine back and the grid caps are off."""
+    from mcgra_b200 import _native as N
+    L = N.lib()
+    saved = {which: L.mcgra_get_engine(which) for which in values}
+    try:
+        for which, value in values.items():
+            assert L.mcgra_set_engine(which, value) == 0, (which, value)
+        for which, cap in (caps or {}).items():
+            assert L.mcgra_set_engine(which, 100 + cap) == 0, (which, cap)
+        yield
+    finally:
+        for which, value in saved.items():
+            assert L.mcgra_set_engine(which, value) == 0, (which, value)
+        for which in (1, 4):
+            assert L.mcgra_set_engine(which, 100) == 0
 
 
 def make_models(d, device):

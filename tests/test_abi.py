@@ -3,6 +3,7 @@ include/mcgra.h declares (no compute calls -- there is no GPU here)."""
 import ctypes
 import os
 import re
+import shutil
 
 import pytest
 
@@ -39,7 +40,17 @@ def test_version_and_tile_count(native):
     assert L.mcgra_tiles_in_rows(2, 4) == 7
 
 
+# bench.py's large_parity restores {0: 5, 1: 3, 2: 2} after its exact-engine run, so these must stay the defaults
 DEFAULT_ENGINES = {0: 5, 1: 3, 2: 2, 4: 1, 5: 1, 6: 1}
+
+
+def test_fresh_library_reports_default_engines(native, tmp_path):
+    # a copy under another path is loaded as a second instance, with engine state no earlier test has touched
+    fresh = tmp_path / "libmcgra_fresh.so"
+    shutil.copyfile(native.LIB_PATH, fresh)
+    L = ctypes.CDLL(str(fresh))
+    assert {which: L.mcgra_get_engine(which) for which in DEFAULT_ENGINES} == DEFAULT_ENGINES
+    assert [L.mcgra_get_engine(which) for which in (-1, 3, 7)] == [-1, -1, -1]
 
 
 def test_set_engine_accepts_only_known_values(native):
@@ -47,14 +58,20 @@ def test_set_engine_accepts_only_known_values(native):
     accepted = {0: [0, 5], 1: [0, 2, 3, 100, 101, 999], 2: [0, 1, 2], 4: [0, 1, 100, 101, 999], 5: [0, 1], 6: [0, 1]}
     rejected = [(3, 1), (3, 2), (3, 116), (0, 3), (0, 1), (0, 101), (1, 1), (1, 4), (1, 1007), (1, 1000), (1, -1),
                 (2, 3), (2, -1), (4, 2), (4, 1000), (5, 2), (6, 2), (6, 101), (7, 0), (-1, 0)]
+    saved = {which: L.mcgra_get_engine(which) for which in accepted}
     try:
         for which, values in accepted.items():
             for value in values:
                 assert L.mcgra_set_engine(which, value) == 0, (which, value)
+                if value < 100:                     # 100 + cap sets the grid cap and leaves the engine as it is
+                    engine = value
+                assert L.mcgra_get_engine(which) == engine, (which, value)
         for which, value in rejected:
+            before = L.mcgra_get_engine(which)
             assert L.mcgra_set_engine(which, value) == -1, (which, value)
+            assert L.mcgra_get_engine(which) == before, (which, value)
     finally:
-        for which, value in DEFAULT_ENGINES.items():
+        for which, value in saved.items():
             assert L.mcgra_set_engine(which, value) == 0
         assert L.mcgra_set_engine(1, 100) == 0 and L.mcgra_set_engine(4, 100) == 0     # grid caps off
 

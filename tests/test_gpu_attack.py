@@ -8,7 +8,7 @@ import pytest
 import torch
 
 import pgd_oracle as O
-from helpers import run_native_case
+from helpers import engines, run_native_case
 
 pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -108,24 +108,25 @@ def test_multi_tile_matches_oracle(n, measure, weights, density):
     np.testing.assert_allclose(got["modified_adj"], ref["modified_adj"].numpy(), rtol=1e-3, atol=1e-3)
 
 
-DEFAULT_ENGINE = {0: 5, 1: 3, 2: 2, 4: 1}      # propagate: tcgen05 fp16x2 (v5); fold: persistent row-run tcgen05 (TMEM-resident A); pairs: tcgen05 (entropy-only) / mma.sync
-
-
-@pytest.mark.parametrize("which,eng", [(0, 5), (1, 2), (1, 3), (2, 1), (4, 1)])
-def test_engines_agree(which, eng):
+@pytest.mark.parametrize("which,eng,case,rtol,dx", [
+    pytest.param(0, 5, "mse_all_n150", 2e-6, 2e-5, id="0-5"),
+    pytest.param(0, 5, "kl_C_n150", 2e-5, 5e-5, id="0-5-kl_C_n150"),
+    pytest.param(1, 2, "mse_all_n150", 2e-6, 2e-5, id="1-2"),
+    pytest.param(1, 3, "mse_all_n150", 2e-6, 2e-5, id="1-3"),
+    pytest.param(2, 1, "mse_all_n150", 2e-6, 2e-5, id="2-1"),
+    pytest.param(4, 1, "mse_all_n150", 2e-6, 2e-5, id="4-1"),
+])
+def test_engines_agree(which, eng, case, rtol, dx):
     """exact-fp32 FFMA engine 0 vs the tensor-core engines of propagate (0: tcgen05 fp16x2) / fold (1: tcgen05 3xTF32,
-    one tile per CTA and persistent row runs) / pairs (2: mma.sync 3xTF32) on the same inputs."""
-    from mcgra_b200 import _native as N
-    d = np.load(os.path.join(GOLDEN, "attack_mse_all_n150.npz"))
-    try:
-        N.lib().mcgra_set_engine(which, 0)
+    one tile per CTA and persistent row runs) / pairs (2: mma.sync 3xTF32) / element-wise pass (4: persistent) on the
+    same inputs."""
+    d = np.load(os.path.join(GOLDEN, f"attack_{case}.npz"))
+    with engines({which: 0}):
         a = run_native_case(d)
-        N.lib().mcgra_set_engine(which, eng)
+    with engines({which: eng}):
         b = run_native_case(d)
-    finally:
-        N.lib().mcgra_set_engine(which, DEFAULT_ENGINE[which])
-    np.testing.assert_allclose(a["loss"], b["loss"], rtol=2e-6)
-    assert np.max(np.abs(np.stack(a["x_iters"]) - np.stack(b["x_iters"]))) < 2e-5
+    np.testing.assert_allclose(a["loss"], b["loss"], rtol=rtol)
+    assert np.max(np.abs(np.stack(a["x_iters"]) - np.stack(b["x_iters"]))) < dx
 
 
 FOLD_WSETS = {"mse_ent": {1: 0.01, 6: 10.0, 7: 10.0, 9: 10.0, 10: 1000.0},       # k_fold_rs<MSE, entropy>
@@ -143,17 +144,11 @@ def test_fold_persistent_engine_multi_tile(eng, density, grid, wset):
     clamped-parameter view from the second iteration (clamped store), density 1 = budget binds (lazily projected view,
     un-clamped store, min / max for the bisection); the weight sets select the kernel's template variants."""
     from helpers import synthetic_case
-    from mcgra_b200 import _native as N
     d = synthetic_case(1500, 40, 5, weights=FOLD_WSETS[wset], epochs=4, density=density, mean_deg=8.0)
-    try:
-        N.lib().mcgra_set_engine(1, 2)
+    with engines({1: 2}):
         a = run_native_case(d)
-        N.lib().mcgra_set_engine(1, eng)
-        N.lib().mcgra_set_engine(1, 100 + grid)
+    with engines({1: eng}, caps={1: grid}):
         b = run_native_case(d)
-    finally:
-        N.lib().mcgra_set_engine(1, 100)
-        N.lib().mcgra_set_engine(1, DEFAULT_ENGINE[1])
     # (not bit-equal: the degree row sums and the norm term are accumulated with float / double atomics in tile order.  When
     #  the budget binds, a bisection decision at the 1e-5 bracket can flip on such a difference -- run to run, with either
     #  engine: the atomics' order is not fixed -- and shift mu, i.e. EVERY free entry, by up to 1e-5 per iteration: up to
@@ -175,17 +170,11 @@ def test_elem_persistent_engine_multi_tile(grid):
     """element-wise pass: bulk-staged persistent kernel (engine 1 of stage 4) against the one-tile-per-CTA kernel with
     several tiles and tile rows per CTA (n = 1500, ragged last row, grid capped to 5 CTAs / uncapped)."""
     from helpers import synthetic_case
-    from mcgra_b200 import _native as N
     d = synthetic_case(1500, 40, 5, weights={1: 0.01, 6: 10.0, 7: 10.0, 9: 10.0, 10: 1000.0}, epochs=4, mean_deg=8.0)
-    try:
-        N.lib().mcgra_set_engine(4, 0)
+    with engines({4: 0}):
         a = run_native_case(d)
-        N.lib().mcgra_set_engine(4, 1)
-        N.lib().mcgra_set_engine(4, 100 + grid)
+    with engines({4: 1}, caps={4: grid}):
         b = run_native_case(d)
-    finally:
-        N.lib().mcgra_set_engine(4, 100)
-        N.lib().mcgra_set_engine(4, DEFAULT_ENGINE[4])
     np.testing.assert_allclose(a["loss"], b["loss"], rtol=1e-6)
     assert np.max(np.abs(np.stack(a["x_iters"]) - np.stack(b["x_iters"]))) < 5e-6
 
@@ -195,18 +184,14 @@ def test_pairs_tcgen05_engine_agrees(n, f, epochs):
     """pairs engine 2 (pairs_tc.cu: gram, coefficient planes and both skinny products on tcgen05, entropy-only
     configuration = README Cora profile) vs the exact fp32 FFMA engine 0; n = 4500 crosses the 32-tile run boundary."""
     from helpers import synthetic_case
-    from mcgra_b200 import _native as N
     if n == 150:
         d = np.load(os.path.join(GOLDEN, "attack_mse_A_n150.npz"))
     else:
         d = synthetic_case(n, f, 5, weights={1: 0.01, 6: 10, 7: 10, 9: 10, 10: 1000}, epochs=epochs, mean_deg=8.0)
-    try:
-        N.lib().mcgra_set_engine(2, 0)
+    with engines({2: 0}):
         a = run_native_case(d, epochs=epochs, trace=(n < 2000))
-        N.lib().mcgra_set_engine(2, 2)
+    with engines({2: 2}):
         b = run_native_case(d, epochs=epochs, trace=(n < 2000))
-    finally:
-        N.lib().mcgra_set_engine(2, DEFAULT_ENGINE[2])
     # c7 = -k mean(q log2 q) is ill-conditioned when the decode gram saturates (q -> 1 - 1e-4: q log2 q ~ -(1 - q) / ln 2, so
     # an fp32 rounding of s = <z_i, z_j> ~ 1e-7 is ~1e-3 of the value -- for the reference's own fp32 GEMM as well): the term
     # is compared on the scale of the loss it enters, the kernels themselves agree with fp64 to 1e-7 on well-conditioned
@@ -222,35 +207,13 @@ def test_pairs_tcgen05_engine_agrees(n, f, epochs):
 
 
 @pytest.mark.parametrize("eng", [5])
-@pytest.mark.parametrize("case", ["mse_all_n150", "kl_C_n150"])
-def test_tcgen05_propagate_engine_agrees(case, eng):
-    """tcgen05 propagate engines (2: direct product on tcgen05/TMEM + mirrored on mma.sync; 4: both on tcgen05 with the
-    transposed operand in tensor memory) vs the exact-fp32 FFMA engine."""
-    from mcgra_b200 import _native as N
-    d = np.load(os.path.join(GOLDEN, f"attack_{case}.npz"))
-    try:
-        N.lib().mcgra_set_engine(0, 0)
-        a = run_native_case(d)
-        N.lib().mcgra_set_engine(0, eng)
-        b = run_native_case(d)
-    finally:
-        N.lib().mcgra_set_engine(0, DEFAULT_ENGINE[0])
-    np.testing.assert_allclose(a["loss"], b["loss"], rtol=2e-5)
-    assert np.max(np.abs(np.stack(a["x_iters"]) - np.stack(b["x_iters"]))) < 5e-5
-
-
-@pytest.mark.parametrize("eng", [5])
 def test_tcgen05_propagate_multi_tile(eng):
     from helpers import synthetic_case
-    from mcgra_b200 import _native as N
     d = synthetic_case(1300, 40, 5, weights={1: 0.5, 2: 0.3, 6: 2.0, 7: 3.0, 9: 1.5, 10: 50.0}, epochs=2, mean_deg=8.0)
-    try:
-        N.lib().mcgra_set_engine(0, 0)
+    with engines({0: 0}):
         a = run_native_case(d)
-        N.lib().mcgra_set_engine(0, eng)
+    with engines({0: eng}):
         b = run_native_case(d)
-    finally:
-        N.lib().mcgra_set_engine(0, DEFAULT_ENGINE[0])
     np.testing.assert_allclose(a["loss"], b["loss"], rtol=2e-5)
     assert np.max(np.abs(np.stack(a["x_iters"]) - np.stack(b["x_iters"]))) < 5e-5
 

@@ -9,7 +9,7 @@ import pytest
 import torch
 
 import pgd_oracle as O
-from helpers import make_args, make_models, synthetic_case
+from helpers import engines, make_args, make_models, synthetic_case
 
 pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -141,15 +141,10 @@ def test_eps_gradient_matches_autograd(eps):
 @pytest.mark.parametrize("which", [0, 1])
 def test_eps_exact_engines_agree(which):
     """exact-fp32 FFMA propagate (0) / fold (1) against the default tensor-core engines on the noisy path."""
-    from mcgra_b200 import _native as N
-    default = {0: 5, 1: 3}[which]
     d = noisy_case(0.05)
     noise = draws(11, 700, 3)
-    try:
-        N.lib().mcgra_set_engine(which, 0)
+    with engines({which: 0}):
         a = run_noisy(d, noise=noise)
-    finally:
-        N.lib().mcgra_set_engine(which, default)
     b = run_noisy(d, noise=noise)
     np.testing.assert_allclose(a["loss"], b["loss"], rtol=5e-6)
     assert np.max(np.abs(np.stack(a["x_iters"]) - np.stack(b["x_iters"]))) < 2e-5

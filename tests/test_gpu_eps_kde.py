@@ -15,7 +15,7 @@ import pytest
 import torch
 
 import pgd_oracle as O
-from helpers import synthetic_case
+from helpers import engines, synthetic_case
 from test_gpu_eps import draws, oracle_noisy, run_noisy
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -97,15 +97,10 @@ def test_eps_kde_trajectory_matches_fp64_oracle(config):
 @pytest.mark.parametrize("which", [0, 1])
 def test_eps_kde_exact_engines_agree(which):
     """exact-fp32 FFMA propagate (0) / fold (1) against the default tensor-core engines on the noisy KDE path."""
-    from mcgra_b200 import _native as N
-    default = {0: 5, 1: 3}[which]
     d = kde_case(ALL, -2.0, 0.05)
     noise = draws(11, 700, 3)
-    try:
-        N.lib().mcgra_set_engine(which, 0)
+    with engines({which: 0}):
         a = run_noisy(d, noise=noise)
-    finally:
-        N.lib().mcgra_set_engine(which, default)
     b = run_noisy(d, noise=noise)
     rel = np.abs(np.asarray(a["loss"]) - b["loss"]) / np.abs(b["loss"])
     dx = [np.abs(u - v) for u, v in zip(a["x_iters"], b["x_iters"])]

@@ -6,6 +6,7 @@ import pytest
 import torch
 
 import pgd_oracle as O
+from helpers import engines
 
 pytestmark = pytest.mark.gpu
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -30,17 +31,13 @@ def test_auc_ap_random(n, ties, engine):
     positives: n = 1.3e6, 2e6, 5e6), sampled keys + search in global memory (~210 000: n = 7e6); engine 0: the
     1024-sample kernel over the sorted positives."""
     from mcgra_b200 import metrics
-    from mcgra_b200 import _native as N
-    N.lib().mcgra_set_engine(6, engine)
     rng = np.random.RandomState(n % 1000)
     y = (rng.random_sample(n) < 0.03).astype(np.uint8)
     s = (rng.standard_normal(n) + 0.8 * y).astype(np.float32)
     if ties:
         s = np.round(s * 20) / 20
-    try:
+    with engines({6: engine}):
         auc, ap = metrics.roc_auc_ap(torch.from_numpy(s).cuda(), torch.from_numpy(y).cuda())
-    finally:
-        N.lib().mcgra_set_engine(6, 1)
     assert abs(auc - O.roc_auc(y, s)) < 1e-10
     assert abs(ap - O.average_precision(y, s)) < 1e-10
 
@@ -123,10 +120,7 @@ def test_fused_ensemble_is_bitwise_the_sequence_of_terms(n, engine):
             e.labels = ptr(t)
     ea.nterms = len(spec)
     fused = torch.full((n, n), float("nan"), device="cuda")
-    N.lib().mcgra_set_engine(5, engine)      # 1: one CTA per block pair (symmetric terms once), 0: one CTA per block
-    try:
+    with engines({5: engine}):      # 1: one CTA per block pair (symmetric terms once), 0: one CTA per block
         call("mcgra_ensemble", ptr(tiles), n, ctypes.byref(ea), ptr(fused), n, 0, n, st)
         torch.cuda.synchronize()
-    finally:
-        N.lib().mcgra_set_engine(5, 1)
     assert torch.equal(fused, seq)

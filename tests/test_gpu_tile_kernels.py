@@ -13,12 +13,13 @@ dyadic feature_adj, every sum below 2^24 units.  Then a dropped, duplicated, mir
 whatever n is.  Elsewhere the bounds are derived from the arithmetic; the constants fixed from the first B200 run are
 stated next to each test.  The references are fp64 (torch on the same device, so that n = 8321 stays fast).
 """
-import contextlib
 import ctypes as C
 
 import numpy as np
 import pytest
 import torch
+
+from helpers import engines
 
 pytestmark = pytest.mark.gpu
 
@@ -26,7 +27,6 @@ TILE = 128
 SIZES = [2, 127, 128, 129, 255, 256, 257, 1000, 8321]
 SPLITS = ["whole", "split3", "last", "empty"]
 U = 2.0 ** -24                     # unit roundoff of fp32
-DEFAULT_ENGINE = {0: 5, 1: 3, 4: 1}
 # parameter views (include/mcgra.h "PARAMETER VIEW"): (name, raw, mu); the random mu is dyadic so that x' - mu is exact
 VIEWS = [("lazy_mu0", 0, 0.0), ("lazy_mu5/16", 0, 0.3125), ("lazy_murand", 0, 181.0 / 512.0), ("raw1", 1, 0.0),
          ("raw2", 2, 0.0)]
@@ -142,20 +142,6 @@ def P(t):
 
 def stream():
     return N().stream_ptr()
-
-
-@contextlib.contextmanager
-def engine(which, value, cap=None):
-    L = N().lib()
-    try:
-        assert L.mcgra_set_engine(which, value) == 0
-        if cap is not None:
-            assert L.mcgra_set_engine(which, 100 + cap) == 0
-        yield
-    finally:
-        if which in (1, 4):
-            L.mcgra_set_engine(which, 100)
-        L.mcgra_set_engine(which, DEFAULT_ENGINE[which])
 
 
 @pytest.fixture(scope="module")
@@ -369,7 +355,7 @@ def test_propagate_exact(dev, n, split, K):
         Y0 = (torch.randint(-16, 17, (n, K), generator=g, device=dev).float() * 0.25).contiguous()
         refs = {p: prop_ref(tr, adj, B, sel, p) for p in (1, 2)}
         for ename, eng, use_ws in PROP_ENGINES:
-            with engine(0, eng):
+            with engines({0: eng}):
                 for products in (1, 2, 3):
                     Y = Y0.clone()
                     run_prop(tr, x, mu, raw, B, K, Y, sh, products, use_ws)
@@ -393,7 +379,7 @@ def test_propagate_two_planes(dev, n, split):
     M = tr.to_dense(Lt) + tr.to_dense(Ut).t()
     B = dyadic_features(n, K, g, dev)
     for ename, eng, use_ws in PROP_ENGINES:
-        with engine(0, eng):
+        with engines({0: eng}):
             for first, second, Mx in ((Lt, Ut, M), (Ut, Lt, M.t())):
                 Y = torch.zeros(n, K, device=dev)
                 run_prop(tr, first, 0.0, 2, B, K, Y, sh, 1, use_ws)
@@ -411,7 +397,7 @@ def test_propagate_rejects_bad_arguments(dev, n):
     ws = torch.empty(N().lib().mcgra_propagate_ws_bytes(n, 32), dtype=torch.uint8, device=dev)
     L = N().lib()
     for _, eng, use_ws in PROP_ENGINES:
-        with engine(0, eng):
+        with engines({0: eng}):
             w = P(ws) if use_ws else None
             for products in (0, 4, -1, 7):
                 assert L.mcgra_propagate_sel(P(x), n, 0, tr.T, None, 2, P(B), 32, P(Y), w, products, stream()) < 0
@@ -448,7 +434,7 @@ def test_propagate_precision(dev, n, split):
             bound5 = 2.0 ** -19 * rowM * B.abs().max(0).values.double()[None, :]
             bound0 = (128 + tr.T) * U * absref
             for ename, eng, use_ws in PROP_ENGINES:
-                with engine(0, eng):
+                with engines({0: eng}):
                     Y = torch.zeros(n, K, device=dev)
                     run_prop(tr, x, mu_r, raw, B, K, Y, sh, 3, use_ws)
                     torch.cuda.synchronize()
@@ -463,7 +449,7 @@ def test_propagate_precision(dev, n, split):
 # ---------------------------------------------------------------------------------------------------------------------
 # 4. element-wise terms
 # ---------------------------------------------------------------------------------------------------------------------
-ELEM_ENGINES = [("stats", 0, None), ("rs_cap5", 1, 5), ("rs", 1, 0)]
+ELEM_ENGINES = [("stats", 0, 0), ("rs_cap5", 1, 5), ("rs", 1, 0)]      # (name, engine, grid cap: 0 = none)
 # Bounds (fp32 arithmetic of the kernels against fp64): acc[C1] / acc[C6] within C_VAL 2^-24 S, S the sum of the absolute
 # values of the summed parts; eps_row[i] within C_ROW 2^-24 sum_j s_ij M_ij r_j, s_ij the absolute size of the parts of
 # e'_ij + e'_ji (MSE: 4|k1|(A + F), KL: |k1|(A_ij + X_ij + A_ji + X_ji)(1 + |lse|), entropy: 2|k6|(|log2 q| + 2)).
@@ -564,7 +550,7 @@ def test_elem_stats(dev, n, measure, k6):
                 eps = torch.zeros(n, device=dev)
                 ea = N().ElemArgs(r=P(r), Ftiles=None, lseA=P(lseA), lseF=P(lseF), measure=measure, k1=k1, k6=k6,
                                   acc=P(acc), eps_row=P(eps), dlse=P(dlse))
-                with engine(4, eng, cap):
+                with engines({4: eng}, caps={4: cap}):
                     for tr0, tr1 in sh:
                         ea.Ftiles = P(sl(Ft, tr0, tr1))
                         N().call("mcgra_elem_stats", P(sl(x, tr0, tr1)), n, tr0, tr1, P(mu_tensor(mu_r, dev)), raw,
@@ -602,7 +588,7 @@ def test_elem_stats(dev, n, measure, k6):
 # ---------------------------------------------------------------------------------------------------------------------
 # 5. gradient fold + Adam
 # ---------------------------------------------------------------------------------------------------------------------
-FOLD_ENGINES = [("ffma", 0, None), ("tc", 2, None), ("rs_cap1", 3, 1), ("rs_cap5", 3, 5), ("rs", 3, 0)]
+FOLD_ENGINES = [("ffma", 0, 0), ("tc", 2, 0), ("rs_cap1", 3, 1), ("rs_cap5", 3, 5), ("rs", 3, 0)]
 # the kernels receive these as fp32: the reference uses the same fp32 values (1 - 0.999f is 1.3e-5 away from 0.001)
 BETA1, BETA2, ADAM_EPS, LR = (float(np.float32(v)) for v in (0.9, 0.999, 1e-8, 0.01))
 STEP = 5
@@ -738,7 +724,7 @@ def fold_call(tr, cfg, d, sh, use_engine):
     f.plain_gd = cfg.get("plain_gd", 0)
     mu = mu_tensor(cfg.get("mu", 0.0), dev)
     _, eng, cap = use_engine
-    with engine(1, eng, cap):
+    with engines({1: eng}, caps={1: cap}):
         for tr0, tr1 in sh:
             f.Ftiles = P(sl(d["Ft"], tr0, tr1)) if cfg["measure"] != 0 else None
             f.Gtiles = P(sl(d["Gt"], tr0, tr1)) if d["Gt"] is not None else None

@@ -4,9 +4,8 @@ import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "oracle")); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import pgd_oracle as O
-from helpers import run_native_case
+from helpers import engines, run_native_case
 import test_gpu_parity_sizes as T
-from mcgra_b200 import _native as N
 
 ds = sys.argv[1] if len(sys.argv) > 1 else "cora"
 ep = int(sys.argv[2]) if len(sys.argv) > 2 else 100
@@ -14,8 +13,8 @@ r, d = T._real_case(ds, ep)
 real = d["adj"].reshape(-1).astype(np.float32)
 res = {}
 for tag, eng in [("e2a", 2), ("e2b", 2), ("e3a", 3), ("e3b", 3)]:
-    N.lib().mcgra_set_engine(1, eng)
-    got = run_native_case(d, trace=False)
+    with engines({1: eng}):
+        got = run_native_case(d, trace=False)
     sc = got["modified_adj"].reshape(-1)
     res[tag] = got
     print(tag, "AUC %.5f AP %.5f" % (O.roc_auc(real, sc), O.average_precision(real, sc)), "loss[-1] %.6e" % got["loss"][-1],

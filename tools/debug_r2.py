@@ -4,7 +4,7 @@ import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, "oracle")); sys.path.insert(0, os.path.join(ROOT, "tests"))
 import pgd_oracle as O
-from helpers import run_native_case, synthetic_case, make_models
+from helpers import engines, run_native_case, synthetic_case, make_models
 from mcgra_b200 import _native as N
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 dev = torch.device("cuda:0")
@@ -48,18 +48,17 @@ def probe_pairs():
         k7 = -10.0 * 10 / n / n
         outs = {}
         for eng in (0, 2):
-            N.lib().mcgra_set_engine(2, eng)
             dz = torch.zeros(n, 16, device=dev)
             acc = torch.zeros(32, dtype=torch.float64, device=dev)
             eps = torch.zeros(n, device=dev)
             r = torch.ones(n, device=dev)
             ws = torch.empty(int(N.lib().mcgra_pairs_ws_bytes(n)), dtype=torch.uint8, device=dev)
             tiles = torch.zeros(T * (T + 1) // 2 * 128 * 128, device=dev)
-            N.call("mcgra_pairs", N.ptr(tiles), n, 0, T, None, 2, N.ptr(z), N.ptr(r), k7, 0.0, None, None, N.ptr(dz), N.ptr(eps),
-                   N.ptr(acc), N.ptr(ws), N.stream_ptr())
-            torch.cuda.synchronize()
+            with engines({2: eng}):
+                N.call("mcgra_pairs", N.ptr(tiles), n, 0, T, None, 2, N.ptr(z), N.ptr(r), k7, 0.0, None, None, N.ptr(dz),
+                       N.ptr(eps), N.ptr(acc), N.ptr(ws), N.stream_ptr())
+                torch.cuda.synchronize()
             outs[eng] = (float(acc[4]), dz.clone())
-        N.lib().mcgra_set_engine(2, 1)
         S = (z.double() @ z.double().t())
         q = S.clamp(min=0).clamp(1e-4, 1 - 1e-4)
         ref = float(k7 * (torch.tril(2 * q * torch.log2(q), -1)).sum())

@@ -17,7 +17,9 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests"))
 import bench  # noqa: E402  (the benchmark's problem builder and kernel timers)
+from helpers import engines  # noqa: E402
 
 HBM_PEAK_GBS = 7700.0      # HGX B200 data sheet, one GPU
 # measure -> (weights w1..w10, lr exponent, description, default output)
@@ -106,7 +108,6 @@ def main():
         a.out = os.path.join(ROOT, "profiles", MEASURES[a.measure][3])
     if not torch.cuda.is_available():
         raise SystemExit("eps_bench needs a CUDA device")
-    from mcgra_b200 import _native as N
     out = {"card": card(), "profile": MEASURES[a.measure][2], "hbm_peak_gbs_datasheet": HBM_PEAK_GBS, "sizes": {}}
     print(out["card"], flush=True)
     for wl in a.sizes.split(","):
@@ -139,9 +140,7 @@ def main():
     # exact-FFMA engines vs defaults on the noisy path, 3 iterations, same injected draws
     wl = a.sizes.split(",")[-1]
     res = []
-    for engines in ((5, 3), (0, 0)):
-        N.lib().mcgra_set_engine(0, engines[0])
-        N.lib().mcgra_set_engine(1, engines[1])
+    for values in ({}, {0: 0, 1: 0}):
         torch.cuda.empty_cache()
 
         def noise(t, dev=torch.device("cuda", 0)):
@@ -149,14 +148,13 @@ def main():
             g.manual_seed(1000 + t)
             n = atk.engine.n
             return torch.randn((n, n), dtype=torch.float32, device=dev, generator=g)
-        atk = build(wl, 0.05, 3, noise=noise, measure=a.measure)
-        atk.engine.run(3)
+        with engines(values):
+            atk = build(wl, 0.05, 3, noise=noise, measure=a.measure)
+            atk.engine.run(3)
         res.append((atk.engine.losses()["loss"], atk.engine.packed_parameter()[:1 << 22].cpu().numpy()))
         atk.engine = None
         del atk
         gc.collect()
-    N.lib().mcgra_set_engine(0, 5)
-    N.lib().mcgra_set_engine(1, 3)
     (la, xa), (lb, xb) = res
     out["exact_vs_default"] = {"size": wl, "iters": 3, "loss_default": list(map(float, la)), "loss_exact": list(map(float, lb)),
                                "rel_loss": float(np.max(np.abs(la - lb) / np.abs(lb))),
