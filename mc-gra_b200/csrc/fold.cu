@@ -587,42 +587,6 @@ struct FoldRsSmem {
   uint32_t tmem_base;
 };
 
-__device__ __forceinline__ void ws_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(tc::smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void ws_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc::smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void ws_bulk_g2s_hint(void* dst, const void* src, uint32_t bytes, uint64_t* bar, uint64_t policy) {
-  asm volatile(
-      "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;" ::"r"(
-          tc::smem_u32(dst)),
-      "l"(src), "r"(bytes), "r"(tc::smem_u32(bar)), "l"(policy)
-      : "memory");
-}
-__device__ __forceinline__ uint64_t l2_policy_evict_first() {
-  uint64_t p;
-  asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
-  return p;
-}
-// single-thread waits of the producer / MMA warps: back off between polls so that the spinning lane does not take issue
-// slots from the streaming warps that share its scheduler
-__device__ __forceinline__ void ws_wait_backoff(uint64_t* bar, uint32_t parity) {
-  uint32_t done = 0;
-  while (true) {
-    asm volatile(
-        "{\n\t.reg .pred P1;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, P1;\n\t}"
-        : "=r"(done)
-        : "r"(tc::smem_u32(bar)), "r"(parity)
-        : "memory");
-    if (done) break;
-    __nanosleep(64);
-  }
-}
-__device__ __forceinline__ void rs_cons_sync() { asm volatile("bar.sync 1, %0;" ::"n"(RS_CW * 32) : "memory"); }
-
 // tile run iterator: storage (row-major triangle) order inside the shard of tile rows [tr0, tr1)
 struct RunIter {
   int I, J;
@@ -662,7 +626,7 @@ k_fold_rs(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restrict
     tc::mbar_init(&sm.dempty, RS_CW);
     sm.dsum[0] = 0.0;
     sm.dsum[1] = 0.0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    tc::fence_mbar_init();
   }
   if (warp == 2) tc::tmem_alloc(&sm.tmem_base, 512);
   if (tid < TILE) { sm.colacc[tid] = 0.f; sm.rowacc[tid] = 0.f; }
@@ -676,19 +640,19 @@ k_fold_rs(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restrict
     if (lane == 0) {
       // the streamed arrays are touched once per launch: evict-first, so that the factor blocks (re-read by every CTA)
       // stay in L2
-      const uint64_t pol = l2_policy_evict_first();
+      const uint64_t pol = tc::l2_policy_evict_first();
       uint32_t s = 0, ph = 0;
       for (int k = 0; k < my_tiles; ++k) {
         const int64_t base = (t_begin + k) * (int64_t)TILE_ELEMS;
 #pragma unroll 1
         for (int ch = 0; ch < TILE / RS_R; ++ch) {
-          ws_wait_backoff(&sm.sempty[s], ph ^ 1u);
+          tc::mbar_wait_backoff(&sm.sempty[s], ph ^ 1u);
           const int64_t o = base + (int64_t)ch * RS_CH;
-          ws_expect_tx(&sm.sfull[s], STAGE_BYTES);
-          ws_bulk_g2s_hint(sm.ring[s][0], tiles + o, RS_CH * 4u, &sm.sfull[s], pol);
-          ws_bulk_g2s_hint(sm.ring[s][1], mbuf + o, RS_CH * 4u, &sm.sfull[s], pol);
-          ws_bulk_g2s_hint(sm.ring[s][2], vbuf + o, RS_CH * 4u, &sm.sfull[s], pol);
-          if (USE_F) ws_bulk_g2s_hint(sm.ring[s][3], fa.Ftiles + o, RS_CH * 4u, &sm.sfull[s], pol);
+          tc::mbar_expect_tx(&sm.sfull[s], STAGE_BYTES);
+          tc::bulk_g2s_hint(sm.ring[s][0], tiles + o, RS_CH * 4u, &sm.sfull[s], pol);
+          tc::bulk_g2s_hint(sm.ring[s][1], mbuf + o, RS_CH * 4u, &sm.sfull[s], pol);
+          tc::bulk_g2s_hint(sm.ring[s][2], vbuf + o, RS_CH * 4u, &sm.sfull[s], pol);
+          if (USE_F) tc::bulk_g2s_hint(sm.ring[s][3], fa.Ftiles + o, RS_CH * 4u, &sm.sfull[s], pol);
           if (++s == RS_S) { s = 0; ph ^= 1u; }
         }
       }
@@ -705,9 +669,9 @@ k_fold_rs(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restrict
 #pragma unroll 1
         for (int qd = 0; qd < 4; ++qd, ++cnt) {
           const uint32_t s = cnt & 1u;
-          ws_wait_backoff(&sm.bempty[s], ((cnt >> 1) & 1u) ^ 1u);
-          ws_expect_tx(&sm.bfull[s], 8u * WSLAB);
-          ws_bulk_g2s_hint(sm.bop[s], blkB + (uint32_t)((8 * qd + 16) & 31) * WSLAB, 8u * WSLAB, &sm.bfull[s], keep);
+          tc::mbar_wait_backoff(&sm.bempty[s], ((cnt >> 1) & 1u) ^ 1u);
+          tc::mbar_expect_tx(&sm.bfull[s], 8u * WSLAB);
+          tc::bulk_g2s_hint(sm.bop[s], blkB + (uint32_t)((8 * qd + 16) & 31) * WSLAB, 8u * WSLAB, &sm.bfull[s], keep);
         }
       }
     }
@@ -719,12 +683,12 @@ k_fold_rs(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restrict
       uint32_t cnt = 0;
       for (int k = 0; k < my_tiles; ++k) {
         // phase k of dempty: the consumers have drained tile k - 1 and (re)loaded A when the tile row changed
-        ws_wait_backoff(&sm.dempty, (uint32_t)(k & 1));
+        tc::mbar_wait_backoff(&sm.dempty, (uint32_t)(k & 1));
         tc::fence_after();
 #pragma unroll 1
         for (int qd = 0; qd < 4; ++qd, ++cnt) {
           const uint32_t s = cnt & 1u;
-          ws_wait_backoff(&sm.bfull[s], (cnt >> 1) & 1u);
+          tc::mbar_wait_backoff(&sm.bfull[s], (cnt >> 1) & 1u);
           tc::fence_after();
           const uint32_t bs = tc::smem_u32(sm.bop[s]);
 #pragma unroll
@@ -802,7 +766,7 @@ k_fold_rs(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restrict
     }
     tc::fence_before();
     __syncwarp();
-    if (lane == 0) ws_arrive(&sm.dempty);                // phase 0: A of the first tile row is in place
+    if (lane == 0) tc::mbar_arrive1(&sm.dempty);         // phase 0: A of the first tile row is in place
 
     double d_sq = 0.0, d_clamp = 0.0;
     uint32_t s = 0, ph = 0;
@@ -815,7 +779,7 @@ k_fold_rs(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restrict
       const int64_t i0 = (int64_t)cur.I * TILE, j0 = (int64_t)cur.J * TILE;
       tc::mbar_wait(&sm.dfull, (uint32_t)(k & 1));
       tc::fence_after();
-      rs_cons_sync();                                    // A: every consumer finished streaming tile k - 1
+      tc::bar_sync_named<RS_CW * 32>();                  // A: every consumer finished streaming tile k - 1
       if (ct < TILE) {
         if (k > 0) {                                     // row / column sums of tile k - 1 -> next iteration's degrees
           const float rs = sm.rowacc[ct], cs = sm.colacc[ct];
@@ -846,8 +810,8 @@ k_fold_rs(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restrict
       if (has_next && nx.I != cur.I) load_A(nx.I);       // (the MMAs that read the old rows completed before dfull)
       tc::fence_before();
       __syncwarp();
-      if (lane == 0) ws_arrive(&sm.dempty);              // the MMA warp may form the product of tile k + 1
-      rs_cons_sync();                                    // B: product tile + node vectors visible
+      if (lane == 0) tc::mbar_arrive1(&sm.dempty);       // the MMA warp may form the product of tile k + 1
+      tc::bar_sync_named<RS_CW * 32>();                  // B: product tile + node vectors visible
       if (has_next) load_consts(nx);                     // (deferring the shared-memory stores to the end of the tile measured slower)
 
       float* xt = tiles + (t_begin + k) * (int64_t)TILE_ELEMS;
@@ -867,7 +831,7 @@ k_fold_rs(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restrict
         const float2 V = *reinterpret_cast<const float2*>(b + 2 * RS_CH);
         const float2 F = USE_F ? *reinterpret_cast<const float2*>(b + 3 * RS_CH) : make_float2(0.f, 0.f);
         __syncwarp();
-        if (lane == 0) ws_arrive(&sm.sempty[s]);         // this warp's part of the stage is in registers
+        if (lane == 0) tc::mbar_arrive1(&sm.sempty[s]);  // this warp's part of the stage is in registers
         if (++s == RS_S) { s = 0; ph ^= 1u; }
         const int a = ch * RS_R + rw;
         const float ri = sm.rI[a], rhoi = sm.rhoI[a];
@@ -916,7 +880,7 @@ k_fold_rs(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restrict
       Iprev = cur.I; Jprev = cur.J;
       cur = nx;
     }
-    rs_cons_sync();
+    tc::bar_sync_named<RS_CW * 32>();
     if (ct < TILE && my_tiles > 0) {
       const float rs = sm.rowacc[ct], cs = sm.colacc[ct];
       const int64_t gi = (int64_t)Iprev * TILE + ct, gj = (int64_t)Jprev * TILE + ct;
@@ -929,7 +893,7 @@ k_fold_rs(float* __restrict__ tiles, float* __restrict__ mbuf, float* __restrict
       atomicAdd(&sm.dsum[0], d_clamp);
       atomicAdd(&sm.dsum[1], d_sq);
     }
-    rs_cons_sync();
+    tc::bar_sync_named<RS_CW * 32>();
     if (ct == 0) {
       if (sm.dsum[0] != 0.0) atomicAdd(fa.acc_next + MCGRA_ACC_SUMCLAMP, sm.dsum[0]);
       if (sm.dsum[1] != 0.0) atomicAdd(fa.acc_next + MCGRA_ACC_SUMSQ, sm.dsum[1]);

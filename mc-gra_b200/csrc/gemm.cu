@@ -81,13 +81,6 @@ __device__ __forceinline__ uint32_t mapa_rank(uint32_t saddr, uint32_t rank) {
   asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(rank));
   return r;
 }
-__device__ __forceinline__ void mbar_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(tc::smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void fence_barrier_init() {
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-
 __device__ __forceinline__ void tma_load_2d(uint32_t dst, const CUtensorMap* map, int c0, int c1, uint32_t mbar) {
   asm volatile(
       "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];" ::
@@ -122,14 +115,6 @@ __device__ __forceinline__ void tmem_dealloc_cg(uint32_t taddr, uint32_t ncols) 
   asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
 
-// instruction descriptor: D = F32, A = B = F16, both K-major, dense
-__device__ __forceinline__ uint32_t idesc_f16(int M, int N) {
-  uint32_t d = 0;
-  d |= 1u << 4;
-  d |= (uint32_t)(N >> 3) << 17;
-  d |= (uint32_t)(M >> 4) << 24;
-  return d;
-}
 // K-major SWIZZLE_128B operand: rows of 128 bytes, 8-row groups 1024 bytes apart (TMA box {64 halves, 128 rows})
 __device__ __forceinline__ uint64_t desc_sw128(uint32_t saddr) {
   return tc::make_desc_sw(saddr, 16, 1024, 2);
@@ -141,7 +126,7 @@ __device__ __forceinline__ void mbar_arrive_rank(uint64_t* bar, uint32_t rank, b
     const uint32_t a = mapa_rank(tc::smem_u32(bar), rank);
     asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(a) : "memory");
   } else {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc::smem_u32(bar)) : "memory");
+    tc::mbar_arrive1(bar);
   }
 }
 
@@ -184,7 +169,7 @@ k_gemm3(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUten
       tc::mbar_init(&acc_full[b], 1);
       tc::mbar_init(&acc_empty[b], 16);        // one arrival per epilogue warp of both CTAs of the pair
     }
-    fence_barrier_init();
+    tc::fence_mbar_init();
   }
   if (warp == 1) tmem_alloc_cg(tmem_slot, 2 * NCOLS);
   tc::fence_before();
@@ -200,7 +185,7 @@ k_gemm3(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUten
         const int s = kb % G_STAGES;
         const uint32_t ph = (uint32_t)(kb / G_STAGES) & 1u;
         tc::mbar_wait(&empty[s], ph ^ 1u);
-        if (cta_rank == 0) mbar_expect_tx(&full[s], (uint32_t)(2 * G_STAGE));
+        if (cta_rank == 0) tc::mbar_expect_tx(&full[s], (uint32_t)(2 * G_STAGE));
         const uint32_t bar = mapa_rank(tc::smem_u32(&full[s]), 0);
         const uint32_t base = tc::smem_u32(smem + s * G_STAGE);
         const int k0 = kb * G_BK;
@@ -213,7 +198,7 @@ k_gemm3(const __grid_constant__ CUtensorMap mapAh, const __grid_constant__ CUten
   } else if (warp == 1) {
     // ===== MMA issuer (leader CTA, one thread) =====
     if (cta_rank == 0 && lane == 0) {
-      const uint32_t idesc = idesc_f16(G_BT, G_BT);
+      const uint32_t idesc = tc::make_idesc_f16(G_BT, G_BT, 0);
       for (int kb = 0; kb < num_kb; ++kb) {
         const int s = kb % G_STAGES;
         const uint32_t ph = (uint32_t)(kb / G_STAGES) & 1u;

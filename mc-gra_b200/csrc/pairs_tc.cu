@@ -27,11 +27,8 @@
 
 namespace {
 
-constexpr int P_RUN = 64;
-constexpr uint32_t P_SJ = 16 * 128 + 16;            // stride between 8-column groups of a plane (padded)
-constexpr uint32_t P_PLANE = 16 * P_SJ;
-constexpr uint32_t ZB_LBO = 32 * 16;                 // [g0 | g1]: 32 rows x 16 B per 8-node K group
-constexpr uint32_t ZB_BLK = 16 * ZB_LBO;             // 8192 B per 128-node block
+constexpr uint32_t ZB_LBO = tc::GBlock<HID>::LBO;   // [g0 | g1] block of 128 nodes (tc_common.cuh)
+constexpr uint32_t ZB_BLK = tc::GBlock<HID>::BYTES;
 constexpr uint32_t ZA_LBO = 16 * 128;                // node x feature image: 16 row groups x 128 B per 8-feature K group
 constexpr uint32_t ZA_PLANE = 2 * ZA_LBO;            // 4096 B (hi), + 4096 B (lo)
 constexpr uint32_t ZA_BLK = 2 * ZA_PLANE;
@@ -39,7 +36,7 @@ constexpr int RING = 4;
 constexpr uint32_t COL_D1 = 0, COL_D2 = 48, COL_S = 256;
 
 struct PairTcSmem {
-  unsigned char tile[2][2][P_PLANE];                 // [buffer][plane h0 / h1]
+  unsigned char tile[2][2][tc::PLANE_BYTES];         // [buffer][plane h0 / h1]
   unsigned char zbJ[RING][ZB_BLK];
   unsigned char zaJ[RING][ZA_BLK];
   unsigned char zbI[ZB_BLK];
@@ -51,41 +48,7 @@ struct PairTcSmem {
   uint32_t tmem_base;
 };
 
-__device__ __forceinline__ uint32_t idesc_f16(int M, int N, int a_mn_major) {
-  uint32_t d = 0;
-  d |= 1u << 4;
-  d |= (uint32_t)(a_mn_major & 1) << 15;
-  d |= (uint32_t)(N >> 3) << 17;
-  d |= (uint32_t)(M >> 4) << 24;
-  return d;
-}
-__device__ __forceinline__ void mma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc::smem_u32(bar)) : "memory");
-}
-
 // ---- operand preparation (once per call) ----
-__global__ void k_ptc_colmax(const float* __restrict__ Z, int64_t n, unsigned int* __restrict__ maxbits) {
-  const int c = threadIdx.x % HID;
-  float m = 0.f;
-  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n * HID; e += (int64_t)gridDim.x * blockDim.x)
-    m = fmaxf(m, fabsf(Z[e]));
-  if (m > 0.f) atomicMax(maxbits + c, __float_as_uint(m));
-}
-__device__ __forceinline__ float col_scale(unsigned int maxbits) {     // power of two s with max * s < 2^14
-  if (maxbits == 0u) return 1.f;
-  int e = (int)((maxbits >> 23) & 0xffu) - 127;
-  int se = 13 - e;
-  se = se > 126 ? 126 : (se < -126 ? -126 : se);
-  return __uint_as_float((uint32_t)(se + 127) << 23);
-}
 __global__ void k_ptc_prep(const float* __restrict__ Z, int64_t n, int64_t npad, const unsigned int* __restrict__ maxbits,
                            unsigned char* __restrict__ Zb, unsigned char* __restrict__ Za, float* __restrict__ scale) {
   const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -94,17 +57,10 @@ __global__ void k_ptc_prep(const float* __restrict__ Z, int64_t n, int64_t npad,
   const int c = (int)(e % HID);
   const float z = node < n ? Z[e] : 0.f;
   const int k = (int)(node & 127);
-  // [g0 | g1] block, K = node: (k/8) * ZB_LBO + (row/8) * 128 + (row%8) * 16 + (k%8) * 2, rows 0-15 g0, 16-31 g1
   {
-    const float s = col_scale(maxbits[c]);
+    const float s = tc::col_scale(maxbits[c]);
     if (node == 0) { scale[c] = s; scale[HID + c] = 1.f / s; }
-    const float g = z * s;
-    const __half g0 = __float2half_rn(g);
-    const __half g1 = __float2half_rn((g - __half2float(g0)) * 2048.f);
-    unsigned char* blk = Zb + (node >> 7) * (int64_t)ZB_BLK + (uint32_t)(k >> 3) * ZB_LBO + (uint32_t)(k & 7) * 2u;
-    *reinterpret_cast<__half*>(blk + (uint32_t)(c >> 3) * 128u + (uint32_t)(c & 7) * 16u) = g0;
-    const int c2 = c + HID;
-    *reinterpret_cast<__half*>(blk + (uint32_t)(c2 >> 3) * 128u + (uint32_t)(c2 & 7) * 16u) = g1;
+    tc::store_gblock<HID>(Zb, node, c, z * s);
   }
   // node x feature image, K = feature: (c/8) * ZA_LBO + (k/8) * 128 + (k%8) * 16 + (c%8) * 2; hi plane, then lo plane
   {
@@ -149,13 +105,9 @@ __device__ __forceinline__ void ptc_flush(float* __restrict__ dz, int64_t n, int
 __global__ void __launch_bounds__(320, 1)
 k_pairs_tc(int64_t n, int tr0, const unsigned char* __restrict__ Zb, const unsigned char* __restrict__ Za,
            const float* __restrict__ scale, float k7, float sc, float* __restrict__ dzhat, double* __restrict__ acc) {
-  const int I = tr0 + (int)blockIdx.y;
-  const int Jbeg = (int)blockIdx.x * P_RUN;
-  if (Jbeg > I) return;
-  const int Jend = min(I + 1, Jbeg + P_RUN);
-  const int nt = Jend - Jbeg;
-  const int rot = (I * 5) % nt;                    // rotated visiting order: neighbouring tile rows hit different dz rows
-  auto tile_of = [&](int k) { const int r = k + rot; return Jbeg + (r >= nt ? r - nt : r); };
+  tc::TileRun run;
+  if (!run.init(tr0)) return;
+  const int I = run.I, nt = run.nt;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   PairTcSmem& sm = *reinterpret_cast<PairTcSmem*>(smem_raw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -171,7 +123,7 @@ k_pairs_tc(int64_t n, int tr0, const unsigned char* __restrict__ Zb, const unsig
     }
     for (int r = 0; r < RING; ++r) { tc::mbar_init(&sm.bfull[r], 1); tc::mbar_init(&sm.bfree[r], 1); }
     tc::mbar_init(&sm.bIfull, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    tc::fence_mbar_init();
   }
   if (tid >= 32 && tid < 32 + HID) sm.inv_s[tid - 32] = scale[HID + tid - 32];
   tc::fence_before();
@@ -188,7 +140,7 @@ k_pairs_tc(int64_t n, int tr0, const unsigned char* __restrict__ Zb, const unsig
       for (int k = 0; k < nt; ++k) {
         const int r = k % RING;
         if (k >= RING) tc::mbar_wait_backoff(&sm.bfree[r], (uint32_t)((k / RING - 1) & 1));   // MMAs of tile k - RING are done
-        const int J = tile_of(k);
+        const int J = run.tile_of(k);
         tc::mbar_expect_tx(&sm.bfull[r], ZB_BLK + ZA_BLK);
         tc::bulk_g2s(sm.zbJ[r], Zb + (int64_t)J * ZB_BLK, ZB_BLK, &sm.bfull[r]);
         tc::bulk_g2s(sm.zaJ[r], Za + (int64_t)J * ZA_BLK, ZA_BLK, &sm.bfull[r]);
@@ -197,9 +149,9 @@ k_pairs_tc(int64_t n, int tr0, const unsigned char* __restrict__ Zb, const unsig
   } else if (warp == 8) {
     // =================================== MMA issuer ===================================
     if (lane == 0) {
-      const uint32_t id_s = idesc_f16(128, 128, 0);
-      const uint32_t id_cat = idesc_f16(128, 2 * HID, 0), id_one = idesc_f16(128, HID, 0);
-      const uint32_t id_cat_t = idesc_f16(128, 2 * HID, 1), id_one_t = idesc_f16(128, HID, 1);
+      const uint32_t id_s = tc::make_idesc_f16(128, 128, 0);
+      const uint32_t id_cat = tc::make_idesc_f16(128, 2 * HID, 0), id_one = tc::make_idesc_f16(128, HID, 0);
+      const uint32_t id_cat_t = tc::make_idesc_f16(128, 2 * HID, 1), id_one_t = tc::make_idesc_f16(128, HID, 1);
       const uint32_t zaI = tc::smem_u32(sm.zaI);
       const uint64_t aIh = tc::make_desc(zaI, ZA_LBO, 128u), aIl = tc::make_desc(zaI + ZA_PLANE, ZA_LBO, 128u);
       const uint64_t bI0 = tc::make_desc(tc::smem_u32(sm.zbI), ZB_LBO, 128u);
@@ -211,9 +163,9 @@ k_pairs_tc(int64_t n, int tr0, const unsigned char* __restrict__ Zb, const unsig
         const uint32_t zaJ = tc::smem_u32(sm.zaJ[k % RING]);
         const uint64_t bJh = tc::make_desc(zaJ, ZA_LBO, 128u), bJl = tc::make_desc(zaJ + ZA_PLANE, ZA_LBO, 128u);
         const uint32_t d = tm + COL_S + (uint32_t)b * 128u;
-        mma_f16(d, aIh, bJh, id_s, 0u);
-        mma_f16(d, aIh, bJl, id_s, 1u);
-        mma_f16(d, aIl, bJh, id_s, 1u);
+        tc::mma_f16(d, aIh, bJh, id_s, 0u);
+        tc::mma_f16(d, aIh, bJl, id_s, 1u);
+        tc::mma_f16(d, aIl, bJh, id_s, 1u);
         tc::mma_commit(&sm.s_ready[b]);
       };
       tc::mbar_wait(&sm.bIfull, 0u);
@@ -231,11 +183,11 @@ k_pairs_tc(int64_t n, int tr0, const unsigned char* __restrict__ Zb, const unsig
           const uint64_t db = (uint64_t)((uint32_t)ks * ((2u * ZB_LBO) >> 4));
           const uint32_t acc1 = (k > 0 || ks > 0) ? 1u : 0u, acc2 = ks > 0 ? 1u : 0u;
           // direct: C as a K-major A operand (M = row, K = column)
-          mma_f16(tm + COL_D1, tc::make_desc(p0 + (uint32_t)ks * 2u * P_SJ, P_SJ, 128u), bJ0 + db, id_cat, acc1);
-          mma_f16(tm + COL_D1 + 2 * HID, tc::make_desc(p1 + (uint32_t)ks * 2u * P_SJ, P_SJ, 128u), bJ0 + db, id_one, acc1);
+          tc::mma_f16(tm + COL_D1, tc::make_desc(p0 + (uint32_t)ks * 2u * tc::PLANE_SJ, tc::PLANE_SJ, 128u), bJ0 + db, id_cat, acc1);
+          tc::mma_f16(tm + COL_D1 + 2 * HID, tc::make_desc(p1 + (uint32_t)ks * 2u * tc::PLANE_SJ, tc::PLANE_SJ, 128u), bJ0 + db, id_one, acc1);
           // mirrored: the same image as an MN-major A operand (M = column, K = row)
-          mma_f16(d2, tc::make_desc(p0 + (uint32_t)ks * 256u, 128u, P_SJ), bI0 + db, id_cat_t, acc2);
-          mma_f16(d2 + 2 * HID, tc::make_desc(p1 + (uint32_t)ks * 256u, 128u, P_SJ), bI0 + db, id_one_t, acc2);
+          tc::mma_f16(d2, tc::make_desc(p0 + (uint32_t)ks * 256u, 128u, tc::PLANE_SJ), bI0 + db, id_cat_t, acc2);
+          tc::mma_f16(d2 + 2 * HID, tc::make_desc(p1 + (uint32_t)ks * 256u, 128u, tc::PLANE_SJ), bI0 + db, id_one_t, acc2);
         }
         tc::mma_commit(&sm.tile_done[b]);
         tc::mma_commit(&sm.bfree[k % RING]);
@@ -251,14 +203,14 @@ k_pairs_tc(int64_t n, int tr0, const unsigned char* __restrict__ Zb, const unsig
     const float k7s2 = 2.f * k7 * sc, k7s2_ln = k7s2 * INV_LN2;
     float v7 = 0.f;
     for (int k = 0; k < nt; ++k) {
-      const int J = tile_of(k), b = k & 1;
+      const int J = run.tile_of(k), b = k & 1;
       const int64_t j0 = (int64_t)J * TILE;
       const bool interior = (J < I) && (i0 + TILE <= n);
       tc::mbar_wait(&sm.s_ready[b], (uint32_t)((k >> 1) & 1));
       if (k >= 2) tc::mbar_wait(&sm.tile_done[b], (uint32_t)(((k - 2) >> 1) & 1));   // planes of buffer b are free
       tc::fence_after();
       unsigned char* pl0 = sm.tile[b][0] + (uint32_t)(row >> 3) * 128u + (uint32_t)(row & 7) * 16u;
-      unsigned char* pl1 = pl0 + P_PLANE;
+      unsigned char* pl1 = pl0 + tc::PLANE_BYTES;
       // the element-wise stage is the bound of this kernel (one MUFU log2 + ~12 ALU ops per pair): interior tiles take
       // the mask-free instantiation, 32-bit indices everywhere
       auto convert = [&](auto interior_tag) {
@@ -288,32 +240,23 @@ k_pairs_tc(int64_t n, int tr0, const unsigned char* __restrict__ Zb, const unsig
                 co[u] = (valid && qq == sv) ? dp : 0.f;
               }
             }
-            const __half2 a01 = __floats2half2_rn(co[0], co[1]), a23 = __floats2half2_rn(co[2], co[3]);
-            const __half2 a45 = __floats2half2_rn(co[4], co[5]), a67 = __floats2half2_rn(co[6], co[7]);
-            const float2 f01 = __half22float2(a01), f23 = __half22float2(a23), f45 = __half22float2(a45), f67 = __half22float2(a67);
-            const __half2 r01 = __floats2half2_rn((co[0] - f01.x) * 2048.f, (co[1] - f01.y) * 2048.f);
-            const __half2 r23 = __floats2half2_rn((co[2] - f23.x) * 2048.f, (co[3] - f23.y) * 2048.f);
-            const __half2 r45 = __floats2half2_rn((co[4] - f45.x) * 2048.f, (co[5] - f45.y) * 2048.f);
-            const __half2 r67 = __floats2half2_rn((co[6] - f67.x) * 2048.f, (co[7] - f67.y) * 2048.f);
-            const uint32_t off = (uint32_t)((c0 >> 3) + g8) * P_SJ;
-            *reinterpret_cast<uint4*>(pl0 + off) =
-                make_uint4(*reinterpret_cast<const uint32_t*>(&a01), *reinterpret_cast<const uint32_t*>(&a23),
-                           *reinterpret_cast<const uint32_t*>(&a45), *reinterpret_cast<const uint32_t*>(&a67));
-            *reinterpret_cast<uint4*>(pl1 + off) =
-                make_uint4(*reinterpret_cast<const uint32_t*>(&r01), *reinterpret_cast<const uint32_t*>(&r23),
-                           *reinterpret_cast<const uint32_t*>(&r45), *reinterpret_cast<const uint32_t*>(&r67));
+            uint32_t hi[4], lo[4];
+            tc::split_pairs<4>(co, hi, lo);
+            const uint32_t off = (uint32_t)((c0 >> 3) + g8) * tc::PLANE_SJ;
+            *reinterpret_cast<uint4*>(pl0 + off) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+            *reinterpret_cast<uint4*>(pl1 + off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
           }
         }
       };
       if (interior) convert(std::true_type{}); else convert(std::false_type{});
       tc::fence_before();
-      mbar_arrive(&sm.s_free[b]);                   // S[b] has been read
+      tc::mbar_arrive1(&sm.s_free[b]);                   // S[b] has been read
       tc::fence_async_smem();
-      mbar_arrive(&sm.ready[b]);                    // planes of tile k are in shared memory
+      tc::mbar_arrive1(&sm.ready[b]);                    // planes of tile k are in shared memory
       if (k >= 1) {                                 // flush the mirrored result of the previous tile
         tc::mbar_wait(&sm.tile_done[b ^ 1], (uint32_t)(((k - 1) >> 1) & 1));
         tc::fence_after();
-        if (flusher) ptc_flush(dzhat, n, (int64_t)tile_of(k - 1) * TILE + row, tlane + COL_D2 + (uint32_t)(b ^ 1) * 48u, sm.inv_s, 1.f / sc);
+        if (flusher) ptc_flush(dzhat, n, (int64_t)run.tile_of(k - 1) * TILE + row, tlane + COL_D2 + (uint32_t)(b ^ 1) * 48u, sm.inv_s, 1.f / sc);
         tc::fence_before();
       }
     }
@@ -321,14 +264,14 @@ k_pairs_tc(int64_t n, int tr0, const unsigned char* __restrict__ Zb, const unsig
     tc::mbar_wait(&sm.tile_done[bl], (uint32_t)(((nt - 1) >> 1) & 1));
     tc::fence_after();
     if (flusher) {
-      ptc_flush(dzhat, n, (int64_t)tile_of(nt - 1) * TILE + row, tlane + COL_D2 + (uint32_t)bl * 48u, sm.inv_s, 1.f / sc);
+      ptc_flush(dzhat, n, (int64_t)run.tile_of(nt - 1) * TILE + row, tlane + COL_D2 + (uint32_t)bl * 48u, sm.inv_s, 1.f / sc);
       ptc_flush(dzhat, n, i0 + row, tlane + COL_D1, sm.inv_s, 1.f / sc);
     }
     // c7 value: sum 2 q log2 q over valid pairs, scaled by k7 (one atomic per CTA); 256 converter threads
     double v = (double)v7 * 2.0 * (double)k7;
     v = warp_sum_d(v);
     if (lane == 0) sm.red[warp] = v;
-    asm volatile("bar.sync 1, 256;" ::: "memory");
+    tc::bar_sync_named<256>();
     if (warp == 0) {
       double s = lane < 8 ? sm.red[lane] : 0.0;
       s = warp_sum_d(s);
@@ -360,7 +303,7 @@ int mcgra_pairs_tc_(int64_t n, int tr0, int tr1, const float* zhat, float k7, fl
   unsigned int* maxbits = reinterpret_cast<unsigned int*>(scale + 2 * HID);
   cudaError_t e = cudaMemsetAsync(maxbits, 0, HID * sizeof(unsigned int), st);
   if (e != cudaSuccess) return (int)e;
-  k_ptc_colmax<<<(unsigned)min((int64_t)592, (n * HID + 255) / 256), 256, 0, st>>>(zhat, n, maxbits);
+  k_colmax<HID><<<(unsigned)min((int64_t)592, (n * HID + 255) / 256), 256, 0, st>>>(zhat, n, maxbits);
   k_ptc_prep<<<(unsigned)((npad * HID + 255) / 256), 256, 0, st>>>(zhat, n, npad, maxbits, Zb, Za, scale);
   // coefficient scale: |dL/dS| <= 2 |k7| (|log2 1e-4| + 1/ln 2) = 29.5 |k7|;  s_c = 2^floor(log2(2^14 / bound))
   const double bound = 29.5 * fabs((double)k7);
@@ -372,9 +315,8 @@ int mcgra_pairs_tc_(int64_t n, int tr0, int tr1, const float* zhat, float k7, fl
   const size_t smem = sizeof(PairTcSmem);
   e = cudaFuncSetAttribute(k_pairs_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  if (tr1 - tr0 > 65535) return -3;
-  dim3 grid((unsigned)((tr1 + P_RUN - 1) / P_RUN), (unsigned)(tr1 - tr0));
-  k_pairs_tc<<<grid, 320, smem, st>>>(n, tr0, Zb, Za, scale, k7, sc, dzhat, acc);
+  if (tr1 - tr0 > tc::RUN_MAX_ROWS) return -3;
+  k_pairs_tc<<<tc::run_grid(tr0, tr1), 320, smem, st>>>(n, tr0, Zb, Za, scale, k7, sc, dzhat, acc);
   MCGRA_LAUNCH_CHECK();
   return 0;
 }

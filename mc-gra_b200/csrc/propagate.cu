@@ -237,7 +237,7 @@ k_row_sumexp(const float* __restrict__ tiles, int64_t n, int64_t t0, const float
 //   D[:, 0:2KC] += h0 * [g0 | g1]      D[:, 2KC:3KC] += h1 * g0       y_c = (d0 + (d1 + d2) * 2^-11) / s_c
 // (mixed f16 x bf16 operands are rejected by the hardware; bf16 x 3 would need 3 planes and 48 MMAs per tile).
 //
-// Plane image: element (i, j) at (j/8)*H_SJ + (i/8)*128 + (i%8)*16 + (j%8)*2, two planes per tile, two tile buffers.
+// Plane image (tc_common.cuh): two planes per tile, two tile buffers.
 // Warps 0-7 convert their prefetched registers into the planes, arrive on ready[b], prefetch the tile after next and
 // flush the mirrored result of the previous tile; warp 8 (one lane) issues the 32 MMAs of a tile and nothing else -- a
 // clock64 trace showed its serial instruction stream to be the bound of the kernel (2.6 k clk of MMA issue + 1.9 k clk of
@@ -246,57 +246,17 @@ k_row_sumexp(const float* __restrict__ tiles, int64_t n, int64_t t0, const float
 // flush of the previous tile, 3-3.4 k clk) became the bound, so the flush moved to warps 8-11; registers are re-partitioned
 // with setmaxnreg (converters keep two prefetched tiles in registers, everything else needs few).  TMEM columns: D1 (even tiles) [0, 3KC) | D1 (odd tiles) [96, 96+3KC) | D2[0] [192, 192+3KC) | D2[1] [288, 288+3KC).
 // ---------------------------------------------------------------------------------------------------------
-constexpr int H_RUN = 64;
-constexpr uint32_t H_SJ = 16 * 128 + 16;           // stride between 8-column groups of a plane (padded: conflict-free stores)
-constexpr uint32_t H_PLANE = 16 * H_SJ;
-
 template <int KC>
 struct PropHSmem {
-  unsigned char tile[2][2][H_PLANE];               // [buffer][plane h0 / h1]
-  unsigned char bkJ[3][16 * (2 * KC) * 16];        // 16 K-groups x (2KC rows [g0 | g1] x 16 B); ring of 3
-  unsigned char bkI[16 * (2 * KC) * 16];
+  unsigned char tile[2][2][tc::PLANE_BYTES];       // [buffer][plane h0 / h1]
+  unsigned char bkJ[3][tc::GBlock<KC>::BYTES];     // ring of 3
+  unsigned char bkI[tc::GBlock<KC>::BYTES];
   uint64_t ready[2], tile_done[2], flushed[2];
   uint64_t bfull[3], bfree[3], bIfull;           // B-block ring (bulk copies by the loader warp)
   float inv_s[32];
   uint32_t tmem_base;
 };
 
-__device__ __forceinline__ uint32_t make_idesc_f16(int M, int N, int a_mn_major) {
-  uint32_t d = 0;
-  d |= 1u << 4;                          // D = F32; A = B = F16 (format 0)
-  d |= (uint32_t)(a_mn_major & 1) << 15;
-  d |= (uint32_t)(N >> 3) << 17;
-  d |= (uint32_t)(M >> 4) << 24;
-  return d;
-}
-__device__ __forceinline__ void mma_f16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc::smem_u32(bar)) : "memory");
-}
-
-// column scales: maxbits[c] = bits of max_i |B[i][c]|
-template <int KC>
-__global__ void k_colmax(const float* __restrict__ B, int64_t n, unsigned int* __restrict__ maxbits) {
-  const int c = threadIdx.x % KC;
-  float m = 0.f;
-  for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n * KC; e += (int64_t)gridDim.x * blockDim.x)
-    m = fmaxf(m, fabsf(B[e]));
-  if (m > 0.f) atomicMax(maxbits + c, __float_as_uint(m));
-}
-__device__ __forceinline__ float h_col_scale(unsigned int maxbits) {     // power of two s with max * s < 2^14
-  if (maxbits == 0u) return 1.f;
-  int e = (int)((maxbits >> 23) & 0xffu) - 127;                          // max < 2^(e+1)
-  int se = 13 - e;
-  se = se > 126 ? 126 : (se < -126 ? -126 : se);
-  return __uint_as_float((uint32_t)(se + 127) << 23);
-}
 // B (n x KC fp32) -> per node tile a K-major [g0 | g1] fp16 block; scale[0:KC] = s_c, scale[KC:2KC] = 1 / s_c
 template <int KC>
 __global__ void k_prep_b16(const float* __restrict__ B, int64_t n, int64_t npad, const unsigned int* __restrict__ maxbits,
@@ -305,26 +265,18 @@ __global__ void k_prep_b16(const float* __restrict__ B, int64_t n, int64_t npad,
   if (e >= npad * KC) return;
   const int64_t node = e / KC;
   const int c = (int)(e % KC);
-  const float s = h_col_scale(maxbits[c]);
+  const float s = tc::col_scale(maxbits[c]);
   if (node == 0) { scale[c] = s; scale[KC + c] = 1.f / s; }
-  const float g = node < n ? B[e] * s : 0.f;
-  const __half g0 = __float2half_rn(g);
-  const __half g1 = __float2half_rn((g - __half2float(g0)) * 2048.f);
-  const int k = (int)(node & 127);
-  unsigned char* blk = Bk + (node >> 7) * (int64_t)(16 * (2 * KC) * 16) + (uint32_t)(k >> 3) * (uint32_t)((2 * KC) * 16) + (uint32_t)(k & 7) * 2u;
-  *reinterpret_cast<__half*>(blk + (uint32_t)(c >> 3) * 128u + (uint32_t)(c & 7) * 16u) = g0;
-  const int c2 = c + KC;
-  *reinterpret_cast<__half*>(blk + (uint32_t)(c2 >> 3) * 128u + (uint32_t)(c2 & 7) * 16u) = g1;
+  tc::store_gblock<KC>(Bk, node, c, node < n ? B[e] * s : 0.f);
 }
 
 // one chunk (4 consecutive tile columns of a row) -> 8 bytes of each fp16 plane
 __device__ __forceinline__ void h_convert_store(float x0, float x1, float x2, float x3, unsigned char* p0, unsigned char* p1) {
-  const __half2 a01 = __floats2half2_rn(x0, x1), a23 = __floats2half2_rn(x2, x3);
-  const float2 f01 = __half22float2(a01), f23 = __half22float2(a23);
-  const __half2 r01 = __floats2half2_rn((x0 - f01.x) * 2048.f, (x1 - f01.y) * 2048.f);
-  const __half2 r23 = __floats2half2_rn((x2 - f23.x) * 2048.f, (x3 - f23.y) * 2048.f);
-  *reinterpret_cast<uint2*>(p0) = make_uint2(*reinterpret_cast<const uint32_t*>(&a01), *reinterpret_cast<const uint32_t*>(&a23));
-  *reinterpret_cast<uint2*>(p1) = make_uint2(*reinterpret_cast<const uint32_t*>(&r01), *reinterpret_cast<const uint32_t*>(&r23));
+  const float x[4] = {x0, x1, x2, x3};
+  uint32_t hi[2], lo[2];
+  tc::split_pairs<2>(x, hi, lo);
+  *reinterpret_cast<uint2*>(p0) = make_uint2(hi[0], hi[1]);
+  *reinterpret_cast<uint2*>(p1) = make_uint2(lo[0], lo[1]);
 }
 // register-array element by run-time index without local memory (rolled generic path)
 __device__ __forceinline__ float4 h_pick(const float4 (&a)[16], int it) {
@@ -392,22 +344,16 @@ __global__ void __launch_bounds__(H_THREADS, 1)
 k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* mu, int raw,
               const unsigned char* __restrict__ Bk, const float* __restrict__ scale, float* __restrict__ Y,
               int products) {
-  const int I = tr0 + (int)blockIdx.y;
-  const int Jbeg = (int)blockIdx.x * H_RUN;
-  if (Jbeg > I) return;
-  const int Jend = min(I + 1, Jbeg + H_RUN);
-  const int nt = Jend - Jbeg;
-  // the tiles of a run are visited in a rotated order (start depends on the tile row) so that concurrently resident
-  // CTAs of neighbouring tile rows do not add their mirrored results to the same rows of Y at the same time
-  const int rot = (I * 5) % nt;
-  auto tile_of = [&](int k) { const int r = k + rot; return Jbeg + (r >= nt ? r - nt : r); };
+  tc::TileRun run;
+  if (!run.init(tr0)) return;
+  const int I = run.I, nt = run.nt;
   extern __shared__ __align__(128) unsigned char smem_raw[];
   PropHSmem<KC>& sm = *reinterpret_cast<PropHSmem<KC>*>(smem_raw);
   const ParamView pv = load_view(mu, raw);
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int64_t i0 = (int64_t)I * TILE;
-  constexpr uint32_t LBO_B = (2 * KC) * 16;
-  constexpr uint32_t BLK = 16 * LBO_B;
+  constexpr uint32_t LBO_B = tc::GBlock<KC>::LBO;
+  constexpr uint32_t BLK = tc::GBlock<KC>::BYTES;
   constexpr uint32_t COL_D1 = 0, COL_D2 = 192;    // D1 of the even / odd tiles at 0 / 96, D2[b] at 192 + 96 b
   const bool tcwarp = warp == 12 || warp == 14;   // two issuing lanes: even / odd tiles of the run
   const bool rows_ok = (i0 + TILE <= n) && (pv.raw == 2);
@@ -421,7 +367,7 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
     tc::mbar_init(&sm.flushed[0], 128); tc::mbar_init(&sm.flushed[1], 128);
     for (int r = 0; r < 3; ++r) { tc::mbar_init(&sm.bfull[r], 1); tc::mbar_init(&sm.bfree[r], 1); }
     tc::mbar_init(&sm.bIfull, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    tc::fence_mbar_init();
   }
   if (tid >= 32 && tid < 32 + KC) sm.inv_s[tid - 32] = scale[KC + tid - 32];
   tc::fence_before();
@@ -439,7 +385,7 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
         const int r = k % 3;
         if (k >= 3) tc::mbar_wait_backoff(&sm.bfree[r], (uint32_t)((k / 3 - 1) & 1));     // MMAs of tile k-3 have read slot r
         tc::mbar_expect_tx(&sm.bfull[r], BLK);
-        tc::bulk_g2s(sm.bkJ[r], Bk + (int64_t)tile_of(k) * BLK, BLK, &sm.bfull[r]);
+        tc::bulk_g2s(sm.bkJ[r], Bk + (int64_t)run.tile_of(k) * BLK, BLK, &sm.bfull[r]);
       }
     }
   } else if (tcwarp) {
@@ -449,8 +395,8 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
     // result of its tiles in its own D1 (summed by the final flush); D2[b] belongs to parity b anyway.
     if (lane == 0) {
       const int par = (warp - 12) >> 1;
-      const uint32_t id_cat = make_idesc_f16(128, 2 * KC, 0), id_one = make_idesc_f16(128, KC, 0);
-      const uint32_t id_cat_t = make_idesc_f16(128, 2 * KC, 1), id_one_t = make_idesc_f16(128, KC, 1);
+      const uint32_t id_cat = tc::make_idesc_f16(128, 2 * KC, 0), id_one = tc::make_idesc_f16(128, KC, 0);
+      const uint32_t id_cat_t = tc::make_idesc_f16(128, 2 * KC, 1), id_one_t = tc::make_idesc_f16(128, KC, 1);
       const uint64_t bI0 = tc::make_desc(tc::smem_u32(sm.bkI), LBO_B, 128u);
       const uint32_t d1 = tm + COL_D1 + (uint32_t)par * 96u, d2 = tm + COL_D2 + (uint32_t)par * 96u;
       tc::mbar_wait(&sm.bIfull, 0u);
@@ -466,15 +412,15 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
         for (int ks = 0; ks < TILE / 16; ++ks) {
           const uint64_t db = (uint64_t)((uint32_t)ks * ((2u * LBO_B) >> 4));
           const uint32_t acc1 = (k > par || ks > 0) ? 1u : 0u, acc2 = ks > 0 ? 1u : 0u;
-          // direct: A K-major (M = row: SBO 128 between 8-row groups; K = column: LBO H_SJ between 8-column groups)
+          // direct: A K-major (M = row: SBO 128 between 8-row groups; K = column: LBO PLANE_SJ between 8-column groups)
           if (do_dir) {
-            mma_f16(d1, tc::make_desc(p0 + (uint32_t)ks * 2u * H_SJ, H_SJ, 128u), bJ0 + db, id_cat, acc1);
-            mma_f16(d1 + 2 * KC, tc::make_desc(p1 + (uint32_t)ks * 2u * H_SJ, H_SJ, 128u), bJ0 + db, id_one, acc1);
+            tc::mma_f16(d1, tc::make_desc(p0 + (uint32_t)ks * 2u * tc::PLANE_SJ, tc::PLANE_SJ, 128u), bJ0 + db, id_cat, acc1);
+            tc::mma_f16(d1 + 2 * KC, tc::make_desc(p1 + (uint32_t)ks * 2u * tc::PLANE_SJ, tc::PLANE_SJ, 128u), bJ0 + db, id_one, acc1);
           }
-          // mirrored: the same image as an MN-major A operand (M = column: SBO H_SJ; K = row: LBO 128)
+          // mirrored: the same image as an MN-major A operand (M = column: SBO PLANE_SJ; K = row: LBO 128)
           if (do_mir) {
-            mma_f16(d2, tc::make_desc(p0 + (uint32_t)ks * 256u, 128u, H_SJ), bI0 + db, id_cat_t, acc2);
-            mma_f16(d2 + 2 * KC, tc::make_desc(p1 + (uint32_t)ks * 256u, 128u, H_SJ), bI0 + db, id_one_t, acc2);
+            tc::mma_f16(d2, tc::make_desc(p0 + (uint32_t)ks * 256u, 128u, tc::PLANE_SJ), bI0 + db, id_cat_t, acc2);
+            tc::mma_f16(d2 + 2 * KC, tc::make_desc(p1 + (uint32_t)ks * 256u, 128u, tc::PLANE_SJ), bI0 + db, id_one_t, acc2);
           }
         }
         tc::mma_commit(&sm.tile_done[b]);
@@ -494,10 +440,10 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
       if (do_mir) {
 #pragma unroll
         for (int cg = 0; cg < KC / 16; ++cg)
-          h_flush<KC>(Y, n, (int64_t)tile_of(k) * TILE + ltid, tlane + COL_D2 + (uint32_t)b * 96u, cg * 16, sm.inv_s + cg * 16);
+          h_flush<KC>(Y, n, (int64_t)run.tile_of(k) * TILE + ltid, tlane + COL_D2 + (uint32_t)b * 96u, cg * 16, sm.inv_s + cg * 16);
       }
       tc::fence_before();
-      mbar_arrive(&sm.flushed[b]);
+      tc::mbar_arrive1(&sm.flushed[b]);
     }
     if (do_dir) {                                        // the run's direct result (complete with the last tile_done)
 #pragma unroll
@@ -515,13 +461,13 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
       for (int it = 0; it < 16; ++it) dst[it] = src[(it * 8 + warp) * 32 + lane];
     };
     auto step = [&](int k, float4 (&cur)[16], float4 (&nxt)[16]) {
-      const int J = tile_of(k), b = k & 1;
+      const int J = run.tile_of(k), b = k & 1;
       const int64_t j0 = (int64_t)J * TILE;
       if (k >= 2) tc::mbar_wait(&sm.tile_done[b], (uint32_t)(((k - 2) >> 1) & 1));   // MMAs of tile k-2 released buffer b
       // this thread's 16 chunks: row = it * 8 + warp, columns 4 * lane .. + 3  ->  8 bytes per plane at
-      // (lane/2) * H_SJ + it * 128 + warp * 16 + (lane%2) * 8
-      unsigned char* pl0 = sm.tile[b][0] + (uint32_t)(lane >> 1) * H_SJ + (uint32_t)warp * 16u + (uint32_t)(lane & 1) * 8u;
-      unsigned char* pl1 = pl0 + H_PLANE;
+      // (lane/2) * PLANE_SJ + it * 128 + warp * 16 + (lane%2) * 8
+      unsigned char* pl0 = sm.tile[b][0] + (uint32_t)(lane >> 1) * tc::PLANE_SJ + (uint32_t)warp * 16u + (uint32_t)(lane & 1) * 8u;
+      unsigned char* pl1 = pl0 + tc::PLANE_BYTES;
       if (rows_ok && J < I) {
 #pragma unroll
         for (int it = 0; it < 16; ++it) h_convert_store(cur[it].x, cur[it].y, cur[it].z, cur[it].w, pl0 + it * 128, pl1 + it * 128);
@@ -547,12 +493,12 @@ k_propagate_h(const float* __restrict__ tiles, int64_t n, int tr0, const float* 
         }
       }
       tc::fence_async_smem();
-      mbar_arrive(&sm.ready[b]);
-      if (k + 2 < nt) fetch(tile_of(k + 2), cur);   // two tiles ahead, into the registers just consumed
+      tc::mbar_arrive1(&sm.ready[b]);
+      if (k + 2 < nt) fetch(run.tile_of(k + 2), cur);   // two tiles ahead, into the registers just consumed
     };
     float4 ra[16], rb[16];
-    fetch(tile_of(0), ra);
-    if (nt > 1) fetch(tile_of(1), rb);
+    fetch(run.tile_of(0), ra);
+    if (nt > 1) fetch(run.tile_of(1), rb);
     for (int k = 0; k < nt; k += 2) {
       step(k, ra, rb);
       if (k + 1 < nt) step(k + 1, rb, ra);
@@ -582,9 +528,8 @@ int launch_prop_h(const float* tiles, int64_t n, int tr0, int tr1, const float* 
   const size_t smem = sizeof(PropHSmem<KC>);
   e = cudaFuncSetAttribute(k_propagate_h<KC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
   if (e != cudaSuccess) return (int)e;
-  if (tr1 - tr0 > 65535) return -3;
-  dim3 grid((unsigned)((tr1 + H_RUN - 1) / H_RUN), (unsigned)(tr1 - tr0));
-  k_propagate_h<KC><<<grid, H_THREADS, smem, st>>>(tiles, n, tr0, mu, raw, Bk, scale, Y, products);
+  if (tr1 - tr0 > tc::RUN_MAX_ROWS) return -3;
+  k_propagate_h<KC><<<tc::run_grid(tr0, tr1), H_THREADS, smem, st>>>(tiles, n, tr0, mu, raw, Bk, scale, Y, products);
   MCGRA_LAUNCH_CHECK();
   return 0;
 }
@@ -741,7 +686,7 @@ k_elem_rs(const float* __restrict__ tiles, int64_t n, int tr0, int64_t ntiles, c
     }
     sm.dsum[0] = 0.0;
     sm.dsum[1] = 0.0;
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    tc::fence_mbar_init();
   }
   if (tid < 2 * TILE) (&sm.colacc[0][0])[tid] = 0.f;
   __syncthreads();
@@ -794,7 +739,7 @@ k_elem_rs(const float* __restrict__ tiles, int64_t n, int tr0, int64_t ntiles, c
     const int p = k & 1;
     int In = I, Jn = J + 1;
     if (Jn > In) { ++In; Jn = 0; }
-    asm volatile("bar.sync 1, %0;" ::"n"(ES_CW * 32) : "memory");   // tile k - 1 complete everywhere; r[p] visible
+    tc::bar_sync_named<ES_CW * 32>();   // tile k - 1 complete everywhere; r[p] visible
     // node vectors of tile k + 1: loads issued now, parked in shared memory after the stream (no stall on their latency)
     float nrI = 0.f, nrJ = 0.f;
     if (k + 1 < my_tiles && ct < TILE) {
@@ -879,7 +824,7 @@ k_elem_rs(const float* __restrict__ tiles, int64_t n, int tr0, int64_t ntiles, c
     Iprev = I; Jprev = J;
     I = In; J = Jn;
   }
-  asm volatile("bar.sync 1, %0;" ::"n"(ES_CW * 32) : "memory");
+  tc::bar_sync_named<ES_CW * 32>();
   if (ct < TILE && my_tiles > 0) flush((my_tiles - 1) & 1, Iprev, Jprev);
   d1 = warp_sum_d(d1);
   d6 = warp_sum_d(d6);
@@ -887,7 +832,7 @@ k_elem_rs(const float* __restrict__ tiles, int64_t n, int tr0, int64_t ntiles, c
     atomicAdd(&sm.dsum[0], d1);
     atomicAdd(&sm.dsum[1], d6);
   }
-  asm volatile("bar.sync 1, %0;" ::"n"(ES_CW * 32) : "memory");
+  tc::bar_sync_named<ES_CW * 32>();
   if (ct == 0) {
     if (sm.dsum[0] != 0.0) atomicAdd(ea.acc + MCGRA_ACC_C1, sm.dsum[0] * (double)ea.k1);
     if (ent && sm.dsum[1] != 0.0) atomicAdd(ea.acc + MCGRA_ACC_C6, sm.dsum[1] * (double)ea.k6);
